@@ -68,6 +68,28 @@ int vtk_patchify(const void* images, const int64_t* img_table, int in_dtype, int
 int vtk_patchify_ex(const void* images, const int64_t* img_table, int in_dtype, int B, int patch, int max_tokens, int out_dtype,
                     void* patches, uint8_t* patch_mask, int64_t* row_idx, int64_t* col_idx, int64_t* time_idx, int64_t* meta, int* status,
                     int max_h, int max_w, void* stream);
+/* resize_to_token_budget | patchify + patch_collate_fn for a ragged batch. vitok/pp/ops.py:169-214, :217-285, vitok/data.py:77-94
+ * img_table  : [B,5] int64 = {element offset, H, W, h', w'} per image; (h', w') is the target size, normally
+ *              _fit_to_token_budget(H, W, patch, max_tokens) (ops.py:169-196).  An axis whose size is unchanged is not resampled,
+ *              so an image with (h', w') == (H, W) comes out bit-identical to vtk_patchify_ex.
+ * resampling : TF.resize(BICUBIC, antialias=True) on the normalised fp32 image = ATen's _upsample_bicubic2d_aa (align_corners=False):
+ *              cubic a = -0.5, support 2 * scale when shrinking, weights divided by their sum; width pass first, then height, each
+ *              output summed in fp32 in tap order.  Weights equal torch's; outputs agree with TF.resize to a few fp32 ulps.
+ * in_dtype / out_dtype / outputs: as vtk_patchify; meta holds the RESIZED height and width (patchify sees the resized tensor).
+ * workspace  : device memory of at least vtk_resize_patchify_workspace_bytes.  Layout: a header of 2B+3 int64 (rounded up to 256
+ *              bytes): [0..B] = offset of each image's region in floats after the header, [B+1..2B+1] = row prefix of the width pass,
+ *              [2B+2] = 1 if the batch was usable.  An image's region holds its resample tables (width then height; only for axes
+ *              that change; [4*ceil(n_in/n_out)+3][n_out] floats, tap-major: row 0 = xmin and row 1 = tap count as int32 bits, then
+ *              one row per tap of weights)
+ *              and, if its width changes, the fp32 [3, H, w'] image of the width pass.
+ * status     : optional device int: 1 if a target grid exceeds max_tokens (only for a target not produced by _fit_to_token_budget);
+ *              2 if a size is < 1 or the workspace is too small (the resized images' patches are then left zero). */
+int vtk_resize_patchify(const void* images, const int64_t* img_table, int in_dtype, int B, int patch, int max_tokens, int out_dtype,
+                        void* patches, uint8_t* patch_mask, int64_t* row_idx, int64_t* col_idx, int64_t* time_idx, int64_t* meta,
+                        void* workspace, size_t workspace_bytes, int* status, void* stream);
+/* Workspace of vtk_resize_patchify for a batch: img_table_host = the same [B,5] table in HOST memory.  Header + per image the tables
+ * and 3 * H * w' * 4 bytes of width-pass scratch (none for an image whose width is unchanged). */
+size_t vtk_resize_patchify_workspace_bytes(const int64_t* img_table_host, int B);
 /* test hook: *mismatches (device int) = number of uint8 values for which the arithmetic to_tensor|normalize of the row kernel differs
  * from the IEEE-division form (u / 255 - 0.5) / 0.5 of vitok/pp/ops.py:140-161; must be 0 */
 int vtk_patchify_selftest(int* mismatches, void* stream);

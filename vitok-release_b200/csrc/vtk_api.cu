@@ -304,6 +304,26 @@ int vtk_patchify_ex(const void* images, const int64_t* img_table, int in_dtype, 
   return launch_patchify(a, (cudaStream_t)stream);
 }
 
+int vtk_resize_patchify(const void* images, const int64_t* img_table, int in_dtype, int B, int patch, int max_tokens, int out_dtype,
+                        void* patches, uint8_t* patch_mask, int64_t* row_idx, int64_t* col_idx, int64_t* time_idx, int64_t* meta,
+                        void* workspace, size_t workspace_bytes, int* status, void* stream) {
+  VTK_REQUIRE(images && img_table && patches && patch_mask && row_idx && col_idx && time_idx && meta && workspace,
+              "vtk_resize_patchify: null pointer");
+  VTK_REQUIRE(in_dtype == 0 || in_dtype == 1, "vtk_resize_patchify: in_dtype must be 0 (f32 CHW) or 1 (u8 HWC)");
+  VTK_REQUIRE(out_dtype == 0 || out_dtype == 1, "vtk_resize_patchify: out_dtype must be 0 (f32) or 1 (bf16)");
+  VTK_REQUIRE(B >= 0 && max_tokens >= 0, "vtk_resize_patchify: negative size");
+  ResizePatchifyArgs a;
+  a.images = images; a.img_table = img_table; a.in_dtype = in_dtype; a.B = B; a.patch = patch; a.max_tokens = max_tokens;
+  a.out_dtype = out_dtype; a.patches = patches; a.patch_mask = patch_mask; a.row_idx = row_idx; a.col_idx = col_idx;
+  a.time_idx = time_idx; a.meta = meta; a.workspace = workspace; a.workspace_bytes = workspace_bytes; a.status = status;
+  return launch_resize_patchify(a, (cudaStream_t)stream);
+}
+
+size_t vtk_resize_patchify_workspace_bytes(const int64_t* img_table_host, int B) {
+  if (!img_table_host || B <= 0) return 0;
+  return resize_workspace_bytes(img_table_host, B);
+}
+
 int vtk_patchify_selftest(int* mismatches, void* stream) {
   VTK_REQUIRE(mismatches, "vtk_patchify_selftest: null pointer");
   return launch_patchify_selftest(mismatches, (cudaStream_t)stream);

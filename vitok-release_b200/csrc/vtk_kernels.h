@@ -208,6 +208,38 @@ struct PatchifyArgs {
 int launch_patchify(const PatchifyArgs& a, cudaStream_t stream);
 int launch_patchify_selftest(int* mismatches, cudaStream_t stream);   // norm_u8_fast == norm_u8 for all 256 inputs
 
+// resize to the token budget + patchify (vtk_pp.cu).  img_table [B, 5] = {element offset, H, W, h', w'}.  The workspace holds a
+// header (per-image offsets, computed on the device) and, per image, its resample tables and width-pass scratch image.
+// Table of one axis n_in -> n_out: [resize_kt + 2][n_out] floats, tap-major: row 0 = xmin, row 1 = taps (int bits), then the
+// weights (zero beyond the tap count); resize_kt bounds
+// ATen's ceil(support) * 2 + 1 taps (support = 2 * n_in / n_out when shrinking, 2 otherwise).
+__host__ __device__ inline int resize_kt(int n_in, int n_out) { return 4 * ((n_in + n_out - 1) / n_out) + 1; }
+struct ResizeImage {
+  long long off;
+  int H, W, h, w;   // source size, target size
+  __host__ __device__ bool sized() const { return H >= 1 && W >= 1 && h >= 1 && w >= 1; }
+  __host__ __device__ long long table_floats() const {
+    if (!sized()) return 0;
+    return (w != W ? (long long)w * (resize_kt(W, w) + 2) : 0) + (h != H ? (long long)h * (resize_kt(H, h) + 2) : 0);
+  }
+  __host__ __device__ long long width_rows() const { return sized() && w != W ? H : 0; }
+  __host__ __device__ long long region_floats() const { return table_floats() + 3 * width_rows() * (sized() ? w : 0); }
+};
+__host__ __device__ inline ResizeImage resize_image(const int64_t* tab, int b) {
+  const int64_t* r = tab + 5 * (long long)b;
+  return ResizeImage{(long long)r[0], (int)r[1], (int)r[2], (int)r[3], (int)r[4]};
+}
+__host__ __device__ inline size_t resize_header_bytes(int B) { return ((size_t)(2 * B + 3) * 8 + 255) / 256 * 256; }
+struct ResizePatchifyArgs {
+  const void* images; const int64_t* img_table;
+  int in_dtype, B, patch, max_tokens, out_dtype;
+  void* patches; uint8_t* patch_mask; int64_t* row_idx; int64_t* col_idx; int64_t* time_idx; int64_t* meta;
+  void* workspace; size_t workspace_bytes;
+  int* status;   // 1: a target grid exceeds max_tokens; 2: a size < 1 or the workspace is too small
+};
+int launch_resize_patchify(const ResizePatchifyArgs& a, cudaStream_t stream);
+size_t resize_workspace_bytes(const int64_t* img_table_host, int B);
+
 struct UnpatchifyArgs {
   const void* patches;         // [B, N, 3 p^2]
   int dtype;                   // 0 fp32, 1 bf16

@@ -5,6 +5,8 @@
 //                row_idx / col_idx / time_idx / orig_height / orig_width / grid_rows / grid_cols.
 //                Optional fused front end: uint8 HWC -> to_tensor | normalize(minus_one_to_one)
 //                (ops.py:140-155) and bf16 output.
+//   resize_patchify  vitok/pp/ops.py:169-214 + :217-285: over-budget images resized (antialiased bicubic, ATen's
+//                _upsample_bicubic2d_aa) to the token budget and patchified in one launch sequence.
 //   unpatchify   vitok/pp/ops.py:295-335: scatter + fold restated as a gather through a cell->token map,
 //                with _convert_format (vitok/pp/io.py:91-121) optionally fused.
 // All integer/byte work is bit-exact against the reference.
@@ -542,6 +544,277 @@ int launch_patchify_selftest(int* mismatches, cudaStream_t stream) {
   if (check_cuda(cudaMemsetAsync(mismatches, 0, sizeof(int), stream), "selftest memset")) return -1;
   patchify_selftest_kernel<<<1, 256, 0, stream>>>(mismatches);
   return check_cuda(cudaGetLastError(), "patchify selftest launch");
+}
+
+// ---------------------------------------------------------------------------------------------
+// resize_to_token_budget + normalize + patchify (vitok/pp/ops.py:169-214, :217-285)
+//
+// The reference resizes an over-budget [3,H,W] fp32 image with TF.resize(BICUBIC, antialias=True), i.e. ATen's CPU
+// _upsample_bicubic2d_aa (align_corners=False): separable, width pass first, an axis whose size is unchanged is not resampled.
+// Here: (1) plan = prefix sums over the batch -> workspace header; (2) per-image resample tables; (3) width pass, one CTA per source
+// row staged in shared memory, into an fp32 [3, H, w'] scratch image; (4) height pass fused with patchify, one warp per token.
+// ---------------------------------------------------------------------------------------------
+static constexpr int RS_ROW_CAP = 4096;   // source rows up to this width are staged in shared memory (3 x 4096 fp32 = 48 KB)
+
+// ATen's cubic filter with a = -0.5 (antialiased bicubic) in fp32.  The CPU build contracts both polynomials into FMAs; so do we
+// (the resulting weights equal torch's one-hot weight matrices exactly).
+__device__ __forceinline__ float aa_cubic(float x) {
+  x = fabsf(x);
+  if (x < 1.f) return __fmaf_rn(__fmul_rn(__fmaf_rn(1.5f, x, -2.5f), x), x, 1.f);
+  if (x < 2.f) return __fmaf_rn(__fmaf_rn(__fmaf_rn(-0.5f, x, 2.5f), x, -4.f), x, 2.f);
+  return 0.f;
+}
+
+// Table column of output coordinate o (ATen _compute_indices_min_size_weights_aa, with its float / double mix), stored with stride
+// n_out (tap-major, so that the lanes of a warp, which own consecutive outputs, read consecutive words): [0] = xmin and [1] = tap
+// count as int bits, [2 ..] = the normalised weights, zero beyond the tap count.
+__device__ void aa_entry(int n_in, int n_out, int o, int kt, float* e) {
+  const int st = n_out;
+  const float scale = __fdiv_rn((float)n_in, (float)n_out);
+  const float support = scale >= 1.f ? __fmul_rn(2.f, scale) : 2.f;
+  const int kmax = (int)ceilf(support) * 2 + 1;
+  const float invscale = scale >= 1.f ? (float)(1.0 / (double)scale) : 1.f;
+  const float center = (float)((double)scale * ((double)o + 0.5));
+  const int xmin = max((int)((double)__fsub_rn(center, support) + 0.5), 0);
+  int xs = min((int)((double)__fadd_rn(center, support) + 0.5), n_in) - xmin;
+  xs = min(max(xs, 0), min(kmax, kt));
+  float* w = e + 2 * st;
+  float tot = 0.f;
+  for (int j = 0; j < xs; ++j) {
+    const float d = __fsub_rn((float)(j + xmin), center);
+    w[j * st] = aa_cubic((float)(((double)d + 0.5) * (double)invscale));
+    tot = __fadd_rn(tot, w[j * st]);
+  }
+  if (tot != 0.f)
+    for (int j = 0; j < xs; ++j) w[j * st] = __fdiv_rn(w[j * st], tot);
+  for (int j = xs; j < kt; ++j) w[j * st] = 0.f;
+  e[0] = __int_as_float(xmin);
+  e[st] = __int_as_float(xs);
+}
+
+// plan: one CTA.  Workspace = header, then one region per image: its resample tables (width, then height), then its width-pass
+// scratch image.  hdr[0 .. B] = region offsets in floats from the end of the header, hdr[B+1 .. 2B+1] = width-pass row prefix,
+// hdr[2B+2] = 1 when the batch is usable (every size >= 1 and the workspace large enough).
+__global__ void __launch_bounds__(1024) resize_plan_kernel(const int64_t* __restrict__ tab, int B, long long ws_bytes, int64_t* hdr,
+                                                           int* status) {
+  pdl_wait();
+  pdl_trigger();
+  __shared__ long long sh[2][1024];
+  __shared__ int bad;
+  const int tid = threadIdx.x, nt = blockDim.x;
+  if (tid == 0) bad = 0;
+  const int per = (B + nt - 1) / nt, b0 = min(B, tid * per), b1 = min(B, b0 + per);
+  long long s[2] = {0, 0};
+  __syncthreads();
+  for (int b = b0; b < b1; ++b) {
+    const ResizeImage im = resize_image(tab, b);
+    if (im.H < 1 || im.W < 1 || im.h < 1 || im.w < 1) bad = 1;
+    s[0] += im.region_floats(); s[1] += im.width_rows();
+  }
+  sh[0][tid] = s[0]; sh[1][tid] = s[1];
+  __syncthreads();
+  for (int d = 1; d < nt; d <<= 1) {                 // inclusive scan of the per-thread sums
+    const long long v0 = tid >= d ? sh[0][tid - d] : 0, v1 = tid >= d ? sh[1][tid - d] : 0;
+    __syncthreads();
+    sh[0][tid] += v0; sh[1][tid] += v1;
+    __syncthreads();
+  }
+  long long r0 = sh[0][tid] - s[0], r1 = sh[1][tid] - s[1];
+  for (int b = b0; b < b1; ++b) {
+    const ResizeImage im = resize_image(tab, b);
+    hdr[b] = r0; hdr[B + 1 + b] = r1;
+    r0 += im.region_floats(); r1 += im.width_rows();
+  }
+  if (tid == nt - 1) {
+    hdr[B] = sh[0][tid]; hdr[2 * B + 1] = sh[1][tid];
+    const bool ok = !bad && sh[1][tid] < (1ll << 31) && resize_header_bytes(B) + 4 * (size_t)sh[0][tid] <= (size_t)ws_bytes;
+    hdr[2 * B + 2] = ok ? 1 : 0;
+    if (!ok && status) atomicExch(status, 2);
+  }
+}
+
+__global__ void __launch_bounds__(256) resize_tables_kernel(const int64_t* __restrict__ tab, int B, const int64_t* __restrict__ hdr,
+                                                            float* data) {
+  pdl_wait();
+  pdl_trigger();
+  if (!hdr[2 * B + 2]) return;
+  for (int b = blockIdx.x; b < B; b += gridDim.x) {
+    const ResizeImage im = resize_image(tab, b);
+    float* t = data + hdr[b];
+    if (im.w != im.W) {
+      const int kt = resize_kt(im.W, im.w);
+      for (int o = threadIdx.x; o < im.w; o += blockDim.x) aa_entry(im.W, im.w, o, kt, t + o);
+      t += (long long)im.w * (kt + 2);
+    }
+    if (im.h != im.H) {
+      const int kt = resize_kt(im.H, im.h);
+      for (int o = threadIdx.x; o < im.h; o += blockDim.x) aa_entry(im.H, im.h, o, kt, t + o);
+    }
+  }
+}
+
+// source pixel (ch, y, x) as the reference's normalised fp32 tensor holds it (the uint8 value is what patchify's front end produces)
+__device__ __forceinline__ float resize_src(const void* images, int in_dtype, long long off, int H, int W, int ch, int y, int x) {
+  if (in_dtype == 1) return norm_u8_fast(__ldg(reinterpret_cast<const uint8_t*>(images) + off + ((long long)y * W + x) * 3 + ch));
+  return __ldg(reinterpret_cast<const float*>(images) + off + ((long long)ch * H + y) * W + x);
+}
+
+// width pass: work item = one source row of an image whose width changes; the row (normalised fp32, 3 planes) is staged in shared
+// memory when it is at most RS_ROW_CAP pixels wide.  Each output sums its taps in order in fp32, every product rounded before it is
+// added (ATen's loop: out = x0 * w0; out += xj * wj).
+__global__ void __launch_bounds__(256) resize_width_kernel(const void* __restrict__ images, int in_dtype, const int64_t* __restrict__ tab,
+                                                           int B, const int64_t* __restrict__ hdr, float* data) {
+  extern __shared__ float row_s[];
+  pdl_wait();
+  pdl_trigger();
+  if (!hdr[2 * B + 2]) return;
+  const int64_t* rows = hdr + B + 1;
+  const int items = (int)rows[B];                    // sum of the heights of the images whose width changes
+  for (int it = blockIdx.x; it < items; it += gridDim.x) {
+    int lo = 0, hi = B - 1;                          // the image b with rows[b] <= it < rows[b + 1]
+    while (lo < hi) {
+      const int mid = (lo + hi + 1) >> 1;
+      if (rows[mid] <= it) lo = mid; else hi = mid - 1;
+    }
+    const int b = lo, y = (int)(it - rows[b]);
+    const ResizeImage im = resize_image(tab, b);
+    const int W = im.W, w2 = im.w, kt = resize_kt(W, w2);
+    const bool staged = W <= RS_ROW_CAP;
+    if (staged) {
+      if (in_dtype == 1) {
+        const uint8_t* src = reinterpret_cast<const uint8_t*>(images) + im.off + (long long)y * W * 3;
+        for (int i = threadIdx.x; i < 3 * W; i += blockDim.x) {
+          const int px = i / 3, ch = i - px * 3;
+          row_s[ch * W + px] = norm_u8_fast(__ldg(src + i));
+        }
+      } else {
+        for (int i = threadIdx.x; i < 3 * W; i += blockDim.x) {
+          const int ch = i / W, x = i - ch * W;
+          row_s[i] = __ldg(reinterpret_cast<const float*>(images) + im.off + ((long long)ch * im.H + y) * W + x);
+        }
+      }
+      __syncthreads();
+    }
+    const float* tw = data + hdr[b];
+    float* dst = data + hdr[b] + im.table_floats() + (long long)y * w2;
+    const long long plane = (long long)im.H * w2;
+    for (int i = threadIdx.x; i < 3 * w2; i += blockDim.x) {
+      const int ch = i / w2, o = i - ch * w2;
+      const float* e = tw + o;                       // column o of the tap-major table (stride w2)
+      const int xmin = __float_as_int(e[0]), xs = __float_as_int(e[w2]);
+      const float* wt = e + 2 * w2;
+      float acc = 0.f;
+      if (staged) {
+        const float* s = row_s + ch * W + xmin;
+        if (xs > 0) acc = __fmul_rn(s[0], wt[0]);
+        for (int j = 1; j < xs; ++j) acc = __fadd_rn(acc, __fmul_rn(s[j], wt[j * w2]));
+      } else {
+        if (xs > 0) acc = __fmul_rn(resize_src(images, in_dtype, im.off, im.H, W, ch, y, xmin), wt[0]);
+        for (int j = 1; j < xs; ++j)
+          acc = __fadd_rn(acc, __fmul_rn(resize_src(images, in_dtype, im.off, im.H, W, ch, y, xmin + j), wt[j * w2]));
+      }
+      dst[ch * plane + o] = acc;
+    }
+    __syncthreads();                                 // row_s is reused by the next item
+  }
+}
+
+// height pass + patchify: one warp per output token, element order ch * p^2 + dy * p + dx.  Pixels come from the width pass's scratch
+// image, or straight from the source when the width is unchanged; an image of unchanged size reads exactly what patchify reads.
+template <typename OutT>
+__global__ void __launch_bounds__(256) resize_patchify_kernel(const ResizePatchifyArgs a, const int64_t* __restrict__ hdr,
+                                                              const float* __restrict__ data) {
+  pdl_wait();
+  pdl_trigger();
+  const int p = a.patch, pp = p * p, P = 3 * pp, T = a.max_tokens, B = a.B;
+  const bool ok = hdr[2 * B + 2] != 0;
+  const int lane = threadIdx.x & 31;
+  const unsigned ntok = (unsigned)B * (unsigned)T;
+  const unsigned nwarp = gridDim.x * (blockDim.x >> 5);
+  for (unsigned bt = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5); bt < ntok; bt += nwarp) {
+    const int b = (int)(bt / (unsigned)T), t = (int)(bt - (unsigned)b * (unsigned)T);
+    const ResizeImage im = resize_image(a.img_table, b);
+    const int h2 = im.h, w2 = im.w;
+    const bool sized = h2 >= 1 && w2 >= 1;
+    const int gr = sized ? (h2 + p - 1) / p : 0, gc = sized ? (w2 + p - 1) / p : 0, n = gr * gc;
+    const bool rs_w = w2 != im.W, rs_h = h2 != im.H;
+    const bool valid = t < n && n <= T;
+    const bool data_ok = valid && (ok || (!rs_w && !rs_h));       // an unusable workspace leaves the resized images' patches zero
+    const int r = valid ? t / gc : 0, c = valid ? t - (t / gc) * gc : 0;
+    OutT* dst = reinterpret_cast<OutT*>(a.patches) + (long long)bt * P;
+    const float* reg = data + (ok ? hdr[b] : 0);
+    const float* scr = reg + (ok ? im.table_floats() : 0);
+    const float* th = reg + (rs_w ? (long long)w2 * (resize_kt(im.W, w2) + 2) : 0);
+    for (int e = lane; e < P; e += 32) {
+      const int ch = e / pp, rem = e - ch * pp, dy = rem / p, dx = rem - dy * p;
+      const int y = r * p + dy, x = c * p + dx;
+      float v = 0.f;                                 // zero padding to the patch grid (ops.py:235-238)
+      if (data_ok && y < h2 && x < w2) {
+        if (rs_h) {
+          const float* ey = th + y;                  // column y of the tap-major table (stride h2)
+          const int ymin = __float_as_int(ey[0]), ys = __float_as_int(ey[h2]);
+          for (int j = 0; j < ys; ++j) {
+            const float s = rs_w ? scr[((long long)ch * im.H + ymin + j) * w2 + x]
+                                 : resize_src(a.images, a.in_dtype, im.off, im.H, im.W, ch, ymin + j, x);
+            const float wj = ey[(2 + j) * h2];
+            v = j == 0 ? __fmul_rn(s, wj) : __fadd_rn(v, __fmul_rn(s, wj));
+          }
+        } else {
+          v = rs_w ? scr[((long long)ch * im.H + y) * w2 + x] : resize_src(a.images, a.in_dtype, im.off, im.H, im.W, ch, y, x);
+        }
+      }
+      if (sizeof(OutT) == 4) reinterpret_cast<float*>(dst)[e] = v;
+      else reinterpret_cast<bf16*>(dst)[e] = __float2bfloat16_rn(v);
+    }
+    if (lane == 0) {
+      a.patch_mask[bt] = valid ? 1 : 0;
+      a.row_idx[bt] = r;
+      a.col_idx[bt] = c;
+      a.time_idx[bt] = 0;
+      if (t == 0) {
+        a.meta[0 * B + b] = h2;                      // the reference's patchify sees the resized tensor
+        a.meta[1 * B + b] = w2;
+        a.meta[2 * B + b] = gr;
+        a.meta[3 * B + b] = gc;
+        if (n > T && a.status) atomicExch(a.status, 1);
+      }
+    }
+  }
+}
+
+int launch_resize_patchify(const ResizePatchifyArgs& a, cudaStream_t stream) {
+  if (a.patch <= 0) { set_error("resize_patchify: patch size must be positive (got %d)", a.patch); return -2; }
+  if (a.B <= 0 || a.max_tokens <= 0) return 0;
+  const long long ntok = (long long)a.B * a.max_tokens;
+  if (ntok >= (1ll << 31)) { set_error("resize_patchify: B * max_tokens too large"); return -2; }
+  const size_t hb = resize_header_bytes(a.B);
+  if (a.workspace_bytes < hb) {
+    set_error("resize_patchify: workspace of %zu bytes is smaller than its %zu-byte header", a.workspace_bytes, hb);
+    return -2;
+  }
+  int64_t* hdr = reinterpret_cast<int64_t*>(a.workspace);
+  float* data = reinterpret_cast<float*>(reinterpret_cast<char*>(a.workspace) + hb);
+  const int sms = num_sms();
+  // the work sizes (rows to resample, table entries) are known only on the device: persistent grids that read them from the header
+  (void)launch_k(resize_plan_kernel, dim3(1), dim3(1024), 0, stream, a.img_table, a.B, (long long)a.workspace_bytes, hdr, a.status);
+  (void)launch_k(resize_tables_kernel, dim3((unsigned)min(a.B, 4 * sms)), dim3(256), 0, stream, a.img_table, a.B, (const int64_t*)hdr,
+                 data);
+  (void)launch_k(resize_width_kernel, dim3((unsigned)(8 * sms)), dim3(256), (size_t)(3 * RS_ROW_CAP * sizeof(float)), stream, a.images,
+                 a.in_dtype, a.img_table, a.B, (const int64_t*)hdr, data);
+  long long blocks = (ntok + 7) / 8;                 // one warp per token, 8 warps per CTA
+  const long long cap = (long long)sms * 8 * 16;
+  if (blocks > cap) blocks = cap;
+  if (a.out_dtype == 0)
+    (void)launch_k(resize_patchify_kernel<float>, dim3((unsigned)blocks), dim3(256), 0, stream, a, (const int64_t*)hdr, (const float*)data);
+  else
+    (void)launch_k(resize_patchify_kernel<bf16>, dim3((unsigned)blocks), dim3(256), 0, stream, a, (const int64_t*)hdr, (const float*)data);
+  return check_cuda(cudaGetLastError(), "resize_patchify launch");
+}
+
+size_t resize_workspace_bytes(const int64_t* img_table_host, int B) {
+  size_t floats = 0;
+  for (int b = 0; b < B; ++b) floats += (size_t)resize_image(img_table_host, b).region_floats();
+  return resize_header_bytes(B) + 4 * floats;
 }
 
 // ---------------------------------------------------------------------------------------------

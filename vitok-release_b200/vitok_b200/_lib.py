@@ -51,6 +51,9 @@ SIGNATURES = {
     "vtk_set_flag": (c_int, [ctypes.c_char_p, c_int]),
     "vtk_patchify": (c_int, [c_vp, c_vp, c_int, c_int, c_int, c_int, c_int, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp]),
     "vtk_patchify_ex": (c_int, [c_vp, c_vp, c_int, c_int, c_int, c_int, c_int, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_int, c_int, c_vp]),
+    "vtk_resize_patchify": (c_int, [c_vp, c_vp, c_int, c_int, c_int, c_int, c_int, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_sz,
+                                    c_vp, c_vp]),
+    "vtk_resize_patchify_workspace_bytes": (c_sz, [c_vp, c_int]),
     "vtk_patchify_selftest": (c_int, [c_vp, c_vp]),
     "vtk_grid_extent": (c_int, [c_vp, c_vp, c_vp, c_int, c_int, c_vp, c_vp]),
     "vtk_unpatchify": (c_int, [c_vp, c_int, c_vp, c_vp, c_vp, c_int, c_int, c_int, c_int, c_int, c_vp, c_vp, c_int, c_vp, c_vp]),

@@ -4,7 +4,9 @@ preprocess : PIL image(s) -> batched patch dict on the GPU.  The DSL string is p
              reference; every op up to ``patchify`` that works on PIL images runs on the host (they are
              not on the hot path), and the trailing ``to_tensor|normalize(minus_one_to_one)|patchify(p,T)``
              is executed as ONE kernel on uint8 HWC pixels (4x fewer H2D bytes than the reference's fp32
-             upload, bit-identical output) writing straight into the batched buffers.
+             upload, bit-identical output) writing straight into the batched buffers.  With ``fuse_resize=True`` a
+             trailing ``...|normalize(minus_one_to_one)|resize_to_token_budget(p,T)|patchify(p,T)`` runs the same way, the
+             resize done on the GPU inside the patchify launch sequence (within a few fp32 ulps of torchvision's resize).
 postprocess: patch dict -> images; unpatchify + format conversion fused in one kernel, then ``unpack``.
 """
 from __future__ import annotations
@@ -21,8 +23,14 @@ _FORMATS = ("minus_one_to_one", "zero_to_one", "0_255")
 
 
 def preprocess(images, pp: str = "to_tensor|normalize(minus_one_to_one)|patchify(16, 256)",
-               device: str = "cuda") -> Dict[str, torch.Tensor]:
-    """PIL image(s) -> batched patch dict with fp32 patches on ``device`` (io.py:18-49)."""
+               device: str = "cuda", fuse_resize: bool = False) -> Dict[str, torch.Tensor]:
+    """PIL image(s) -> batched patch dict with fp32 patches on ``device`` (io.py:18-49).
+
+    fuse_resize: when the pipeline ends in ``to_tensor|normalize(minus_one_to_one)|resize_to_token_budget(p,T)|patchify(p,T)``
+    (same p and T in both ops), decode to uint8 and resize + normalize + patchify on the GPU (``patchify_batch(...,
+    resize_to_budget=True)``) instead of running torchvision's resize per image on the host.  Off by default: the GPU resize
+    is not bit-identical to torchvision's.
+    """
     if not isinstance(images, (list, tuple)):
         images = [images]
     steps = parse_pipeline(pp)
@@ -38,8 +46,14 @@ def preprocess(images, pp: str = "to_tensor|normalize(minus_one_to_one)|patchify
     probe = OPS["patchify"](*pargs, **pkw)
     patch, max_tokens = probe.patch, probe.max_tokens
     head = steps[:-1]
+    resize = fuse_resize and len(head) >= 3 and head[-1][0] == "resize_to_token_budget" and \
+        _budget_args(head[-1]) == (patch, max_tokens)
+    if resize:
+        head = head[:-1]
     fused = (len(head) >= 2 and head[-2][0] == "to_tensor" and head[-1][0] == "normalize"
              and (head[-1][1] + ("minus_one_to_one",))[0] == "minus_one_to_one" and not head[-1][2])
+    if resize and not fused:            # the resize only fuses behind to_tensor|normalize(minus_one_to_one): keep it a host step
+        head, resize = steps[:-1], False
     host_steps = head[:-2] if fused else head
     fns = [OPS[n](*a, **k) for n, a, k in host_steps]
     outs = []
@@ -54,8 +68,16 @@ def preprocess(images, pp: str = "to_tensor|normalize(minus_one_to_one)|patchify
             if a.ndim != 3 or a.shape[2] != 3 or a.dtype != np.uint8:
                 raise ValueError("preprocess: expected 8-bit RGB PIL images")
             arrs.append(np.ascontiguousarray(a))
-        return patchify_batch(arrs, patch, max_tokens, torch.float32, device)
+        return patchify_batch(arrs, patch, max_tokens, torch.float32, device, resize_to_budget=resize)
     return patchify_batch(outs, patch, max_tokens, torch.float32, device)
+
+
+def _budget_args(step):
+    """(patch, max_tokens) of a parsed ``resize_to_token_budget(...)`` step."""
+    import inspect
+    _, args, kwargs = step
+    bound = inspect.signature(OPS["resize_to_token_budget"]).bind(*args, **kwargs).arguments
+    return int(bound["patch"]), int(bound["max_tokens"])
 
 
 def postprocess(output: Union[torch.Tensor, Dict[str, torch.Tensor]], output_format: str = "minus_one_to_one",

@@ -28,14 +28,18 @@ def _grid(h: int, w: int, patch: int) -> Tuple[int, int]:
 
 def patchify_batch(images: Union[torch.Tensor, Sequence[torch.Tensor], Sequence[np.ndarray]], patch: int = 16,
                    max_tokens: int = 256, out_dtype: torch.dtype = torch.float32,
-                   device: Union[str, torch.device] = "cuda") -> Dict[str, torch.Tensor]:
+                   device: Union[str, torch.device] = "cuda", resize_to_budget: bool = False) -> Dict[str, torch.Tensor]:
     """patchify + collate for a whole (possibly ragged) batch in one kernel launch.
 
     images: a [B,3,H,W] float32 tensor, or a list of [3,H_i,W_i] float32 tensors (already normalised,
     i.e. the output of ``to_tensor|normalize``), or a list of uint8 HWC arrays/tensors (then
     ``to_tensor|normalize(minus_one_to_one)`` is fused into the kernel).  Returns the batched NaFlex
     dict of vitok/pp/ops.py:274-284 + vitok/data.py:77-94 on ``device``.
-    Raises RuntimeError when an image's patch grid exceeds ``max_tokens`` (reference: ops.py:260).
+    Raises RuntimeError when an image's patch grid exceeds ``max_tokens`` (reference: ops.py:260), unless
+    ``resize_to_budget``: then such images are first resized on the device to ``_fit_to_token_budget(h, w, patch,
+    max_tokens)`` as ``resize_to_token_budget`` does (ops.py:169-214; antialiased bicubic, within a few fp32 ulps of
+    torchvision's, not bit-identical), in the same launch sequence as the patchify.  ``orig_height`` / ``orig_width``
+    are then the resized sizes.
     """
     dev = torch.device(device)
     if dev.type != "cuda":
@@ -46,7 +50,8 @@ def patchify_batch(images: Union[torch.Tensor, Sequence[torch.Tensor], Sequence[
         # to_tensor|normalize(minus_one_to_one) fused into the kernel (ops.py:140-161)
         B, H, W, _ = images.shape
         packed = images.to(dev, non_blocking=True).reshape(-1)
-        return _patchify_packed(packed, [i * H * W * 3 for i in range(B)], [(H, W)] * B, 1, patch, max_tokens, out_dtype, dev)
+        return _patchify_packed(packed, [i * H * W * 3 for i in range(B)], [(H, W)] * B, 1, patch, max_tokens, out_dtype, dev,
+                                resize_to_budget)
     if isinstance(images, torch.Tensor) and images.dim() == 4:
         imgs: List = list(images.unbind(0)) if not images.is_contiguous() else None
         if imgs is None:
@@ -57,7 +62,7 @@ def patchify_batch(images: Union[torch.Tensor, Sequence[torch.Tensor], Sequence[
             packed = images.to(dev).reshape(-1)
             offsets = [i * 3 * H * W for i in range(B)]
             in_dtype = 0
-            return _patchify_packed(packed, offsets, sizes, in_dtype, patch, max_tokens, out_dtype, dev)
+            return _patchify_packed(packed, offsets, sizes, in_dtype, patch, max_tokens, out_dtype, dev, resize_to_budget)
         images = imgs
     imgs = [torch.from_numpy(i) if isinstance(i, np.ndarray) else i for i in images]
     if not imgs:
@@ -87,7 +92,7 @@ def patchify_batch(images: Union[torch.Tensor, Sequence[torch.Tensor], Sequence[
         for t, o in zip(flat, offsets):
             host[o:o + t.numel()] = t.cpu()
         packed = host.to(dev, non_blocking=True)
-    return _patchify_packed(packed, offsets, sizes, 1 if u8 else 0, patch, max_tokens, out_dtype, dev)
+    return _patchify_packed(packed, offsets, sizes, 1 if u8 else 0, patch, max_tokens, out_dtype, dev, resize_to_budget)
 
 
 def pack_images(images: Sequence[Union[torch.Tensor, np.ndarray]], pin: bool = True):
@@ -116,21 +121,26 @@ def pack_images(images: Sequence[Union[torch.Tensor, np.ndarray]], pin: bool = T
 
 
 def patchify_packed(flat: torch.Tensor, offsets: Sequence[int], sizes: Sequence[Tuple[int, int]], patch: int = 16,
-                    max_tokens: int = 256, out_dtype: torch.dtype = torch.float32) -> Dict[str, torch.Tensor]:
-    """patchify + collate of a batch laid out by ``pack_images`` (``flat`` already on the GPU): one kernel launch."""
+                    max_tokens: int = 256, out_dtype: torch.dtype = torch.float32,
+                    resize_to_budget: bool = False) -> Dict[str, torch.Tensor]:
+    """patchify + collate of a batch laid out by ``pack_images`` (``flat`` already on the GPU): one kernel launch.
+    ``resize_to_budget``: as in ``patchify_batch``."""
     if not flat.is_cuda:
         raise RuntimeError("vitok_b200.patchify_packed: the packed image buffer must be on a CUDA device")
     if flat.dtype not in (torch.uint8, torch.float32):
         raise ValueError("patchify_packed: the packed buffer must be uint8 (HWC images) or float32 (CHW images)")
     return _patchify_packed(flat, list(offsets), list(sizes), 1 if flat.dtype == torch.uint8 else 0, patch, max_tokens,
-                            out_dtype, flat.device)
+                            out_dtype, flat.device, resize_to_budget)
 
 
 _TABLE_CACHE: Dict = {}
 
 
-def _patchify_packed(packed, offsets, sizes, in_dtype, patch, max_tokens, out_dtype, dev):
+def _patchify_packed(packed, offsets, sizes, in_dtype, patch, max_tokens, out_dtype, dev, resize_to_budget=False):
     B = len(sizes)
+    targets = [_fit_to_token_budget(h, w, patch, max_tokens) for (h, w) in sizes] if resize_to_budget else sizes
+    if list(targets) != list(sizes):
+        return _resize_patchify_packed(packed, offsets, sizes, targets, in_dtype, patch, max_tokens, out_dtype, dev)
     for (h, w) in sizes:
         gr, gc = _grid(h, w, patch)
         if gr * gc > max_tokens:
@@ -156,6 +166,41 @@ def _patchify_packed(packed, offsets, sizes, in_dtype, patch, max_tokens, out_dt
                                                0 if out_dtype == torch.float32 else 1, patches.data_ptr(), mask.data_ptr(),
                                                idx[0].data_ptr(), idx[1].data_ptr(), idx[2].data_ptr(), meta.data_ptr(), None,
                                                max(h for h, _ in sizes), max(w for _, w in sizes), _lib.stream_ptr()))
+    return {"patches": patches, "patch_mask": mask, "row_idx": idx[0], "col_idx": idx[1], "time_idx": idx[2],
+            "orig_height": meta[0], "orig_width": meta[1], "grid_rows": meta[2], "grid_cols": meta[3]}
+
+
+def _resize_patchify_packed(packed, offsets, sizes, targets, in_dtype, patch, max_tokens, out_dtype, dev):
+    """Over-budget images of the batch resized to ``targets`` on the device, fused with patchify (vtk_resize_patchify)."""
+    if out_dtype not in (torch.float32, torch.bfloat16):
+        raise ValueError("patchify: out_dtype must be float32 or bfloat16")
+    for (h, w), (th, tw) in zip(sizes, targets):
+        gr, gc = _grid(th, tw, patch)
+        if gr * gc > max_tokens:    # _fit_to_token_budget keeps a 1-patch side at 1 patch: 1 x 4500 -> 1 x 4288 at p = 16
+            raise RuntimeError(f"patchify: image {h}x{w} resized to {th}x{tw} needs {gr}x{gc}={gr * gc} patches > "
+                               f"max_tokens={max_tokens} (the reference's patchify raises here too)")
+    B = len(sizes)
+    key = ("resize", dev, tuple(offsets), tuple(sizes), tuple(targets))
+    cached = _TABLE_CACHE.get(key)
+    if cached is None:      # {offset, H, W, h', w'} per image + the workspace size it needs
+        if len(_TABLE_CACHE) > 64:
+            _TABLE_CACHE.clear()
+        host = torch.tensor([[o, h, w, th, tw] for o, (h, w), (th, tw) in zip(offsets, sizes, targets)], dtype=torch.int64)
+        cached = (host.to(dev), int(_lib.load().vtk_resize_patchify_workspace_bytes(host.data_ptr(), B)))
+        _TABLE_CACHE[key] = cached
+    table, ws_bytes = cached
+    P = 3 * patch * patch
+    T = max_tokens
+    patches = torch.empty(B, T, P, dtype=out_dtype, device=dev)
+    mask = torch.empty(B, T, dtype=torch.bool, device=dev)
+    idx = torch.empty(3, B, T, dtype=torch.int64, device=dev)
+    meta = torch.empty(4, B, dtype=torch.int64, device=dev)
+    ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
+    with _lib.device_of(packed, patches):
+        _lib.check(_lib.load().vtk_resize_patchify(packed.data_ptr(), table.data_ptr(), in_dtype, B, patch, T,
+                                                   0 if out_dtype == torch.float32 else 1, patches.data_ptr(), mask.data_ptr(),
+                                                   idx[0].data_ptr(), idx[1].data_ptr(), idx[2].data_ptr(), meta.data_ptr(),
+                                                   ws.data_ptr(), ws_bytes, None, _lib.stream_ptr()))
     return {"patches": patches, "patch_mask": mask, "row_idx": idx[0], "col_idx": idx[1], "time_idx": idx[2],
             "orig_height": meta[0], "orig_width": meta[1], "grid_rows": meta[2], "grid_cols": meta[3]}
 
