@@ -98,8 +98,8 @@ def test_uint8_batched_tensor_frontend_and_u8_roundtrip():
 
 
 def test_arithmetic_normalisation_equals_ieee_division_for_all_bytes():
-    """The row-coalesced uint8 front end normalises with three FMAs instead of u / 255 (no table, no division sequence): bit-identical
-    to (u / 255 - 0.5) / 0.5 for all 256 inputs (device-side exhaustive check), and the kernel's output equals numpy's on them."""
+    """The three-FMA normalisation (no table, no division sequence) is bit-identical to (u / 255 - 0.5) / 0.5 for all 256 inputs
+    (device-side exhaustive check), and the uint8 front end's output equals numpy's on them."""
     import vitok_b200 as vb
     from vitok_b200 import _lib
     bad = torch.full((1,), -1, dtype=torch.int32, device="cuda")
@@ -112,33 +112,33 @@ def test_arithmetic_normalisation_equals_ieee_division_for_all_bytes():
 
 
 @pytest.mark.parametrize("out_format", ["as_is", "0_255", "zero_to_one"])
-def test_unpatchify_row_and_cell_kernels_agree(out_format):
-    """unpatchify has two kernels (row-coalesced writes for p = 16 / 32, cell-per-warp for any other patch size); on a ragged batch with
-    padded tokens and a canvas larger than every image they produce identical bytes (p = 16 / 32 vs the same data pushed through the
-    generic kernel by choosing p = 8 is not comparable, so the A/B is done through an env switch in a subprocess)."""
-    import os, subprocess, sys, tempfile
-    code = r"""
-import sys, numpy as np, torch
-sys.path.insert(0, %r); sys.path.insert(0, %r)
-import vitok_b200 as vb
-rng = np.random.default_rng(5)
-imgs = [torch.from_numpy(rng.standard_normal((3, h, w)).astype(np.float32)) for h, w in [(128, 128), (96, 64), (50, 120), (16, 16)]]
-for dt in (torch.float32, torch.bfloat16):
-    d = vb.patchify_batch(imgs, 16, 64, out_dtype=dt)
-    out = vb.unpatchify(d, 16, max_grid_size=9, output_format=%r)
-    np.save(sys.argv[1] + str(dt)[-4:] + ".npy", out.float().cpu().numpy())
-"""
-    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    outs = {}
-    with tempfile.TemporaryDirectory() as td:
-        for mode in ("1", "0"):
-            env = dict(os.environ, VTK_UNPATCHIFY_ROWS=mode)
-            r = subprocess.run([sys.executable, "-c", code % (root, os.path.join(root, "vitok-release_b200"), out_format), os.path.join(td, mode)],
-                               env=env, capture_output=True, text=True, timeout=300)
-            assert r.returncode == 0, r.stderr[-2000:]
-            outs[mode] = [np.load(os.path.join(td, mode + sfx + ".npy")) for sfx in ("at32", "at16")]
-    for a, b in zip(outs["1"], outs["0"]):
-        assert np.array_equal(a, b)
+def test_unpatchify_row_and_cell_kernels_match_reference(out_format):
+    """unpatchify has two kernels (row-coalesced writes for p = 16 / 32, cell-per-warp for any other patch size).  On a ragged batch
+    with padding tokens and a canvas larger than every image, both equal the reference: fp32 patches bit for bit the numpy oracle,
+    bf16 patches the io.py:91-121 operations evaluated by torch on a bf16 CPU tensor (each eager op rounds to bf16)."""
+    import vitok_b200 as vb
+
+    def io_convert(x):   # vitok/pp/io.py:91-121 from "minus_one_to_one"
+        if out_format == "0_255":
+            return ((x.clamp(-1.0, 1.0) + 1.0) / 2.0 * 255).round().to(torch.uint8)
+        if out_format == "zero_to_one":
+            return ((x + 1.0) / 2.0).clamp(0.0, 1.0)
+        return x
+
+    rng = np.random.default_rng(5)
+    imgs = [torch.from_numpy(rng.standard_normal((3, h, w)).astype(np.float32)) for h, w in [(128, 128), (96, 64), (50, 120), (16, 16)]]
+    for p, T, grid in ((8, 256, 18), (16, 64, 9)):       # generic kernel, row kernel
+        for dt in (torch.float32, torch.bfloat16):
+            d = vb.patchify_batch(imgs, p, T, out_dtype=dt)
+            got = vb.unpatchify(d, p, max_grid_size=grid, output_format=out_format).cpu()
+            canvas = pp_oracle.unpatchify({k: v.float().cpu().numpy() if k == "patches" else v.cpu().numpy() for k, v in d.items()},
+                                          p, max_grid_size=grid)
+            if dt == torch.float32:
+                want = pp_oracle.convert_format(canvas, "minus_one_to_one", out_format)
+                assert np.array_equal(got.numpy(), want), (p, dt)
+            else:
+                want = io_convert(torch.from_numpy(canvas).to(torch.bfloat16))
+                assert got.dtype == want.dtype and torch.equal(got, want), (p, dt)
 
 
 def test_full_size_roundtrip_and_bf16():

@@ -48,7 +48,7 @@ t1 = timeit(lambda: _lib.qkv_swiglu(h, wp, D, d, Hf, qp, nq, nk, table))
 t2 = timeit(lambda: _lib.proj_residual(a2, wo, gamma, x))
 f1 = 2.0 * M * D * (3 * D + 2 * Hf)
 f2 = 2.0 * M * (D + Hf) * D
-print(f"{which} debug={os.environ.get('VTK_EPI_DEBUG', '0')}: qkv_swiglu {t1*1e3:.1f} us {f1/t1/1e9:.0f} TF/s | proj_resid {t2*1e3:.1f} us {f2/t2/1e9:.0f} TF/s")
+print(f"{which}: qkv_swiglu {t1*1e3:.1f} us {f1/t1/1e9:.0f} TF/s | proj_resid {t2*1e3:.1f} us {f2/t2/1e9:.0f} TF/s")
 
 if len(sys.argv) > 2 and sys.argv[2] == "sustain":
     # 2 s of back-to-back launches per GEMM with nvidia-smi clock sampling: is the kernel power-capped?

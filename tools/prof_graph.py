@@ -8,7 +8,7 @@ sys.path.insert(0, os.path.join(ROOT, "vitok-release_b200"))
 import torch  # noqa: E402
 import vitok_b200 as vb  # noqa: E402
 
-print(f"VTK_PDL={os.environ.get('VTK_PDL', '1')} VTK_GEMM_CL4={os.environ.get('VTK_GEMM_CL4', 'auto')}")
+print(f"VTK_PDL={os.environ.get('VTK_PDL', '1')}")
 
 cfg = vb.decode_variant("Ld4-Ld24/1x16x64")
 torch.manual_seed(0)

@@ -1,6 +1,6 @@
 """Per-kernel times of one 350M transformer block at small per-GPU batches (the strong-scaling shards of c2: 8 / 16 / 32 images),
 each kernel replayed back to back from a CUDA graph (20 launches per replay, PDL edges like in the model) so that launch latency is
-hidden the same way it is in the graphed step.  Env knobs (read once per process): VTK_PDL, VTK_GEMM_ALLHALF, VTK_GEMM_CL4, VTK_GEMM_PAIR."""
+hidden the same way it is in the graphed step.  Env knob (read once per process): VTK_PDL."""
 import math
 import os
 import sys
@@ -48,7 +48,7 @@ def graph_time(fn):
     return e0.elapsed_time(e1) / 10 / REP * 1e3
 
 
-tag = " ".join(f"{k}={os.environ[k]}" for k in ("VTK_PDL", "VTK_GEMM_ALLHALF", "VTK_GEMM_CL4", "VTK_GEMM_PAIR", "VTK_QKV_BN") if k in os.environ) or "default"
+tag = " ".join(f"{k}={os.environ[k]}" for k in ("VTK_PDL",) if k in os.environ) or "default"
 for B in [int(a) for a in sys.argv[1:]] or [8, 16, 32, 64]:
     M = B * N
     h = rn(M, D)

@@ -1,7 +1,7 @@
 """The three GEMM kinds of the 5B training step (BASELINE config 5: M = 8192 tokens, D = 3072, Hf = 8192) timed alone:
 forward (K-major operands), data gradient (B read MN-major, `vtk_linear_nn_acc_bf16`) and weight gradient (both operands MN-major,
 `vtk_linear_tn_bf16`), each at the shapes the step launches.  CUDA events over 10 back-to-back launches (operands larger than L2 in
-total; no profiler).  Env switches are read by the library: VTK_GEMM_CL4_TRANS=1, VTK_GEMM_PROF=1 (per-role cycle report)."""
+total; no profiler).  VTK_GEMM_PROF=1 makes the library print a per-role cycle report after every launch."""
 import os
 import sys
 
@@ -43,7 +43,7 @@ out_w = torch.empty(2 * Hf, D, dtype=torch.bfloat16, device=dev)
 out_w2 = torch.empty(D, Hf, dtype=torch.bfloat16, device=dev)
 out_a = torch.empty(M, Hf, dtype=torch.bfloat16, device=dev)
 f = 2.0 * M * D * 2 * Hf
-print(f"--- c5 shapes: M = {M}, D = {D}, Hf = {Hf}; env CL4_TRANS={os.environ.get('VTK_GEMM_CL4_TRANS', '0')}")
+print(f"--- c5 shapes: M = {M}, D = {D}, Hf = {Hf}")
 timed("forward  h[M,D] x W1[2Hf,D]^T            (K-major)", lambda: T._linear(h, D, w1, None, M, 2 * Hf, D, out=out_f), f)
 timed("dgrad    dz[M,2Hf] x W1[2Hf,D]           (B MN-major)", lambda: T._dgrad(dz1, 2 * Hf, w1, M, D, 2 * Hf, out=out_d), f)
 timed("dgrad    dy[M,D] x W2[D,Hf]              (B MN-major)", lambda: T._dgrad(dy, D, w2, M, Hf, D, out=out_a), 2.0 * M * D * Hf)

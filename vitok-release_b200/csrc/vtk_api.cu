@@ -454,7 +454,7 @@ int vtk_linear2_bf16(const void* A, int64_t lda, const void* W0, int64_t ldw0, c
   VTK_REQUIRE(A && W0 && W1 && out, "vtk_linear2_bf16: null pointer");
   VTK_REQUIRE(ldo % 8 == 0 && K0 > 0 && K1 > 0, "vtk_linear2_bf16: ldo must be a multiple of 8 and both K parts non-empty");
   const bool aligned = ((reinterpret_cast<uintptr_t>(W1) | reinterpret_cast<uintptr_t>(A)) & 15) == 0;
-  if (M > 128 && N > 128 && K0 % 64 == 0 && ldw1 % 8 == 0 && aligned && !(getenv("VTK_GEMM_PAIR") && atoi(getenv("VTK_GEMM_PAIR")) == 0)) {
+  if (M > 128 && N > 128 && K0 % 64 == 0 && ldw1 % 8 == 0 && aligned) {
     GemmArgs g = base_args(A, lda, W0, ldw0, N, M, N, K0 + K1);       // one accumulator over both K ranges
     g.B2 = (const bf16*)W1; g.ldb2 = ldw1; g.epi.k_split = K0;
     g.epi.out = (bf16*)out; g.epi.ldo = ldo;
@@ -735,10 +735,9 @@ size_t vtk_ae_workspace_bytes(vtk_ae_t h, int side, int B, int N) {
 }
 
 // Token packing is used whenever a mask is given and the attention kernel has the packed variant (head_dim 64).
-// vtk_ae_set_packing(h, 0) / VTK_NO_PACK=1 keep the padded [B, N] layout with in-kernel key masking (A/B experiments, parity tests).
+// vtk_ae_set_packing(h, 0) keeps the padded [B, N] layout with in-kernel key masking (parity tests).
 static bool use_packing(const vtk_ae_s* h, const Side& s, const uint8_t* patch_mask) {
-  static const int off = getenv("VTK_NO_PACK") ? atoi(getenv("VTK_NO_PACK")) : 0;
-  return patch_mask != nullptr && s.depth > 0 && (s.head_dim() == 64 || s.head_dim() == 128) && h->packing && !off;
+  return patch_mask != nullptr && s.depth > 0 && (s.head_dim() == 64 || s.head_dim() == 128) && h->packing;
 }
 
 // rows = row capacity of the activation buffers; with `pl` the kernels read the live row count from pl->m_dev()

@@ -35,7 +35,7 @@ static constexpr int BLK = 16384;    // one [128 x 64] bf16 swizzled block
 static constexpr float RESCALE_THRESHOLD = 8.0f;  // log2 units
 
 // NQ = query tiles per CTA.  NQ = 2 (one CTA per SM): two softmax warpgroups ping-pong on the tensor core and
-// share every K/V tile.  NQ = 1 (d = 64 only): 112 KB of shared memory and 256 TMEM columns, so TWO CTAs are
+// share every K/V tile.  NQ = 1 (the persistent d = 64 kernel): 112 KB of shared memory and 256 TMEM columns, so TWO CTAs are
 // resident per SM and hide each other's load / MMA / store latencies -- the better shape for the short
 // sequences of the 256 px configs (N = 256: two K/V tiles per CTA, latency-bound otherwise).
 template <int DH, int NQ> struct AttnShape {
@@ -610,14 +610,14 @@ __device__ __forceinline__ bool item_at(int k, int total, int& w) {
   return base < total;
 }
 
-template <int DH, bool SNAKE, bool PTMEM>
+template <int DH, bool SNAKE>
 __global__ void __launch_bounds__(192, 2)
 attn_persist_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__ CUtensorMap tmK,
                     const __grid_constant__ CUtensorMap tmV, const __grid_constant__ CUtensorMap tmO, const AttnParams p,
                     const int total_items_host, const int qtiles) {
   using S = AttnShape<DH, 1>;
   static_assert(DH == 64, "persistent attention: d = 64 only");
-  constexpr uint32_t P_COL = S::O_COL0 + DH;   // PTMEM: P (bf16, 128 keys = 64 columns) after S [0,128) and O [128,192)
+  constexpr uint32_t P_COL = S::O_COL0 + DH;   // P (bf16, 128 keys = 64 columns) after S [0,128) and O [128,192)
   const int warp = threadIdx.x >> 5;
   const int lane = threadIdx.x & 31;
   const int W = p.window;
@@ -700,7 +700,7 @@ attn_persist_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_consta
       const uint32_t idesc_o = make_idesc_bf16(ATT_BQ, DH, 0, 1);   // B (= V) is MN-major
       uint32_t n_item = 0, n_k = 0, n_v = 0, n_t = 0;   // n_t = key tiles whose S has been issued so far
       uint32_t n_pv = 0;                                 // key tiles whose PV has been issued so far
-      const uint32_t qa = smem_u32(sQ), pa = smem_u32(sP);
+      const uint32_t qa = smem_u32(sQ);
       auto issue_s = [&]() {   // S(tile n_t) = Q K^T; waits for the K tile and for the S buffer
         const uint32_t slot = n_k % S::RK;
         mbar_wait(&k_full[slot], (n_k / S::RK) & 1u);
@@ -733,12 +733,8 @@ attn_persist_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_consta
 #pragma unroll
           for (int kk = 0; kk < ATT_BKV / 16; ++kk) {
             const uint64_t bdesc = make_smem_desc(va + kk * 2048, BLK, 1024, 2);
-            if (PTMEM) {   // A = P from tensor memory: 16 keys = 8 packed 32-bit columns per MMA
-              umma_bf16_ts(tmem_base + S::O_COL0, tmem_base + P_COL + kk * 8, bdesc, idesc_o, (jj | kk) != 0 ? 1u : 0u);
-            } else {
-              const uint64_t adesc = make_desc_kmajor_sw128(pa + (kk >> 2) * BLK + (kk & 3) * 32);
-              umma_bf16_ss(tmem_base + S::O_COL0, adesc, bdesc, idesc_o, (jj | kk) != 0 ? 1u : 0u);
-            }
+            // A = P from tensor memory: 16 keys = 8 packed 32-bit columns per MMA
+            umma_bf16_ts(tmem_base + S::O_COL0, tmem_base + P_COL + kk * 8, bdesc, idesc_o, (jj | kk) != 0 ? 1u : 0u);
           }
           umma_commit(&v_empty[slot]);
           umma_commit(pv_done);
@@ -754,7 +750,6 @@ attn_persist_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_consta
     const uint32_t lane_base = (uint32_t)(quarter * 32) << 16;
     const uint32_t tS = tmem_base + lane_base;
     const uint32_t tO = tmem_base + lane_base + S::O_COL0;
-    uint8_t* prow = sP + r * 128;
     const float sc = p.scale_log2;
     uint32_t n_t = 0;          // key tiles processed so far by this CTA (phase of s_full / p_full / pv_done)
     bool store_pending = false;
@@ -816,26 +811,16 @@ attn_persist_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_consta
         const float m_sub = (m_use == -INFINITY) ? 0.f : m_use;
         const uint64_t sc2 = f2_pack(sc, sc), nm2 = f2_pack(-m_sub, -m_sub);
         uint64_t sum2a = 0ull, sum2b = 0ull;
-        // the P buffer is free once the previous tile's PV (this item's or the previous item's last) has completed,
-        // and once the O tile staged in it by the previous item's epilogue has been read by its TMA store
+        // P's tensor-memory columns are free once the previous tile's PV (this item's or the previous item's last) has completed
         const long long k3 = PCLK();
         if (n_t > 0) {
           mbar_wait(pv_done, (n_t - 1) & 1u);
           __syncwarp();
           tc_fence_after();
         }
-        if (!PTMEM && store_pending) {   // (PTMEM: the staging buffer is not P's; it is awaited in the epilogue)
-          if (lane == 0) tma_store_wait_read();
-          __syncwarp();
-          store_pending = false;
-        }
         const long long k4 = PCLK();
-        if (PTMEM) {
-          softmax_exp_tile_tmem(v, sc2, nm2, tmem_base + lane_base + P_COL, sum2a, sum2b);
-          tmem_wait_st();
-        } else {
-          softmax_exp_tile(v, sc2, nm2, prow, r, sum2a, sum2b);
-        }
+        softmax_exp_tile_tmem(v, sc2, nm2, tmem_base + lane_base + P_COL, sum2a, sum2b);
+        tmem_wait_st();
         const long long k5 = PCLK();
         float sum0, sum1;
         f2_unpack(f2_add(sum2a, sum2b), sum0, sum1);
@@ -878,12 +863,12 @@ attn_persist_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_consta
       tmem_wait_ld();
       tc_fence_before();
       if (p.tma_out && (!SNAKE || it.q0 + ATT_BQ <= it.nrows)) {   // packed: only full tiles leave through TMA (a partial tile shares rows with the next image)
-        if (PTMEM && store_pending) {   // the previous item's TMA store has read the staging rows
+        if (store_pending) {   // the previous item's TMA store has read the staging rows
           if (lane == 0) tma_store_wait_read();
           __syncwarp();
           store_pending = false;
         }
-        uint8_t* srow = sP + r * 128;   // O staged in block 0 of the P buffer (free: its last PV has completed)
+        uint8_t* srow = sP + r * 128;   // (P lives in tensor memory: sP is only the O staging buffer here)
 #pragma unroll
         for (int c = 0; c < DH / 32; ++c)
 #pragma unroll
@@ -971,10 +956,8 @@ static int launch_attention_persist(const AttnArgs& a, cudaStream_t stream) {
   }
   p.scale_log2 = (float)((1.0 / sqrt((double)a.d)) * 1.4426950408889634);
   // P stays in tensor memory (A operand of the PV MMA read from TMEM, no 32 KB shared-memory round trip per tile): 3-4 % faster
-  // than the shared-memory P buffer (43.9 vs 45.6 us at the c2 shape); VTK_ATTN_PTMEM=0 selects the shared-memory variant
-  static const int ptmem = getenv("VTK_ATTN_PTMEM") ? atoi(getenv("VTK_ATTN_PTMEM")) : 1;
-  auto kern = packed ? (ptmem ? attn_persist_kernel<64, true, true> : attn_persist_kernel<64, true, false>)
-                     : (ptmem ? attn_persist_kernel<64, false, true> : attn_persist_kernel<64, false, false>);
+  // than a shared-memory P buffer (43.9 vs 45.6 us at the c2 shape)
+  auto kern = packed ? attn_persist_kernel<64, true> : attn_persist_kernel<64, false>;
   if (ensure_max_smem(reinterpret_cast<const void*>(kern), S::SMEM_BYTES, "cudaFuncSetAttribute(attn_persist)")) return -1;
   const int qtiles = (a.N + ATT_BQ - 1) / ATT_BQ;
   const long long total = packed ? (long long)a.grp_cap * a.heads : (long long)a.B * a.heads * qtiles;
@@ -1049,12 +1032,7 @@ int launch_attention(const AttnArgs& a, cudaStream_t stream) {
   if (a.B <= 0 || a.N <= 0 || a.heads <= 0) { set_error("attention: empty problem"); return -2; }
   if ((a.ld_qkv % 8) || (a.ld_out % 8)) { set_error("attention: row strides must be multiples of 8"); return -2; }
   if (a.cu && a.d != 64 && a.d != 128) { set_error("attention: the packed layout is implemented for head_dim 64 and 128"); return -3; }
-  if (a.d == 64) {
-    // perf experiments: VTK_ATTN_NQ = 0 (default) persistent kernel, 1 = one-shot CTAs (2 per SM), 2 = one-shot, one CTA per SM
-    static const int nq = getenv("VTK_ATTN_NQ") ? atoi(getenv("VTK_ATTN_NQ")) : 0;
-    if (nq == 0 || a.cu) return launch_attention_persist(a, stream);
-    return nq == 2 ? launch_attention_t<64, 2>(a, stream) : launch_attention_t<64, 1>(a, stream);
-  }
+  if (a.d == 64) return launch_attention_persist(a, stream);
   if (a.d == 128) return launch_attention_t<128, 2>(a, stream);
   set_error("attention: head_dim %d unsupported (64 or 128)", a.d);
   return -3;

@@ -53,7 +53,6 @@ template <int BN> struct GemmShape {
 struct OutStage {
   uint8_t* base;     // two granule buffers per warp: the TMA store of one drains while the next is filled
   int lane, row0, cur;
-  bool store;
   __device__ __forceinline__ void begin() {
     cur ^= 1;
     if (lane == 0) tma_store_wait_read_le1();   // the store issued from this buffer two granules ago has read it
@@ -66,7 +65,7 @@ struct OutStage {
   __device__ __forceinline__ void flush(const CUtensorMap* tm, int col) {
     fence_proxy_async_smem();
     __syncwarp();
-    if (lane == 0 && store) {
+    if (lane == 0) {
       tma_store_2d(tm, base + cur * OUT_GRANULE_BYTES, col, row0);
       tma_store_commit();
     }
@@ -662,14 +661,13 @@ gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUt
     st.lane = lane;
     st.row0 = 0;
     st.cur = 0;
-    st.store = epi.debug != 1;
     int acc = 0;
     uint32_t acc_ph = 0;
     for (int t = blockIdx.x; t < sched.total_tiles; t += gridDim.x) {
       int m0, n0, width;
       sched.decode(t, m0, n0, width);
       const int row = m0 + quarter * 32 + lane;
-      const bool row_ok = row < M && epi.debug != 1;
+      const bool row_ok = row < M;
       st.row0 = m0 + quarter * 32;
       const int rrow = row_ok ? row : (M - 1);
       uint64_t rs2 = 0ull;
@@ -677,9 +675,7 @@ gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUt
       mbar_wait(&tfull[acc], acc_ph);
       tc_fence_after();
       const uint32_t taddr = tmem_base + lane_base + (uint32_t)(acc * BN);
-      if (epi.debug == 2) {
-        // experiment: no epilogue work at all
-      } else if (EPI == EPI_BIAS_LN) {
+      if (EPI == EPI_BIAS_LN) {
         epi_bias_ln_row(epi, taddr, row, row_ok, N);
       } else {
         const int U = (EPI == EPI_QKV_SWIGLU && epi.d > 64) ? epi.d : 64;
@@ -974,7 +970,6 @@ gemm2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CU
     st.lane = lane;
     st.row0 = 0;
     st.cur = 0;
-    st.store = epi.debug != 1;
     int acc = 0;
     uint32_t acc_ph = 0;
     long long w_tfull = 0, w_work = 0;
@@ -984,7 +979,7 @@ gemm2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CU
       sched.decode(t, m0, n0, width);
       m0 += (int)rrank * BM;
       const int row = m0 + quarter * 32 + lane;
-      const bool row_ok = row < M && epi.debug != 1;
+      const bool row_ok = row < M;
       st.row0 = m0 + quarter * 32;
       const int rrow = row < M ? row : (M - 1);
       uint64_t rs2 = 0ull;
@@ -1039,13 +1034,11 @@ gemm2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CU
         mbar_wait(part_full, 0);   // all 128 KB of the partner's accumulator have landed in this CTA's ring
         partial = sA + (uint32_t)(quarter * 8) * 4096u + (uint32_t)lane * 128u;
       }
-      if (epi.debug != 2) {
-        const int U = (EPI == EPI_QKV_SWIGLU && epi.d > 64) ? epi.d : 64;
-        for (int c0 = half * U; c0 < width; c0 += NHALF * U) {
-          if (EPI == EPI_BIAS) epi_bias_unit(epi, taddr + c0, row, row_ok, n0 + c0, N, U);
-          if (EPI == EPI_RESID) epi_resid_unit(epi, taddr + c0, row, row < M, n0 + c0, N, U, st, &tmO0, rs2, partial, c0);
-          if (EPI == EPI_QKV_SWIGLU) epi_qkv_swiglu_unit(epi, taddr + c0, rrow, n0 + c0, U, normw_s, st, &tmO0, &tmO1, rs2);
-        }
+      const int U = (EPI == EPI_QKV_SWIGLU && epi.d > 64) ? epi.d : 64;
+      for (int c0 = half * U; c0 < width; c0 += NHALF * U) {
+        if (EPI == EPI_BIAS) epi_bias_unit(epi, taddr + c0, row, row_ok, n0 + c0, N, U);
+        if (EPI == EPI_RESID) epi_resid_unit(epi, taddr + c0, row, row < M, n0 + c0, N, U, st, &tmO0, rs2, partial, c0);
+        if (EPI == EPI_QKV_SWIGLU) epi_qkv_swiglu_unit(epi, taddr + c0, rrow, n0 + c0, U, normw_s, st, &tmO0, &tmO1, rs2);
       }
       tc_fence_before();
       __syncwarp();
@@ -1069,7 +1062,7 @@ gemm2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CU
   }
 }
 
-// 4-CTA-cluster launch (gemm2_kernel<..., CL = 4>): super-tiles of 512 x 256, no half-width tiles; the number of co-resident
+// 4-CTA-cluster launch (gemm2_kernel<..., CL = 4>, residual and plain epilogues): super-tiles of 512 x 256, no half-width tiles; the number of co-resident
 // clusters is what the hardware can place (GPCs whose SM count is not a multiple of 4 leave SMs unused)
 // split-K launch (gemm2_kernel<..., CL = 4, SK = true>): one 256 x 256 tile per 4-CTA cluster, K halved between its two pairs
 template <int NEPI, int G2_STAGES>
@@ -1107,8 +1100,7 @@ static int launch_gemm2_cl4(const GemmArgs& a, const CUtensorMap& tmA, const CUt
   sc.bm = 4 * BM;
   sc.split = 0;
   sc.gm_cap = sc.gm_cap > 1 ? sc.gm_cap / 2 : 1;   // the band height was sized for 256-row tiles: keep the A panel of a band at ~32 MB
-  constexpr bool kStaged = (EPI == EPI_QKV_SWIGLU || EPI == EPI_RESID);
-  const int smem_bytes = g2_smem_bytes(G2_STAGES, kStaged ? NEPI : 0);
+  const int smem_bytes = g2_smem_bytes(G2_STAGES, EPI == EPI_RESID ? NEPI : 0);
   auto kern = a.fp8 ? gemm2_kernel<EPI, NEPI, G2_STAGES, false, true, 0, 4> : gemm2_kernel<EPI, NEPI, G2_STAGES, false, false, 0, 4>;
   if constexpr (EPI == EPI_BIAS) {   // transposed-operand variants (the training step's data / weight gradients)
     if (a.trans == 3) kern = gemm2_kernel<EPI, NEPI, G2_STAGES, false, false, 3, 4>;
@@ -1134,10 +1126,7 @@ static int launch_gemm2_cl4(const GemmArgs& a, const CUtensorMap& tmA, const CUt
   const int big = sc.num_m * sc.num_n;
   const int clusters = big < avail ? big : avail;
   CUtensorMap tmO0 = tmA, tmO1 = tmA;
-  if (EPI == EPI_QKV_SWIGLU) {
-    if (encode_tmap_bf16(&tmO0, a.epi.qkv, (uint64_t)3 * a.epi.D, (uint64_t)a.M, (uint64_t)a.epi.ld_qkv, 32, 32, 64)) return -1;
-    if (encode_tmap_bf16(&tmO1, a.epi.act, (uint64_t)a.epi.Hf, (uint64_t)a.M, (uint64_t)a.epi.ld_act, 32, 32, 64)) return -1;
-  } else if (EPI == EPI_RESID) {
+  if (EPI == EPI_RESID) {
     if (encode_tmap_bf16(&tmO0, a.epi.out, (uint64_t)a.N, (uint64_t)a.M, (uint64_t)a.epi.ldo, 32, 32, 64)) return -1;
   } else if (EPI == EPI_BIAS && a.epi.k_split > 0) {
     if (encode_tmap_bf16_sw128(&tmO1, a.B2, (uint64_t)(a.K - a.epi.k_split), (uint64_t)a.b_rows, (uint64_t)a.ldb2, 64)) return -1;
@@ -1145,8 +1134,6 @@ static int launch_gemm2_cl4(const GemmArgs& a, const CUtensorMap& tmA, const CUt
   return check_cuda(launch_k(kern, dim3(4 * clusters), dim3(128 + 32 * NEPI), smem_bytes, stream, tmA, tmB, tmO0, tmO1, a.M, a.N, a.K, sc,
                              a.epi), "gemm2 (4-CTA cluster) launch");
 }
-
-static int env_int(const char* name, int dflt);
 
 template <int EPI, int NEPI, int G2_STAGES>
 static int launch_gemm2_s(const GemmArgs& a, cudaStream_t stream) {
@@ -1169,15 +1156,9 @@ static int launch_gemm2_s(const GemmArgs& a, cudaStream_t stream) {
   {
     const long long panel = 2ll * BM * a.K * 2;
     long long gm = (32ll << 20) / (panel > 0 ? panel : 1);
-    if (const char* e = getenv("VTK_GEMM_GM")) gm = atoi(e) > 0 ? atoi(e) : gm;
     sc.gm_cap = (int)(gm < 1 ? 1 : gm > (1 << 20) ? (1 << 20) : gm);
   }
-  sc.split = env_int("VTK_GEMM_ALLHALF", 1) ? 1 : 3;   // perf experiments: 0 keeps full-width tiles (split bit 2 = no all-half mode)
-  // 4-CTA clusters (two pairs sharing the B tile by TMA multicast): bf16 / fp8 K-major operands, enough M for two 256-row tiles
-  // Measured (B200, c2 / c4 in the bench pipeline): out_proj+fc2 residual GEMM 3.19 -> 3.11 ms / 21.5 -> 20.5 ms, but the QKV+fc1 GEMM
-  // 6.99 -> 7.18 / 43.9 -> 45.2 ms -- only 33 clusters (132 of 148 SMs) are co-resident, which the epilogue-heavy kernel feels more than
-  // it gains from the lighter L2 traffic.  Default: the light epilogues (residual, plain / bias; the 5B training step's forward GEMMs
-  // gain 1 %).  VTK_GEMM_CL4 = 0 never, 1 every epilogue kind.
+  sc.split = 1;
   // Split-K for the residual GEMM of small batches: at most pairs / 2 tiles (half of the SMs would idle) and a long K
   if constexpr (EPI == EPI_RESID) {
     const long long tiles2 = (long long)((a.M + 2 * BM - 1) / (2 * BM)) * sc.num_n;
@@ -1187,16 +1168,18 @@ static int launch_gemm2_s(const GemmArgs& a, cudaStream_t stream) {
       if (r || taken) return r;
     }
   }
-  static const int cl4_mode = getenv("VTK_GEMM_CL4") ? atoi(getenv("VTK_GEMM_CL4")) : -1;
-  // ... and only when the 512-row super tiles fill the ~33 co-resident clusters at least once: below that (the small per-GPU
-  // batches of a strong-scaled job) the pair kernel with half-width tiles keeps more SMs busy
-  const long long tiles4 = (long long)((a.M + 4 * BM - 1) / (4 * BM)) * sc.num_n;
-  // ... the transposed-operand variants (data / weight gradients of the training step) included: alone wgrad 1333-1365 -> 1414-1441 TF/s,
-  // dgrad 1395 -> 1439 TF/s, 5B step 302.8 -> 296.3 ms (VTK_GEMM_CL4_TRANS=0 keeps them on CTA pairs)
-  static const int cl4_trans = env_int("VTK_GEMM_CL4_TRANS", 1);
-  const bool cl4 = (cl4_mode == 1 || (cl4_mode == -1 && (EPI == EPI_RESID || EPI == EPI_BIAS) && tiles4 >= num_sms() / 4 - 4)) &&
-                   (!a.trans || (cl4_trans && EPI == EPI_BIAS)) && !a.epi.prof && a.M > 2 * BM;
-  if (cl4) return launch_gemm2_cl4<EPI, NEPI, G2_STAGES>(a, tmA, tmB, sc, stream);
+  // 4-CTA clusters (two pairs sharing the B tile by TMA multicast): bf16 / fp8 K-major operands, enough M for two 256-row tiles
+  // Measured (B200, c2 / c4 in the bench pipeline): out_proj+fc2 residual GEMM 3.19 -> 3.11 ms / 21.5 -> 20.5 ms, but the QKV+fc1 GEMM
+  // 6.99 -> 7.18 / 43.9 -> 45.2 ms -- only 33 clusters (132 of 148 SMs) are co-resident, which the epilogue-heavy kernel feels more than
+  // it gains from the lighter L2 traffic.  So: the light epilogues only (residual, plain / bias; the 5B training step's forward GEMMs
+  // gain 1 %), and the transposed-operand variants (data / weight gradients of the training step) included: alone wgrad 1333-1365 ->
+  // 1414-1441 TF/s, dgrad 1395 -> 1439 TF/s, 5B step 302.8 -> 296.3 ms.
+  if constexpr (EPI == EPI_RESID || EPI == EPI_BIAS) {
+    // ... and only when the 512-row super tiles fill the ~33 co-resident clusters at least once: below that (the small per-GPU
+    // batches of a strong-scaled job) the pair kernel with half-width tiles keeps more SMs busy
+    const long long tiles4 = (long long)((a.M + 4 * BM - 1) / (4 * BM)) * sc.num_n;
+    if (tiles4 >= num_sms() / 4 - 4 && !a.epi.prof && a.M > 2 * BM) return launch_gemm2_cl4<EPI, NEPI, G2_STAGES>(a, tmA, tmB, sc, stream);
+  }
   const int pairs = usable_sms() / 2;
   sc.setup(a.M, pairs);
   const int clusters = sc.workers;
@@ -1211,50 +1194,20 @@ static int launch_gemm2_s(const GemmArgs& a, cudaStream_t stream) {
     if (encode_tmap_bf16_sw128(&tmO1, a.B2, (uint64_t)(a.K - a.epi.k_split), (uint64_t)a.b_rows, (uint64_t)a.ldb2, 64)) return -1;
   }
   const int smem_bytes = g2_smem_bytes(G2_STAGES, kStaged ? NEPI : 0);
-  auto kern = a.trans == 3 ? (a.epi.prof ? gemm2_kernel<EPI, NEPI, G2_STAGES, true, false, 3> : gemm2_kernel<EPI, NEPI, G2_STAGES, false, false, 3>)
-              : a.trans == 2 ? (a.epi.prof ? gemm2_kernel<EPI, NEPI, G2_STAGES, true, false, 2> : gemm2_kernel<EPI, NEPI, G2_STAGES, false, false, 2>)
-              : a.fp8 ? gemm2_kernel<EPI, NEPI, G2_STAGES, false, true>
+  auto kern = a.fp8 ? gemm2_kernel<EPI, NEPI, G2_STAGES, false, true>
               : a.epi.prof ? gemm2_kernel<EPI, NEPI, G2_STAGES, true> : gemm2_kernel<EPI, NEPI, G2_STAGES, false>;
+  if constexpr (EPI == EPI_BIAS) {   // transposed-operand variants (launch_gemm_inner accepts trans with this epilogue only)
+    if (a.trans == 3) kern = a.epi.prof ? gemm2_kernel<EPI, NEPI, G2_STAGES, true, false, 3> : gemm2_kernel<EPI, NEPI, G2_STAGES, false, false, 3>;
+    else if (a.trans == 2) kern = a.epi.prof ? gemm2_kernel<EPI, NEPI, G2_STAGES, true, false, 2> : gemm2_kernel<EPI, NEPI, G2_STAGES, false, false, 2>;
+  }
   if (ensure_max_smem(reinterpret_cast<const void*>(kern), smem_bytes, "cudaFuncSetAttribute(gemm2)")) return -1;
   return check_cuda(launch_k(kern, dim3(2 * clusters), dim3(128 + 32 * NEPI), smem_bytes, stream, tmA, tmB, tmO0, tmO1, a.M, a.N, a.K, sc,
                              a.epi), "gemm2 launch");
 }
 
-static int env_int(const char* name, int dflt) {
-  const char* e = getenv(name);
-  return e ? atoi(e) : dflt;
-}
-
-// perf experiments: VTK_G2_STAGES (4 | 6), VTK_G2_NEPI (8 | 16)
-template <int EPI, int NEPI_DEFAULT>
-static int launch_gemm2_t(const GemmArgs& a, cudaStream_t stream) {
-  static const int stages = env_int("VTK_G2_STAGES", 6), nepi = env_int("VTK_G2_NEPI", NEPI_DEFAULT);
-  if (nepi == 8) return stages == 4 ? launch_gemm2_s<EPI, 8, 4>(a, stream) : launch_gemm2_s<EPI, 8, 6>(a, stream);
-  return stages == 4 ? launch_gemm2_s<EPI, 16, 4>(a, stream) : launch_gemm2_s<EPI, 16, 6>(a, stream);
-}
-
-static int gemm_pair_mode() {   // VTK_GEMM_PAIR=0 forces the single-CTA kernel (perf experiments)
-  static int mode = -1;
-  if (mode < 0) {
-    const char* e = getenv("VTK_GEMM_PAIR");
-    mode = e ? atoi(e) : 1;
-  }
-  return mode;
-}
-
 int launch_gemm_inner(EpiKind kind, const GemmArgs& a, cudaStream_t stream);
 
-static int epi_debug_mode() {
-  static int mode = -1;
-  if (mode < 0) {
-    const char* e = getenv("VTK_EPI_DEBUG");
-    mode = e ? atoi(e) : 0;
-  }
-  return mode;
-}
-
 static unsigned long long* g_prof = nullptr;
-static int env_int(const char* name, int dflt);
 
 // VTK_GEMM_PROF=1: every pair-kernel launch is followed by a sync and a per-role cycle report on stderr.
 static void prof_report(const char* what, int NEPI) {
@@ -1271,7 +1224,6 @@ static void prof_report(const char* what, int NEPI) {
 
 int launch_gemm(EpiKind kind, const GemmArgs& a_in, cudaStream_t stream) {
   GemmArgs a = a_in;
-  a.epi.debug = epi_debug_mode();
   a.epi.prof = nullptr;
   static int prof_mode = -1;
   if (prof_mode < 0) { const char* e = getenv("VTK_GEMM_PROF"); prof_mode = e ? atoi(e) : 0; }
@@ -1280,7 +1232,7 @@ int launch_gemm(EpiKind kind, const GemmArgs& a_in, cudaStream_t stream) {
     cudaMemsetAsync(g_prof, 0, 64 * sizeof(unsigned long long), stream);
     a.epi.prof = g_prof;
     const int r = launch_gemm_inner(kind, a, stream);
-    if (r == 0) prof_report(kind == EPI_QKV_SWIGLU ? "qkv_swiglu" : kind == EPI_RESID ? "proj_resid" : "linear", env_int("VTK_G2_NEPI", 8));
+    if (r == 0) prof_report(kind == EPI_QKV_SWIGLU ? "qkv_swiglu" : kind == EPI_RESID ? "proj_resid" : "linear", 8);
     return r;
   }
   return launch_gemm_inner(kind, a, stream);
@@ -1298,11 +1250,11 @@ int launch_gemm_inner(EpiKind kind, const GemmArgs& a, cudaStream_t stream) {
   }
   if (a.epi.k_split > 0) {   // two weight matrices, one accumulator: pair kernel only (the caller checks the shape)
     if (kind != EPI_BIAS || a.trans || a.fp8 || !a.B2 || (a.epi.k_split % BK) || a.epi.k_split >= a.K || (a.ldb2 % 8) || a.M <= BM || a.N <= 128 ||
-        !gemm_pair_mode() || (reinterpret_cast<uintptr_t>(a.B2) & 15)) {
+        (reinterpret_cast<uintptr_t>(a.B2) & 15)) {
       set_error("gemm(k_split): needs the bf16 pair kernel (M > 128, N > 128), k_split %% 64 == 0 inside K, a 16-byte aligned second matrix");
       return -3;
     }
-    return launch_gemm2_t<EPI_BIAS, 8>(a, stream);
+    return launch_gemm2_s<EPI_BIAS, 8, 6>(a, stream);
   }
   if (a.trans) {   // transposed operands (weight gradients): CTA-pair kernel, plain epilogue
     if (kind != EPI_BIAS || a.fp8 || (a.trans != 2 && a.trans != 3)) {
@@ -1335,7 +1287,7 @@ int launch_gemm_inner(EpiKind kind, const GemmArgs& a, cudaStream_t stream) {
     case EPI_BIAS:
       if (a.N <= 64) return launch_gemm_t<64, EPI_BIAS, 8>(a, false, stream);
       if (a.N <= 128) return launch_gemm_t<128, EPI_BIAS, 8>(a, false, stream);
-      if (gemm_pair_mode() && a.M > BM) return launch_gemm2_t<EPI_BIAS, 8>(a, stream);
+      if (a.M > BM) return launch_gemm2_s<EPI_BIAS, 8, 6>(a, stream);
       return launch_gemm_t<256, EPI_BIAS, 16>(a, true, stream);
     case EPI_BIAS_LN:
       if (a.N % 16 || a.N > 256 || !a.epi.bias) { set_error("gemm: LN epilogue needs N%%16==0, N<=256 and a bias (N=%d)", a.N); return -2; }
@@ -1348,10 +1300,10 @@ int launch_gemm_inner(EpiKind kind, const GemmArgs& a, cudaStream_t stream) {
                   a.epi.d, a.epi.Hf, a.epi.qp);
         return -3;
       }
-      if (gemm_pair_mode() && a.M > BM) return launch_gemm2_t<EPI_QKV_SWIGLU, 8>(a, stream);
+      if (a.M > BM) return launch_gemm2_s<EPI_QKV_SWIGLU, 8, 6>(a, stream);
       return launch_gemm_t<256, EPI_QKV_SWIGLU, 8>(a, true, stream);
     case EPI_RESID:
-      if (gemm_pair_mode() && a.M > BM) return launch_gemm2_t<EPI_RESID, 8>(a, stream);
+      if (a.M > BM) return launch_gemm2_s<EPI_RESID, 8, 6>(a, stream);
       return launch_gemm_t<256, EPI_RESID, 8>(a, true, stream);
   }
   set_error("gemm: unknown epilogue %d", (int)kind);

@@ -90,7 +90,6 @@ struct EpiParams {
   const int* m_dev;     // optional: number of rows to process, read on the device (<= GemmArgs::M, which is then the row
                         // capacity of the buffers); used by the packed NaFlex path where sum(n_i) is only known on the GPU
   unsigned long long* prof;  // perf experiments only (env VTK_GEMM_PROF): per-role clock64 accumulators, or null
-  int debug;            // perf experiments only (env VTK_EPI_DEBUG): 1 = no global stores, 2 = skip epilogue math+stores
 };
 
 struct GemmArgs {

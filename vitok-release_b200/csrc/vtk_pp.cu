@@ -10,8 +10,6 @@
 //   unpatchify   vitok/pp/ops.py:295-335: scatter + fold restated as a gather through a cell->token map,
 //                with _convert_format (vitok/pp/io.py:91-121) optionally fused.
 // All integer/byte work is bit-exact against the reference.
-#include <stdlib.h>
-
 #include "vtk_common.cuh"
 #include "vtk_kernels.h"
 
@@ -194,94 +192,7 @@ __global__ void __launch_bounds__(256) patchify_kernel(const PatchifyArgs a) {
   }
 }
 
-// uint8 HWC input, row-coalesced: thread <-> 16 consecutive pixels of one image row (48 contiguous bytes = three 16-byte loads; a warp
-// reads 1.5 KB of a row instead of eight 48-byte pieces), normalised arithmetically and written as 16-element runs of the three channel
-// planes of the token (64 B of fp32 / 32 B of bf16 each: whole sectors).  Work item = (image, y, 16-pixel group) over the bounding box of
-// the batch; tokens beyond an image's grid (padding tokens) and the index arrays are written by a second pass over tokens.
-template <typename OutT, int PT>
-__global__ void __launch_bounds__(256) patchify_u8_rows_kernel(const PatchifyArgs a, const int max_w16, const int max_rows) {
-  pdl_wait();
-  pdl_trigger();
-  constexpr int p = PT, pp = p * p, P = 3 * pp;
-  const int T = a.max_tokens;
-  // ---- pass 1: pixels.  idx -> (b, y, x16) over the bounding box [max_rows x max_w16] of the batch (threads outside an image idle)
-  const long long per_img = (long long)max_rows * max_w16;
-  const long long total = per_img * a.B;
-  for (long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x; idx < total; idx += (long long)gridDim.x * blockDim.x) {
-    const int b = (int)(idx / per_img);
-    const int rem = (int)(idx - (long long)b * per_img);
-    const int y = rem / max_w16, x = (rem - y * max_w16) << 4;
-    const int H = (int)a.img_table[3 * b + 1], W = (int)a.img_table[3 * b + 2];
-    const int gr = (H + p - 1) / p, gc = (W + p - 1) / p;
-    if (gr * gc > T || y >= gr * p || x >= gc * p) continue;        // outside this image's patch grid
-    const int r = y / p, dy = y - r * p, c = x / p, dx = x - c * p;
-    OutT* dst = reinterpret_cast<OutT*>(a.patches) + ((long long)b * T + r * gc + c) * P + dy * p + dx;
-    uint32_t w[12];
-#pragma unroll
-    for (int k = 0; k < 12; ++k) w[k] = 0u;
-    int np = 0;                                                      // pixels of this run inside the image
-    if (y < H && x < W) {
-      np = min(16, W - x);
-      const uint8_t* src = reinterpret_cast<const uint8_t*>(a.images) + a.img_table[3 * b] + ((long long)y * W + x) * 3;
-      if (np == 16 && (reinterpret_cast<uintptr_t>(src) & 15) == 0) {
-        const uint4 q0 = __ldg(reinterpret_cast<const uint4*>(src)), q1 = __ldg(reinterpret_cast<const uint4*>(src) + 1),
-                    q2 = __ldg(reinterpret_cast<const uint4*>(src) + 2);
-        w[0] = q0.x; w[1] = q0.y; w[2] = q0.z; w[3] = q0.w; w[4] = q1.x; w[5] = q1.y; w[6] = q1.z; w[7] = q1.w;
-        w[8] = q2.x; w[9] = q2.y; w[10] = q2.z; w[11] = q2.w;
-      } else if (np == 16 && (reinterpret_cast<uintptr_t>(src) & 3) == 0) {
-#pragma unroll
-        for (int k = 0; k < 12; ++k) w[k] = __ldg(reinterpret_cast<const uint32_t*>(src) + k);
-      } else {
-#pragma unroll
-        for (int k = 0; k < 48; ++k)        // (fully unrolled: w[] must stay in registers)
-          if (k < np * 3) w[k >> 2] |= (uint32_t)src[k] << (8 * (k & 3));
-      }
-    }
-    // byte i of the run = pixel i / 3, channel i % 3; pixels at or beyond np stay 0.0 (zero padding is applied AFTER normalize)
-#pragma unroll
-    for (int ch = 0; ch < 3; ++ch) {
-      float v[16];
-#pragma unroll
-      for (int px = 0; px < 16; ++px) {
-        const int i = 3 * px + ch;
-        const float f = norm_u8_fast((w[i >> 2] >> (8 * (i & 3))) & 255u);
-        v[px] = px < np ? f : 0.f;
-      }
-#pragma unroll
-      for (int g = 0; g < 4; ++g) store4(dst + ch * pp + 4 * g, make_float4(v[4 * g], v[4 * g + 1], v[4 * g + 2], v[4 * g + 3]));
-    }
-  }
-  // ---- pass 2: per token -- index arrays, metadata, and the zero rows of padding tokens (one warp per token)
-  const int lane = threadIdx.x & 31;
-  const unsigned ntok = (unsigned)a.B * (unsigned)T;
-  const unsigned nwarp = gridDim.x * (blockDim.x >> 5);
-  for (unsigned bt = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5); bt < ntok; bt += nwarp) {
-    const int b = (int)(bt / (unsigned)T), t = (int)(bt - (unsigned)b * (unsigned)T);
-    const int H = (int)a.img_table[3 * b + 1], W = (int)a.img_table[3 * b + 2];
-    const int gr = (H + p - 1) / p, gc = (W + p - 1) / p;
-    const int n = gr * gc;
-    const bool valid = t < n && n <= T;
-    if (!valid) {
-      OutT* dst = reinterpret_cast<OutT*>(a.patches) + (long long)bt * P;
-      for (int e4 = lane; e4 < (P >> 2); e4 += 32) store4(dst + (e4 << 2), make_float4(0.f, 0.f, 0.f, 0.f));
-    }
-    if (lane == 0) {
-      a.patch_mask[bt] = valid ? 1 : 0;
-      a.row_idx[bt] = valid ? t / gc : 0;
-      a.col_idx[bt] = valid ? t - (t / gc) * gc : 0;
-      a.time_idx[bt] = 0;
-      if (t == 0) {
-        a.meta[0 * a.B + b] = H;
-        a.meta[1 * a.B + b] = W;
-        a.meta[2 * a.B + b] = gr;
-        a.meta[3 * a.B + b] = gc;
-        if (n > T && a.status) atomicExch(a.status, 1);
-      }
-    }
-  }
-}
-
-// uint8 HWC input, staged through shared memory (round 2, second rewrite).  The row kernel above reads coalesced but every one of its
+// uint8 HWC input, staged through shared memory (round 2, second rewrite).  A register-only row kernel reads coalesced but every one of its
 // store instructions touches 32 different 128-byte lines (a lane owns one image row of one token = 16 elements of a plane, the next lane
 // the next TOKEN), and the load/store unit needs one pass per line: ncu 1.8 TB/s, LSU wavefronts 71 % of peak.  Here a persistent CTA walks
 // STRIPS = the PT image rows of one token row x up to 256 pixels:
@@ -505,32 +416,12 @@ int launch_patchify(const PatchifyArgs& a, cudaStream_t stream) {
   const long long ntok = (long long)a.B * a.max_tokens;
   if (ntok >= (1ll << 31)) { set_error("patchify: B * max_tokens too large"); return -2; }
   if (a.in_dtype == 1 && (a.patch == 16 || a.patch == 32) && a.max_h > 0 && a.max_w > 0) {
-    // uint8 HWC front end over the batch's bounding box (the caller knows every image size): the shared-memory-staged strip kernel;
-    // VTK_PATCHIFY_U8=rows keeps the register-only row kernel for A/B (byte-identical output)
-    static const bool use_rows = getenv("VTK_PATCHIFY_U8") && getenv("VTK_PATCHIFY_U8")[0] == 'r';
-    if (!use_rows) {
-      int rc;
-      if (a.out_dtype == 0) rc = a.patch == 16 ? patchify_u8_strip_launch<float, 16>(a, stream) : patchify_u8_strip_launch<float, 32>(a, stream);
-      else rc = a.patch == 16 ? patchify_u8_strip_launch<bf16, 16>(a, stream) : patchify_u8_strip_launch<bf16, 32>(a, stream);
-      if (rc) return rc;
-      return check_cuda(cudaGetLastError(), "patchify (uint8 strips) launch");
-    }
-    const int p = a.patch;
-    const int max_rows = (a.max_h + p - 1) / p * p, max_w4 = ((a.max_w + p - 1) / p * p) >> 4;   // 16-pixel runs per bounding-box row
-    const long long total = (long long)a.B * max_rows * max_w4;
-    long long blocks = (total + 255) / 256;
-    const long long cap = (long long)num_sms() * 8 * 16;
-    if (blocks > cap) blocks = cap;
-    if (blocks < (ntok + 7) / 8 && (ntok + 7) / 8 <= cap) blocks = (ntok + 7) / 8;   // enough warps for the per-token pass
-    const dim3 g((unsigned)blocks), b(256);
-    if (a.out_dtype == 0) {
-      if (p == 16) (void)launch_k(patchify_u8_rows_kernel<float, 16>, g, b, 0, stream, a, max_w4, max_rows);
-      else (void)launch_k(patchify_u8_rows_kernel<float, 32>, g, b, 0, stream, a, max_w4, max_rows);
-    } else {
-      if (p == 16) (void)launch_k(patchify_u8_rows_kernel<bf16, 16>, g, b, 0, stream, a, max_w4, max_rows);
-      else (void)launch_k(patchify_u8_rows_kernel<bf16, 32>, g, b, 0, stream, a, max_w4, max_rows);
-    }
-    return check_cuda(cudaGetLastError(), "patchify (uint8 rows) launch");
+    // uint8 HWC front end over the batch's bounding box (the caller knows every image size): the shared-memory-staged strip kernel
+    int rc;
+    if (a.out_dtype == 0) rc = a.patch == 16 ? patchify_u8_strip_launch<float, 16>(a, stream) : patchify_u8_strip_launch<float, 32>(a, stream);
+    else rc = a.patch == 16 ? patchify_u8_strip_launch<bf16, 16>(a, stream) : patchify_u8_strip_launch<bf16, 32>(a, stream);
+    if (rc) return rc;
+    return check_cuda(cudaGetLastError(), "patchify (uint8 strips) launch");
   }
   long long blocks = (ntok + 7) / 8;                   // one warp per token, 8 warps per CTA: the block scheduler balances the tail
   const long long cap = (long long)num_sms() * 8 * 16;  // (a fixed grid of one wave left the last tokens to a few warps); warp-stride beyond
@@ -878,13 +769,13 @@ __device__ __forceinline__ uint32_t to_u8x4(const float (&v)[4], bool bf16_math)
 }
 
 // One warp per canvas cell (b, r, c): the token that owns the cell is looked up once, its 3p^2 elements are read as
-// contiguous 8 / 16-byte chunks (coalesced) and written as p-pixel row segments of the three channel planes.  PT = compile-
-// time patch size (16 / 32; 0 = any multiple of 4) so the per-chunk index math is shifts, not divisions.
-template <typename T, int PT>
+// contiguous 8 / 16-byte chunks (coalesced) and written as p-pixel row segments of the three channel planes.  Patch sizes
+// other than 16 / 32 (any multiple of 4); those two have the row kernel below.
+template <typename T>
 __global__ void __launch_bounds__(256) unpatchify_kernel(const UnpatchifyArgs a) {
   pdl_wait();      // PDL (vtk_common.cuh): this kernel may have been launched before its predecessor finished
   pdl_trigger();
-  const int p = PT ? PT : a.patch, pp = p * p, P = 3 * pp, p4 = p >> 2, chunks = pp >> 2;
+  const int p = a.patch, pp = p * p, P = 3 * pp, p4 = p >> 2, chunks = pp >> 2;
   const int Hc = a.gy * p, Wc = a.gx * p;
   const int cells_per_img = a.gy * a.gx;
   const unsigned ncell = (unsigned)a.B * (unsigned)cells_per_img;
@@ -1025,15 +916,9 @@ static void unpatchify_rows_launch(const UnpatchifyArgs& a, cudaStream_t stream)
 
 template <typename T>
 static void unpatchify_dispatch(const UnpatchifyArgs& a, int blocks, cudaStream_t stream) {
-  static const int rows_mode = getenv("VTK_UNPATCHIFY_ROWS") ? atoi(getenv("VTK_UNPATCHIFY_ROWS")) : 1;   // 0: cell-per-warp kernel (A/B)
-  if (rows_mode && (a.patch == 16 || a.patch == 32)) {
-    if (a.patch == 16) unpatchify_rows_launch<T, 16>(a, stream);
-    else unpatchify_rows_launch<T, 32>(a, stream);
-    return;
-  }
-  if (a.patch == 16) (void)launch_k(unpatchify_kernel<T, 16>, dim3(blocks), dim3(256), 0, stream, a);
-  else if (a.patch == 32) (void)launch_k(unpatchify_kernel<T, 32>, dim3(blocks), dim3(256), 0, stream, a);
-  else (void)launch_k(unpatchify_kernel<T, 0>, dim3(blocks), dim3(256), 0, stream, a);
+  if (a.patch == 16) unpatchify_rows_launch<T, 16>(a, stream);
+  else if (a.patch == 32) unpatchify_rows_launch<T, 32>(a, stream);
+  else (void)launch_k(unpatchify_kernel<T>, dim3(blocks), dim3(256), 0, stream, a);
 }
 
 int launch_unpatchify(const UnpatchifyArgs& a, cudaStream_t stream) {

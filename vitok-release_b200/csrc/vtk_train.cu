@@ -1009,9 +1009,8 @@ int launch_qk_norm_rope_fwd(const bf16* zraw, long long ldz, const bf16* wq, con
                             long long ldq, int M, int heads, int d, float eps, cudaStream_t st) {
   VTK_TRAIN_CHECK(d == 64 || d == 128, "qk_norm_rope: head_dim %d unsupported (64 or 128)", d);
   if (M <= 0) return 0;
-  static const int v1 = getenv("VTK_TRAIN_V1") ? atoi(getenv("VTK_TRAIN_V1")) : 0;   // 1: the round-1 kernels (A/B)
   const int hpw = 32 / (d / 8);
-  if (!v1 && heads % hpw == 0 && ldz % 8 == 0 && ldq % 8 == 0 && (long long)M * (3 * heads / hpw) < (1ll << 31) &&
+  if (heads % hpw == 0 && ldz % 8 == 0 && ldq % 8 == 0 && (long long)M * (3 * heads / hpw) < (1ll << 31) &&
       ((reinterpret_cast<uintptr_t>(zraw) | reinterpret_cast<uintptr_t>(qkv) | reinterpret_cast<uintptr_t>(wq) | reinterpret_cast<uintptr_t>(wk) |
         reinterpret_cast<uintptr_t>(rope)) & 15) == 0) {
     const int g16 = grid_for(((long long)M * (3 * heads / hpw) + 3) / 4, 8, 8);
@@ -1075,9 +1074,8 @@ int launch_qk_norm_rope_bwd(bf16* dz, long long lddz, const bf16* zraw, long lon
                             const bf16* rope, float* dw, int M, int heads, int d, float eps, cudaStream_t st) {
   VTK_TRAIN_CHECK(d == 64 || d == 128, "qk_norm_rope_bwd: head_dim %d unsupported (64 or 128)", d);
   if (M <= 0) return 0;
-  static const int v1 = getenv("VTK_TRAIN_V1") ? atoi(getenv("VTK_TRAIN_V1")) : 0;
   const int hpw = 32 / (d / 8);
-  if (!v1 && heads % hpw == 0 && ldz % 8 == 0 && lddz % 8 == 0 && (long long)M * (2 * heads / hpw) < (1ll << 31) &&
+  if (heads % hpw == 0 && ldz % 8 == 0 && lddz % 8 == 0 && (long long)M * (2 * heads / hpw) < (1ll << 31) &&
       ((reinterpret_cast<uintptr_t>(zraw) | reinterpret_cast<uintptr_t>(dz) | reinterpret_cast<uintptr_t>(wq) | reinterpret_cast<uintptr_t>(wk) |
         reinterpret_cast<uintptr_t>(rope)) & 15) == 0) {
     const int g16 = grid_for(((long long)M * (2 * heads / hpw) + 3) / 4, 8, 4);
@@ -1094,8 +1092,7 @@ int launch_rmsnorm_bwd(const bf16* x, const bf16* dh, const bf16* w, const bf16*
                        float eps, cudaStream_t st) {
   VTK_TRAIN_CHECK(D % 8 == 0 && D <= 4096, "rmsnorm_bwd: D %% 8 == 0 and D <= 4096 required (D=%d)", D);
   if (M <= 0) return 0;
-  static const int v1 = getenv("VTK_TRAIN_V1") ? atoi(getenv("VTK_TRAIN_V1")) : 0;
-  if (!v1 && ((reinterpret_cast<uintptr_t>(x) | reinterpret_cast<uintptr_t>(dh) | reinterpret_cast<uintptr_t>(w) |
+  if (((reinterpret_cast<uintptr_t>(x) | reinterpret_cast<uintptr_t>(dh) | reinterpret_cast<uintptr_t>(w) |
                reinterpret_cast<uintptr_t>(dx_res) | reinterpret_cast<uintptr_t>(dx_out)) & 15) == 0) {
     const int threads = ((D / 8) + 31) / 32 * 32;                       // <= 512 for D <= 4096
     const int per_sm = threads <= 192 ? 4 : threads <= 384 ? 2 : 1;

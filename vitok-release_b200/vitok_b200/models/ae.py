@@ -21,8 +21,6 @@ Training: ``model(batch)`` in train mode builds one autograd node (vitok_b200/tr
 """
 from __future__ import annotations
 
-import os
-
 import ctypes
 import itertools
 import re
@@ -258,7 +256,7 @@ class AE(nn.Module):
         self.token_packing = True
         # Block.norm1 fused into the GEMM epilogues (widths that are multiples of 256): no RMSNorm kernel, no h buffer
         # round trip.  False keeps the separate RMSNorm kernel (rounds h to bf16 exactly where the reference does).
-        self.fuse_norm = os.environ.get("VTK_NO_FUSE_NORM", "0") != "1"
+        self.fuse_norm = True
         # quantize(): dynamic FP8 activation scale per "row" (default: finer, no extra pass over the activations) or per "tensor"
         # (torchao's default granularity for Float8DynamicActivationFloat8WeightConfig, the reference's numerics)
         self.fp8_activation_scale = "row"

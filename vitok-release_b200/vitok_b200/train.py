@@ -145,15 +145,12 @@ def enable_grad_sync(model, process_group=None, broadcast_parameters: bool = Tru
     ``broadcast_parameters`` the parameters of rank 0 are copied to every rank first (what DDP's constructor does).
     ``reserve_sms``: SMs the persistent GEMM / attention kernels leave free for NCCL's all-reduce CTAs, which run next to the
     backward kernels (include/vitok_b200.h: vtk_set_flag "reserve_sms"); None keeps the process-wide setting."""
-    import os
     import torch.distributed as dist
     if reserve_sms is not None:
         _lib.set_flag("reserve_sms", int(reserve_sms))
-    if (process_group is None and dist.get_world_size() > 1 and dist.get_backend() == "nccl"
-            and os.environ.get("VTK_GRAD_SYNC_HIPRIO", "1") != "0"):
+    if process_group is None and dist.get_world_size() > 1 and dist.get_backend() == "nccl":
         # The per-block all-reduces run NEXT TO the backward kernels: give them their own communicator on a high-priority stream so
-        # that their CTAs are placed as soon as SMs free up instead of queueing behind the next GEMM's grid (VTK_GRAD_SYNC_HIPRIO=0:
-        # the default process group).
+        # that their CTAs are placed as soon as SMs free up instead of queueing behind the next GEMM's grid.
         try:
             opts = dist.ProcessGroupNCCL.Options(is_high_priority_stream=True)
             process_group = dist.new_group(backend="nccl", pg_options=opts)
