@@ -204,6 +204,14 @@ int vtk_attention_packed_bf16(const void* q, const void* k, const void* v, int64
                               int64_t row_cap, int grp_cap, void* stream);
 /* lse (optional, may be null): [B*N, heads] fp32, log2-domain logsumexp of the scaled scores (+inf for zeroed rows);
  * the training backward (vtk_attention_bwd_bf16) consumes it. */
+/* The packed form with lse, for the training step on packed rows (vitok/models/modules/attention.py:118-127 under autograd):
+ * lse [row_cap, heads] fp32.  For image b it writes packed rows [cu[b], cu[b+1]) only: rows below n_valid[b] get out and lse as in
+ * vtk_attention_packed_bf16 (equal to vtk_attention_bf16 with kv_len = n_valid and zero_invalid_rows = 1), the image's pad rows
+ * [cu[b] + n_valid[b], cu[b+1]) get out = 0 and lse = +inf.  Rows of other images -- the rest of a partial last tile -- are not
+ * touched.  qrows of the plan: 128 (d = 64) or 256 (d = 128), as above. */
+int vtk_attention_packed_lse_bf16(const void* q, const void* k, const void* v, int64_t ld_qkv, void* out, int64_t ld_out,
+                                  const int* n_valid, const int* cu, const int* cuq, const int* grp_img, const int* grp_order, int B, int N,
+                                  int heads, int d, int64_t row_cap, int grp_cap, float* lse, void* stream);
 
 /* out [M,N] (+)= A [M,K] @ Bt [K,N] with B read as stored (the data gradient dX = dY W; vtk_linear_nn_bf16); accumulate != 0 adds to
  * what `out` already holds, in fp32 before the bf16 rounding (dh = dz_qkv Wqkv + dz_fc1 W1 without a separate add pass). */
@@ -281,6 +289,17 @@ int vtk_attn_delta(const void* o, int64_t ldo, const void* dout, int64_t lddo, f
 int vtk_attention_bwd_bf16(const void* q, const void* k, const void* v, int64_t ld_qkv, const void* dout, int64_t ld_do,
                            const float* lse, const float* delta, void* dq, void* dk, void* dv, int64_t ld_d, const int* kv_len,
                            int B, int N, int heads, int d, int zero_invalid_rows, int window, void* stream);
+/* The same on the packed NaFlex layout (autograd of modules/attention.py:118-127 for the packed training step), d = 64 or 128:
+ * lse from vtk_attention_packed_lse_bf16, delta [row_cap, heads] from vtk_attn_delta over the packed rows.  The plan must have
+ * qrows = 128 for both head dims (the d = 128 forward's plan has qrows = 256: a second plan of the same mask, whose n_valid / cu
+ * are the same).  Two passes, each one CTA per (128-row group, head) taken in grp_order: dK/dV per key tile, then dQ per query
+ * tile; grp_cap (>= cuq[B], CTAs beyond cuq[B] exit) sizes the grid.  For image b it writes dq / dk / dv rows [cu[b], cu[b+1])
+ * only: gradients for rows below n_valid[b], zeros for the image's pad rows; rows of other images are not touched.  Query rows
+ * past n_valid[b] in a partial last tile (the next image's rows) contribute nothing to dK / dV whatever their dO. */
+int vtk_attention_bwd_packed_bf16(const void* q, const void* k, const void* v, int64_t ld_qkv, const void* dout, int64_t ld_do,
+                                  const float* lse, const float* delta, void* dq, void* dk, void* dv, int64_t ld_d, const int* n_valid,
+                                  const int* cu, const int* cuq, const int* grp_img, const int* grp_order, int B, int heads, int d,
+                                  int64_t row_cap, int grp_cap, void* stream);
 
 /* test-only: D[128,N] fp32 = A[128,K] * op(B) through one tcgen05 tile with explicit descriptor fields */
 int vtk_umma_probe(const void* A, const void* B, float* D, int N, int K, int b_mn_major, uint32_t lbo_bytes,

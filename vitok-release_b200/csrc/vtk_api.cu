@@ -545,6 +545,19 @@ int vtk_attention_packed_bf16(const void* q, const void* k, const void* v, int64
   return launch_attention(a, (cudaStream_t)stream);
 }
 
+int vtk_attention_packed_lse_bf16(const void* q, const void* k, const void* v, int64_t ld_qkv, void* out, int64_t ld_out,
+                                  const int* n_valid, const int* cu, const int* cuq, const int* grp_img, const int* grp_order, int B, int N,
+                                  int heads, int d, int64_t row_cap, int grp_cap, float* lse, void* stream) {
+  VTK_REQUIRE(q && k && v && out && n_valid && cu && cuq && grp_img && grp_order && lse, "vtk_attention_packed_lse_bf16: null pointer");
+  AttnArgs a;
+  a.q = (const bf16*)q; a.k = (const bf16*)k; a.v = (const bf16*)v; a.ld_qkv = ld_qkv; a.out = (bf16*)out; a.ld_out = ld_out;
+  a.kv_len = n_valid; a.key_mask = nullptr; a.prefix_flag = nullptr; a.B = B; a.N = N; a.heads = heads; a.d = d;
+  a.zero_invalid_rows = 1;   // the image's pad rows: out 0, lse +inf
+  a.window = -1; a.lse = lse;
+  a.cu = cu; a.cuq = cuq; a.grp_img = grp_img; a.grp_order = grp_order; a.row_cap = row_cap; a.grp_cap = grp_cap;
+  return launch_attention(a, (cudaStream_t)stream);
+}
+
 int vtk_umma_probe(const void* A, const void* B, float* D, int N, int K, int b_mn_major, uint32_t lbo_bytes,
                    uint32_t sbo_bytes, uint32_t kstep_bytes, void* stream) {
   VTK_REQUIRE(A && B && D, "vtk_umma_probe: null pointer");
@@ -656,6 +669,20 @@ int vtk_attention_bwd_bf16(const void* q, const void* k, const void* v, int64_t 
   a.q = (const bf16*)q; a.k = (const bf16*)k; a.v = (const bf16*)v; a.ld_qkv = ld_qkv; a.dout = (const bf16*)dout; a.ld_do = ld_do;
   a.lse = lse; a.delta = delta; a.dq = (bf16*)dq; a.dk = (bf16*)dk; a.dv = (bf16*)dv; a.ld_d = ld_d; a.kv_len = kv_len;
   a.B = B; a.N = N; a.heads = heads; a.d = d; a.zero_invalid_rows = zero_invalid_rows; a.window = window;
+  return launch_attention_bwd(a, (cudaStream_t)stream);
+}
+
+int vtk_attention_bwd_packed_bf16(const void* q, const void* k, const void* v, int64_t ld_qkv, const void* dout, int64_t ld_do,
+                                  const float* lse, const float* delta, void* dq, void* dk, void* dv, int64_t ld_d, const int* n_valid,
+                                  const int* cu, const int* cuq, const int* grp_img, const int* grp_order, int B, int heads, int d,
+                                  int64_t row_cap, int grp_cap, void* stream) {
+  VTK_REQUIRE(q && k && v && dout && lse && delta && dq && dk && dv && n_valid && cu && cuq && grp_img && grp_order,
+              "vtk_attention_bwd_packed_bf16: null pointer");
+  AttnBwdArgs a;
+  a.q = (const bf16*)q; a.k = (const bf16*)k; a.v = (const bf16*)v; a.ld_qkv = ld_qkv; a.dout = (const bf16*)dout; a.ld_do = ld_do;
+  a.lse = lse; a.delta = delta; a.dq = (bf16*)dq; a.dk = (bf16*)dk; a.dv = (bf16*)dv; a.ld_d = ld_d; a.kv_len = n_valid;
+  a.B = B; a.N = 0; a.heads = heads; a.d = d; a.zero_invalid_rows = 1; a.window = -1;
+  a.cu = cu; a.cuq = cuq; a.grp_img = grp_img; a.grp_order = grp_order; a.row_cap = row_cap; a.grp_cap = grp_cap;
   return launch_attention_bwd(a, (cudaStream_t)stream);
 }
 

@@ -63,7 +63,7 @@ struct AttnParams {
   int window;         // sliding window |i - j| <= window on the token index (flash backend, attention.py:113-116); < 0 = none
   float scale_log2;   // (1/sqrt(d)) * log2(e)
   unsigned long long* prof;   // perf experiments (env VTK_ATTN_PROF): clock64 accumulators, or null
-  float* lse;                 // [B*N, heads] log2-domain logsumexp of the scaled scores (training), or null; +inf for zero rows
+  float* lse;                 // [rows, heads] log2-domain logsumexp of the scaled scores (training), or null; +inf for zero rows
   // packed NaFlex batches: image b owns packed rows [cu[b], cu[b+1]) and holds kv_len[b] valid tokens at the front; work group g
   // (128 query rows for the persistent kernel, NQ * 128 for the one-shot kernel) is the (g - cuq[img])-th group of image
   // img = grp_img[g]; cuq[B] (= *n_grp) groups exist; grp_order lists them longest image first
@@ -207,7 +207,9 @@ attn_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__ CUt
     row0 = p.cu[img];
     q0 = (grp - p.cuq[img]) * (NQ * ATT_BQ);
     kvlen = p.kv_len[img];
-    N = kvlen;                           // rows >= kvlen of the last tile belong to the next image: never stored
+    // rows stored: the valid ones, plus (zero_invalid: the training forward, which needs lse) the image's pad rows as 0 / +inf.
+    // Rows past cu[img + 1] belong to the next image and are never stored.
+    N = p.zero_invalid ? p.cu[img + 1] - (int)row0 : kvlen;
   } else {
     q0 = blockIdx.x * (NQ * ATT_BQ);
     img = blockIdx.z;
@@ -568,7 +570,8 @@ __device__ __forceinline__ AttnItem attn_item(const AttnParams& p, int w, int qt
     it.row0 = p.cu[it.img];
     it.q0 = (grp - p.cuq[it.img]) * ATT_BQ;
     it.kvlen = p.kv_len[it.img];
-    it.nrows = it.kvlen;                     // rows >= kvlen of the last tile belong to the next image: never stored
+    // rows stored: the valid ones (+ the image's pad rows as 0 / +inf under zero_invalid); rows past cu[img + 1] belong to the next image
+    it.nrows = p.zero_invalid ? p.cu[it.img + 1] - (int)it.row0 : it.kvlen;
   } else {
     const int per_img = qtiles * p.heads;
     it.img = w / per_img;

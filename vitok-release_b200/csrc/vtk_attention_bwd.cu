@@ -19,6 +19,10 @@
 // Two compute warpgroups (warps 0-3 and 8-11) split every [128 x 128] S / dP tile by columns (64 keys each; a warp may
 // only read the TMEM lanes of its quarter, so both groups own the same rows), which halves the P / dS latency that
 // sits between the two MMA groups; tiles that need no masking skip the per-element key test.
+// Packed NaFlex layout (vtk_attention_bwd_packed_bf16, the training step with AE.train_token_packing): the same two passes over
+// 128-row tiles of one image, image b at packed rows [cu[b], cu[b] + n_valid[b]); the grid is the plan's compact work list of
+// (128-row group, head) instead of (tiles, heads, B).  Stores stay inside [cu[b], cu[b+1]) (zeros for the image's pad rows), and MODE 0
+// masks query rows >= n_valid[b] explicitly: after a partial last tile they are the next image's rows, whose dO is not 0.
 #include <math.h>
 #include <stdio.h>
 
@@ -58,13 +62,17 @@ struct BwdParams {
   const int* kv_len;
   int N, heads, zero_invalid, window;
   float scale, scale_log2;
+  // packed layout (PACKED kernels): image b = rows [cu[b], cu[b+1]), kv_len[b] valid tokens in front; 128-row group g is the
+  // (g - cuq[img])-th tile of img = grp_img[g]; *n_grp groups exist, grp_order lists them longest image first
+  const int* cu; const int* cuq; const int* grp_img; const int* grp_order; const int* n_grp;
 };
 
 // P and dS of one 32-key chunk of a row: P = exp2(S * scale*log2e - lse), dS = P * (dP - delta) * scale, written as bf16
-// into the row's 128B-swizzled slots.  MASKED = false: every key of the chunk is live (no per-element test).
+// into the row's 128B-swizzled slots.  MASKED = false: every key of the chunk is live (no per-element test).  qlive = false
+// (packed MODE 0: a query row past the image end, which belongs to the next image): P and dS of the whole row are 0.
 template <int MODE, bool MASKED>
 __device__ __forceinline__ void bwd_chunk(const uint32_t (&sv)[32], const uint32_t (&dv)[32], float lse_r, float delta_r,
-                                          float scale_log2, float scale, int kc0, int kvlen, int W, int qi, uint8_t* prow,
+                                          float scale_log2, float scale, int kc0, int kvlen, int W, int qi, bool qlive, uint8_t* prow,
                                           uint8_t* dsrow, int c, int r) {
 #pragma unroll
   for (int g = 0; g < 4; ++g) {
@@ -78,11 +86,12 @@ __device__ __forceinline__ void bwd_chunk(const uint32_t (&sv)[32], const uint32
         float pe = ex2_approx_bwd(fmaf(__uint_as_float(sv[col]), scale_log2, -lse_r));
         if (MASKED) {
           const int kc = kc0 + col;
-          const bool ok = kc < kvlen && (W < 0 || abs(kc - qi) <= W);
+          const bool ok = qlive && kc < kvlen && (W < 0 || abs(kc - qi) <= W);
           pe = ok ? pe : 0.f;
         }
         pv[e] = pe;
         dsv[e] = pe * (__uint_as_float(dv[col]) - delta_r) * scale;
+        if (MASKED) dsv[e] = qlive ? dsv[e] : 0.f;   // the next image's dP may be anything: no 0 * inf
       }
       pp[i] = bf2_cvt(pv[0], pv[1]);
       dd[i] = bf2_cvt(dsv[0], dsv[1]);
@@ -94,19 +103,38 @@ __device__ __forceinline__ void bwd_chunk(const uint32_t (&sv)[32], const uint32
   }
 }
 
-template <int DH, int MODE>
+// PACKED: the packed NaFlex layout.  One CTA per (128-row group of one image, head) from the plan's work list instead of a
+// (tiles, heads, B) grid; N becomes the image's packed row count (valid rows, then its pad rows, which get zero gradients), and
+// MODE 0 masks query rows >= kv_len explicitly: in the padded layout those rows are the image's own padding (dO = 0, lse = +inf),
+// here the rows after a partial last query tile belong to the next image.
+template <int DH, int MODE, bool PACKED>
 __global__ void __launch_bounds__(384, 1)
 attn_bwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__ CUtensorMap tmK,
                 const __grid_constant__ CUtensorMap tmV, const __grid_constant__ CUtensorMap tmDO, const BwdParams p) {
   using S = BwdShape<DH>;
-  const int tile0 = blockIdx.x * BWD_T;   // MODE 0: first key of this CTA; MODE 1: first query
-  const int head = blockIdx.y, img = blockIdx.z;
+  int tile0, head, img, N, kvlen;   // tile0 = MODE 0: first key of this CTA; MODE 1: first query
+  long long row0;
+  if (PACKED) {
+    const int rank = blockIdx.x / p.heads;
+    if (rank >= __ldg(p.n_grp)) return;   // beyond the groups of this batch (whole CTA)
+    head = blockIdx.x - rank * p.heads;
+    const int grp = p.grp_order[rank];
+    img = p.grp_img[grp];
+    row0 = p.cu[img];
+    N = p.cu[img + 1] - (int)row0;
+    kvlen = p.kv_len[img];
+    tile0 = (grp - p.cuq[img]) * BWD_T;
+  } else {
+    tile0 = blockIdx.x * BWD_T;
+    head = blockIdx.y;
+    img = blockIdx.z;
+    N = p.N;
+    kvlen = p.kv_len ? p.kv_len[img] : N;
+    kvlen = kvlen < N ? kvlen : N;
+    row0 = (long long)img * N;
+  }
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int N = p.N;
-  int kvlen = p.kv_len ? p.kv_len[img] : N;
-  kvlen = kvlen < N ? kvlen : N;
   const int qlimit = p.zero_invalid ? kvlen : N;
-  const long long row0 = (long long)img * N;
   const int W = p.window;
 
   // the range of the OTHER dimension's tiles this CTA visits
@@ -306,7 +334,10 @@ attn_bwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__
         mbar_wait(&s1_free[(t - 1) % NB1], (uint32_t)((t - 1) / NB1) & 1u);
         __syncwarp();
       }
-      const bool need_mask = (k0 + BWD_T > kvlen) || W >= 0;   // warp-uniform
+      // warp-uniform; packed MODE 0 also masks the query rows of an image's partial last query tile
+      const bool row_mask = PACKED && MODE == 0 && other0 + BWD_T > qlimit;
+      const bool need_mask = (k0 + BWD_T > kvlen) || W >= 0 || row_mask;
+      const bool qlive = !row_mask || qi < qlimit;
 #pragma unroll
       for (int cc = 0; cc < 2; ++cc) {
         const int c = 2 * half + cc;
@@ -314,8 +345,8 @@ attn_bwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__
         tmem_ld32(tmem_base + lane_base + c * 32, sv);
         tmem_ld32(tmem_base + lane_base + 128 + c * 32, dv);
         tmem_wait_ld();
-        if (need_mask) bwd_chunk<MODE, true>(sv, dv, lse_r, delta_r, p.scale_log2, p.scale, k0 + c * 32, kvlen, W, qi, prow, dsrow, c, r);
-        else bwd_chunk<MODE, false>(sv, dv, lse_r, delta_r, p.scale_log2, p.scale, k0 + c * 32, kvlen, W, qi, prow, dsrow, c, r);
+        if (need_mask) bwd_chunk<MODE, true>(sv, dv, lse_r, delta_r, p.scale_log2, p.scale, k0 + c * 32, kvlen, W, qi, qlive, prow, dsrow, c, r);
+        else bwd_chunk<MODE, false>(sv, dv, lse_r, delta_r, p.scale_log2, p.scale, k0 + c * 32, kvlen, W, qi, true, prow, dsrow, c, r);
       }
       tc_fence_before();
       mbar_arrive(sdp_free);
@@ -360,10 +391,10 @@ attn_bwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__
   }
 }
 
-template <int DH>
+template <int DH, bool PACKED>
 static int launch_bwd_t(const AttnBwdArgs& a, cudaStream_t stream) {
   using S = BwdShape<DH>;
-  const long long Mrows = (long long)a.B * a.N;
+  const long long Mrows = PACKED ? a.row_cap : (long long)a.B * a.N;
   const long long cols = (long long)a.heads * a.d;
   CUtensorMap tmQ, tmK, tmV, tmDO;
   if (encode_tmap_bf16_sw128(&tmQ, a.q, cols, Mrows, a.ld_qkv, BWD_T)) return -1;
@@ -372,14 +403,16 @@ static int launch_bwd_t(const AttnBwdArgs& a, cudaStream_t stream) {
   if (encode_tmap_bf16_sw128(&tmDO, a.dout, cols, Mrows, a.ld_do, BWD_T)) return -1;
   BwdParams p;
   p.lse = a.lse; p.delta = a.delta; p.dq = a.dq; p.dk = a.dk; p.dv = a.dv; p.ld_d = a.ld_d; p.kv_len = a.kv_len;
-  p.N = a.N; p.heads = a.heads; p.zero_invalid = a.zero_invalid_rows; p.window = a.window;
+  p.N = a.N; p.heads = a.heads; p.zero_invalid = PACKED ? 1 : a.zero_invalid_rows; p.window = PACKED ? -1 : a.window;
   p.scale = (float)(1.0 / sqrt((double)a.d));
   p.scale_log2 = (float)((1.0 / sqrt((double)a.d)) * 1.4426950408889634);
-  auto k0 = attn_bwd_kernel<DH, 0>;
-  auto k1 = attn_bwd_kernel<DH, 1>;
+  p.cu = a.cu; p.cuq = a.cuq; p.grp_img = a.grp_img; p.grp_order = a.grp_order; p.n_grp = a.cuq ? a.cuq + a.B : nullptr;
+  auto k0 = attn_bwd_kernel<DH, 0, PACKED>;
+  auto k1 = attn_bwd_kernel<DH, 1, PACKED>;
   if (ensure_max_smem(reinterpret_cast<const void*>(k0), S::SMEM_BYTES, "attr(attn_bwd0)")) return -1;
   if (ensure_max_smem(reinterpret_cast<const void*>(k1), S::SMEM_BYTES, "attr(attn_bwd1)")) return -1;
   dim3 grid((a.N + BWD_T - 1) / BWD_T, a.heads, a.B);
+  if (PACKED) grid = dim3((unsigned)((long long)a.grp_cap * a.heads));
   k0<<<grid, 384, S::SMEM_BYTES, stream>>>(tmQ, tmK, tmV, tmDO, p);
   if (check_cuda(cudaGetLastError(), "attention bwd (dK/dV) launch")) return -1;
   k1<<<grid, 384, S::SMEM_BYTES, stream>>>(tmQ, tmK, tmV, tmDO, p);
@@ -387,10 +420,16 @@ static int launch_bwd_t(const AttnBwdArgs& a, cudaStream_t stream) {
 }
 
 int launch_attention_bwd(const AttnBwdArgs& a, cudaStream_t stream) {
-  if (a.B <= 0 || a.N <= 0 || a.heads <= 0) { set_error("attention_bwd: empty problem"); return -2; }
+  const bool packed = a.cu != nullptr;   // (N is not used by the packed layout)
+  if (a.B <= 0 || (!packed && a.N <= 0) || a.heads <= 0) { set_error("attention_bwd: empty problem"); return -2; }
   if ((a.ld_qkv % 8) || (a.ld_do % 8) || (a.ld_d % 8)) { set_error("attention_bwd: row strides must be multiples of 8"); return -2; }
-  if (a.d == 64) return launch_bwd_t<64>(a, stream);
-  if (a.d == 128) return launch_bwd_t<128>(a, stream);
+  if (packed && (!a.cuq || !a.grp_img || !a.grp_order || !a.kv_len || a.row_cap <= 0 || a.grp_cap <= 0 ||
+                 (long long)a.grp_cap * a.heads >= (1ll << 31))) {
+    set_error("attention_bwd: packed layout needs cu/cuq/grp_img/grp_order/kv_len and positive row and group capacities");
+    return -2;
+  }
+  if (a.d == 64) return packed ? launch_bwd_t<64, true>(a, stream) : launch_bwd_t<64, false>(a, stream);
+  if (a.d == 128) return packed ? launch_bwd_t<128, true>(a, stream) : launch_bwd_t<128, false>(a, stream);
   set_error("attention_bwd: head_dim %d unsupported (64 or 128)", a.d);
   return -3;
 }

@@ -121,7 +121,7 @@ struct AttnArgs {
   const uint8_t* key_mask;      // [B, N] or null
   const int* prefix_flag;       // [B] or null: 1 = key_mask[b] is a pure prefix (kv_len alone describes it)
   int B, N, heads, d;
-  int zero_invalid_rows;        // 1: rows >= kv_len[b] (or with key_mask 0) are written as 0
+  int zero_invalid_rows;        // 1: rows >= kv_len[b] (or with key_mask 0) are written as 0 (packed: the image's pad rows)
   int window;                   // sliding window: keys j with |i - j| <= window (flash_attn window_size=(w,w)); < 0 = none
   float* lse;                   // optional [B*N, heads] fp32: log2-domain logsumexp of the scaled scores (for the backward pass)
   // packed NaFlex layout (PackPlan): rows of image b start at cu[b] and hold kv_len[b] valid tokens, no key_mask; work group g
@@ -137,10 +137,15 @@ int launch_attention(const AttnArgs& a, cudaStream_t stream);
 struct AttnBwdArgs {
   const bf16* q; const bf16* k; const bf16* v; long long ld_qkv;
   const bf16* dout; long long ld_do;
-  const float* lse; const float* delta;   // [B*N, heads]
+  const float* lse; const float* delta;   // [B*N, heads] (packed: [row_cap, heads])
   bf16* dq; bf16* dk; bf16* dv; long long ld_d;
   const int* kv_len;
   int B, N, heads, d, zero_invalid_rows, window;
+  // packed NaFlex layout (PackPlan with qrows = 128): image b = rows [cu[b], cu[b+1]) with kv_len[b] valid tokens in front; one CTA
+  // per (128-row group, head) of each pass, groups taken in grp_order
+  const int* cu = nullptr; const int* cuq = nullptr; const int* grp_img = nullptr; const int* grp_order = nullptr;
+  long long row_cap = 0;   // rows of the q / k / v / dO / dq / dk / dv buffers
+  int grp_cap = 0;         // groups the grid covers (>= cuq[B]; CTAs beyond cuq[B] exit at once)
 };
 int launch_attention_bwd(const AttnBwdArgs& a, cudaStream_t stream);
 

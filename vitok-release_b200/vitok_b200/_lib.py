@@ -85,6 +85,8 @@ SIGNATURES = {
                                    c_int, c_int, c_vp, c_vp]),
     "vtk_attention_packed_bf16": (c_int, [c_vp, c_vp, c_vp, c_i64, c_vp, c_i64, c_vp, c_vp, c_vp, c_vp, c_vp, c_int, c_int, c_int, c_int,
                                           c_i64, c_int, c_vp]),
+    "vtk_attention_packed_lse_bf16": (c_int, [c_vp, c_vp, c_vp, c_i64, c_vp, c_i64, c_vp, c_vp, c_vp, c_vp, c_vp, c_int, c_int, c_int,
+                                              c_int, c_i64, c_int, c_vp, c_vp]),
     "vtk_qk_norm_rope_fwd": (c_int, [c_vp, c_i64, c_vp, c_vp, c_vp, c_vp, c_i64, c_int, c_int, c_int, c_f32, c_vp]),
     "vtk_swiglu_fwd": (c_int, [c_vp, c_i64, c_int, c_vp, c_i64, c_int, c_int, c_int, c_vp]),
     "vtk_resid_fwd": (c_int, [c_vp, c_vp, c_vp, c_vp, c_int, c_int, c_vp]),
@@ -101,6 +103,8 @@ SIGNATURES = {
     "vtk_attn_delta": (c_int, [c_vp, c_i64, c_vp, c_i64, c_vp, c_int, c_int, c_int, c_vp]),
     "vtk_attention_bwd_bf16": (c_int, [c_vp, c_vp, c_vp, c_i64, c_vp, c_i64, c_vp, c_vp, c_vp, c_vp, c_vp, c_i64, c_vp,
                                        c_int, c_int, c_int, c_int, c_int, c_int, c_vp]),
+    "vtk_attention_bwd_packed_bf16": (c_int, [c_vp, c_vp, c_vp, c_i64, c_vp, c_i64, c_vp, c_vp, c_vp, c_vp, c_vp, c_i64, c_vp, c_vp,
+                                              c_vp, c_vp, c_vp, c_int, c_int, c_int, c_i64, c_int, c_vp]),
     "vtk_umma_probe": (c_int, [c_vp, c_vp, c_vp, c_int, c_int, c_int, c_u32, c_u32, c_u32, c_vp]),
     "vtk_ae_create": (c_int, [ctypes.POINTER(AEConfig), ctypes.POINTER(c_vp)]),
     "vtk_ae_destroy": (c_int, [c_vp]),
@@ -425,13 +429,19 @@ def umma_probe(a: torch.Tensor, b: torch.Tensor, n: int, k: int, b_mn_major: boo
 
 
 @_on_device
-def attention_packed(qkv: torch.Tensor, plan: dict, B: int, N: int, heads: int, d: int) -> torch.Tensor:
+def attention_packed(qkv: torch.Tensor, plan: dict, B: int, N: int, heads: int, d: int, lse: Optional[torch.Tensor] = None,
+                     out: Optional[torch.Tensor] = None) -> torch.Tensor:
     """Attention over the packed NaFlex layout of ``pack_plan`` (qkv [row capacity, 3*heads*d]; the plan's qrows must be 128 for
-    d = 64, 256 for d = 128)."""
+    d = 64, 256 for d = 128).  Without ``lse`` the pad rows of ``out`` are never written; with ``lse`` ([rows, heads] fp32,
+    vtk_attention_packed_lse_bf16) they are written as 0 and lse as +inf.  ``out`` (optional) = a preallocated [rows, heads*d]."""
     D = heads * d
-    out = torch.empty(qkv.shape[0], D, dtype=torch.bfloat16, device=qkv.device)   # pad rows are never written
+    if out is None:
+        out = torch.empty(qkv.shape[0], D, dtype=torch.bfloat16, device=qkv.device)
     base = qkv.data_ptr()
-    check(load().vtk_attention_packed_bf16(base, base + 2 * D, base + 4 * D, qkv.stride(0), ptr(out), out.stride(0), ptr(plan["n_valid"]),
-                                           ptr(plan["cu"]), ptr(plan["cuq"]), ptr(plan["grp_img"]), ptr(plan["grp_order"]), B, N, heads, d,
-                                           qkv.shape[0], plan["grp_img"].numel(), stream_ptr()))
+    args = (base, base + 2 * D, base + 4 * D, qkv.stride(0), ptr(out), out.stride(0), ptr(plan["n_valid"]), ptr(plan["cu"]), ptr(plan["cuq"]),
+            ptr(plan["grp_img"]), ptr(plan["grp_order"]), B, N, heads, d, qkv.shape[0], plan["grp_img"].numel())
+    if lse is None:
+        check(load().vtk_attention_packed_bf16(*args, stream_ptr()))
+    else:
+        check(load().vtk_attention_packed_lse_bf16(*args, ptr(lse), stream_ptr()))
     return out

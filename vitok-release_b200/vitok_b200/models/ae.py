@@ -254,6 +254,10 @@ class AE(nn.Module):
         # NaFlex token packing for masked (sdpa-backend) batches: only valid tokens go through the layer stack
         # (include/vitok_b200.h, vtk_ae_set_packing).  False keeps the padded layout with in-kernel key masking.
         self.token_packing = True
+        # The same for the training step (train mode, sdpa backend with a patch_mask; vitok_b200/train.py: _Packing): GEMMs, kernels
+        # and saved activations cover the valid tokens only.  Off by default: the result differs from the padded step in the order of
+        # the weight-gradient sums, and masked tokens of the output are 0.  No effect without a mask or under the flash backend.
+        self.train_token_packing = False
         # Block.norm1 fused into the GEMM epilogues (widths that are multiples of 256): no RMSNorm kernel, no h buffer
         # round trip.  False keeps the separate RMSNorm kernel (rounds h to bf16 exactly where the reference does).
         self.fuse_norm = True

@@ -21,6 +21,10 @@ reference does (``keep_prob + torch.rand((B, 1, 1), dtype)`` floored), one draw 
 Any ``patch_mask`` is accepted under the sdpa backend: tokens are permuted so that each image's valid tokens come first
 (the model is equivariant to token order: positions travel in row_idx / col_idx), which turns every mask into the prefix
 mask the attention backward understands; the output is permuted back.
+``AE.train_token_packing`` (sdpa backend with a ``patch_mask``): the step runs on the packed NaFlex layout instead (``_Packing``,
+include/vitok_b200.h: vtk_pack_plan) -- every image's valid tokens, in token order, padded to 16 rows, so every GEMM, elementwise
+kernel and saved activation covers the valid tokens only; attention forward / backward are the packed kernels
+(vtk_attention_packed_lse_bf16, vtk_attention_bwd_packed_bf16).  No permutation is needed for masks with holes.
 """
 from __future__ import annotations
 
@@ -199,8 +203,63 @@ class _SideWeights:
         self.wa, self.ba, self.wb, self.bb = b16(lin_a.weight), b16(lin_a.bias), b16(lin_b.weight), b16(lin_b.bias)
 
 
-def _block_forward(lib, blk, x: torch.Tensor, rope, kv, pf, m8, B: int, N: int, dims, window: int, keep, keep_prob: float):
-    """One transformer block (ae.py:55-65) with everything the backward needs: returns (x_new, (h, zraw, qkv, a2, lse, y))."""
+class _Packing:
+    """The packed NaFlex layout of one training step: image b owns rows [cu[b], cu[b+1]) -- its valid tokens in token order, then
+    zero rows up to a multiple of 16 -- and the step runs on M = cu[B] rows.  ``plan`` (128-row attention groups) is the work list of
+    the attention backward at both head dims and of the d = 64 forward; the d = 128 forward takes 256-row groups (a second plan of
+    the same mask: same rows, other groups).  Reading n_valid is the step's one host sync; it sizes every buffer."""
+
+    def __init__(self, mask: torch.Tensor, B: int, N: int):
+        self.B, self.N = B, N
+        self.mask = mask.bool().contiguous()
+        self.plan = _lib.pack_plan(self.mask, 16, 128)
+        nv = self.plan["n_valid"].cpu().long()
+        self.M = int(((nv + 15) // 16 * 16).sum())
+        if self.M == 0:
+            raise ValueError("vitok_b200 training: the batch has no valid token (patch_mask is all False)")
+        self.groups = {q: int(((nv + q - 1) // q).sum()) for q in (128, 256)}
+        self._plans = {128: self.plan}
+        self._row_img = None
+
+    def attn_plan(self, qrows: int) -> dict:
+        if qrows not in self._plans:
+            self._plans[qrows] = _lib.pack_plan(self.mask, 16, qrows)
+        return self._plans[qrows]
+
+    def pack(self, x: torch.Tensor) -> torch.Tensor:
+        """[B*N, W] bf16 rows -> [M, W] (pad rows 0) with vtk_pack_rows."""
+        W = x.shape[1]
+        out = torch.empty(self.M, W, dtype=BF, device=x.device)
+        _check(_lib.load().vtk_pack_rows(x.data_ptr(), x.stride(0), self.plan["src"].data_ptr(), self.plan["cu"].data_ptr(), self.B,
+                                         self.M, out.data_ptr(), W, W, _lib.stream_ptr()))
+        return out
+
+    def unpack(self, x: torch.Tensor) -> torch.Tensor:
+        """[M, W] -> [B, N, W] (masked tokens 0) with vtk_unpack_rows."""
+        W = x.shape[1]
+        out = torch.empty(self.B, self.N, W, dtype=BF, device=x.device)
+        _check(_lib.load().vtk_unpack_rows(x.data_ptr(), x.stride(0), self.plan["rel"].data_ptr(), self.plan["cu"].data_ptr(), self.B,
+                                           self.N, out.data_ptr(), W, W, _lib.stream_ptr()))
+        return out
+
+    def pack_index(self, idx: torch.Tensor) -> torch.Tensor:
+        """[B, N] int64 token indices (row_idx / col_idx) -> [M], 0 on pad rows."""
+        src = self.plan["src"][:self.M].long()
+        return torch.where(src >= 0, idx.reshape(-1)[src.clamp_min(0)], 0).contiguous()
+
+    def per_row(self, keep: torch.Tensor) -> torch.Tensor:
+        """[B] per-image values -> [M] per packed row (a pad row takes its image's value)."""
+        if self._row_img is None:
+            cu = self.plan["cu"]
+            self._row_img = torch.repeat_interleave(torch.arange(self.B, device=cu.device), (cu[1:] - cu[:-1]).long(),
+                                                    output_size=self.M)
+        return keep[self._row_img].contiguous()
+
+
+def _block_forward(lib, blk, x: torch.Tensor, rope, kv, pf, m8, B: int, N: int, dims, window: int, keep, keep_prob: float,
+                   pk: Optional[_Packing] = None):
+    """One transformer block (ae.py:55-65) with everything the backward needs: returns (x_new, (h, zraw, qkv, a2, lse, y)).
+    ``pk``: the packed layout (M = pk.M rows; ``keep`` then holds one entry per row)."""
     M, D, heads, d, Hf, qp, ZP, kp = dims
     wqkv, w1, w_o, w_2, n1, nq, nk, gamma = blk
     st = _lib.stream_ptr()
@@ -220,22 +279,30 @@ def _block_forward(lib, blk, x: torch.Tensor, rope, kv, pf, m8, B: int, N: int, 
         a2[:, D + Hf:].zero_()
     lse = torch.empty(M, heads, dtype=torch.float32, device=dev)
     base = qkv.data_ptr()
-    _check(lib.vtk_attention_bf16(base, base + 2 * D, base + 4 * D, 3 * D, a2.data_ptr(), kp, _lib.ptr(kv),
-                                  _lib.ptr(m8), _lib.ptr(pf), B, N, heads, d, 1 if m8 is not None else 0, window,
-                                  lse.data_ptr(), st))
+    if pk is None:
+        _check(lib.vtk_attention_bf16(base, base + 2 * D, base + 4 * D, 3 * D, a2.data_ptr(), kp, _lib.ptr(kv),
+                                      _lib.ptr(m8), _lib.ptr(pf), B, N, heads, d, 1 if m8 is not None else 0, window,
+                                      lse.data_ptr(), st))
+    else:
+        qrows = 128 if d == 64 else 256
+        pl = pk.attn_plan(qrows)
+        _check(lib.vtk_attention_packed_lse_bf16(base, base + 2 * D, base + 4 * D, 3 * D, a2.data_ptr(), kp, pl["n_valid"].data_ptr(),
+                                                 pl["cu"].data_ptr(), pl["cuq"].data_ptr(), pl["grp_img"].data_ptr(),
+                                                 pl["grp_order"].data_ptr(), B, N, heads, d, M, pk.groups[qrows], lse.data_ptr(), st))
     _check(lib.vtk_swiglu_fwd(zraw.data_ptr(), ZP, qp, a2.data_ptr() + 2 * D, kp, M, Hf, 1, st))
     y = _linear2(a2, kp, w_o, w_2, M, D)
     x_new = torch.empty(M, D, dtype=BF, device=dev)
-    _check(lib.vtk_resid_fwd_dp(x.data_ptr(), y.data_ptr(), gamma.data_ptr(), x_new.data_ptr(), M, D, _lib.ptr(keep), N,
-                                float(keep_prob), st))
+    _check(lib.vtk_resid_fwd_dp(x.data_ptr(), y.data_ptr(), gamma.data_ptr(), x_new.data_ptr(), M, D, _lib.ptr(keep),
+                                N if pk is None else 1, float(keep_prob), st))
     return x_new, (h, zraw, qkv, a2, lse, y)
 
 
-def _side_forward(lib, model, sw: _SideWeights, side: int, xin: torch.Tensor, row, col, m8, B: int, N: int, saved: Dict):
+def _side_forward(lib, model, sw: _SideWeights, side: int, xin: torch.Tensor, row, col, m8, B: int, N: int, saved: Dict,
+                  pk: Optional[_Packing] = None):
     width = model.encoder_width if side == 0 else model.decoder_width
     heads = model.encoder_heads if side == 0 else model.decoder_heads
     d = width // heads
-    M, D = B * N, width
+    M, D = (B * N if pk is None else pk.M), width
     from .models.ae import _ffn_hidden
     Hf = _ffn_hidden(width, model.mlp_factor)
     qp = ((3 * D + 255) // 256) * 256
@@ -251,7 +318,7 @@ def _side_forward(lib, model, sw: _SideWeights, side: int, xin: torch.Tensor, ro
         inv = (1.0 / (model.rope_theta ** (torch.arange(0, d // 2, 2).float() / (d // 2)))).to(dev)
         rope = torch.zeros((M + 31) // 32 * 32, 2 * d, dtype=BF, device=dev)
         _check(lib.vtk_rope_table(row.data_ptr(), col.data_ptr(), inv.data_ptr(), rope.data_ptr(), M, d, st))
-        if m8 is not None:
+        if m8 is not None and pk is None:
             kv, pf = _lib.kv_len(m8.view(B, N))     # train_forward has made every mask a prefix mask
     window = int(model.sw) if (model.sw and m8 is None) else -1
     ck = int(getattr(model, "checkpoint", 0) or 0)
@@ -264,11 +331,13 @@ def _side_forward(lib, model, sw: _SideWeights, side: int, xin: torch.Tensor, ro
             # torch's CUDA generator, one per block in block order, so a seeded run drops the same images as the reference
             keep_prob = 1.0 - rate
             keep = (keep_prob + torch.rand((B, 1, 1), dtype=BF, device=dev)).floor_().float().reshape(B).contiguous()
-        x_new, inner = _block_forward(lib, blk, x, rope, kv, pf, m8, B, N, dims, window, keep, keep_prob)
+            if pk is not None:
+                keep = pk.per_row(keep)
+        x_new, inner = _block_forward(lib, blk, x, rope, kv, pf, m8, B, N, dims, window, keep, keep_prob, pk)
         # activation checkpointing (ae.py:159-160): block i with i % checkpoint == 0 keeps its input only
         layers.append((x, None if (ck > 0 and li % ck == 0) else inner, keep, keep_prob))
         x = x_new
-    saved.update(dict(layers=layers, x_final=x, rope=rope, kv=kv, pf=pf, m8=m8, window=window, xin=xin, dims=dims))
+    saved.update(dict(layers=layers, x_final=x, rope=rope, kv=kv, pf=pf, m8=m8, window=window, xin=xin, dims=dims, pk=pk))
     return x
 
 
@@ -279,19 +348,19 @@ def _side_backward(lib, model, sw: _SideWeights, side: int, dx: torch.Tensor, sa
     M, D, heads, d, Hf, qp, ZP, kp = dims
     st = _lib.stream_ptr()
     dev = dx.device
-    rope, kv, window = saved["rope"], saved["kv"], saved["window"]
+    rope, kv, window, pk = saved["rope"], saved["kv"], saved["window"], saved["pk"]
     grads: List[Dict[str, torch.Tensor]] = []
     for li in range(len(sw.blocks) - 1, -1, -1):
         wqkv, w1, w_o, w_2, n1, nq, nk, gamma = sw.blocks[li]
         x, inner, keep, keep_prob = saved["layers"][li]
         if inner is None:      # checkpointed block: re-run its forward from x (same stochastic-depth draw)
-            _, inner = _block_forward(lib, sw.blocks[li], x, rope, kv, saved["pf"], saved["m8"], B, N, dims, window, keep, keep_prob)
+            _, inner = _block_forward(lib, sw.blocks[li], x, rope, kv, saved["pf"], saved["m8"], B, N, dims, window, keep, keep_prob, pk)
         h, zraw, qkv, a2, lse, y = inner
         saved["layers"][li] = None                                                 # free this block's activations as we go
         dy = torch.empty(M, D, dtype=BF, device=dev)
         dgamma = torch.zeros(D, dtype=torch.float32, device=dev)
         _check(lib.vtk_resid_bwd_dp(dx.data_ptr(), y.data_ptr(), gamma.data_ptr(), dy.data_ptr(), dgamma.data_ptr(), M, D,
-                                    _lib.ptr(keep), N, float(keep_prob), st))
+                                    _lib.ptr(keep), N if pk is None else 1, float(keep_prob), st))
         # the four weight gradients of the block live in ONE flat buffer so that they leave as one all-reduce
         n_qkv, n_fc1, n_o, n_f2 = 3 * D * D, 2 * Hf * D, D * D, D * Hf
         flat = torch.empty(n_qkv + n_fc1 + n_o + n_f2, dtype=BF, device=dev)
@@ -311,9 +380,16 @@ def _side_backward(lib, model, sw: _SideWeights, side: int, dx: torch.Tensor, sa
         delta = torch.empty(M, heads, dtype=torch.float32, device=dev)
         _check(lib.vtk_attn_delta(a2.data_ptr(), kp, da2.data_ptr(), kp, delta.data_ptr(), M, heads, d, st))
         qb, zb = qkv.data_ptr(), dz.data_ptr()
-        _check(lib.vtk_attention_bwd_bf16(qb, qb + 2 * D, qb + 4 * D, 3 * D, da2.data_ptr(), kp, lse.data_ptr(), delta.data_ptr(),
-                                          zb, zb + 2 * D, zb + 4 * D, ZP, _lib.ptr(kv), B, N, heads, d,
-                                          1 if kv is not None else 0, window, st))
+        if pk is None:
+            _check(lib.vtk_attention_bwd_bf16(qb, qb + 2 * D, qb + 4 * D, 3 * D, da2.data_ptr(), kp, lse.data_ptr(), delta.data_ptr(),
+                                              zb, zb + 2 * D, zb + 4 * D, ZP, _lib.ptr(kv), B, N, heads, d,
+                                              1 if kv is not None else 0, window, st))
+        else:
+            pl = pk.plan
+            _check(lib.vtk_attention_bwd_packed_bf16(qb, qb + 2 * D, qb + 4 * D, 3 * D, da2.data_ptr(), kp, lse.data_ptr(),
+                                                     delta.data_ptr(), zb, zb + 2 * D, zb + 4 * D, ZP, pl["n_valid"].data_ptr(),
+                                                     pl["cu"].data_ptr(), pl["cuq"].data_ptr(), pl["grp_img"].data_ptr(),
+                                                     pl["grp_order"].data_ptr(), B, heads, d, M, pk.groups[128], st))
         dwqk = torch.zeros(2, d, dtype=torch.float32, device=dev)
         _check(lib.vtk_qk_norm_rope_bwd(dz.data_ptr(), ZP, zraw.data_ptr(), ZP, nq.data_ptr(), nk.data_ptr(), rope.data_ptr(),
                                         dwqk.data_ptr(), M, heads, d, 1e-6, st))
@@ -356,7 +432,8 @@ class AETrainFunction(torch.autograd.Function):
         lib = _lib.load()
         B, N, P = patches.shape
         dev = patches.device
-        if (B * N) % 8:
+        pk = _Packing(mask.to(dev), B, N) if _packs(model, mask) else None    # (packed row counts are multiples of 16)
+        if pk is None and (B * N) % 8:
             raise ValueError("vitok_b200 training: B * N must be a multiple of 8 (token count is the K dimension of the wgrad GEMMs)")
         enc_w, dec_w = _SideWeights(model, 0), _SideWeights(model, 1)
         row = row.to(device=dev, dtype=torch.int64).contiguous()
@@ -364,12 +441,14 @@ class AETrainFunction(torch.autograd.Function):
         m8 = mask.to(dev).bool().contiguous().view(torch.uint8) if mask is not None else None
         xin = (_lib.cast_to_bf16(patches) if patches.dtype == torch.float32 else patches).contiguous().view(B * N, P)
         M, C = B * N, model.channels_per_token
+        if pk is not None:
+            xin, row, col, M = pk.pack(xin), pk.pack_index(row), pk.pack_index(col), pk.M
         s_enc, s_dec = {}, {}
-        x = _side_forward(lib, model, enc_w, 0, xin, row, col, m8, B, N, s_enc)
+        x = _side_forward(lib, model, enc_w, 0, xin, row, col, m8, B, N, s_enc, pk)
         zlin = _linear(x, x.shape[1], enc_w.wb, enc_w.bb, M, C, x.shape[1])
         z = torch.empty(M, C, dtype=BF, device=dev)
         _check(lib.vtk_layernorm_fwd(zlin.data_ptr(), z.data_ptr(), M, C, 1e-6, _lib.stream_ptr()))
-        xd = _side_forward(lib, model, dec_w, 1, z, row, col, m8, B, N, s_dec)
+        xd = _side_forward(lib, model, dec_w, 1, z, row, col, m8, B, N, s_dec, pk)
         out = _linear(xd, xd.shape[1], dec_w.wb, dec_w.bb, M, P, xd.shape[1])
         # activations live on ctx (not save_for_backward: they are workspace of the backward kernels, freed block by block while it
         # runs); a second backward through the same graph is therefore refused with a clear error in backward()
@@ -377,7 +456,8 @@ class AETrainFunction(torch.autograd.Function):
         ctx.zlin, ctx.shape, ctx.names = zlin, (B, N, P, C), [n for n, _ in model.named_parameters()]
         ctx.param_dtypes = [p.dtype for p in params]
         ctx.patches_dtype = patches.dtype
-        return out.view(B, N, P)
+        ctx.pk = pk
+        return out.view(B, N, P) if pk is None else pk.unpack(out)
 
     @staticmethod
     def backward(ctx, dout):
@@ -393,8 +473,11 @@ class AETrainFunction(torch.autograd.Function):
         lib = _lib.load()
         model, enc_w, dec_w = ctx.model, ctx.enc_w, ctx.dec_w
         B, N, P, C = ctx.shape
-        M = B * N
-        dout = dout.to(BF).contiguous().view(M, P)
+        pk = ctx.pk
+        M = B * N if pk is None else pk.M
+        dout = dout.to(BF).contiguous().view(B * N, P)
+        if pk is not None:
+            dout = pk.pack(dout)           # pad rows 0: no gradient enters them, every weight gradient sums over valid tokens only
         g: Dict[str, torch.Tensor] = {}
         # decoder: to_pixels, blocks, decoder_embed
         xd = ctx.s_dec["x_final"]
@@ -427,9 +510,9 @@ class AETrainFunction(torch.autograd.Function):
         for name, dt in zip(ctx.names, ctx.param_dtypes):
             t = g.get(name)
             grads.append(None if t is None else t.to(dt).contiguous())
-        ctx.s_enc = ctx.s_dec = ctx.zlin = None
+        ctx.s_enc = ctx.s_dec = ctx.zlin = ctx.pk = None
         if dpatches is not None:
-            dpatches = dpatches.view(B, N, P).to(ctx.patches_dtype)
+            dpatches = (dpatches.view(B, N, P) if pk is None else pk.unpack(dpatches)).to(ctx.patches_dtype)
         return (None, dpatches, None, None, None, *grads)
 
 
@@ -442,6 +525,11 @@ def _name_block(g: Dict[str, torch.Tensor], prefix: str, bg: Dict[str, torch.Ten
     g[prefix + "attn.norm_q.weight"] = bg["norm_q"]
     g[prefix + "attn.norm_k.weight"] = bg["norm_k"]
     g[prefix + "layer_scale.gamma"] = bg["gamma"]
+
+
+def _packs(model, mask: Optional[torch.Tensor]) -> bool:
+    """The training step runs on packed rows: opt-in (AE.train_token_packing) and only for a masked (sdpa) batch."""
+    return mask is not None and bool(getattr(model, "train_token_packing", False))
 
 
 def _prefix_permutation(mask: torch.Tensor):
@@ -468,7 +556,8 @@ def train_forward(model, patch_dict: Dict[str, torch.Tensor]) -> Dict[str, torch
     mask = patch_dict.get("patch_mask") if model.attn_backend == "sdpa" else None
     params = [p for _, p in model.named_parameters()]
     row, col = patch_dict["row_idx"], patch_dict["col_idx"]
-    pp = _prefix_permutation(mask.to(patches.device)) if mask is not None else None
+    # (the packed layout keeps every image's valid tokens in order for any mask: no permutation)
+    pp = _prefix_permutation(mask.to(patches.device)) if mask is not None and not _packs(model, mask) else None
     if pp is None:
         out = AETrainFunction.apply(model, patches, row, col, mask, *params)
     else:
