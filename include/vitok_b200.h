@@ -25,7 +25,7 @@ extern "C" {
 #pragma GCC visibility push(default)
 #endif
 
-#define VTK_ABI_VERSION 5
+#define VTK_ABI_VERSION 6
 
 typedef enum {
   VTK_OK = 0,
@@ -58,13 +58,10 @@ int vtk_set_flag(const char* name, int value);
  * out_dtype  : 0 = float32 (what the reference returns), 1 = bfloat16.
  * outputs    : patches [B,T,3p^2], patch_mask [B,T] (bool bytes), row/col/time_idx [B,T] int64,
  *              meta [4,B] int64 = orig_height, orig_width, grid_rows, grid_cols.
- * status     : optional device int, set to 1 if an image's grid exceeds max_tokens (the reference raises at :260). */
-int vtk_patchify(const void* images, const int64_t* img_table, int in_dtype, int B, int patch, int max_tokens,
-                 int out_dtype, void* patches, uint8_t* patch_mask, int64_t* row_idx, int64_t* col_idx,
-                 int64_t* time_idx, int64_t* meta, int* status, void* stream);
-/* The same with a host-side hint: max_h / max_w = the largest image height / width of the batch (0 = unknown).  With the hint the
- * uint8 front end runs a row-coalesced kernel over the batch's bounding box (thread = 4 pixels of an image row, 384 contiguous bytes
- * per warp) with the normalisation done arithmetically; results are bit-identical to vtk_patchify. */
+ * status     : optional device int, set to 1 if an image's grid exceeds max_tokens (the reference raises at :260).
+ * max_h/max_w: a host-side hint, the largest image height / width of the batch (0 = unknown).  With the hint the uint8 front end
+ *              runs a row-coalesced kernel over the batch's bounding box (thread = 4 pixels of an image row, 384 contiguous bytes
+ *              per warp) with the normalisation done arithmetically; results are bit-identical to the call without it. */
 int vtk_patchify_ex(const void* images, const int64_t* img_table, int in_dtype, int B, int patch, int max_tokens, int out_dtype,
                     void* patches, uint8_t* patch_mask, int64_t* row_idx, int64_t* col_idx, int64_t* time_idx, int64_t* meta, int* status,
                     int max_h, int max_w, void* stream);
@@ -75,7 +72,7 @@ int vtk_patchify_ex(const void* images, const int64_t* img_table, int in_dtype, 
  * resampling : TF.resize(BICUBIC, antialias=True) on the normalised fp32 image = ATen's _upsample_bicubic2d_aa (align_corners=False):
  *              cubic a = -0.5, support 2 * scale when shrinking, weights divided by their sum; width pass first, then height, each
  *              output summed in fp32 in tap order.  Weights equal torch's; outputs agree with TF.resize to a few fp32 ulps.
- * in_dtype / out_dtype / outputs: as vtk_patchify; meta holds the RESIZED height and width (patchify sees the resized tensor).
+ * in_dtype / out_dtype / outputs: as vtk_patchify_ex; meta holds the RESIZED height and width (patchify sees the resized tensor).
  * workspace  : device memory of at least vtk_resize_patchify_workspace_bytes.  Layout: a header of 2B+3 int64 (rounded up to 256
  *              bytes): [0..B] = offset of each image's region in floats after the header, [B+1..2B+1] = row prefix of the width pass,
  *              [2B+2] = 1 if the batch was usable.  An image's region holds its resample tables (width then height; only for axes
@@ -121,10 +118,9 @@ int vtk_rope_table(const int64_t* row_idx, const int64_t* col_idx, const float* 
                    void* stream);
 
 int vtk_cast_f32_to_bf16(const float* in, void* out, int64_t n, void* stream);
-int vtk_cast_bf16_to_f32(const void* in, float* out, int64_t n, void* stream);
 
-/* kv_len[b] = 1 + last valid index, is_prefix[b] = mask is contiguous from 0.   vitok/models/ae.py:173-187 */
-int vtk_kv_len(const uint8_t* patch_mask, int* kv_len, int* is_prefix, int B, int N, void* stream);
+/* kv_len[b] = 1 + last valid index: the key length of a prefix mask.   vitok/models/ae.py:173-187 */
+int vtk_kv_len(const uint8_t* patch_mask, int* kv_len, int B, int N, void* stream);
 
 /* NaFlex token packing plan for a masked [B, N] batch (replaces the reference's [B,1,N,N] mask, vitok/models/ae.py:173-187,
  * and its work on padded tokens).  Valid tokens are packed image after image, each image padded to `pad` rows (a multiple
@@ -149,9 +145,6 @@ int vtk_unpack_rows(const void* packed, int64_t ld_packed, const int* rel, const
 /* out [M, N] = At^T Bt for At [K, M] and Bt [K, N] row-major (row strides lda / ldb): the weight gradient dW = dY^T X of the
  * training step without transposing either operand (the tensor core reads both tiles MN-major).  M, N multiples of 8. */
 int vtk_linear_tn_bf16(const void* At, int64_t lda, const void* Bt, int64_t ldb, void* out, int64_t ldo, int M, int N, int K,
-                       void* stream);
-/* out [M, N] = A Bt for A [M, K] and Bt [K, N] row-major: the data gradient dX = dY W with the weight W [out, in] used as stored. */
-int vtk_linear_nn_bf16(const void* A, int64_t lda, const void* Bt, int64_t ldb, void* out, int64_t ldo, int M, int N, int K,
                        void* stream);
 
 /* FP8 inference building blocks (reference AE.quantize, vitok/models/ae.py:253-270 = torchao
@@ -189,32 +182,29 @@ int vtk_proj_residual_bf16(const void* A, int64_t lda, const void* W, int64_t ld
                            int64_t ldx, int M, int N, int K, void* stream);
 
 /* softmax(q k^T / sqrt(d)) v per (image, head); q,k,v,out rows = tokens, heads along columns.
- * kv_len/key_mask/is_prefix null = no masking (reference flash backend, modules/attention.py:109-117);
- * otherwise the sdpa backend's key masking (modules/attention.py:118-127).
+ * kv_len null = no masking (reference flash backend, modules/attention.py:109-117); otherwise image b attends to its first
+ * kv_len[b] keys: the sdpa backend's key masking (modules/attention.py:118-127) for a prefix mask (vtk_kv_len).
+ * zero_invalid_rows = 1: query rows >= kv_len[b] are written as 0 (lse +inf).
  * window >= 0: sliding-window attention, query i sees keys j with |i - j| <= window on the token index, i.e.
- * flash_attn_func(window_size=(window, window)) as called at modules/attention.py:113-116; window < 0 = full. */
+ * flash_attn_func(window_size=(window, window)) as called at modules/attention.py:113-116; window < 0 = full.
+ * lse (optional, may be null): [B*N, heads] fp32, log2-domain logsumexp of the scaled scores (+inf for zeroed rows);
+ * the training backward (vtk_attention_bwd_bf16) consumes it. */
 int vtk_attention_bf16(const void* q, const void* k, const void* v, int64_t ld_qkv, void* out, int64_t ld_out,
-                       const int* kv_len, const uint8_t* key_mask, const int* is_prefix, int B, int N, int heads, int d,
-                       int zero_invalid_rows, int window, float* lse, void* stream);
+                       const int* kv_len, int B, int N, int heads, int d, int zero_invalid_rows, int window, float* lse, void* stream);
 /* The same on the packed NaFlex layout of vtk_pack_plan (the form the layer stack runs masked batches in): image b owns packed rows
  * [cu[b], cu[b+1]) with its n_valid[b] tokens in front; q / k / v / out have row_cap rows.  qrows of the plan must be 128 (d = 64)
- * or 256 (d = 128). */
-int vtk_attention_packed_bf16(const void* q, const void* k, const void* v, int64_t ld_qkv, void* out, int64_t ld_out, const int* n_valid,
-                              const int* cu, const int* cuq, const int* grp_img, const int* grp_order, int B, int N, int heads, int d,
-                              int64_t row_cap, int grp_cap, void* stream);
-/* lse (optional, may be null): [B*N, heads] fp32, log2-domain logsumexp of the scaled scores (+inf for zeroed rows);
- * the training backward (vtk_attention_bwd_bf16) consumes it. */
-/* The packed form with lse, for the training step on packed rows (vitok/models/modules/attention.py:118-127 under autograd):
- * lse [row_cap, heads] fp32.  For image b it writes packed rows [cu[b], cu[b+1]) only: rows below n_valid[b] get out and lse as in
- * vtk_attention_packed_bf16 (equal to vtk_attention_bf16 with kv_len = n_valid and zero_invalid_rows = 1), the image's pad rows
- * [cu[b] + n_valid[b], cu[b+1]) get out = 0 and lse = +inf.  Rows of other images -- the rest of a partial last tile -- are not
- * touched.  qrows of the plan: 128 (d = 64) or 256 (d = 128), as above. */
+ * or 256 (d = 128).  For image b it writes packed rows [cu[b], cu[b+1]) only, and rows below n_valid[b] get out as
+ * vtk_attention_bf16 with kv_len = n_valid.  Rows of other images -- the rest of a partial last tile -- are not touched.
+ * lse (optional, may be null; the training step on packed rows, vitok/models/modules/attention.py:118-127 under autograd):
+ * [row_cap, heads] fp32.  With lse, the image's pad rows [cu[b] + n_valid[b], cu[b+1]) get out = 0 and lse = +inf; without it,
+ * they are not written. */
 int vtk_attention_packed_lse_bf16(const void* q, const void* k, const void* v, int64_t ld_qkv, void* out, int64_t ld_out,
                                   const int* n_valid, const int* cu, const int* cuq, const int* grp_img, const int* grp_order, int B, int N,
                                   int heads, int d, int64_t row_cap, int grp_cap, float* lse, void* stream);
 
-/* out [M,N] (+)= A [M,K] @ Bt [K,N] with B read as stored (the data gradient dX = dY W; vtk_linear_nn_bf16); accumulate != 0 adds to
- * what `out` already holds, in fp32 before the bf16 rounding (dh = dz_qkv Wqkv + dz_fc1 W1 without a separate add pass). */
+/* out [M,N] (+)= A [M,K] @ Bt [K,N] with B read as stored: the data gradient dX = dY W with the weight W [out, in] used as stored.
+ * accumulate != 0 adds to what `out` already holds, in fp32 before the bf16 rounding (dh = dz_qkv Wqkv + dz_fc1 W1 without a
+ * separate add pass). */
 int vtk_linear_nn_acc_bf16(const void* A, int64_t lda, const void* Bt, int64_t ldb, void* out, int64_t ldo, int M, int N, int K,
                            int accumulate, void* stream);
 /* out [M,N] = A[:, :K0] W0^T + A[:, K0:K0+K1] W1^T with W0 [N,K0], W1 [N,K1] as stored: out_proj(attn) + fc2(act)
@@ -225,9 +215,10 @@ int vtk_linear2_bf16(const void* A, int64_t lda, const void* W0, int64_t ldw0, c
 
 /* ------------------------------------------------------------------------------------------------
  * Training step (BASELINE config 5; scripts/train_vae.py:304-320,371-372 = forward, Charbonnier loss, backward,
- * AdamW).  The GEMMs of forward and backward are vtk_linear_bf16 calls (dgrad against transposed weight copies,
- * wgrad on vtk_transpose_bf16'd activations); everything else is below.  All tensors bf16 unless noted;
- * gradient accumulators of norm weights / gamma / biases are fp32 and ADDED to (zero them first).
+ * AdamW).  The GEMMs of forward and backward are vtk_linear_bf16 (forward), vtk_linear2_bf16 (out_proj + fc2),
+ * vtk_linear_nn_acc_bf16 (dgrad against the weights as stored) and vtk_linear_tn_bf16 (wgrad) calls; everything else is
+ * below.  All tensors bf16 unless noted; gradient accumulators of norm weights / gamma / biases are fp32 and ADDED to (zero
+ * them first).
  * ---------------------------------------------------------------------------------------------- */
 /* zraw [M, >=3D] raw q|k|v -> qkv [M,3D]: QK-RMSNorm over d + 2D RoPE, v copied (modules/attention.py:95-107) */
 int vtk_qk_norm_rope_fwd(const void* zraw, int64_t ldz, const void* norm_q, const void* norm_k, const void* rope_table,
@@ -235,21 +226,18 @@ int vtk_qk_norm_rope_fwd(const void* zraw, int64_t ldz, const void* norm_q, cons
 /* zraw[:, qp:] (16-col groups value|gate, the packed fc1 order) -> act [M,Hf] = silu(g) * v (modules/mlp.py:21-22) */
 /* layout: 0 = 16-column (value16 | gate16) groups (the packed w_in of the inference path), 1 = [value Hf | gate Hf] (fc1 rows as stored) */
 int vtk_swiglu_fwd(const void* zraw, int64_t ldz, int qp, void* act, int64_t ld_act, int M, int Hf, int layout, void* stream);
-/* out = x + gamma * y (vitok/models/ae.py:64-65); contiguous [M,D] */
-int vtk_resid_fwd(const void* x, const void* y, const void* gamma, void* out, int M, int D, void* stream);
-/* The same with stochastic depth (drop_path, vitok/models/ae.py:15-30,65; decoder blocks in train mode): keep [B] fp32 holds the
- * per-image draw floor(keep_prob + U[0,1)) in {0, 1}, image b = rows [b * rows_per_image, (b+1) * rows_per_image):
- * out = x + bf16(bf16(gamma * y) / keep_prob) * keep[b].  keep == NULL: identical to vtk_resid_fwd. */
+/* out = x + gamma * y (vitok/models/ae.py:64-65); contiguous [M,D].  With stochastic depth (drop_path, vitok/models/ae.py:15-30,65;
+ * decoder blocks in train mode): keep [B] fp32 holds the per-image draw floor(keep_prob + U[0,1)) in {0, 1}, image b = rows
+ * [b * rows_per_image, (b+1) * rows_per_image): out = x + bf16(bf16(gamma * y) / keep_prob) * keep[b].  keep == NULL: no
+ * stochastic depth. */
 int vtk_resid_fwd_dp(const void* x, const void* y, const void* gamma, void* out, int M, int D, const float* keep, int rows_per_image,
                      float keep_prob, void* stream);
 /* backward of vtk_resid_fwd_dp: the LayerScale output's gradient is bf16(dx * keep[b] / keep_prob); dy = that * gamma,
- * dgamma[D] += colsum(that * y) */
+ * dgamma[D] += colsum(that * y).  keep == NULL: dy = dx * gamma, dgamma[D] += colsum(dx * y) */
 int vtk_resid_bwd_dp(const void* dx, const void* y, const void* gamma, void* dy, float* dgamma, int M, int D, const float* keep,
                      int rows_per_image, float keep_prob, void* stream);
 /* out = LayerNorm_noaffine(x) over C <= 256 (modules/norm.py:28-39) */
 int vtk_layernorm_fwd(const void* x, void* out, int M, int C, float eps, void* stream);
-/* dy = dx * gamma; dgamma[D] += colsum(dx * y) */
-int vtk_resid_bwd(const void* dx, const void* y, const void* gamma, void* dy, float* dgamma, int M, int D, void* stream);
 /* out[C] += colsum(in [M,C]) (bias gradients) */
 int vtk_colsum(const void* in, int64_t ld, float* out, int M, int C, void* stream);
 /* d_act [M,Hf] + zraw -> dz[:, qp:] in the packed (value|gate) order */
@@ -262,15 +250,10 @@ int vtk_qk_norm_rope_bwd(void* dz, int64_t lddz, const void* zraw, int64_t ldz, 
 int vtk_rmsnorm_bwd(const void* x, const void* dh, const void* w, const void* dx_res, void* dx_out, float* dw, int M, int D,
                     float eps, void* stream);
 int vtk_layernorm_bwd(const void* zlin, const void* dz, void* dx, int M, int C, float eps, void* stream);
-/* out [C,R] = in [R,C]^T */
-int vtk_transpose_bf16(const void* in, int64_t ldi, void* out, int64_t ldo, int R, int C, void* stream);
 /* Charbonnier loss (scripts/train_vae.py:314-320): loss_sum[B] fp32 += per-image masked mean (caller zeroes it and takes the
  * batch mean); dpred (optional) = d(batch-mean loss)/d pred; n_valid[B] int32 = clamp_min(patch_mask.sum(1), 1) */
 int vtk_charbonnier(const void* pred, const void* target, const uint8_t* patch_mask, const int* n_valid, float* loss_sum,
                     void* dpred, int B, int N, int P, float eps, void* stream);
-/* fused AdamW on bf16 param/grad/exp_avg/exp_avg_sq, fp32 math (torch.optim.AdamW semantics; scripts/train_vae.py:200-208) */
-int vtk_adamw_bf16(void* p, const void* g, void* m, void* v, int64_t n, float lr, float beta1, float beta2, float eps,
-                   float weight_decay, int step, float grad_scale, void* stream);
 /* Multi-tensor AdamW with the reference's optimizer precision (scripts/train_vae.py:200-208: fp32 parameters and fp32 Adam moments under
  * autocast).  Per tensor: `master` = fp32 parameter values (for an fp32 model parameter: the parameter itself), `p16` = the bf16 model
  * parameter re-emitted from the master in the same pass (NULL for fp32 parameters), `g` = gradient (bf16, or fp32 when g_is_f32),
@@ -335,7 +318,12 @@ int vtk_ae_destroy(vtk_ae_t h);
 int vtk_ae_set_weights(vtk_ae_t h, int side, const void* w_a, const void* b_a, const void* w_b, const void* b_b,
                        const vtk_block_weights* blocks, int nblocks, const float* inv_freq_host, int n_inv_freq);
 size_t vtk_ae_workspace_bytes(vtk_ae_t h, int side, int B, int N);
-/* AE.encode (vitok/models/ae.py:189-216): patches [B,N,P] bf16 -> z [B,N,C] bf16.  patch_mask null = flash semantics. */
+/* AE.encode (vitok/models/ae.py:189-216): patches [B,N,P] bf16 -> z [B,N,C] bf16.  patch_mask null = flash semantics.
+ * NaFlex token packing: when a patch_mask is given, vtk_ae_encode/decode gather the valid tokens of every image into a packed
+ * row range (each image padded to 16 rows), run every kernel of the layer stack over the packed rows only -- the packed row count
+ * stays in device memory, nothing syncs -- and scatter the result back; masked tokens of the output are 0.  This replaces the
+ * reference's [B,1,N,N] mask (vitok/models/ae.py:173-187) and its work on padded tokens.  A side without blocks keeps the padded
+ * rows (it has no attention to mask). */
 int vtk_ae_encode(vtk_ae_t h, const void* patches, const int64_t* row_idx, const int64_t* col_idx,
                   const uint8_t* patch_mask, int B, int N, void* z_out, void* workspace, size_t workspace_bytes,
                   void* stream);
@@ -361,16 +349,9 @@ typedef struct vtk_block_fp8 {
   float w_out_scale;
 } vtk_block_fp8;
 int vtk_ae_set_fp8_weights(vtk_ae_t h, int side, const vtk_block_fp8* blocks, int nblocks);
-/* NaFlex token packing (default on).  When a patch_mask is given, vtk_ae_encode/decode gather the
- * valid tokens of every image into a packed row range (each image padded to 16 rows), run every kernel
- * of the layer stack over the packed rows only -- the packed row count stays in device memory, nothing syncs -- and
- * scatter the result back; masked tokens of the output are 0.  This replaces the reference's [B,1,N,N] mask
- * (vitok/models/ae.py:173-187) and its work on padded tokens.  enable = 0 keeps the padded [B, N] layout with
- * in-kernel key masking (results on valid tokens are identical for prefix masks). */
 /* FP8 activation scale granularity of the quantised block GEMMs: 0 = per row (default: finer, no extra pass), 1 = per tensor
  * (torchao-equivalent numerics). */
 int vtk_ae_set_fp8_granularity(vtk_ae_t h, int per_tensor);
-int vtk_ae_set_packing(vtk_ae_t h, int enable);
 /* number of kernels launched by the last vtk_ae_encode/decode on this handle (for gpu_launches accounting) */
 int vtk_ae_last_launch_count(vtk_ae_t h);
 /* Optional per-launch CUDA-event timing (bench.py's live roofline).  With timing enabled every kernel launched by

@@ -45,12 +45,27 @@ def test_attention_prefix_mask(L, N, heads, d, lens):
 
 
 def test_attention_general_mask(L):
+    """A mask with holes runs on the packed layout, as the model runs it: pack_plan -> pack_rows -> attention_packed ->
+    unpack_rows (masked tokens read 0, like the oracle's masked query rows)."""
     B, N, heads, d = 2, 256, 2, 64
     qkv = bf16_randn(B * N, 3 * heads * d, seed=42)
     g = torch.Generator().manual_seed(5)
     mask = torch.rand(B, N, generator=g) > 0.4
-    out = L.attention(qkv, B, N, heads, d, mask.cuda())
+    plan = L.pack_plan(mask.cuda())
+    packed = L.attention_packed(L.pack_rows(qkv.view(B, N, -1), plan), plan, B, N, heads, d)
+    out = L.unpack_rows(packed, plan, B, N).view(B * N, heads * d)
     report("attn general mask", out, _ref(qkv, B, N, heads, d, mask).float(), max_abs=3e-2, rel_fro=1e-2)
+
+
+def test_attention_rejects_mask_with_holes(L):
+    """The padded layout masks keys by length only: a mask with holes is refused (it runs on the packed layout instead)."""
+    B, N, heads, d = 2, 256, 2, 64
+    qkv = bf16_randn(B * N, 3 * heads * d, seed=42)
+    mask = torch.zeros(B, N, dtype=torch.bool)
+    mask[:, :100] = True
+    mask[1, 50] = False
+    with pytest.raises(ValueError, match="prefix mask"):
+        L.attention(qkv, B, N, heads, d, mask.cuda())
 
 
 def test_masked_equals_unpadded(L):

@@ -72,6 +72,4 @@ def test_kv_len(L):
     m[3, 5:9] = True          # not a prefix
     m[4, :100] = True
     m[4, 50] = False          # hole
-    kl, pf = L.kv_len(m.cuda())
-    assert kl.tolist() == [300, 17, 0, 9, 100]
-    assert pf.tolist() == [1, 1, 1, 0, 0]
+    assert L.kv_len(m.cuda()).tolist() == [300, 17, 0, 9, 100]

@@ -128,7 +128,7 @@ def test_packed_attention_backward_matches_padded(L, heads, d):
     lse_pad = torch.empty(B * N, heads, dtype=torch.float32, device="cuda")
     out_pad = L.attention(qkv, B, N, heads, d, mask, lse=lse_pad)
     delta_pad = _attn_delta(L, out_pad, do, B * N, heads, d)
-    kl = L.kv_len(mask)[0]
+    kl = L.kv_len(mask)
     dqkv_pad = torch.empty(B * N, 3 * D, dtype=BF, device="cuda")
     b0, g0 = qkv.data_ptr(), dqkv_pad.data_ptr()
     L.check(L.load().vtk_attention_bwd_bf16(b0, b0 + 2 * D, b0 + 4 * D, 3 * D, do.data_ptr(), D, lse_pad.data_ptr(), delta_pad.data_ptr(),

@@ -20,7 +20,7 @@ def test_library_exports_every_declared_symbol():
     assert declared == set(_lib.SIGNATURES), declared ^ set(_lib.SIGNATURES)
     for name in declared:
         assert hasattr(lib, name), name
-    assert lib.vtk_abi_version() == 5
+    assert lib.vtk_abi_version() == 6
 
 
 def test_decode_variant_matches_reference(golden_dir):

@@ -3,7 +3,7 @@
 
     c2         64 images x 16 heads x N = 256, d = 64           c4   8 images x 24 heads x N = 1024, d = 128
     c3-packed  64 mixed-aspect images (bench.py's seeded list, 64..1024 tokens each), 16 heads, d = 64: flash_attn_varlen_func on the
-               concatenated valid tokens vs vtk_attention_packed_bf16 on the packed NaFlex layout
+               concatenated valid tokens vs vtk_attention_packed_lse_bf16 (lse = NULL) on the packed NaFlex layout
     2048px     1 image x 16 heads x N = 16384, d = 64 (dense), and the same with a sliding window of 1024 tokens
 
 Both are replayed from CUDA graphs (20 calls per replay) so that the host-side wrappers do not enter the number; outputs are

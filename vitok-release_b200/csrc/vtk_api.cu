@@ -163,7 +163,6 @@ struct Workspace {
   float *sx, *sa;
   float* amax;          // FP8 per-tensor activation scale: two device floats (x, [attn | act])
   float* ss;            // [rows, D / 64] per-unit sums of squares of x (fused norm1)
-  int *kv_len, *is_prefix;
   PackPlan plan;        // NaFlex token packing (masked batches): plan arrays + packed input / output staging rows
   bf16 *pin, *pout;
   size_t bytes;
@@ -198,10 +197,8 @@ static Workspace carve(const Side& s, void* base, int B, int N, int io_cols) {
     w.sa = static_cast<float*>(take((size_t)M * 4));
     w.amax = static_cast<float*>(take(1024));
   }
-  w.kv_len = static_cast<int*>(take((size_t)B * 4));
-  w.is_prefix = static_cast<int*>(take((size_t)B * 4));
   w.plan.B = B; w.plan.N = N; w.plan.pad = 16; w.plan.qrows = qrows;
-  w.plan.n_valid = w.kv_len;
+  w.plan.n_valid = static_cast<int*>(take((size_t)B * 4));
   w.plan.rel = static_cast<int*>(take((size_t)B * N * 4));
   w.plan.cu = static_cast<int*>(take((size_t)(B + 1) * 4));
   w.plan.cuq = static_cast<int*>(take((size_t)(B + 1) * 4));
@@ -225,7 +222,6 @@ struct vtk_ae_s {
   vtk_ae_config cfg;
   vtk::Side side[2];
   int last_launches = 0;
-  bool packing = true;   // NaFlex token packing for masked batches (vtk_ae_set_packing)
   bool fp8_per_tensor = false;   // FP8 activations quantised with one dynamic scale per tensor instead of per row (vtk_ae_set_fp8_granularity)
   // timing: one (start, stop) event pair per launch of the last encode/decode call
   bool timing = false;
@@ -273,21 +269,6 @@ int vtk_set_flag(const char* name, int value) {
   if (!strcmp(name, "reserve_sms")) { g_flag_reserve = value < 0 ? 0 : value; return VTK_OK; }
   set_error("vtk_set_flag: unknown flag '%s' (pdl, gemm_splitk, reserve_sms)", name);
   return VTK_ERR_BAD_ARG;
-}
-
-int vtk_patchify(const void* images, const int64_t* img_table, int in_dtype, int B, int patch, int max_tokens,
-                 int out_dtype, void* patches, uint8_t* patch_mask, int64_t* row_idx, int64_t* col_idx,
-                 int64_t* time_idx, int64_t* meta, int* status, void* stream) {
-  VTK_REQUIRE(images && img_table && patches && patch_mask && row_idx && col_idx && time_idx && meta,
-              "vtk_patchify: null pointer");
-  VTK_REQUIRE(in_dtype == 0 || in_dtype == 1, "vtk_patchify: in_dtype must be 0 (f32 CHW) or 1 (u8 HWC)");
-  VTK_REQUIRE(out_dtype == 0 || out_dtype == 1, "vtk_patchify: out_dtype must be 0 (f32) or 1 (bf16)");
-  VTK_REQUIRE(B >= 0 && max_tokens >= 0, "vtk_patchify: negative size");
-  PatchifyArgs a;
-  a.images = images; a.img_table = img_table; a.in_dtype = in_dtype; a.B = B; a.patch = patch; a.max_tokens = max_tokens;
-  a.out_dtype = out_dtype; a.patches = patches; a.patch_mask = patch_mask; a.row_idx = row_idx; a.col_idx = col_idx;
-  a.time_idx = time_idx; a.meta = meta; a.status = status;
-  return launch_patchify(a, (cudaStream_t)stream);
 }
 
 int vtk_patchify_ex(const void* images, const int64_t* img_table, int in_dtype, int B, int patch, int max_tokens, int out_dtype,
@@ -364,14 +345,10 @@ int vtk_cast_f32_to_bf16(const float* in, void* out, int64_t n, void* stream) {
   VTK_REQUIRE(in && out, "vtk_cast_f32_to_bf16: null pointer");
   return launch_cast_f32_bf16(in, (bf16*)out, n, (cudaStream_t)stream);
 }
-int vtk_cast_bf16_to_f32(const void* in, float* out, int64_t n, void* stream) {
-  VTK_REQUIRE(in && out, "vtk_cast_bf16_to_f32: null pointer");
-  return launch_cast_bf16_f32((const bf16*)in, out, n, (cudaStream_t)stream);
-}
 
-int vtk_kv_len(const uint8_t* patch_mask, int* kv_len, int* is_prefix, int B, int N, void* stream) {
+int vtk_kv_len(const uint8_t* patch_mask, int* kv_len, int B, int N, void* stream) {
   VTK_REQUIRE(patch_mask && kv_len, "vtk_kv_len: null pointer");
-  return launch_kv_len(patch_mask, kv_len, is_prefix, B, N, (cudaStream_t)stream);
+  return launch_kv_len(patch_mask, kv_len, B, N, (cudaStream_t)stream);
 }
 
 int vtk_pack_plan(const uint8_t* patch_mask, int B, int N, int pad, int qrows, int* n_valid, int* rel, int* cu, int* cuq,
@@ -425,16 +402,6 @@ int vtk_linear_tn_bf16(const void* At, int64_t lda, const void* Bt, int64_t ldb,
   VTK_REQUIRE(ldo % 8 == 0, "vtk_linear_tn_bf16: ldo must be a multiple of 8");
   GemmArgs g = base_args(At, lda, Bt, ldb, N, M, N, K);
   g.trans = 3;
-  g.epi.out = (bf16*)out; g.epi.ldo = ldo;
-  return launch_gemm(EPI_BIAS, g, (cudaStream_t)stream);
-}
-
-int vtk_linear_nn_bf16(const void* A, int64_t lda, const void* Bt, int64_t ldb, void* out, int64_t ldo, int M, int N, int K,
-                       void* stream) {
-  VTK_REQUIRE(A && Bt && out, "vtk_linear_nn_bf16: null pointer");
-  VTK_REQUIRE(ldo % 8 == 0, "vtk_linear_nn_bf16: ldo must be a multiple of 8");
-  GemmArgs g = base_args(A, lda, Bt, ldb, N, M, N, K);
-  g.trans = 2;
   g.epi.out = (bf16*)out; g.epi.ldo = ldo;
   return launch_gemm(EPI_BIAS, g, (cudaStream_t)stream);
 }
@@ -521,38 +488,25 @@ int vtk_proj_residual_fp8(const void* A8, int64_t lda, const float* a_scale, con
 }
 
 int vtk_attention_bf16(const void* q, const void* k, const void* v, int64_t ld_qkv, void* out, int64_t ld_out,
-                       const int* kv_len, const uint8_t* key_mask, const int* is_prefix, int B, int N, int heads, int d,
-                       int zero_invalid_rows, int window, float* lse, void* stream) {
+                       const int* kv_len, int B, int N, int heads, int d, int zero_invalid_rows, int window, float* lse, void* stream) {
   VTK_REQUIRE(q && k && v && out, "vtk_attention_bf16: null pointer");
   AttnArgs a;
   a.q = (const bf16*)q; a.k = (const bf16*)k; a.v = (const bf16*)v; a.ld_qkv = ld_qkv; a.out = (bf16*)out; a.ld_out = ld_out;
-  a.kv_len = kv_len; a.key_mask = key_mask; a.prefix_flag = is_prefix; a.B = B; a.N = N; a.heads = heads; a.d = d;
+  a.kv_len = kv_len; a.B = B; a.N = N; a.heads = heads; a.d = d;
   a.zero_invalid_rows = zero_invalid_rows;
   a.window = window;
   a.lse = lse;
   return launch_attention(a, (cudaStream_t)stream);
 }
 
-int vtk_attention_packed_bf16(const void* q, const void* k, const void* v, int64_t ld_qkv, void* out, int64_t ld_out, const int* n_valid,
-                              const int* cu, const int* cuq, const int* grp_img, const int* grp_order, int B, int N, int heads, int d,
-                              int64_t row_cap, int grp_cap, void* stream) {
-  VTK_REQUIRE(q && k && v && out && n_valid && cu && cuq && grp_img && grp_order, "vtk_attention_packed_bf16: null pointer");
-  AttnArgs a;
-  a.q = (const bf16*)q; a.k = (const bf16*)k; a.v = (const bf16*)v; a.ld_qkv = ld_qkv; a.out = (bf16*)out; a.ld_out = ld_out;
-  a.kv_len = n_valid; a.key_mask = nullptr; a.prefix_flag = nullptr; a.B = B; a.N = N; a.heads = heads; a.d = d;
-  a.zero_invalid_rows = 0; a.window = -1; a.lse = nullptr;
-  a.cu = cu; a.cuq = cuq; a.grp_img = grp_img; a.grp_order = grp_order; a.row_cap = row_cap; a.grp_cap = grp_cap;
-  return launch_attention(a, (cudaStream_t)stream);
-}
-
 int vtk_attention_packed_lse_bf16(const void* q, const void* k, const void* v, int64_t ld_qkv, void* out, int64_t ld_out,
                                   const int* n_valid, const int* cu, const int* cuq, const int* grp_img, const int* grp_order, int B, int N,
                                   int heads, int d, int64_t row_cap, int grp_cap, float* lse, void* stream) {
-  VTK_REQUIRE(q && k && v && out && n_valid && cu && cuq && grp_img && grp_order && lse, "vtk_attention_packed_lse_bf16: null pointer");
+  VTK_REQUIRE(q && k && v && out && n_valid && cu && cuq && grp_img && grp_order, "vtk_attention_packed_lse_bf16: null pointer");
   AttnArgs a;
   a.q = (const bf16*)q; a.k = (const bf16*)k; a.v = (const bf16*)v; a.ld_qkv = ld_qkv; a.out = (bf16*)out; a.ld_out = ld_out;
-  a.kv_len = n_valid; a.key_mask = nullptr; a.prefix_flag = nullptr; a.B = B; a.N = N; a.heads = heads; a.d = d;
-  a.zero_invalid_rows = 1;   // the image's pad rows: out 0, lse +inf
+  a.kv_len = n_valid; a.B = B; a.N = N; a.heads = heads; a.d = d;
+  a.zero_invalid_rows = lse ? 1 : 0;   // with lse: the image's pad rows get out 0, lse +inf; without: they are not written
   a.window = -1; a.lse = lse;
   a.cu = cu; a.cuq = cuq; a.grp_img = grp_img; a.grp_order = grp_order; a.row_cap = row_cap; a.grp_cap = grp_cap;
   return launch_attention(a, (cudaStream_t)stream);
@@ -579,10 +533,6 @@ int vtk_swiglu_fwd(const void* zraw, int64_t ldz, int qp, void* act, int64_t ld_
   VTK_REQUIRE(layout == 0 || layout == 1, "vtk_swiglu_fwd: layout must be 0 (16-column value|gate groups) or 1 ([value | gate])");
   return launch_swiglu_fwd((const bf16*)zraw, ldz, qp, (bf16*)act, ld_act, M, Hf, layout, (cudaStream_t)stream);
 }
-int vtk_resid_fwd(const void* x, const void* y, const void* gamma, void* out, int M, int D, void* stream) {
-  VTK_REQUIRE(x && y && gamma && out, "vtk_resid_fwd: null pointer");
-  return launch_resid_fwd((const bf16*)x, (const bf16*)y, (const bf16*)gamma, (bf16*)out, M, D, (cudaStream_t)stream);
-}
 int vtk_resid_fwd_dp(const void* x, const void* y, const void* gamma, void* out, int M, int D, const float* keep, int rows_per_image,
                      float keep_prob, void* stream) {
   VTK_REQUIRE(x && y && gamma && out, "vtk_resid_fwd_dp: null pointer");
@@ -598,10 +548,6 @@ int vtk_resid_bwd_dp(const void* dx, const void* y, const void* gamma, void* dy,
 int vtk_layernorm_fwd(const void* x, void* out, int M, int C, float eps, void* stream) {
   VTK_REQUIRE(x && out, "vtk_layernorm_fwd: null pointer");
   return launch_ln_fwd((const bf16*)x, (bf16*)out, M, C, eps, (cudaStream_t)stream);
-}
-int vtk_resid_bwd(const void* dx, const void* y, const void* gamma, void* dy, float* dgamma, int M, int D, void* stream) {
-  VTK_REQUIRE(dx && y && gamma && dy && dgamma, "vtk_resid_bwd: null pointer");
-  return launch_resid_bwd((const bf16*)dx, (const bf16*)y, (const bf16*)gamma, (bf16*)dy, dgamma, M, D, (cudaStream_t)stream);
 }
 int vtk_colsum(const void* in, int64_t ld, float* out, int M, int C, void* stream) {
   VTK_REQUIRE(in && out, "vtk_colsum: null pointer");
@@ -629,22 +575,12 @@ int vtk_layernorm_bwd(const void* zlin, const void* dz, void* dx, int M, int C, 
   VTK_REQUIRE(zlin && dz && dx, "vtk_layernorm_bwd: null pointer");
   return launch_ln_bwd((const bf16*)zlin, (const bf16*)dz, (bf16*)dx, M, C, eps, (cudaStream_t)stream);
 }
-int vtk_transpose_bf16(const void* in, int64_t ldi, void* out, int64_t ldo, int R, int C, void* stream) {
-  VTK_REQUIRE(in && out, "vtk_transpose_bf16: null pointer");
-  return launch_transpose((const bf16*)in, ldi, (bf16*)out, ldo, R, C, (cudaStream_t)stream);
-}
 int vtk_charbonnier(const void* pred, const void* target, const uint8_t* patch_mask, const int* n_valid, float* loss_sum,
                     void* dpred, int B, int N, int P, float eps, void* stream) {
   VTK_REQUIRE(pred && target && loss_sum, "vtk_charbonnier: null pointer");
   VTK_REQUIRE(!patch_mask || n_valid, "vtk_charbonnier: n_valid is required with a patch_mask");
   return launch_charbonnier((const bf16*)pred, (const bf16*)target, patch_mask, n_valid, loss_sum, (bf16*)dpred, B, N, P, eps,
                             (cudaStream_t)stream);
-}
-int vtk_adamw_bf16(void* p, const void* g, void* m, void* v, int64_t n, float lr, float beta1, float beta2, float eps,
-                   float weight_decay, int step, float grad_scale, void* stream) {
-  VTK_REQUIRE(p && g && m && v, "vtk_adamw_bf16: null pointer");
-  return launch_adamw((bf16*)p, (const bf16*)g, (bf16*)m, (bf16*)v, n, lr, beta1, beta2, eps, weight_decay, step, grad_scale,
-                      (cudaStream_t)stream);
 }
 int vtk_adamw_multi(const vtk_adamw_tensor* tensors, int n_tensors, float lr, float beta1, float beta2, float eps, int step,
                     float grad_scale, void* stream) {
@@ -761,15 +697,12 @@ size_t vtk_ae_workspace_bytes(vtk_ae_t h, int side, int B, int N) {
   return carve(h->side[side], nullptr, B, N, io_cols(h->cfg)).bytes;
 }
 
-// Token packing is used whenever a mask is given and the attention kernel has the packed variant (head_dim 64).
-// vtk_ae_set_packing(h, 0) keeps the padded [B, N] layout with in-kernel key masking (parity tests).
-static bool use_packing(const vtk_ae_s* h, const Side& s, const uint8_t* patch_mask) {
-  return patch_mask != nullptr && s.depth > 0 && (s.head_dim() == 64 || s.head_dim() == 128) && h->packing;
-}
+// A masked batch runs on its packed valid tokens.  A side without blocks keeps the padded rows: it has no attention to mask.
+static bool use_packing(const Side& s, const uint8_t* patch_mask) { return patch_mask != nullptr && s.depth > 0; }
 
 // rows = row capacity of the activation buffers; with `pl` the kernels read the live row count from pl->m_dev()
-static int run_blocks(vtk_ae_s* h, const Side& s, const Workspace& w, const int64_t* row_idx, const int64_t* col_idx,
-                      const uint8_t* patch_mask, int B, int N, int rows, const PackPlan* pl, cudaStream_t st, int& launches) {
+static int run_blocks(vtk_ae_s* h, const Side& s, const Workspace& w, const int64_t* row_idx, const int64_t* col_idx, int B, int N,
+                      int rows, const PackPlan* pl, cudaStream_t st, int& launches) {
   const int M = rows, D = s.width, d = s.head_dim(), Hf = s.hidden, qp = s.qp(), kp = s.kp();
   const float eps = h->cfg.norm_eps;
   const int* m_dev = pl ? pl->m_dev() : nullptr;
@@ -778,11 +711,6 @@ static int run_blocks(vtk_ae_s* h, const Side& s, const Workspace& w, const int6
     { LaunchTimer t(h, st, CLS_MISC); r = launch_rope_table(row_idx, col_idx, s.inv_freq, w.rope, M, d, st, pl ? pl->src : nullptr, m_dev); }
     if (r) return r;
     ++launches;
-    if (patch_mask && !pl) {
-      { LaunchTimer t(h, st, CLS_MISC); r = launch_kv_len(patch_mask, w.kv_len, w.is_prefix, B, N, st); }
-      if (r) return r;
-      ++launches;
-    }
   }
   for (int i = 0; i < s.depth; ++i) {
     const vtk_block_weights& b = s.blocks[i];
@@ -811,19 +739,19 @@ static int run_blocks(vtk_ae_s* h, const Side& s, const Workspace& w, const int6
     AttnArgs a;
     a.q = w.qkv; a.k = w.qkv + D; a.v = w.qkv + 2 * D; a.ld_qkv = 3 * D; a.out = w.a2; a.ld_out = kp;
     a.B = B; a.N = N; a.heads = s.heads; a.d = d;
+    a.zero_invalid_rows = 0;
+    a.lse = nullptr;
     if (pl) {
       // packed: image b = packed rows [cu[b], cu[b+1]) with its n_valid[b] tokens in front -- no key mask left
-      a.kv_len = pl->n_valid; a.key_mask = nullptr; a.prefix_flag = nullptr; a.zero_invalid_rows = 0;
+      a.kv_len = pl->n_valid;
       a.cu = pl->cu; a.cuq = pl->cuq; a.grp_img = pl->grp_img; a.grp_order = pl->grp_order; a.row_cap = M;
       a.grp_cap = (int)PackPlan::group_capacity(B, N, pl->qrows);
       a.window = -1;
     } else {
-      a.kv_len = patch_mask ? w.kv_len : nullptr; a.key_mask = patch_mask; a.prefix_flag = patch_mask ? w.is_prefix : nullptr;
-      a.zero_invalid_rows = patch_mask ? 1 : 0;
-      // sliding window: flash backend only (attention.py:113-116); the sdpa backend (patch_mask given) ignores it
-      a.window = (!patch_mask && h->cfg.sliding_window > 0) ? h->cfg.sliding_window : -1;
+      // no mask: every key of the image, or those of the sliding window (flash backend, attention.py:113-116)
+      a.kv_len = nullptr;
+      a.window = h->cfg.sliding_window > 0 ? h->cfg.sliding_window : -1;
     }
-    a.lse = nullptr;
     { LaunchTimer t(h, st, CLS_ATTENTION); r = launch_attention(a, st); }
     if (r) return r;
     if (f8) {
@@ -850,7 +778,7 @@ static int run_side(vtk_ae_s* h, int side, const void* in, const int64_t* row_id
   const int P = h->cfg.pixels_per_token, C = h->cfg.channels_per_token, D = s.width;
   const int cin = side == 0 ? P : C, cout = side == 0 ? C : P;
   Workspace w = carve(s, workspace, B, N, io_cols(h->cfg));
-  const bool packed = use_packing(h, s, patch_mask);
+  const bool packed = use_packing(s, patch_mask);
   const PackPlan* pl = packed ? &w.plan : nullptr;
   const int rows = packed ? (int)PackPlan::row_capacity(B, N, w.plan.pad) : B * N;   // capacity; the live count is pl->m_dev()
   const int* m_dev = packed ? pl->m_dev() : nullptr;
@@ -871,7 +799,7 @@ static int run_side(vtk_ae_s* h, int side, const void* in, const int64_t* row_id
   { LaunchTimer t(h, st, CLS_LINEAR); r = launch_gemm(EPI_BIAS, g, st); }
   if (r) return r;
   ++launches;
-  if ((r = run_blocks(h, s, w, row_idx, col_idx, patch_mask, B, N, rows, pl, st, launches))) return r;
+  if ((r = run_blocks(h, s, w, row_idx, col_idx, B, N, rows, pl, st, launches))) return r;
   bf16* o = packed ? w.pout : (bf16*)out;
   GemmArgs gz = base_args(w.x, D, s.w_b, D, cout, rows, cout, D);
   gz.epi.out = o; gz.epi.ldo = cout; gz.epi.bias = s.b_b; gz.epi.eps = h->cfg.norm_eps; gz.epi.m_dev = m_dev;
@@ -942,12 +870,6 @@ int vtk_ae_set_fp8_weights(vtk_ae_t h, int side, const vtk_block_fp8* blocks, in
 int vtk_ae_set_fp8_granularity(vtk_ae_t h, int per_tensor) {
   VTK_REQUIRE(h, "vtk_ae_set_fp8_granularity: null handle");
   h->fp8_per_tensor = per_tensor != 0;
-  return VTK_OK;
-}
-
-int vtk_ae_set_packing(vtk_ae_t h, int enable) {
-  VTK_REQUIRE(h, "vtk_ae_set_packing: null handle");
-  h->packing = enable != 0;
   return VTK_OK;
 }
 

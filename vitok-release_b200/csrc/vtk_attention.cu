@@ -4,8 +4,9 @@
 // reference: out = softmax(q k^T / sqrt(d)) v per (image, head), q/k already QK-normed + RoPE'd by the
 // QKV GEMM epilogue.  The reference's sdpa backend masks keys with patch_mask (ae.py:173-187) by
 // materialising a [B,1,N,N] bool mask; here the mask is a per-image key length (padded keys are never
-// loaded -- whole kv tiles past kv_len[b] are skipped, padded query tiles exit at once) plus an optional
-// per-key byte mask for non-prefix masks.  The flash backend's semantics (no mask) = kv_len null.
+// loaded -- whole kv tiles past kv_len[b] are skipped, padded query tiles exit at once).  Masked inference runs
+// on the packed NaFlex layout, where every image's valid tokens form a prefix of its rows; the padded training
+// step permutes tokens so that every mask is a prefix mask.  The flash backend's semantics (no mask) = kv_len null.
 //
 // One CTA per (256-query block, head, image) = two 128-query tiles A and B that share every K/V tile:
 //   warps 0-3 : softmax warpgroup A   (one query row per thread, TMEM lane = row)
@@ -58,7 +59,7 @@ template <int DH, int NQ> struct AttnShape {
 
 struct AttnParams {
   bf16* out; long long ld_out;
-  const int* kv_len; const uint8_t* key_mask; const int* prefix_flag;
+  const int* kv_len;
   int N, heads, zero_invalid, tma_out;
   int window;         // sliding window |i - j| <= window on the token index (flash backend, attention.py:113-116); < 0 = none
   float scale_log2;   // (1/sqrt(d)) * log2(e)
@@ -81,14 +82,13 @@ __device__ __forceinline__ float ex2_approx(float x) {
   return y;
 }
 
-// Set the masked scores of one 128-key tile to -inf.  The common case -- the tail tile of an image whose valid keys are a
-// prefix (what patchify emits, and always the case in the packed layout), no byte mask, no window -- is handled per
-// 32-column chunk with warp-uniform branches: chunks entirely inside kvlen are skipped and only the chunks at / beyond
+// Set the masked scores of one 128-key tile to -inf.  The common case -- the tail tile of an image, no window -- is handled
+// per 32-column chunk with warp-uniform branches: chunks entirely inside kvlen are skipped and only the chunks at / beyond
 // the boundary pay a compare + select per column (the general per-element test costs ~12 instructions per score and
 // made a masked tile 8x as expensive as an unmasked one).
 template <int NCH>
-__device__ __forceinline__ void mask_scores(uint32_t (&v)[NCH][32], int kv0, int kvlen, const uint8_t* kmask, int W, int qi) {
-  if (kmask == nullptr && W < 0) {
+__device__ __forceinline__ void mask_scores(uint32_t (&v)[NCH][32], int kv0, int kvlen, int W, int qi) {
+  if (W < 0) {
     const int lim = kvlen - kv0;   // columns >= lim are masked
 #pragma unroll
     for (int c = 0; c < NCH; ++c) {
@@ -106,7 +106,7 @@ __device__ __forceinline__ void mask_scores(uint32_t (&v)[NCH][32], int kv0, int
 #pragma unroll
     for (int i = 0; i < 32; ++i) {
       const int kc = kv0 + c * 32 + i;
-      const bool ok = kc < kvlen && (kmask == nullptr || kmask[kc] != 0) && (W < 0 || abs(kc - qi) <= W);
+      const bool ok = kc < kvlen && abs(kc - qi) <= W;
       if (!ok) v[c][i] = 0xff800000u;   // -inf
     }
 }
@@ -388,8 +388,6 @@ attn_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__ CUt
     const uint32_t lane_base = (uint32_t)(quarter * 32) << 16;
     const uint32_t tS = tmem_base + lane_base + q * 128;
     const uint32_t tO = tmem_base + lane_base + S::O_COL0 + q * DH;
-    const bool general_mask = p.key_mask != nullptr && !(p.prefix_flag != nullptr && p.prefix_flag[img] != 0);
-    const uint8_t* kmask = general_mask ? p.key_mask + row0 : nullptr;
     uint8_t* prow = sP + q * S::P_BYTES + r * 128;
     const float sc = p.scale_log2;
     float m_run = -INFINITY, l_run = 0.f;
@@ -399,7 +397,7 @@ attn_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__ CUt
       const int kv0 = (j_lo + j) * ATT_BKV;
       const int qt0 = q0 + q * ATT_BQ;
       const bool win_mask = W >= 0 && (kv0 < qt0 + ATT_BQ - 1 - W || kv0 + ATT_BKV - 1 > qt0 + W);
-      const bool need_mask = (kv0 + ATT_BKV > kvlen) || (kmask != nullptr) || win_mask;
+      const bool need_mask = (kv0 + ATT_BKV > kvlen) || win_mask;
       const long long ta = p.prof ? clock64() : 0;
       mbar_wait(&s_full[q], (uint32_t)j & 1u);
       if (p.prof) { const long long tb = clock64(); if (j == 0) t_first = tb - t_sync; else w_s += tb - ta; }
@@ -413,7 +411,7 @@ attn_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__ CUt
       tmem_wait_ld();
       tc_fence_before();
       mbar_arrive(&s_empty[q]);   // S is in registers: the tensor core may overwrite it with S(j+1)
-      if (need_mask) mask_scores(v, kv0, kvlen, kmask, W, qi);
+      if (need_mask) mask_scores(v, kv0, kvlen, W, qi);
       float mx0 = -INFINITY, mx1 = -INFINITY, mx2 = -INFINITY, mx3 = -INFINITY;
 #pragma unroll
       for (int i = 0; i < 32; i += 2) {   // FMNMX3: two elements per instruction
@@ -472,8 +470,7 @@ attn_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__ CUt
     __syncwarp();
     tc_fence_after();
     const float inv = l_run > 0.f ? 1.f / l_run : 0.f;
-    bool zero_row = false;
-    if (p.zero_invalid) zero_row = (qi >= kvlen) || (kmask != nullptr && qi < N && kmask[qi] == 0);
+    const bool zero_row = p.zero_invalid && qi >= kvlen;
     const float osc = zero_row ? 0.f : inv;
     if (p.lse && qi < N) p.lse[(row0 + qi) * p.heads + head] = (zero_row || !(l_run > 0.f)) ? INFINITY : m_run + log2f(l_run);
     bf16* op = p.out + (row0 + qi) * p.ld_out + head * DH;
@@ -775,13 +772,11 @@ attn_persist_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_consta
         continue;
       }
       const int kvlen = it.kvlen;
-      const bool general_mask = p.key_mask != nullptr && !(p.prefix_flag != nullptr && p.prefix_flag[it.img] != 0);
-      const uint8_t* kmask = general_mask ? p.key_mask + row0 : nullptr;
       float m_run = -INFINITY, l_run = 0.f;
       for (int j = 0; j < it.Tn; ++j, ++n_t) {
         const int kv0 = (it.j_lo + j) * ATT_BKV;
         const bool win_mask = W >= 0 && (kv0 < it.q0 + ATT_BQ - 1 - W || kv0 + ATT_BKV - 1 > it.q0 + W);
-        const bool need_mask = (kv0 + ATT_BKV > kvlen) || (kmask != nullptr) || win_mask;
+        const bool need_mask = (kv0 + ATT_BKV > kvlen) || win_mask;
         const long long k0 = PCLK();
         mbar_wait(s_full, n_t & 1u);
         __syncwarp();
@@ -796,7 +791,7 @@ attn_persist_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_consta
         tc_fence_before();
         mbar_arrive(s_empty);   // S is in registers: the tensor core may overwrite it with the next tile's S
         const long long k2 = PCLK();
-        if (need_mask) mask_scores(v, kv0, kvlen, kmask, W, qi);
+        if (need_mask) mask_scores(v, kv0, kvlen, W, qi);
         float mx0 = -INFINITY, mx1 = -INFINITY, mx2 = -INFINITY, mx3 = -INFINITY;
 #pragma unroll
         for (int i = 0; i < 32; i += 2) {
@@ -856,8 +851,7 @@ attn_persist_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_consta
       tc_fence_after();
       const long long e1 = PCLK();
       const float inv = l_run > 0.f ? 1.f / l_run : 0.f;
-      bool zero_row = false;
-      if (p.zero_invalid) zero_row = (qi >= kvlen) || (kmask != nullptr && qi < N && kmask[qi] == 0);
+      const bool zero_row = p.zero_invalid && qi >= kvlen;
       const float osc = zero_row ? 0.f : inv;
       if (p.lse && qi < N) p.lse[(row0 + qi) * p.heads + it.head] = (zero_row || !(l_run > 0.f)) ? INFINITY : m_run + log2f(l_run);
       uint32_t o[DH / 32][32];
@@ -932,8 +926,8 @@ static int launch_attention_persist(const AttnArgs& a, cudaStream_t stream) {
   const bool packed = a.cu != nullptr;
   const long long Mrows = packed ? a.row_cap : (long long)a.B * a.N;
   const long long cols = (long long)a.heads * a.d;
-  if (packed && (!a.cuq || !a.grp_img || !a.grp_order || !a.kv_len || a.key_mask || a.window >= 0 || a.row_cap <= 0 || a.grp_cap <= 0)) {
-    set_error("attention: packed layout needs cu/cuq/grp_img/grp_order/kv_len, row and group capacities, no key mask and no window");
+  if (packed && (!a.cuq || !a.grp_img || !a.grp_order || !a.kv_len || a.window >= 0 || a.row_cap <= 0 || a.grp_cap <= 0)) {
+    set_error("attention: packed layout needs cu/cuq/grp_img/grp_order/kv_len, row and group capacities and no window");
     return -2;
   }
   CUtensorMap tmQ, tmK, tmV, tmO;
@@ -943,7 +937,7 @@ static int launch_attention_persist(const AttnArgs& a, cudaStream_t stream) {
   if (encode_tmap_bf16(&tmO, a.out, cols, Mrows, a.ld_out, 64, 32, 128)) return -1;
   AttnParams p;
   p.out = a.out; p.ld_out = a.ld_out;
-  p.kv_len = a.kv_len; p.key_mask = a.key_mask; p.prefix_flag = a.prefix_flag;
+  p.kv_len = a.kv_len;
   p.N = a.N; p.heads = a.heads; p.zero_invalid = a.zero_invalid_rows;
   p.tma_out = (packed || a.N % ATT_BQ == 0) ? 1 : 0;
   p.window = a.window;
@@ -984,8 +978,8 @@ template <int DH, int NQ>
 static int launch_attention_t(const AttnArgs& a, cudaStream_t stream) {
   using S = AttnShape<DH, NQ>;
   const bool packed = a.cu != nullptr;
-  if (packed && (!a.cuq || !a.grp_img || !a.kv_len || a.key_mask || a.window >= 0 || a.row_cap <= 0 || a.grp_cap <= 0)) {
-    set_error("attention: packed layout needs cu/cuq/grp_img/kv_len, row and group capacities, no key mask and no window");
+  if (packed && (!a.cuq || !a.grp_img || !a.kv_len || a.window >= 0 || a.row_cap <= 0 || a.grp_cap <= 0)) {
+    set_error("attention: packed layout needs cu/cuq/grp_img/kv_len, row and group capacities and no window");
     return -2;
   }
   const long long Mrows = packed ? a.row_cap : (long long)a.B * a.N;
@@ -998,7 +992,7 @@ static int launch_attention_t(const AttnArgs& a, cudaStream_t stream) {
   if (encode_tmap_bf16(&tmO, a.out, cols, Mrows, a.ld_out, 64, 32, 128)) return -1;
   AttnParams p;
   p.out = a.out; p.ld_out = a.ld_out;
-  p.kv_len = a.kv_len; p.key_mask = a.key_mask; p.prefix_flag = a.prefix_flag;
+  p.kv_len = a.kv_len;
   p.N = a.N; p.heads = a.heads; p.zero_invalid = a.zero_invalid_rows;
   p.tma_out = (packed || a.N % ATT_BQ == 0) ? 1 : 0;
   p.window = a.window;

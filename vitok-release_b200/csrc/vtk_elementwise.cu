@@ -190,12 +190,6 @@ __global__ void cast_f32_bf16_kernel(const float* __restrict__ in, bf16* __restr
   for (long long i = (nvec << 3) + (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride)
     out[i] = __float2bfloat16_rn(in[i]);
 }
-__global__ void cast_bf16_f32_kernel(const bf16* __restrict__ in, float* __restrict__ out, long long n) {
-  pdl_wait();      // PDL (vtk_common.cuh): this kernel may have been launched before its predecessor finished
-  pdl_trigger();
-  const long long stride = (long long)gridDim.x * blockDim.x;
-  for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) out[i] = __bfloat162float(in[i]);
-}
 static int cast_grid(long long n) {
   long long blocks = (n / 8 + 255) / 256 + 1;
   const long long cap = (long long)num_sms() * 16;
@@ -205,11 +199,6 @@ int launch_cast_f32_bf16(const float* in, bf16* out, long long n, cudaStream_t s
   if (n <= 0) return 0;
   if ((reinterpret_cast<uintptr_t>(in) | reinterpret_cast<uintptr_t>(out)) & 15) { set_error("cast: pointers must be 16-byte aligned"); return -2; }
   (void)launch_k(cast_f32_bf16_kernel, dim3(cast_grid(n)), dim3(256), 0, stream, in, out, n);
-  return check_cuda(cudaGetLastError(), "cast launch");
-}
-int launch_cast_bf16_f32(const bf16* in, float* out, long long n, cudaStream_t stream) {
-  if (n <= 0) return 0;
-  (void)launch_k(cast_bf16_f32_kernel, dim3(cast_grid(n)), dim3(256), 0, stream, in, out, n);
   return check_cuda(cudaGetLastError(), "cast launch");
 }
 
@@ -303,32 +292,24 @@ int launch_quant_rows_e4m3(const bf16* x, long long ldx, uint8_t* q, long long l
   return check_cuda(cudaGetLastError(), "quant_rows launch");
 }
 
-// one warp per image: kv_len = 1 + index of the last valid token (0 if none); is_prefix = mask is all-ones
-// on [0, kv_len).
-__global__ void kv_len_kernel(const uint8_t* __restrict__ mask, int* __restrict__ kv_len, int* __restrict__ is_prefix,
-                              int B, int N) {
+// one warp per image: kv_len = 1 + index of the last valid token (0 if none)
+__global__ void kv_len_kernel(const uint8_t* __restrict__ mask, int* __restrict__ kv_len, int B, int N) {
   pdl_wait();      // PDL (vtk_common.cuh): this kernel may have been launched before its predecessor finished
   pdl_trigger();
   const int b = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
   if (b >= B) return;
   const int lane = threadIdx.x & 31;
-  int last = -1, count = 0;
+  int last = -1;
   for (int i = lane; i < N; i += 32) {
-    if (mask[(long long)b * N + i]) { last = i; ++count; }
+    if (mask[(long long)b * N + i]) last = i;
   }
 #pragma unroll
-  for (int o = 16; o > 0; o >>= 1) {
-    last = max(last, __shfl_xor_sync(0xffffffffu, last, o));
-    count += __shfl_xor_sync(0xffffffffu, count, o);
-  }
-  if (lane == 0) {
-    kv_len[b] = last + 1;
-    if (is_prefix) is_prefix[b] = (count == last + 1) ? 1 : 0;
-  }
+  for (int o = 16; o > 0; o >>= 1) last = max(last, __shfl_xor_sync(0xffffffffu, last, o));
+  if (lane == 0) kv_len[b] = last + 1;
 }
-int launch_kv_len(const uint8_t* mask, int* kv_len, int* is_prefix, int B, int N, cudaStream_t stream) {
+int launch_kv_len(const uint8_t* mask, int* kv_len, int B, int N, cudaStream_t stream) {
   if (B <= 0) return 0;
-  (void)launch_k(kv_len_kernel, dim3((B + 3) / 4), dim3(128), 0, stream, mask, kv_len, is_prefix, B, N);
+  (void)launch_k(kv_len_kernel, dim3((B + 3) / 4), dim3(128), 0, stream, mask, kv_len, B, N);
   return check_cuda(cudaGetLastError(), "kv_len launch");
 }
 

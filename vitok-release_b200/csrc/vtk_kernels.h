@@ -111,20 +111,17 @@ int launch_umma_probe(const bf16* A, const bf16* B, float* D, int N, int K, int 
 
 // ---------------------------------------------------------------------------------------------
 // attention (vtk_attention.cu): softmax(q k^T / sqrt(d)) v per (image, head); q/k/v rows are
-// [B*N, ld] with heads along columns.  kv_len[b] = number of leading key rows to visit
-// (null = N); key_mask [B, N] bytes (null = none) masks individual keys inside kv_len.
+// [B*N, ld] with heads along columns.  kv_len[b] = number of leading key rows to visit (null = N).
 // ---------------------------------------------------------------------------------------------
 struct AttnArgs {
   const bf16* q; const bf16* k; const bf16* v; long long ld_qkv;  // row stride (elements)
   bf16* out; long long ld_out;
   const int* kv_len;            // [B] or null
-  const uint8_t* key_mask;      // [B, N] or null
-  const int* prefix_flag;       // [B] or null: 1 = key_mask[b] is a pure prefix (kv_len alone describes it)
   int B, N, heads, d;
-  int zero_invalid_rows;        // 1: rows >= kv_len[b] (or with key_mask 0) are written as 0 (packed: the image's pad rows)
+  int zero_invalid_rows;        // 1: rows >= kv_len[b] are written as 0 (packed: the image's pad rows)
   int window;                   // sliding window: keys j with |i - j| <= window (flash_attn window_size=(w,w)); < 0 = none
   float* lse;                   // optional [B*N, heads] fp32: log2-domain logsumexp of the scaled scores (for the backward pass)
-  // packed NaFlex layout (PackPlan): rows of image b start at cu[b] and hold kv_len[b] valid tokens, no key_mask; work group g
+  // packed NaFlex layout (PackPlan): rows of image b start at cu[b] and hold kv_len[b] valid tokens; work group g
   // (128 query rows at d = 64, 256 at d = 128) belongs to image grp_img[g] and is the (g - cuq[grp_img[g]])-th of that image
   const int* cu = nullptr; const int* cuq = nullptr; const int* grp_img = nullptr; const int* grp_order = nullptr;
   long long row_cap = 0;   // rows of the q / k / v / out buffers
@@ -185,12 +182,11 @@ int launch_pack_rows(const bf16* in, long long ld_in, const PackPlan& pl, long l
 int launch_unpack_rows(const bf16* packed, long long ld_p, const PackPlan& pl, bf16* out, long long ld_out, int width,
                        cudaStream_t stream);
 int launch_cast_f32_bf16(const float* in, bf16* out, long long n, cudaStream_t stream);
-int launch_cast_bf16_f32(const bf16* in, float* out, long long n, cudaStream_t stream);
 // dynamic per-row FP8 (e4m3) quantisation: q[row, :K] = e4m3(x[row, :K] / scale[row]), scale[row] = amax(row) / 448
 // amax_ws (optional, one device float): per-TENSOR scale instead (amax of the whole tensor, torchao's default granularity)
 int launch_quant_rows_e4m3(const bf16* x, long long ldx, uint8_t* q, long long ldq, float* scale, int M, int K, const int* m_dev,
                            cudaStream_t stream, float* amax_ws = nullptr);
-int launch_kv_len(const uint8_t* mask, int* kv_len, int* is_prefix, int B, int N, cudaStream_t stream);
+int launch_kv_len(const uint8_t* mask, int* kv_len, int B, int N, cudaStream_t stream);
 
 // ---------------------------------------------------------------------------------------------
 // NaFlex pre/post-processing (vtk_pp.cu)
@@ -278,11 +274,8 @@ int launch_qk_norm_rope_bwd(bf16* dz, long long lddz, const bf16* zraw, long lon
 int launch_rmsnorm_bwd(const bf16* x, const bf16* dh, const bf16* w, const bf16* dx_res, bf16* dx_out, float* dw, int M, int D,
                        float eps, cudaStream_t st);
 int launch_ln_bwd(const bf16* zlin, const bf16* dz, bf16* dx, int M, int C, float eps, cudaStream_t st);
-int launch_transpose(const bf16* in, long long ldi, bf16* out, long long ldo, int R, int C, cudaStream_t st);
 int launch_charbonnier(const bf16* pred, const bf16* target, const uint8_t* mask, const int* n_valid, float* loss_sum, bf16* dpred,
                        int B, int N, int P, float eps, cudaStream_t st);
-int launch_adamw(bf16* p, const bf16* g, bf16* m, bf16* v, long long n, float lr, float b1, float b2, float eps, float wd, int step,
-                 float grad_scale, cudaStream_t st);
 int launch_attn_delta(const bf16* o, long long ldo, const bf16* dob, long long lddo, float* delta, int M, int heads, int d,
                       cudaStream_t st);
 // one tensor of a multi-tensor AdamW step (mirrors vtk_adamw_tensor of include/vitok_b200.h)

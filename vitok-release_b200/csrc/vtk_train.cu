@@ -11,7 +11,7 @@
 //   AdamW (multi-tensor)     scripts/train_vae.py:185-208    torch.optim.AdamW semantics, fp32 master weights + fp32 moments
 //
 // GEMMs of the backward pass (dgrad / wgrad) run on the tcgen05 GEMM of vtk_gemm.cu with transposed-operand variants (the
-// weights and activations are read MN-major as stored: no transposed copies; transpose_kernel below is kept for tests only).
+// weights and activations are read MN-major as stored: no transposed copies).
 #include <stdlib.h>
 
 #include <algorithm>
@@ -481,40 +481,6 @@ __global__ void __launch_bounds__(256) ln_bwd_kernel(const bf16* __restrict__ zl
   }
 }
 
-// out [C, R] = in [R, C]^T  (bf16; R, C multiples of 8; row strides in elements).  64 x 64 tiles through
-// shared memory, 16-byte global accesses on both sides.
-__global__ void __launch_bounds__(256) transpose_kernel(const bf16* __restrict__ in, long long ldi, bf16* __restrict__ out,
-                                                        long long ldo, int R, int C) {
-  __shared__ uint16_t tile[64][64 + 2];
-  const int r0 = blockIdx.y * 64, c0 = blockIdx.x * 64;
-  const int t = threadIdx.x;
-  // load: 64 rows x 8 vectors of 8 columns; thread -> (row = t / 8 + 32 * pass, vec = t % 8)
-#pragma unroll
-  for (int pass = 0; pass < 2; ++pass) {
-    const int r = (t >> 3) + 32 * pass, v = t & 7;
-    uint4 q = make_uint4(0, 0, 0, 0);
-    if (r0 + r < R && c0 + 8 * v < C) q = ld_global_nc_v4(in + (long long)(r0 + r) * ldi + c0 + 8 * v);
-    const uint32_t u[4] = {q.x, q.y, q.z, q.w};
-#pragma unroll
-    for (int k = 0; k < 4; ++k) {
-      tile[r][8 * v + 2 * k] = (uint16_t)(u[k] & 0xFFFFu);
-      tile[r][8 * v + 2 * k + 1] = (uint16_t)(u[k] >> 16);
-    }
-  }
-  __syncthreads();
-#pragma unroll
-  for (int pass = 0; pass < 2; ++pass) {
-    const int c = (t >> 3) + 32 * pass, v = t & 7;   // output row = input column c, output columns 8v..8v+7 = input rows
-    if (c0 + c < C && r0 + 8 * v < R) {
-      uint32_t u[4];
-#pragma unroll
-      for (int k = 0; k < 4; ++k)
-        u[k] = (uint32_t)tile[8 * v + 2 * k][c] | ((uint32_t)tile[8 * v + 2 * k + 1][c] << 16);
-      *reinterpret_cast<uint4*>(out + (long long)(c0 + c) * ldo + r0 + 8 * v) = make_uint4(u[0], u[1], u[2], u[3]);
-    }
-  }
-}
-
 // Charbonnier loss (scripts/train_vae.py:314-320): per token mean over P of sqrt(diff^2 + eps^2) with
 // diff = float(pred) - float(target); per image mean over its valid tokens; batch mean.
 //   loss_sum[b] += per-token means of image b (fp32 atomics);  n_valid[b] is computed by the caller
@@ -551,7 +517,7 @@ __global__ void __launch_bounds__(256) charbonnier_kernel(const bf16* __restrict
   }
 }
 
-// fused AdamW on bf16 params / grads / moments with fp32 math (torch.optim.AdamW(fused=True) semantics):
+// one AdamW element update in fp32 (torch.optim.AdamW semantics):
 //   p *= 1 - lr * wd;  m = b1 m + (1 - b1) g;  v = b2 v + (1 - b2) g^2;  p -= lr / bc1 * m / (sqrt(v) / sqrt(bc2) + eps)
 __device__ __forceinline__ void adamw_one(float& pf, float gf, float& mf, float& vf, float lr, float b1, float b2, float eps,
                                           float wd, float bc1, float bc2_sqrt) {
@@ -560,41 +526,6 @@ __device__ __forceinline__ void adamw_one(float& pf, float gf, float& mf, float&
   vf = b2 * vf + (1.f - b2) * gf * gf;
   const float denom = sqrtf(vf) / bc2_sqrt + eps;
   pf -= (lr / bc1) * (mf / denom);
-}
-
-// 8 elements (16 bytes of each of p, g, m, v) per thread and iteration: 4 coalesced 16-byte loads, 3 stores -- the optimizer
-// step is pure HBM streaming (14 bytes per parameter).  VEC = false: scalar fallback for unaligned / short tensors.
-template <bool VEC>
-__global__ void __launch_bounds__(256) adamw_kernel(bf16* __restrict__ p, const bf16* __restrict__ g, bf16* __restrict__ m,
-                                                    bf16* __restrict__ v, long long n, float lr, float b1, float b2, float eps,
-                                                    float wd, float bc1, float bc2_sqrt, float grad_scale) {
-  const long long stride = (long long)gridDim.x * blockDim.x;
-  const long long tid = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-  long long done = 0;
-  if (VEC) {
-    const long long nvec = n >> 3;
-    for (long long i = tid; i < nvec; i += stride) {
-      const uint4 pq = ld_global_v4(p + 8 * i), gq = ld_global_nc_v4(g + 8 * i), mq = ld_global_v4(m + 8 * i), vq = ld_global_v4(v + 8 * i);
-      float pf[8], gf[8], mf[8], vf[8];
-      unpack8(pq, pf); unpack8(gq, gf); unpack8(mq, mf); unpack8(vq, vf);
-#pragma unroll
-      for (int k = 0; k < 8; ++k) adamw_one(pf[k], gf[k] * grad_scale, mf[k], vf[k], lr, b1, b2, eps, wd, bc1, bc2_sqrt);
-      const uint4 po = pack8(pf), mo = pack8(mf), vo = pack8(vf);
-      st_global_v4(p + 8 * i, po.x, po.y, po.z, po.w);
-      st_global_v4(m + 8 * i, mo.x, mo.y, mo.z, mo.w);
-      st_global_v4(v + 8 * i, vo.x, vo.y, vo.z, vo.w);
-    }
-    done = nvec << 3;
-  }
-  for (long long i = done + tid; i < n; i += stride) {
-    float pf = __bfloat162float(p[i]);
-    const float gf = __bfloat162float(g[i]) * grad_scale;
-    float mf = __bfloat162float(m[i]), vf = __bfloat162float(v[i]);
-    adamw_one(pf, gf, mf, vf, lr, b1, b2, eps, wd, bc1, bc2_sqrt);
-    p[i] = __float2bfloat16_rn(pf);
-    m[i] = __float2bfloat16_rn(mf);
-    v[i] = __float2bfloat16_rn(vf);
-  }
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -1120,30 +1051,12 @@ int launch_ln_bwd(const bf16* zlin, const bf16* dz, bf16* dx, int M, int C, floa
   ln_bwd_kernel<<<grid_for(M, 8), 256, 0, st>>>(zlin, dz, dx, M, C, eps);
   return check_cuda(cudaGetLastError(), "ln_bwd launch");
 }
-int launch_transpose(const bf16* in, long long ldi, bf16* out, long long ldo, int R, int C, cudaStream_t st) {
-  VTK_TRAIN_CHECK(R % 8 == 0 && C % 8 == 0 && ldi % 8 == 0 && ldo % 8 == 0, "transpose: sizes and strides must be multiples of 8");
-  if (R <= 0 || C <= 0) return 0;
-  dim3 grid((C + 63) / 64, (R + 63) / 64);
-  transpose_kernel<<<grid, 256, 0, st>>>(in, ldi, out, ldo, R, C);
-  return check_cuda(cudaGetLastError(), "transpose launch");
-}
 int launch_charbonnier(const bf16* pred, const bf16* target, const uint8_t* mask, const int* n_valid, float* loss_sum, bf16* dpred,
                        int B, int N, int P, float eps, cudaStream_t st) {
   VTK_TRAIN_CHECK(P % 8 == 0, "charbonnier: P %% 8 required");
   if (B <= 0 || N <= 0) return 0;
   charbonnier_kernel<<<grid_for((long long)B * N, 8), 256, 0, st>>>(pred, target, mask, n_valid, loss_sum, dpred, B, N, P, eps);
   return check_cuda(cudaGetLastError(), "charbonnier launch");
-}
-int launch_adamw(bf16* p, const bf16* g, bf16* m, bf16* v, long long n, float lr, float b1, float b2, float eps, float wd, int step,
-                 float grad_scale, cudaStream_t st) {
-  if (n <= 0) return 0;
-  VTK_TRAIN_CHECK(step >= 1, "adamw: step must be >= 1");
-  const float bc1 = 1.f - powf(b1, (float)step), bc2s = sqrtf(1.f - powf(b2, (float)step));
-  const bool vec = ((reinterpret_cast<uintptr_t>(p) | reinterpret_cast<uintptr_t>(g) | reinterpret_cast<uintptr_t>(m) |
-                     reinterpret_cast<uintptr_t>(v)) & 15) == 0 && n >= 8;
-  if (vec) adamw_kernel<true><<<grid_for((n + 7) / 8, 256, 8), 256, 0, st>>>(p, g, m, v, n, lr, b1, b2, eps, wd, bc1, bc2s, grad_scale);
-  else adamw_kernel<false><<<grid_for(n, 256), 256, 0, st>>>(p, g, m, v, n, lr, b1, b2, eps, wd, bc1, bc2s, grad_scale);
-  return check_cuda(cudaGetLastError(), "adamw launch");
 }
 int launch_adamw_multi(const AdamwTensor* tensors, int n_tensors, float lr, float b1, float b2, float eps, int step, float grad_scale,
                        cudaStream_t st) {

@@ -49,7 +49,6 @@ SIGNATURES = {
     "vtk_abi_version": (c_int, []),
     "vtk_sm_count": (c_int, []),
     "vtk_set_flag": (c_int, [ctypes.c_char_p, c_int]),
-    "vtk_patchify": (c_int, [c_vp, c_vp, c_int, c_int, c_int, c_int, c_int, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp]),
     "vtk_patchify_ex": (c_int, [c_vp, c_vp, c_int, c_int, c_int, c_int, c_int, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_int, c_int, c_vp]),
     "vtk_resize_patchify": (c_int, [c_vp, c_vp, c_int, c_int, c_int, c_int, c_int, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_sz,
                                     c_vp, c_vp]),
@@ -60,8 +59,7 @@ SIGNATURES = {
     "vtk_rmsnorm_bf16": (c_int, [c_vp, c_i64, c_vp, c_vp, c_i64, c_int, c_int, c_f32, c_vp]),
     "vtk_rope_table": (c_int, [c_vp, c_vp, c_vp, c_vp, c_int, c_int, c_vp]),
     "vtk_cast_f32_to_bf16": (c_int, [c_vp, c_vp, c_i64, c_vp]),
-    "vtk_cast_bf16_to_f32": (c_int, [c_vp, c_vp, c_i64, c_vp]),
-    "vtk_kv_len": (c_int, [c_vp, c_vp, c_vp, c_int, c_int, c_vp]),
+    "vtk_kv_len": (c_int, [c_vp, c_vp, c_int, c_int, c_vp]),
     "vtk_pack_plan": (c_int, [c_vp, c_int, c_int, c_int, c_int, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp]),
     "vtk_pack_rows": (c_int, [c_vp, c_i64, c_vp, c_vp, c_int, c_i64, c_vp, c_i64, c_int, c_vp]),
     "vtk_unpack_rows": (c_int, [c_vp, c_i64, c_vp, c_vp, c_int, c_int, c_vp, c_i64, c_int, c_vp]),
@@ -70,7 +68,6 @@ SIGNATURES = {
     "vtk_proj_residual_fp8": (c_int, [c_vp, c_i64, c_vp, c_vp, c_i64, c_f32, c_vp, c_vp, c_i64, c_int, c_int, c_int, c_vp]),
     "vtk_linear_bf16": (c_int, [c_vp, c_i64, c_vp, c_i64, c_vp, c_vp, c_i64, c_int, c_int, c_int, c_vp]),
     "vtk_linear_tn_bf16": (c_int, [c_vp, c_i64, c_vp, c_i64, c_vp, c_i64, c_int, c_int, c_int, c_vp]),
-    "vtk_linear_nn_bf16": (c_int, [c_vp, c_i64, c_vp, c_i64, c_vp, c_i64, c_int, c_int, c_int, c_vp]),
     "vtk_linear_nn_acc_bf16": (c_int, [c_vp, c_i64, c_vp, c_i64, c_vp, c_i64, c_int, c_int, c_int, c_int, c_vp]),
     "vtk_linear2_bf16": (c_int, [c_vp, c_i64, c_vp, c_i64, c_vp, c_i64, c_vp, c_i64, c_int, c_int, c_int, c_int, c_vp]),
     "vtk_resid_fwd_dp": (c_int, [c_vp, c_vp, c_vp, c_vp, c_int, c_int, c_vp, c_int, c_f32, c_vp]),
@@ -81,25 +78,18 @@ SIGNATURES = {
     "vtk_qkv_swiglu_bf16": (c_int, [c_vp, c_i64, c_vp, c_i64, c_i64, c_int, c_int, c_int, c_int, c_int, c_vp, c_vp, c_vp,
                                     c_f32, c_vp, c_i64, c_vp, c_i64, c_vp]),
     "vtk_proj_residual_bf16": (c_int, [c_vp, c_i64, c_vp, c_i64, c_vp, c_vp, c_i64, c_int, c_int, c_int, c_vp]),
-    "vtk_attention_bf16": (c_int, [c_vp, c_vp, c_vp, c_i64, c_vp, c_i64, c_vp, c_vp, c_vp, c_int, c_int, c_int, c_int,
-                                   c_int, c_int, c_vp, c_vp]),
-    "vtk_attention_packed_bf16": (c_int, [c_vp, c_vp, c_vp, c_i64, c_vp, c_i64, c_vp, c_vp, c_vp, c_vp, c_vp, c_int, c_int, c_int, c_int,
-                                          c_i64, c_int, c_vp]),
+    "vtk_attention_bf16": (c_int, [c_vp, c_vp, c_vp, c_i64, c_vp, c_i64, c_vp, c_int, c_int, c_int, c_int, c_int, c_int, c_vp, c_vp]),
     "vtk_attention_packed_lse_bf16": (c_int, [c_vp, c_vp, c_vp, c_i64, c_vp, c_i64, c_vp, c_vp, c_vp, c_vp, c_vp, c_int, c_int, c_int,
                                               c_int, c_i64, c_int, c_vp, c_vp]),
     "vtk_qk_norm_rope_fwd": (c_int, [c_vp, c_i64, c_vp, c_vp, c_vp, c_vp, c_i64, c_int, c_int, c_int, c_f32, c_vp]),
     "vtk_swiglu_fwd": (c_int, [c_vp, c_i64, c_int, c_vp, c_i64, c_int, c_int, c_int, c_vp]),
-    "vtk_resid_fwd": (c_int, [c_vp, c_vp, c_vp, c_vp, c_int, c_int, c_vp]),
     "vtk_layernorm_fwd": (c_int, [c_vp, c_vp, c_int, c_int, c_f32, c_vp]),
-    "vtk_resid_bwd": (c_int, [c_vp, c_vp, c_vp, c_vp, c_vp, c_int, c_int, c_vp]),
     "vtk_colsum": (c_int, [c_vp, c_i64, c_vp, c_int, c_int, c_vp]),
     "vtk_swiglu_bwd": (c_int, [c_vp, c_i64, c_vp, c_i64, c_int, c_vp, c_i64, c_int, c_int, c_int, c_vp]),
     "vtk_qk_norm_rope_bwd": (c_int, [c_vp, c_i64, c_vp, c_i64, c_vp, c_vp, c_vp, c_vp, c_int, c_int, c_int, c_f32, c_vp]),
     "vtk_rmsnorm_bwd": (c_int, [c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_int, c_int, c_f32, c_vp]),
     "vtk_layernorm_bwd": (c_int, [c_vp, c_vp, c_vp, c_int, c_int, c_f32, c_vp]),
-    "vtk_transpose_bf16": (c_int, [c_vp, c_i64, c_vp, c_i64, c_int, c_int, c_vp]),
     "vtk_charbonnier": (c_int, [c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_int, c_int, c_int, c_f32, c_vp]),
-    "vtk_adamw_bf16": (c_int, [c_vp, c_vp, c_vp, c_vp, c_i64, c_f32, c_f32, c_f32, c_f32, c_f32, c_int, c_f32, c_vp]),
     "vtk_attn_delta": (c_int, [c_vp, c_i64, c_vp, c_i64, c_vp, c_int, c_int, c_int, c_vp]),
     "vtk_attention_bwd_bf16": (c_int, [c_vp, c_vp, c_vp, c_i64, c_vp, c_i64, c_vp, c_vp, c_vp, c_vp, c_vp, c_i64, c_vp,
                                        c_int, c_int, c_int, c_int, c_int, c_int, c_vp]),
@@ -115,7 +105,6 @@ SIGNATURES = {
     "vtk_ae_decode": (c_int, [c_vp, c_vp, c_vp, c_vp, c_vp, c_int, c_int, c_vp, c_vp, c_sz, c_vp]),
     "vtk_ae_last_launch_count": (c_int, [c_vp]),
     "vtk_ae_set_timing": (c_int, [c_vp, c_int]),
-    "vtk_ae_set_packing": (c_int, [c_vp, c_int]),
     "vtk_ae_set_fp8_granularity": (c_int, [c_vp, c_int]),
     "vtk_ae_set_fp8_weights": (c_int, [c_vp, c_int, ctypes.POINTER(BlockFp8), c_int]),
     "vtk_ae_set_norm_folded": (c_int, [c_vp, c_int, c_int]),
@@ -252,7 +241,7 @@ def linear_nn(a: torch.Tensor, bt: torch.Tensor) -> torch.Tensor:
     M, K = a.shape
     N = bt.shape[1]
     out = torch.empty(M, N, dtype=torch.bfloat16, device=a.device)
-    check(load().vtk_linear_nn_bf16(ptr(a), a.stride(0), ptr(bt), bt.stride(0), ptr(out), out.stride(0), M, N, K, stream_ptr()))
+    check(load().vtk_linear_nn_acc_bf16(ptr(a), a.stride(0), ptr(bt), bt.stride(0), ptr(out), out.stride(0), M, N, K, 0, stream_ptr()))
     return out
 
 
@@ -305,13 +294,13 @@ def cast_to_bf16(x: torch.Tensor) -> torch.Tensor:
 
 
 @_on_device
-def kv_len(mask: torch.Tensor):
+def kv_len(mask: torch.Tensor) -> torch.Tensor:
+    """[B] int32: 1 + index of the last valid token of each image (the key length of a prefix mask)."""
     B, N = mask.shape
     m = mask.contiguous().view(torch.uint8) if mask.dtype == torch.bool else mask.contiguous()
     kl = torch.empty(B, dtype=torch.int32, device=mask.device)
-    pf = torch.empty(B, dtype=torch.int32, device=mask.device)
-    check(load().vtk_kv_len(ptr(m), ptr(kl), ptr(pf), B, N, stream_ptr()))
-    return kl, pf
+    check(load().vtk_kv_len(ptr(m), ptr(kl), B, N, stream_ptr()))
+    return kl
 
 
 @_on_device
@@ -407,17 +396,21 @@ def proj_residual(a, w, gamma, x):
 @_on_device
 def attention(qkv: torch.Tensor, B: int, N: int, heads: int, d: int, mask: Optional[torch.Tensor] = None,
               window: int = -1, lse: Optional[torch.Tensor] = None) -> torch.Tensor:
-    """qkv [B*N, 3*heads*d] (q | k | v).  mask [B,N] bool -> sdpa semantics; None -> flash semantics.
+    """qkv [B*N, 3*heads*d] (q | k | v).  mask [B,N] bool -> sdpa semantics (masked query rows read 0); None -> flash semantics.
+    The mask must be a prefix mask (every image's valid tokens first, what patchify emits): a mask with holes raises ValueError
+    (a host check; masked batches with holes run on the packed layout, see ``attention_packed``).
     window >= 0: sliding window |i - j| <= window (flash_attn window_size=(window, window))."""
     D = heads * d
     out = torch.empty(B * N, D, dtype=torch.bfloat16, device=qkv.device)
-    kl = pf = m8 = None
+    kl = None
     if mask is not None:
-        m8 = mask.contiguous().view(torch.uint8)
-        kl, pf = kv_len(mask)
+        m = mask.bool()
+        if not bool((m == (torch.arange(N, device=m.device) < m.sum(dim=1, keepdim=True))).all()):
+            raise ValueError("vitok_b200.attention: the mask must be a prefix mask (valid tokens first in every image)")
+        kl = kv_len(mask)
     base = qkv.data_ptr()
     check(load().vtk_attention_bf16(base, base + 2 * D, base + 4 * D, qkv.stride(0), ptr(out), out.stride(0), ptr(kl),
-                                    ptr(m8), ptr(pf), B, N, heads, d, 1 if mask is not None else 0, int(window), ptr(lse), stream_ptr()))
+                                    B, N, heads, d, 1 if mask is not None else 0, int(window), ptr(lse), stream_ptr()))
     return out
 
 
@@ -432,16 +425,14 @@ def umma_probe(a: torch.Tensor, b: torch.Tensor, n: int, k: int, b_mn_major: boo
 def attention_packed(qkv: torch.Tensor, plan: dict, B: int, N: int, heads: int, d: int, lse: Optional[torch.Tensor] = None,
                      out: Optional[torch.Tensor] = None) -> torch.Tensor:
     """Attention over the packed NaFlex layout of ``pack_plan`` (qkv [row capacity, 3*heads*d]; the plan's qrows must be 128 for
-    d = 64, 256 for d = 128).  Without ``lse`` the pad rows of ``out`` are never written; with ``lse`` ([rows, heads] fp32,
-    vtk_attention_packed_lse_bf16) they are written as 0 and lse as +inf.  ``out`` (optional) = a preallocated [rows, heads*d]."""
+    d = 64, 256 for d = 128).  Without ``lse`` the pad rows of ``out`` are never written; with ``lse`` ([rows, heads] fp32) they
+    are written as 0 and lse as +inf.  ``out`` (optional) = a preallocated [rows, heads*d]."""
     D = heads * d
     if out is None:
         out = torch.empty(qkv.shape[0], D, dtype=torch.bfloat16, device=qkv.device)
     base = qkv.data_ptr()
-    args = (base, base + 2 * D, base + 4 * D, qkv.stride(0), ptr(out), out.stride(0), ptr(plan["n_valid"]), ptr(plan["cu"]), ptr(plan["cuq"]),
-            ptr(plan["grp_img"]), ptr(plan["grp_order"]), B, N, heads, d, qkv.shape[0], plan["grp_img"].numel())
-    if lse is None:
-        check(load().vtk_attention_packed_bf16(*args, stream_ptr()))
-    else:
-        check(load().vtk_attention_packed_lse_bf16(*args, ptr(lse), stream_ptr()))
+    check(load().vtk_attention_packed_lse_bf16(base, base + 2 * D, base + 4 * D, qkv.stride(0), ptr(out), out.stride(0),
+                                               ptr(plan["n_valid"]), ptr(plan["cu"]), ptr(plan["cuq"]), ptr(plan["grp_img"]),
+                                               ptr(plan["grp_order"]), B, N, heads, d, qkv.shape[0], plan["grp_img"].numel(), ptr(lse),
+                                               stream_ptr()))
     return out

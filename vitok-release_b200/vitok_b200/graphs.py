@@ -63,8 +63,7 @@ class GraphedAE:
 
     def _state(self):
         m = self.model
-        return (m._signature(), bool(m.token_packing), bool(m.fuse_norm), bool(m._quantization_applied), m.fp8_activation_scale,
-                m.attn_backend, m.sw)
+        return (m._signature(), bool(m.fuse_norm), bool(m._quantization_applied), m.fp8_activation_scale, m.attn_backend, m.sw)
 
     def _forward(self, d):
         m = self.model
@@ -76,7 +75,7 @@ class GraphedAE:
 
     def __call__(self, batch: Dict[str, torch.Tensor]) -> Dict[str, Optional[torch.Tensor]]:
         if self._state() != self._sig:
-            raise RuntimeError("GraphedAE: the model's parameters or its token_packing / fuse_norm / quantize state changed since "
+            raise RuntimeError("GraphedAE: the model's parameters or its fuse_norm / quantize state changed since "
                                "capture; build a new GraphedAE")
         for k in _STATIC_KEYS:
             src = batch.get(k)

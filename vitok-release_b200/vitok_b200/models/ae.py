@@ -251,9 +251,7 @@ class AE(nn.Module):
         self.last_launch_count = 0
         self._model_id = next(_MODEL_IDS)       # key of this instance for the vitok_b200::ae_run op
         _MODELS[self._model_id] = self
-        # NaFlex token packing for masked (sdpa-backend) batches: only valid tokens go through the layer stack
-        # (include/vitok_b200.h, vtk_ae_set_packing).  False keeps the padded layout with in-kernel key masking.
-        self.token_packing = True
+        # Masked (sdpa-backend) inference batches always run on their packed valid tokens (include/vitok_b200.h: vtk_ae_encode).
         # The same for the training step (train mode, sdpa backend with a patch_mask; vitok_b200/train.py: _Packing): GEMMs, kernels
         # and saved activations cover the valid tokens only.  Off by default: the result differs from the padded step in the order of
         # the weight-gradient sums, and masked tokens of the output are 0.  No effect without a mask or under the flash backend.
@@ -451,7 +449,6 @@ class AE(nn.Module):
         ws_ptr = (ws.data_ptr() + 1023) // 1024 * 1024
         out = torch.empty(B, N, out_cols, dtype=torch.bfloat16, device=x.device)
         fn = lib.vtk_ae_encode if side == 0 else lib.vtk_ae_decode
-        _lib.check(lib.vtk_ae_set_packing(h, 1 if self.token_packing else 0))
         _lib.check(lib.vtk_ae_set_fp8_granularity(h, 1 if self.fp8_activation_scale == "tensor" else 0))
         _lib.check(fn(h, xin.data_ptr(), row.data_ptr(), col.data_ptr(), m8.data_ptr() if m8 is not None else None,
                       B, N, out.data_ptr(), ws_ptr, ws.numel() - (ws_ptr - ws.data_ptr()), _lib.stream_ptr()))

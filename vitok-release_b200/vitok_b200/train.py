@@ -256,7 +256,7 @@ class _Packing:
         return keep[self._row_img].contiguous()
 
 
-def _block_forward(lib, blk, x: torch.Tensor, rope, kv, pf, m8, B: int, N: int, dims, window: int, keep, keep_prob: float,
+def _block_forward(lib, blk, x: torch.Tensor, rope, kv, B: int, N: int, dims, window: int, keep, keep_prob: float,
                    pk: Optional[_Packing] = None):
     """One transformer block (ae.py:55-65) with everything the backward needs: returns (x_new, (h, zraw, qkv, a2, lse, y)).
     ``pk``: the packed layout (M = pk.M rows; ``keep`` then holds one entry per row)."""
@@ -280,9 +280,8 @@ def _block_forward(lib, blk, x: torch.Tensor, rope, kv, pf, m8, B: int, N: int, 
     lse = torch.empty(M, heads, dtype=torch.float32, device=dev)
     base = qkv.data_ptr()
     if pk is None:
-        _check(lib.vtk_attention_bf16(base, base + 2 * D, base + 4 * D, 3 * D, a2.data_ptr(), kp, _lib.ptr(kv),
-                                      _lib.ptr(m8), _lib.ptr(pf), B, N, heads, d, 1 if m8 is not None else 0, window,
-                                      lse.data_ptr(), st))
+        _check(lib.vtk_attention_bf16(base, base + 2 * D, base + 4 * D, 3 * D, a2.data_ptr(), kp, _lib.ptr(kv), B, N, heads, d,
+                                      1 if kv is not None else 0, window, lse.data_ptr(), st))
     else:
         qrows = 128 if d == 64 else 256
         pl = pk.attn_plan(qrows)
@@ -297,7 +296,7 @@ def _block_forward(lib, blk, x: torch.Tensor, rope, kv, pf, m8, B: int, N: int, 
     return x_new, (h, zraw, qkv, a2, lse, y)
 
 
-def _side_forward(lib, model, sw: _SideWeights, side: int, xin: torch.Tensor, row, col, m8, B: int, N: int, saved: Dict,
+def _side_forward(lib, model, sw: _SideWeights, side: int, xin: torch.Tensor, row, col, kv, window: int, B: int, N: int, saved: Dict,
                   pk: Optional[_Packing] = None):
     width = model.encoder_width if side == 0 else model.decoder_width
     heads = model.encoder_heads if side == 0 else model.decoder_heads
@@ -313,14 +312,11 @@ def _side_forward(lib, model, sw: _SideWeights, side: int, xin: torch.Tensor, ro
     dev = xin.device
     cin = xin.shape[-1]
     x = _linear(xin, cin, sw.wa, sw.ba, M, D, cin)
-    rope = kv = pf = None
+    rope = None
     if sw.blocks:
         inv = (1.0 / (model.rope_theta ** (torch.arange(0, d // 2, 2).float() / (d // 2)))).to(dev)
         rope = torch.zeros((M + 31) // 32 * 32, 2 * d, dtype=BF, device=dev)
         _check(lib.vtk_rope_table(row.data_ptr(), col.data_ptr(), inv.data_ptr(), rope.data_ptr(), M, d, st))
-        if m8 is not None and pk is None:
-            kv, pf = _lib.kv_len(m8.view(B, N))     # train_forward has made every mask a prefix mask
-    window = int(model.sw) if (model.sw and m8 is None) else -1
     ck = int(getattr(model, "checkpoint", 0) or 0)
     layers = []
     for li, blk in enumerate(sw.blocks):
@@ -333,11 +329,11 @@ def _side_forward(lib, model, sw: _SideWeights, side: int, xin: torch.Tensor, ro
             keep = (keep_prob + torch.rand((B, 1, 1), dtype=BF, device=dev)).floor_().float().reshape(B).contiguous()
             if pk is not None:
                 keep = pk.per_row(keep)
-        x_new, inner = _block_forward(lib, blk, x, rope, kv, pf, m8, B, N, dims, window, keep, keep_prob, pk)
+        x_new, inner = _block_forward(lib, blk, x, rope, kv, B, N, dims, window, keep, keep_prob, pk)
         # activation checkpointing (ae.py:159-160): block i with i % checkpoint == 0 keeps its input only
         layers.append((x, None if (ck > 0 and li % ck == 0) else inner, keep, keep_prob))
         x = x_new
-    saved.update(dict(layers=layers, x_final=x, rope=rope, kv=kv, pf=pf, m8=m8, window=window, xin=xin, dims=dims, pk=pk))
+    saved.update(dict(layers=layers, x_final=x, rope=rope, kv=kv, window=window, xin=xin, dims=dims, pk=pk))
     return x
 
 
@@ -354,7 +350,7 @@ def _side_backward(lib, model, sw: _SideWeights, side: int, dx: torch.Tensor, sa
         wqkv, w1, w_o, w_2, n1, nq, nk, gamma = sw.blocks[li]
         x, inner, keep, keep_prob = saved["layers"][li]
         if inner is None:      # checkpointed block: re-run its forward from x (same stochastic-depth draw)
-            _, inner = _block_forward(lib, sw.blocks[li], x, rope, kv, saved["pf"], saved["m8"], B, N, dims, window, keep, keep_prob, pk)
+            _, inner = _block_forward(lib, sw.blocks[li], x, rope, kv, B, N, dims, window, keep, keep_prob, pk)
         h, zraw, qkv, a2, lse, y = inner
         saved["layers"][li] = None                                                 # free this block's activations as we go
         dy = torch.empty(M, D, dtype=BF, device=dev)
@@ -438,17 +434,20 @@ class AETrainFunction(torch.autograd.Function):
         enc_w, dec_w = _SideWeights(model, 0), _SideWeights(model, 1)
         row = row.to(device=dev, dtype=torch.int64).contiguous()
         col = col.to(device=dev, dtype=torch.int64).contiguous()
-        m8 = mask.to(dev).bool().contiguous().view(torch.uint8) if mask is not None else None
+        # padded step: each image's key length (train_forward has made every mask a prefix mask); the packed step's attention
+        # reads the lengths from its plan.  The sdpa backend (a mask given) ignores the sliding window.
+        kv = _lib.kv_len(mask.to(dev).bool()) if mask is not None and pk is None else None
+        window = int(model.sw) if (model.sw and mask is None) else -1
         xin = (_lib.cast_to_bf16(patches) if patches.dtype == torch.float32 else patches).contiguous().view(B * N, P)
         M, C = B * N, model.channels_per_token
         if pk is not None:
             xin, row, col, M = pk.pack(xin), pk.pack_index(row), pk.pack_index(col), pk.M
         s_enc, s_dec = {}, {}
-        x = _side_forward(lib, model, enc_w, 0, xin, row, col, m8, B, N, s_enc, pk)
+        x = _side_forward(lib, model, enc_w, 0, xin, row, col, kv, window, B, N, s_enc, pk)
         zlin = _linear(x, x.shape[1], enc_w.wb, enc_w.bb, M, C, x.shape[1])
         z = torch.empty(M, C, dtype=BF, device=dev)
         _check(lib.vtk_layernorm_fwd(zlin.data_ptr(), z.data_ptr(), M, C, 1e-6, _lib.stream_ptr()))
-        xd = _side_forward(lib, model, dec_w, 1, z, row, col, m8, B, N, s_dec, pk)
+        xd = _side_forward(lib, model, dec_w, 1, z, row, col, kv, window, B, N, s_dec, pk)
         out = _linear(xd, xd.shape[1], dec_w.wb, dec_w.bb, M, P, xd.shape[1])
         # activations live on ctx (not save_for_backward: they are workspace of the backward kernels, freed block by block while it
         # runs); a second backward through the same graph is therefore refused with a clear error in backward()
