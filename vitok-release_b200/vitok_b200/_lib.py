@@ -133,7 +133,8 @@ def load() -> ctypes.CDLL:
 
 
 def set_flag(name: str, value: int) -> None:
-    """Process-wide kernel switch (include/vitok_b200.h: vtk_set_flag): "pdl", "gemm_splitk"."""
+    """Process-wide kernel switch (include/vitok_b200.h: vtk_set_flag): "pdl", "gemm_splitk", "reserve_sms" (the persistent
+    kernels -- GEMMs and d = 64 attention -- size their grids for that many SMs fewer)."""
     check(load().vtk_set_flag(name.encode(), int(value)))
 
 
