@@ -31,7 +31,8 @@ typedef enum {
   VTK_OK = 0,
   VTK_ERR_CUDA = -1,        /* CUDA runtime / driver error, text in vtk_last_error()          -> RuntimeError */
   VTK_ERR_BAD_ARG = -2,     /* shape / alignment / null-pointer violation                      -> ValueError   */
-  VTK_ERR_UNSUPPORTED = -3  /* valid in the reference but not implemented here (e.g. head_dim) -> NotImplementedError */
+  VTK_ERR_UNSUPPORTED = -3  /* valid in the reference but not implemented here (e.g. a head_dim outside d % 8 == 0, 8 <= d <= 128)
+                               -> NotImplementedError */
 } vtk_status;
 
 const char* vtk_last_error(void);
@@ -171,7 +172,9 @@ int vtk_linear_ln_bf16(const void* A, int64_t lda, const void* W, int64_t ldw, c
 /* Fused first half of Block.forward after norm1 (vitok/models/ae.py:61-63):
  *   qkv_proj -> norm_q/norm_k -> 2-D RoPE (modules/attention.py:95-107) and fc1 -> silu(g)*v (modules/mlp.py:21-22).
  * Wp [w_rows, K=D] is the packed weight [Wq; Wk; Wv; 0-pad to qp; interleave16(W1_v, W1_g)]; qp = 3D rounded up to 256.
- * qkv [M,3D] receives roped q, roped k, v; act [M,Hf] receives silu(g)*v. */
+ * qkv [M,3D] receives roped q, roped k, v; act [M,Hf] receives silu(g)*v.  head_dim d: d % 8 == 0, 8 <= d <= 128.  At d = 32, 64 and
+ * 128 the GEMM epilogue normalises and ropes q / k; at the other d it writes them raw and vtk_qk_norm_rope_fwd runs in place on
+ * qkv after the GEMM, on the same stream (same rounding points). */
 int vtk_qkv_swiglu_bf16(const void* h, int64_t ldh, const void* Wp, int64_t ldw, int64_t w_rows, int M, int D, int d,
                         int Hf, int qp, const void* norm_q, const void* norm_k, const void* rope_table, float eps,
                         void* qkv, int64_t ld_qkv, void* act, int64_t ld_act, void* stream);
@@ -188,12 +191,14 @@ int vtk_proj_residual_bf16(const void* A, int64_t lda, const void* W, int64_t ld
  * window >= 0: sliding-window attention, query i sees keys j with |i - j| <= window on the token index, i.e.
  * flash_attn_func(window_size=(window, window)) as called at modules/attention.py:113-116; window < 0 = full.
  * lse (optional, may be null): [B*N, heads] fp32, log2-domain logsumexp of the scaled scores (+inf for zeroed rows);
- * the training backward (vtk_attention_bwd_bf16) consumes it. */
+ * the training backward (vtk_attention_bwd_bf16) consumes it.
+ * head_dim d: d % 8 == 0 and 8 <= d <= 128 (else VTK_ERR_UNSUPPORTED).  d <= 64 runs on the d = 64 kernel, 64 < d <= 128 on the
+ * d = 128 one; only the d columns of each head are read and written.  Row strides and q / k / v / out: multiples of 8 elements. */
 int vtk_attention_bf16(const void* q, const void* k, const void* v, int64_t ld_qkv, void* out, int64_t ld_out,
                        const int* kv_len, int B, int N, int heads, int d, int zero_invalid_rows, int window, float* lse, void* stream);
 /* The same on the packed NaFlex layout of vtk_pack_plan (the form the layer stack runs masked batches in): image b owns packed rows
- * [cu[b], cu[b+1]) with its n_valid[b] tokens in front; q / k / v / out have row_cap rows.  qrows of the plan must be 128 (d = 64)
- * or 256 (d = 128).  For image b it writes packed rows [cu[b], cu[b+1]) only, and rows below n_valid[b] get out as
+ * [cu[b], cu[b+1]) with its n_valid[b] tokens in front; q / k / v / out have row_cap rows.  qrows of the plan must be 128 (d <= 64)
+ * or 256 (64 < d <= 128).  For image b it writes packed rows [cu[b], cu[b+1]) only, and rows below n_valid[b] get out as
  * vtk_attention_bf16 with kv_len = n_valid.  Rows of other images -- the rest of a partial last tile -- are not touched.
  * lse (optional, may be null; the training step on packed rows, vitok/models/modules/attention.py:118-127 under autograd):
  * [row_cap, heads] fp32.  With lse, the image's pad rows [cu[b] + n_valid[b], cu[b+1]) get out = 0 and lse = +inf; without it,
@@ -220,7 +225,8 @@ int vtk_linear2_bf16(const void* A, int64_t lda, const void* W0, int64_t ldw0, c
  * below.  All tensors bf16 unless noted; gradient accumulators of norm weights / gamma / biases are fp32 and ADDED to (zero
  * them first).
  * ---------------------------------------------------------------------------------------------- */
-/* zraw [M, >=3D] raw q|k|v -> qkv [M,3D]: QK-RMSNorm over d + 2D RoPE, v copied (modules/attention.py:95-107) */
+/* zraw [M, >=3D] raw q|k|v -> qkv [M,3D]: QK-RMSNorm over d + 2D RoPE, v copied (modules/attention.py:95-107).
+ * d % 8 == 0, 8 <= d <= 128.  qkv == zraw (with ld_qkv == ldz) runs in place and leaves v as it is. */
 int vtk_qk_norm_rope_fwd(const void* zraw, int64_t ldz, const void* norm_q, const void* norm_k, const void* rope_table,
                          void* qkv, int64_t ld_qkv, int M, int heads, int d, float eps, void* stream);
 /* zraw[:, qp:] (16-col groups value|gate, the packed fc1 order) -> act [M,Hf] = silu(g) * v (modules/mlp.py:21-22) */
@@ -243,7 +249,8 @@ int vtk_colsum(const void* in, int64_t ld, float* out, int M, int C, void* strea
 /* d_act [M,Hf] + zraw -> dz[:, qp:] in the packed (value|gate) order */
 int vtk_swiglu_bwd(const void* dact, int64_t ldd, const void* zraw, int64_t ldz, int qp, void* dz, int64_t lddz, int M, int Hf, int layout,
                    void* stream);
-/* in place on dz[:, 0:2D] (dq|dk w.r.t. roped q/k) -> gradient w.r.t. raw q/k; dw [2][d] fp32 += norm_q / norm_k grads */
+/* in place on dz[:, 0:2D] (dq|dk w.r.t. roped q/k) -> gradient w.r.t. raw q/k; dw [2][d] fp32 += norm_q / norm_k grads;
+ * d % 8 == 0, 8 <= d <= 128 */
 int vtk_qk_norm_rope_bwd(void* dz, int64_t lddz, const void* zraw, int64_t ldz, const void* norm_q, const void* norm_k,
                          const void* rope_table, float* dw, int M, int heads, int d, float eps, void* stream);
 /* dx_out = dx_res + RMSNorm'(x; w)^T dh; dw[D] += colsum(dh * xhat) */
@@ -266,15 +273,16 @@ int vtk_adamw_multi(const vtk_adamw_tensor* tensors, int n_tensors, float lr, fl
                     float grad_scale, void* stream);
 /* x [n] bf16 *= *scale (fp32 scalar in device memory): the loss gradient arriving at vtk_charbonnier's dpred */
 int vtk_scale_by_dev(void* x, const float* scale, int64_t n, void* stream);
-/* delta [M, heads] fp32 = rowsum over d of dO * O */
+/* delta [M, heads] fp32 = rowsum over d of dO * O; d % 8 == 0, 8 <= d <= 128 */
 int vtk_attn_delta(const void* o, int64_t ldo, const void* dout, int64_t lddo, float* delta, int M, int heads, int d, void* stream);
-/* attention backward: dq, dk, dv (row stride ld_d) from q,k,v,dO, lse (from vtk_attention_bf16) and delta */
+/* attention backward: dq, dk, dv (row stride ld_d) from q,k,v,dO, lse (from vtk_attention_bf16) and delta; the head dims of
+ * vtk_attention_bf16, only the d columns of each head written */
 int vtk_attention_bwd_bf16(const void* q, const void* k, const void* v, int64_t ld_qkv, const void* dout, int64_t ld_do,
                            const float* lse, const float* delta, void* dq, void* dk, void* dv, int64_t ld_d, const int* kv_len,
                            int B, int N, int heads, int d, int zero_invalid_rows, int window, void* stream);
-/* The same on the packed NaFlex layout (autograd of modules/attention.py:118-127 for the packed training step), d = 64 or 128:
+/* The same on the packed NaFlex layout (autograd of modules/attention.py:118-127 for the packed training step), same head dims:
  * lse from vtk_attention_packed_lse_bf16, delta [row_cap, heads] from vtk_attn_delta over the packed rows.  The plan must have
- * qrows = 128 for both head dims (the d = 128 forward's plan has qrows = 256: a second plan of the same mask, whose n_valid / cu
+ * qrows = 128 at every head dim (the forward's plan at 64 < d <= 128 has qrows = 256: a second plan of the same mask, whose n_valid / cu
  * are the same).  Two passes, each one CTA per (128-row group, head) taken in grp_order: dK/dV per key tile, then dQ per query
  * tile; grp_cap (>= cuq[B], CTAs beyond cuq[B] exit) sizes the grid.  For image b it writes dq / dk / dv rows [cu[b], cu[b+1])
  * only: gradients for rows below n_valid[b], zeros for the image's pad rows; rows of other images are not touched.  Query rows

@@ -140,6 +140,24 @@ int encode_tmap_bf16_sw128(CUtensorMap* out, const void* base, uint64_t inner_el
   return encode_tmap_bf16(out, base, inner_elems, rows, row_stride_elems, 64, box_rows, 128);
 }
 
+int encode_tmap_heads(CUtensorMap* out, const void* base, int d, int heads, uint64_t rows, uint64_t row_stride_elems, uint32_t box_rows) {
+  EncodeTiledFn fn = get_encode_fn();
+  if (!fn) return VTK_ERR_CUDA;
+  cuuint64_t gdim[3] = {(cuuint64_t)d, (cuuint64_t)heads, rows};
+  cuuint64_t gstride[2] = {(cuuint64_t)d * 2, row_stride_elems * 2};
+  cuuint32_t box[3] = {64, 1, box_rows};
+  cuuint32_t estr[3] = {1, 1, 1};
+  CUresult r = fn(out, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 3, const_cast<void*>(base), gdim, gstride, box, estr,
+                  CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
+                  CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+  if (r != CUDA_SUCCESS) {
+    set_error("cuTensorMapEncodeTiled(heads) failed (CUresult %d) base=%p d=%d heads=%d rows=%llu stride=%llu box_rows=%u", (int)r,
+              base, d, heads, (unsigned long long)rows, (unsigned long long)row_stride_elems, box_rows);
+    return VTK_ERR_CUDA;
+  }
+  return 0;
+}
+
 // -------------------------------------------------------------------------------------------------
 // AE handle
 // -------------------------------------------------------------------------------------------------
@@ -179,7 +197,7 @@ static Workspace carve(const Side& s, void* base, int B, int N, int io_cols) {
     off += align_up(nbytes, 1024);
     return p;
   };
-  const int qrows = s.head_dim() == 128 ? 256 : 128;      // query rows per attention work group
+  const int qrows = head_tile(s.head_dim()) == 128 ? 256 : 128;   // query rows per attention work group
   const long long M = PackPlan::row_capacity(B, N, 16);   // >= B * N, so it also holds the padded (un-packed) layout
   const long long G = PackPlan::group_capacity(B, N, qrows);
   const long long D = s.width, d = s.head_dim();
@@ -456,7 +474,10 @@ int vtk_qkv_swiglu_bf16(const void* h, int64_t ldh, const void* Wp, int64_t ldw,
   g.epi.qkv = (bf16*)qkv; g.epi.ld_qkv = ld_qkv; g.epi.act = (bf16*)act; g.epi.ld_act = ld_act;
   g.epi.normq = (const bf16*)norm_q; g.epi.normk = (const bf16*)norm_k; g.epi.rope = (const bf16*)rope_table;
   g.epi.D = D; g.epi.d = d; g.epi.Hf = Hf; g.epi.qp = qp; g.epi.eps = eps;
-  return launch_gemm(EPI_QKV_SWIGLU, g, (cudaStream_t)stream);
+  int r = launch_gemm(EPI_QKV_SWIGLU, g, (cudaStream_t)stream);
+  if (r || qk_norm_fused(d)) return r;
+  return launch_qk_norm_rope_fwd((const bf16*)qkv, ld_qkv, (const bf16*)norm_q, (const bf16*)norm_k, (const bf16*)rope_table, (bf16*)qkv,
+                                 ld_qkv, M, D / d, d, eps, (cudaStream_t)stream);
 }
 
 int vtk_proj_residual_bf16(const void* A, int64_t lda, const void* W, int64_t ldw, const void* gamma, void* x,
@@ -644,8 +665,8 @@ int vtk_ae_create(const vtk_ae_config* cfg, vtk_ae_t* out) {
       return VTK_ERR_BAD_ARG;
     }
     const int hd = sd.head_dim();
-    if (sd.depth > 0 && !(hd == 64 || hd == 128)) {
-      set_error("vtk_ae_create: head_dim %d unsupported by the sm_100a attention kernel (64 or 128)", hd);
+    if (sd.depth > 0 && !head_dim_supported(hd)) {
+      set_error("vtk_ae_create: head_dim %d unsupported by the sm_100a attention kernels (supported: multiples of 8 from 8 to 128)", hd);
       delete h;
       return VTK_ERR_UNSUPPORTED;
     }
@@ -736,6 +757,12 @@ static int run_blocks(vtk_ae_s* h, const Side& s, const Workspace& w, const int6
     g1.epi.m_dev = m_dev;
     { LaunchTimer t(h, st, CLS_QKV_SWIGLU); r = launch_gemm(EPI_QKV_SWIGLU, g1, st); }
     if (r) return r;
+    if (!qk_norm_fused(d)) {   // the epilogue copied q and k raw: QK-norm + RoPE in place on the qkv rows
+      LaunchTimer t(h, st, CLS_MISC);
+      r = launch_qk_norm_rope_fwd(w.qkv, 3 * D, (const bf16*)b.norm_q, (const bf16*)b.norm_k, w.rope, w.qkv, 3 * D, M, s.heads, d, eps, st);
+      if (r) return r;
+      ++launches;
+    }
     AttnArgs a;
     a.q = w.qkv; a.k = w.qkv + D; a.v = w.qkv + 2 * D; a.ld_qkv = 3 * D; a.out = w.a2; a.ld_out = kp;
     a.B = B; a.N = N; a.heads = s.heads; a.d = d;

@@ -19,6 +19,9 @@
 // TMEM only when its running max moved by more than 2^8 (lazy rescale; the stale max cancels in O / l).
 // While warpgroup A exponentiates, the tensor core works for B and vice versa.
 // V is consumed as an MN-major B operand straight from its [key, d] layout (no transpose pass).
+// Head dims: any d % 8 == 0 up to 128 runs on the kernel of the next tile width DH (d <= 64: the persistent d = 64 kernel, else the
+// d = 128 one).  Q / K / V / O move through 3-D tensor maps {d, heads, rows}, so the tile columns d..DH-1 load as zeros (they add
+// nothing to S or to P V) and only the head's d columns are stored.
 #include <math.h>
 #include <stdio.h>
 #include <stdlib.h>
@@ -60,7 +63,7 @@ template <int DH, int NQ> struct AttnShape {
 struct AttnParams {
   bf16* out; long long ld_out;
   const int* kv_len;
-  int N, heads, zero_invalid, tma_out;
+  int N, heads, d, zero_invalid, tma_out;   // d = the true head width (<= DH; columns d..DH-1 of a tile are TMA zero fill)
   int window;         // sliding window |i - j| <= window on the token index (flash backend, attention.py:113-116); < 0 = none
   float scale_log2;   // (1/sqrt(d)) * log2(e)
   unsigned long long* prof;   // perf experiments (env VTK_ATTN_PROF): clock64 accumulators, or null
@@ -228,8 +231,8 @@ attn_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__ CUt
     if (wg >= nact) {
       const int qi = q0 + wg * ATT_BQ + (warp & 3) * 32 + lane;
       if (qi < N) {
-        bf16* op = p.out + (row0 + qi) * p.ld_out + head * DH;
-        for (int c = 0; c < DH; c += 8) st_global_v4(op + c, 0u, 0u, 0u, 0u);
+        bf16* op = p.out + (row0 + qi) * p.ld_out + head * p.d;
+        for (int c = 0; c < p.d; c += 8) st_global_v4(op + c, 0u, 0u, 0u, 0u);
         if (p.lse) p.lse[(row0 + qi) * p.heads + head] = INFINITY;
       }
     }
@@ -286,10 +289,10 @@ attn_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__ CUt
     mbar_expect_tx(q_full, (uint32_t)(nact * S::TILE_BYTES));
     for (int t = 0; t < nact; ++t)
       for (int nb = 0; nb < S::NB; ++nb)
-        tma_load_2d(sQ + t * S::TILE_BYTES + nb * BLK, &tmQ, q_full, head * DH + nb * 64, (int)(row0 + q0 + t * ATT_BQ));
+        tma_load_3d(sQ + t * S::TILE_BYTES + nb * BLK, &tmQ, q_full, nb * 64, head, (int)(row0 + q0 + t * ATT_BQ));
     mbar_expect_tx(&k_full[0], S::TILE_BYTES);
     for (int nb = 0; nb < S::NB; ++nb)
-      tma_load_2d(sK + nb * BLK, &tmK, &k_full[0], head * DH + nb * 64, (int)(row0 + (long long)j_lo * ATT_BKV));
+      tma_load_3d(sK + nb * BLK, &tmK, &k_full[0], nb * 64, head, (int)(row0 + (long long)j_lo * ATT_BKV));
   }
   tc_fence_before();
   __syncthreads();
@@ -306,7 +309,7 @@ attn_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__ CUt
         mbar_wait(&k_empty[slot], ((uint32_t)(jj / S::RK) & 1u) ^ 1u);
         mbar_expect_tx(&k_full[slot], S::TILE_BYTES);
         for (int nb = 0; nb < S::NB; ++nb)
-          tma_load_2d(sK + slot * S::TILE_BYTES + nb * BLK, &tmK, &k_full[slot], head * DH + nb * 64,
+          tma_load_3d(sK + slot * S::TILE_BYTES + nb * BLK, &tmK, &k_full[slot], nb * 64, head,
                       (int)(row0 + (long long)(j_lo + jj) * ATT_BKV));
       };
       for (int jj = 0; jj < Tn; ++jj) {
@@ -315,7 +318,7 @@ attn_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__ CUt
         mbar_wait(&v_empty[slot], ((uint32_t)(jj / S::RV) & 1u) ^ 1u);
         mbar_expect_tx(&v_full[slot], S::TILE_BYTES);
         for (int nb = 0; nb < S::NB; ++nb)
-          tma_load_2d(sV + slot * S::TILE_BYTES + nb * BLK, &tmV, &v_full[slot], head * DH + nb * 64,
+          tma_load_3d(sV + slot * S::TILE_BYTES + nb * BLK, &tmV, &v_full[slot], nb * 64, head,
                       (int)(row0 + (long long)(j_lo + jj) * ATT_BKV));
       }
     }
@@ -473,7 +476,7 @@ attn_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__ CUt
     const bool zero_row = p.zero_invalid && qi >= kvlen;
     const float osc = zero_row ? 0.f : inv;
     if (p.lse && qi < N) p.lse[(row0 + qi) * p.heads + head] = (zero_row || !(l_run > 0.f)) ? INFINITY : m_run + log2f(l_run);
-    bf16* op = p.out + (row0 + qi) * p.ld_out + head * DH;
+    bf16* op = p.out + (row0 + qi) * p.ld_out + head * p.d;
     uint32_t o[DH / 32][32];
 #pragma unroll
     for (int c = 0; c < DH / 32; ++c) tmem_ld32(tO + c * 32, o[c]);
@@ -499,7 +502,7 @@ attn_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__ CUt
       if (lane == 0) {
 #pragma unroll
         for (int nb = 0; nb < S::NB; ++nb)
-          tma_store_2d(&tmO, sQ + q * S::TILE_BYTES + nb * BLK + quarter * 32 * 128, head * DH + nb * 64,
+          tma_store_3d(&tmO, sQ + q * S::TILE_BYTES + nb * BLK + quarter * 32 * 128, nb * 64, head,
                        (int)(row0 + q0 + q * ATT_BQ + quarter * 32));
         tma_store_commit();
         tma_store_wait_read();
@@ -509,6 +512,7 @@ attn_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__ CUt
       for (int c = 0; c < DH / 32; ++c)
 #pragma unroll
         for (int g = 0; g < 4; ++g) {
+          if (c * 32 + 8 * g >= p.d) break;   // the tile's zero columns past the head width
           uint32_t w[4];
 #pragma unroll
           for (int i = 0; i < 4; ++i)
@@ -673,13 +677,13 @@ attn_persist_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_consta
         const long long row0 = it.row0;
         if (n_item > 0) mbar_wait(q_empty, (n_item - 1) & 1u);     // last S MMA of the previous item has read Q
         mbar_expect_tx(q_full, S::TILE_BYTES);
-        tma_load_2d(sQ, &tmQ, q_full, it.head * DH, (int)(row0 + it.q0));
+        tma_load_3d(sQ, &tmQ, q_full, 0, it.head, (int)(row0 + it.q0));
         ++n_item;
         auto load_k = [&](int jj) {
           const uint32_t slot = n_k % S::RK;
           mbar_wait(&k_empty[slot], ((n_k / S::RK) & 1u) ^ 1u);
           mbar_expect_tx(&k_full[slot], S::TILE_BYTES);
-          tma_load_2d(sK + slot * S::TILE_BYTES, &tmK, &k_full[slot], it.head * DH, (int)(row0 + (long long)(it.j_lo + jj) * ATT_BKV));
+          tma_load_3d(sK + slot * S::TILE_BYTES, &tmK, &k_full[slot], 0, it.head, (int)(row0 + (long long)(it.j_lo + jj) * ATT_BKV));
           ++n_k;
         };
         load_k(0);
@@ -688,7 +692,7 @@ attn_persist_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_consta
           const uint32_t slot = n_v % S::RV;
           mbar_wait(&v_empty[slot], ((n_v / S::RV) & 1u) ^ 1u);
           mbar_expect_tx(&v_full[slot], S::TILE_BYTES);
-          tma_load_2d(sV + slot * S::TILE_BYTES, &tmV, &v_full[slot], it.head * DH, (int)(row0 + (long long)(it.j_lo + jj) * ATT_BKV));
+          tma_load_3d(sV + slot * S::TILE_BYTES, &tmV, &v_full[slot], 0, it.head, (int)(row0 + (long long)(it.j_lo + jj) * ATT_BKV));
           ++n_v;
         }
       }
@@ -765,8 +769,8 @@ attn_persist_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_consta
       const int qi = it.q0 + r;
       if (!it.active) {   // nothing to attend to: the output rows are 0
         if (qi < N) {
-          bf16* op = p.out + (row0 + qi) * p.ld_out + it.head * DH;
-          for (int c = 0; c < DH; c += 8) st_global_v4(op + c, 0u, 0u, 0u, 0u);
+          bf16* op = p.out + (row0 + qi) * p.ld_out + it.head * p.d;
+          for (int c = 0; c < p.d; c += 8) st_global_v4(op + c, 0u, 0u, 0u, 0u);
           if (p.lse) p.lse[(row0 + qi) * p.heads + it.head] = INFINITY;
         }
         continue;
@@ -881,12 +885,12 @@ attn_persist_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_consta
         fence_proxy_async_smem();
         __syncwarp();
         if (lane == 0) {
-          tma_store_2d(&tmO, sP + quarter * 32 * 128, it.head * DH, (int)(row0 + it.q0 + quarter * 32));
+          tma_store_3d(&tmO, sP + quarter * 32 * 128, 0, it.head, (int)(row0 + it.q0 + quarter * 32));
           tma_store_commit();
         }
         store_pending = true;
       } else if (qi < N) {
-        bf16* op = p.out + (row0 + qi) * p.ld_out + it.head * DH;
+        bf16* op = p.out + (row0 + qi) * p.ld_out + it.head * p.d;
 #pragma unroll
         for (int c = 0; c < DH / 32; ++c)
 #pragma unroll
@@ -895,7 +899,7 @@ attn_persist_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_consta
 #pragma unroll
             for (int i = 0; i < 4; ++i)
               wv[i] = bf2_cvt(__uint_as_float(o[c][8 * g + 2 * i]) * osc, __uint_as_float(o[c][8 * g + 2 * i + 1]) * osc);
-            st_global_v4(op + c * 32 + 8 * g, wv[0], wv[1], wv[2], wv[3]);
+            if (c * 32 + 8 * g < p.d) st_global_v4(op + c * 32 + 8 * g, wv[0], wv[1], wv[2], wv[3]);   // not the zero columns past d
           }
       }
       if (prof) { c_epi_wait += e1 - e0; c_epi += clock64() - e1; }
@@ -921,24 +925,29 @@ attn_persist_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_consta
   }
 }
 
+// Q / K / V / O of every kernel: one head per map coordinate, so a head narrower than the kernel's tile width (d < DH) loads its
+// pad columns as zeros -- they add nothing to S = Q K^T or to P V -- and stores only its own d columns.
+static int encode_attn_maps(const AttnArgs& a, long long Mrows, CUtensorMap* tmQ, CUtensorMap* tmK, CUtensorMap* tmV, CUtensorMap* tmO) {
+  if (encode_tmap_heads(tmQ, a.q, a.d, a.heads, Mrows, a.ld_qkv, ATT_BQ)) return -1;
+  if (encode_tmap_heads(tmK, a.k, a.d, a.heads, Mrows, a.ld_qkv, ATT_BKV)) return -1;
+  if (encode_tmap_heads(tmV, a.v, a.d, a.heads, Mrows, a.ld_qkv, ATT_BKV)) return -1;
+  return encode_tmap_heads(tmO, a.out, a.d, a.heads, Mrows, a.ld_out, 32);
+}
+
 static int launch_attention_persist(const AttnArgs& a, cudaStream_t stream) {
   using S = AttnShape<64, 1>;
   const bool packed = a.cu != nullptr;
   const long long Mrows = packed ? a.row_cap : (long long)a.B * a.N;
-  const long long cols = (long long)a.heads * a.d;
   if (packed && (!a.cuq || !a.grp_img || !a.grp_order || !a.kv_len || a.window >= 0 || a.row_cap <= 0 || a.grp_cap <= 0)) {
     set_error("attention: packed layout needs cu/cuq/grp_img/grp_order/kv_len, row and group capacities and no window");
     return -2;
   }
   CUtensorMap tmQ, tmK, tmV, tmO;
-  if (encode_tmap_bf16_sw128(&tmQ, a.q, cols, Mrows, a.ld_qkv, ATT_BQ)) return -1;
-  if (encode_tmap_bf16_sw128(&tmK, a.k, cols, Mrows, a.ld_qkv, ATT_BKV)) return -1;
-  if (encode_tmap_bf16_sw128(&tmV, a.v, cols, Mrows, a.ld_qkv, ATT_BKV)) return -1;
-  if (encode_tmap_bf16(&tmO, a.out, cols, Mrows, a.ld_out, 64, 32, 128)) return -1;
+  if (encode_attn_maps(a, Mrows, &tmQ, &tmK, &tmV, &tmO)) return -1;
   AttnParams p;
   p.out = a.out; p.ld_out = a.ld_out;
   p.kv_len = a.kv_len;
-  p.N = a.N; p.heads = a.heads; p.zero_invalid = a.zero_invalid_rows;
+  p.N = a.N; p.heads = a.heads; p.d = a.d; p.zero_invalid = a.zero_invalid_rows;
   p.tma_out = (packed || a.N % ATT_BQ == 0) ? 1 : 0;
   p.window = a.window;
   p.lse = a.lse;
@@ -983,17 +992,12 @@ static int launch_attention_t(const AttnArgs& a, cudaStream_t stream) {
     return -2;
   }
   const long long Mrows = packed ? a.row_cap : (long long)a.B * a.N;
-  const long long cols = (long long)a.heads * a.d;
-  CUtensorMap tmQ, tmK, tmV;
-  if (encode_tmap_bf16_sw128(&tmQ, a.q, cols, Mrows, a.ld_qkv, ATT_BQ)) return -1;
-  if (encode_tmap_bf16_sw128(&tmK, a.k, cols, Mrows, a.ld_qkv, ATT_BKV)) return -1;
-  if (encode_tmap_bf16_sw128(&tmV, a.v, cols, Mrows, a.ld_qkv, ATT_BKV)) return -1;
-  CUtensorMap tmO;
-  if (encode_tmap_bf16(&tmO, a.out, cols, Mrows, a.ld_out, 64, 32, 128)) return -1;
+  CUtensorMap tmQ, tmK, tmV, tmO;
+  if (encode_attn_maps(a, Mrows, &tmQ, &tmK, &tmV, &tmO)) return -1;
   AttnParams p;
   p.out = a.out; p.ld_out = a.ld_out;
   p.kv_len = a.kv_len;
-  p.N = a.N; p.heads = a.heads; p.zero_invalid = a.zero_invalid_rows;
+  p.N = a.N; p.heads = a.heads; p.d = a.d; p.zero_invalid = a.zero_invalid_rows;
   p.tma_out = (packed || a.N % ATT_BQ == 0) ? 1 : 0;
   p.window = a.window;
   p.lse = a.lse;
@@ -1028,11 +1032,12 @@ static int launch_attention_t(const AttnArgs& a, cudaStream_t stream) {
 int launch_attention(const AttnArgs& a, cudaStream_t stream) {
   if (a.B <= 0 || a.N <= 0 || a.heads <= 0) { set_error("attention: empty problem"); return -2; }
   if ((a.ld_qkv % 8) || (a.ld_out % 8)) { set_error("attention: row strides must be multiples of 8"); return -2; }
-  if (a.cu && a.d != 64 && a.d != 128) { set_error("attention: the packed layout is implemented for head_dim 64 and 128"); return -3; }
-  if (a.d == 64) return launch_attention_persist(a, stream);
-  if (a.d == 128) return launch_attention_t<128, 2>(a, stream);
-  set_error("attention: head_dim %d unsupported (64 or 128)", a.d);
-  return -3;
+  if (!head_dim_supported(a.d)) {
+    set_error("attention: head_dim %d unsupported (supported: multiples of 8 from 8 to 128)", a.d);
+    return -3;
+  }
+  if (head_tile(a.d) == 64) return launch_attention_persist(a, stream);
+  return launch_attention_t<128, 2>(a, stream);
 }
 
 }  // namespace vtk

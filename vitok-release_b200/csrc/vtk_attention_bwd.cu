@@ -60,7 +60,7 @@ struct BwdParams {
   const float* lse; const float* delta;
   bf16* dq; bf16* dk; bf16* dv; long long ld_d;
   const int* kv_len;
-  int N, heads, zero_invalid, window;
+  int N, heads, d, zero_invalid, window;   // d = the true head width (<= DH; columns d..DH-1 of a tile are TMA zero fill)
   float scale, scale_log2;
   // packed layout (PACKED kernels): image b = rows [cu[b], cu[b+1]), kv_len[b] valid tokens in front; 128-row group g is the
   // (g - cuq[img])-th tile of img = grp_img[g]; *n_grp groups exist, grp_order lists them longest image first
@@ -160,12 +160,12 @@ attn_bwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__
       const int ri = tile0 + warp * 32 + lane;
       if (ri < N) {
         if (MODE == 0) {
-          bf16* a = p.dk + (row0 + ri) * p.ld_d + head * DH;
-          bf16* b = p.dv + (row0 + ri) * p.ld_d + head * DH;
-          for (int c = 0; c < DH; c += 8) { st_global_v4(a + c, 0u, 0u, 0u, 0u); st_global_v4(b + c, 0u, 0u, 0u, 0u); }
+          bf16* a = p.dk + (row0 + ri) * p.ld_d + head * p.d;
+          bf16* b = p.dv + (row0 + ri) * p.ld_d + head * p.d;
+          for (int c = 0; c < p.d; c += 8) { st_global_v4(a + c, 0u, 0u, 0u, 0u); st_global_v4(b + c, 0u, 0u, 0u, 0u); }
         } else {
-          bf16* a = p.dq + (row0 + ri) * p.ld_d + head * DH;
-          for (int c = 0; c < DH; c += 8) st_global_v4(a + c, 0u, 0u, 0u, 0u);
+          bf16* a = p.dq + (row0 + ri) * p.ld_d + head * p.d;
+          for (int c = 0; c < p.d; c += 8) st_global_v4(a + c, 0u, 0u, 0u, 0u);
         }
       }
     }
@@ -226,8 +226,8 @@ attn_bwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__
       const CUtensorMap* mS1 = MODE == 0 ? &tmDO : &tmV;
       mbar_expect_tx(res_full, 2 * S::TILE);
       for (int nb = 0; nb < S::NB; ++nb) {
-        tma_load_2d(sR0 + nb * BWD_BLK, mR0, res_full, head * DH + nb * 64, (int)(row0 + tile0));
-        tma_load_2d(sR1 + nb * BWD_BLK, mR1, res_full, head * DH + nb * 64, (int)(row0 + tile0));
+        tma_load_3d(sR0 + nb * BWD_BLK, mR0, res_full, nb * 64, head, (int)(row0 + tile0));
+        tma_load_3d(sR1 + nb * BWD_BLK, mR1, res_full, nb * 64, head, (int)(row0 + tile0));
       }
       // issue order: tile 0 of step t, then tile 1 of step t -- with NB1 = 1 the wait for tile 1's buffer (the previous step's second MMA
       // group) comes AFTER tile 0 of this step has been requested, so tile 0 always runs a step ahead
@@ -236,10 +236,10 @@ attn_bwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__
         const int b0 = t % NB0, b1 = t % NB1;
         if (t >= NB0) mbar_wait(&s0_free[b0], (uint32_t)(t / NB0 - 1) & 1u);   // the step that used this buffer last is done with it
         mbar_expect_tx(&s0_full[b0], S::TILE);
-        for (int nb = 0; nb < S::NB; ++nb) tma_load_2d(sSb0[b0] + nb * BWD_BLK, mS0, &s0_full[b0], head * DH + nb * 64, (int)(row0 + other0));
+        for (int nb = 0; nb < S::NB; ++nb) tma_load_3d(sSb0[b0] + nb * BWD_BLK, mS0, &s0_full[b0], nb * 64, head, (int)(row0 + other0));
         if (t >= NB1) mbar_wait(&s1_free[b1], (uint32_t)(t / NB1 - 1) & 1u);
         mbar_expect_tx(&s1_full[b1], S::TILE);
-        for (int nb = 0; nb < S::NB; ++nb) tma_load_2d(sSb1[b1] + nb * BWD_BLK, mS1, &s1_full[b1], head * DH + nb * 64, (int)(row0 + other0));
+        for (int nb = 0; nb < S::NB; ++nb) tma_load_3d(sSb1[b1] + nb * BWD_BLK, mS1, &s1_full[b1], nb * 64, head, (int)(row0 + other0));
       }
     }
   } else if (warp == 5) {
@@ -361,7 +361,7 @@ attn_bwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__
 #pragma unroll
     for (int a = 0; a < (MODE == 0 ? 2 : 1); ++a) {
       bf16* base = MODE == 0 ? (a == 0 ? p.dv : p.dk) : p.dq;
-      bf16* op = base + (row0 + ri) * p.ld_d + head * DH;
+      bf16* op = base + (row0 + ri) * p.ld_d + head * p.d;
       const bool live = MODE == 0 ? (ri < kvlen) : (ri < qlimit);
 #pragma unroll
       for (int c = half * (DH / 2); c < (half + 1) * (DH / 2); c += 32) {
@@ -371,6 +371,7 @@ attn_bwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__
         if (ri < N) {
 #pragma unroll
           for (int g = 0; g < 4; ++g) {
+            if (c + 8 * g >= p.d) break;   // the tile's columns past the head width
             uint32_t w[4];
 #pragma unroll
             for (int i = 0; i < 4; ++i)
@@ -395,15 +396,15 @@ template <int DH, bool PACKED>
 static int launch_bwd_t(const AttnBwdArgs& a, cudaStream_t stream) {
   using S = BwdShape<DH>;
   const long long Mrows = PACKED ? a.row_cap : (long long)a.B * a.N;
-  const long long cols = (long long)a.heads * a.d;
+  // one head per map coordinate: at d < DH the pad columns of Q, K, V and dO load as zeros (dP = dO V^T needs them in dO too)
   CUtensorMap tmQ, tmK, tmV, tmDO;
-  if (encode_tmap_bf16_sw128(&tmQ, a.q, cols, Mrows, a.ld_qkv, BWD_T)) return -1;
-  if (encode_tmap_bf16_sw128(&tmK, a.k, cols, Mrows, a.ld_qkv, BWD_T)) return -1;
-  if (encode_tmap_bf16_sw128(&tmV, a.v, cols, Mrows, a.ld_qkv, BWD_T)) return -1;
-  if (encode_tmap_bf16_sw128(&tmDO, a.dout, cols, Mrows, a.ld_do, BWD_T)) return -1;
+  if (encode_tmap_heads(&tmQ, a.q, a.d, a.heads, Mrows, a.ld_qkv, BWD_T)) return -1;
+  if (encode_tmap_heads(&tmK, a.k, a.d, a.heads, Mrows, a.ld_qkv, BWD_T)) return -1;
+  if (encode_tmap_heads(&tmV, a.v, a.d, a.heads, Mrows, a.ld_qkv, BWD_T)) return -1;
+  if (encode_tmap_heads(&tmDO, a.dout, a.d, a.heads, Mrows, a.ld_do, BWD_T)) return -1;
   BwdParams p;
   p.lse = a.lse; p.delta = a.delta; p.dq = a.dq; p.dk = a.dk; p.dv = a.dv; p.ld_d = a.ld_d; p.kv_len = a.kv_len;
-  p.N = a.N; p.heads = a.heads; p.zero_invalid = PACKED ? 1 : a.zero_invalid_rows; p.window = PACKED ? -1 : a.window;
+  p.N = a.N; p.heads = a.heads; p.d = a.d; p.zero_invalid = PACKED ? 1 : a.zero_invalid_rows; p.window = PACKED ? -1 : a.window;
   p.scale = (float)(1.0 / sqrt((double)a.d));
   p.scale_log2 = (float)((1.0 / sqrt((double)a.d)) * 1.4426950408889634);
   p.cu = a.cu; p.cuq = a.cuq; p.grp_img = a.grp_img; p.grp_order = a.grp_order; p.n_grp = a.cuq ? a.cuq + a.B : nullptr;
@@ -428,10 +429,12 @@ int launch_attention_bwd(const AttnBwdArgs& a, cudaStream_t stream) {
     set_error("attention_bwd: packed layout needs cu/cuq/grp_img/grp_order/kv_len and positive row and group capacities");
     return -2;
   }
-  if (a.d == 64) return packed ? launch_bwd_t<64, true>(a, stream) : launch_bwd_t<64, false>(a, stream);
-  if (a.d == 128) return packed ? launch_bwd_t<128, true>(a, stream) : launch_bwd_t<128, false>(a, stream);
-  set_error("attention_bwd: head_dim %d unsupported (64 or 128)", a.d);
-  return -3;
+  if (!head_dim_supported(a.d)) {
+    set_error("attention_bwd: head_dim %d unsupported (supported: multiples of 8 from 8 to 128)", a.d);
+    return -3;
+  }
+  if (head_tile(a.d) == 64) return packed ? launch_bwd_t<64, true>(a, stream) : launch_bwd_t<64, false>(a, stream);
+  return packed ? launch_bwd_t<128, true>(a, stream) : launch_bwd_t<128, false>(a, stream);
 }
 
 }  // namespace vtk

@@ -276,40 +276,47 @@ __device__ __forceinline__ void epi_resid_unit(const EpiParams& p, uint32_t tadd
   }
 }
 
-// LayerNorm without affine over all N (= C) columns of the row; the reference rounds the Linear output to
+// bias[c, c + 16) as fp32; a last group of 8 columns (N % 16 == 8) reads zeros for the 8 past N
+__device__ __forceinline__ void load_bias16(const bf16* bias, int c, int N, float (&b)[16]) {
+  load_bf16x8(bias + c, *reinterpret_cast<float(*)[8]>(&b[0]));
+  if (c + 8 < N) load_bf16x8(bias + c + 8, *reinterpret_cast<float(*)[8]>(&b[8]));
+  else
+#pragma unroll
+    for (int i = 8; i < 16; ++i) b[i] = 0.f;
+}
+
+// LayerNorm without affine over all N (= C, a multiple of 8) columns of the row; the reference rounds the Linear output to
 // bf16 first (nn.Linear in bf16), normalises in fp32 and rounds again (norm.py:39).
 __device__ __forceinline__ void epi_bias_ln_row(const EpiParams& p, uint32_t taddr, int row, bool row_ok, int N) {
   float sum = 0.f;
   for (int c = 0; c < N; c += 16) {
     float b[16];
-    load_bf16x8(p.bias + c, *reinterpret_cast<float(*)[8]>(&b[0]));
-    load_bf16x8(p.bias + c + 8, *reinterpret_cast<float(*)[8]>(&b[8]));
+    load_bias16(p.bias, c, N, b);
     uint32_t r[16];
     tmem_ld16(taddr + c, r);
     tmem_wait_ld();
 #pragma unroll
-    for (int i = 0; i < 16; ++i) sum += bf16r(__uint_as_float(r[i]) + b[i]);
+    for (int i = 0; i < 16; ++i)
+      if (i < 8 || c + 8 < N) sum += bf16r(__uint_as_float(r[i]) + b[i]);
   }
   const float mean = sum / (float)N;
   float var = 0.f;
   for (int c = 0; c < N; c += 16) {
     float b[16];
-    load_bf16x8(p.bias + c, *reinterpret_cast<float(*)[8]>(&b[0]));
-    load_bf16x8(p.bias + c + 8, *reinterpret_cast<float(*)[8]>(&b[8]));
+    load_bias16(p.bias, c, N, b);
     uint32_t r[16];
     tmem_ld16(taddr + c, r);
     tmem_wait_ld();
 #pragma unroll
     for (int i = 0; i < 16; ++i) {
       float dv = bf16r(__uint_as_float(r[i]) + b[i]) - mean;
-      var += dv * dv;
+      if (i < 8 || c + 8 < N) var += dv * dv;
     }
   }
   const float rstd = rsqrtf(var / (float)N + p.eps);
   for (int c = 0; c < N; c += 16) {
     float b[16];
-    load_bf16x8(p.bias + c, *reinterpret_cast<float(*)[8]>(&b[0]));
-    load_bf16x8(p.bias + c + 8, *reinterpret_cast<float(*)[8]>(&b[8]));
+    load_bias16(p.bias, c, N, b);
     uint32_t r[16];
     tmem_ld16(taddr + c, r);
     tmem_wait_ld();
@@ -323,7 +330,7 @@ __device__ __forceinline__ void epi_bias_ln_row(const EpiParams& p, uint32_t tad
     if (row_ok) {
       bf16* op = p.out + (long long)row * p.ldo + c;
       st_global_v4(op, o[0], o[1], o[2], o[3]);
-      st_global_v4(op + 8, o[4], o[5], o[6], o[7]);
+      if (c + 8 < N) st_global_v4(op + 8, o[4], o[5], o[6], o[7]);
     }
   }
 }
@@ -455,23 +462,29 @@ __device__ __forceinline__ void epi_qkv_swiglu_unit(const EpiParams& p, uint32_t
                                                     const CUtensorMap* tmACT, uint64_t rs2) {
   if (n < p.qp) {
     const int threeD = 3 * p.D;
+    // plain bf16 copy of 32 columns (V; q and k too at the head dims whose QK-norm + RoPE run after the GEMM)
+    auto copy32 = [&](uint32_t ta, int col) {
+      uint32_t r[32];
+      tmem_ld32(ta, r);
+      tmem_wait_ld();
+      st.begin();
+#pragma unroll
+      for (int j = 0; j < 4; ++j)
+        st.put(j, cvt_acc2(r[8 * j], r[8 * j + 1], rs2), cvt_acc2(r[8 * j + 2], r[8 * j + 3], rs2),
+               cvt_acc2(r[8 * j + 4], r[8 * j + 5], rs2), cvt_acc2(r[8 * j + 6], r[8 * j + 7], rs2));
+      st.flush(tmQKV, col);
+    };
+    if (!qk_norm_fused(p.d)) {   // a head may straddle two units here: copy the unit, columns past 3D are clipped by the store
+      for (int cc = 0; cc < ucols && n + cc < threeD; cc += 32) copy32(taddr + cc, n + cc);
+      return;
+    }
     const uint4* rope_row = rope_row_ptr(p, rrow);
     for (int hc = 0; hc < ucols; hc += p.d) {
       const int ncol = n + hc;
       if (ncol >= threeD) break;  // zero-padded columns between 3D and qp
       const int seg = ncol / p.D;
       if (seg == 2) {  // V: plain bf16 copy
-        for (int cc = 0; cc < p.d; cc += 32) {
-          uint32_t r[32];
-          tmem_ld32(taddr + hc + cc, r);
-          tmem_wait_ld();
-          st.begin();
-#pragma unroll
-          for (int j = 0; j < 4; ++j)
-            st.put(j, cvt_acc2(r[8 * j], r[8 * j + 1], rs2), cvt_acc2(r[8 * j + 2], r[8 * j + 3], rs2),
-                   cvt_acc2(r[8 * j + 4], r[8 * j + 5], rs2), cvt_acc2(r[8 * j + 6], r[8 * j + 7], rs2));
-          st.flush(tmQKV, ncol + cc);
-        }
+        for (int cc = 0; cc < p.d; cc += 32) copy32(taddr + hc + cc, ncol + cc);
       } else {
         if (p.d == 64) epi_qk_head64(p, taddr + hc, rope_row, ncol, normw_s + seg * 128, st, tmQKV, rs2);
         else epi_qk_head(p, taddr + hc, rope_row, ncol, normw_s + seg * 128, st, tmQKV, rs2);
@@ -678,7 +691,7 @@ gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUt
       if (EPI == EPI_BIAS_LN) {
         epi_bias_ln_row(epi, taddr, row, row_ok, N);
       } else {
-        const int U = (EPI == EPI_QKV_SWIGLU && epi.d > 64) ? epi.d : 64;
+        const int U = (EPI == EPI_QKV_SWIGLU && epi.d == 128) ? 128 : 64;   // a fused-norm unit holds whole heads
         for (int c0 = half * U; c0 < width; c0 += NHALF * U) {
           if (EPI == EPI_BIAS) epi_bias_unit(epi, taddr + c0, row, row_ok, n0 + c0, N, U);
           if (EPI == EPI_RESID) epi_resid_unit(epi, taddr + c0, row, row < M, n0 + c0, N, U, st, &tmO0, f2_pack(1.f, 1.f));
@@ -1034,7 +1047,7 @@ gemm2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CU
         mbar_wait(part_full, 0);   // all 128 KB of the partner's accumulator have landed in this CTA's ring
         partial = sA + (uint32_t)(quarter * 8) * 4096u + (uint32_t)lane * 128u;
       }
-      const int U = (EPI == EPI_QKV_SWIGLU && epi.d > 64) ? epi.d : 64;
+      const int U = (EPI == EPI_QKV_SWIGLU && epi.d == 128) ? 128 : 64;   // a fused-norm unit holds whole heads
       for (int c0 = half * U; c0 < width; c0 += NHALF * U) {
         if (EPI == EPI_BIAS) epi_bias_unit(epi, taddr + c0, row, row_ok, n0 + c0, N, U);
         if (EPI == EPI_RESID) epi_resid_unit(epi, taddr + c0, row, row < M, n0 + c0, N, U, st, &tmO0, rs2, partial, c0);
@@ -1270,7 +1283,7 @@ int launch_gemm_inner(EpiKind kind, const GemmArgs& a, cudaStream_t stream) {
   if (a.fp8) {   // e4m3 operands: CTA-pair kernel only (any M: rows beyond M are zero-filled by TMA and never stored)
     if ((a.K % 16) || (a.lda % 16) || (a.ldb % 16)) { set_error("gemm(fp8): K and the row strides must be multiples of 16 bytes"); return -2; }
     if (kind == EPI_QKV_SWIGLU) {
-      if (!(a.epi.d == 32 || a.epi.d == 64 || a.epi.d == 128) || a.epi.qp % 256 || a.epi.D % a.epi.d || a.epi.Hf % 16) {
+      if (!head_dim_supported(a.epi.d) || a.epi.qp % 256 || a.epi.D % a.epi.d || a.epi.Hf % 16) {
         set_error("gemm(fp8): unsupported attention geometry D=%d d=%d Hf=%d qp=%d", a.epi.D, a.epi.d, a.epi.Hf, a.epi.qp);
         return -3;
       }
@@ -1290,13 +1303,13 @@ int launch_gemm_inner(EpiKind kind, const GemmArgs& a, cudaStream_t stream) {
       if (a.M > BM) return launch_gemm2_s<EPI_BIAS, 8, 6>(a, stream);
       return launch_gemm_t<256, EPI_BIAS, 16>(a, true, stream);
     case EPI_BIAS_LN:
-      if (a.N % 16 || a.N > 256 || !a.epi.bias) { set_error("gemm: LN epilogue needs N%%16==0, N<=256 and a bias (N=%d)", a.N); return -2; }
+      if (a.N % 8 || a.N > 256 || !a.epi.bias) { set_error("gemm: LN epilogue needs N%%8==0, N<=256 and a bias (N=%d)", a.N); return -2; }
       if (a.N <= 64) return launch_gemm_t<64, EPI_BIAS_LN, 4>(a, false, stream);
       if (a.N <= 128) return launch_gemm_t<128, EPI_BIAS_LN, 4>(a, false, stream);
       return launch_gemm_t<256, EPI_BIAS_LN, 4>(a, false, stream);
     case EPI_QKV_SWIGLU:
-      if (!(a.epi.d == 32 || a.epi.d == 64 || a.epi.d == 128) || a.epi.qp % 256 || a.epi.D % a.epi.d || a.epi.Hf % 16) {
-        set_error("gemm: unsupported attention geometry D=%d d=%d Hf=%d qp=%d (head_dim must be 32/64/128)", a.epi.D,
+      if (!head_dim_supported(a.epi.d) || a.epi.qp % 256 || a.epi.D % a.epi.d || a.epi.Hf % 16) {
+        set_error("gemm: unsupported attention geometry D=%d d=%d Hf=%d qp=%d (head_dim: multiples of 8 from 8 to 128)", a.epi.D,
                   a.epi.d, a.epi.Hf, a.epi.qp);
         return -3;
       }

@@ -47,6 +47,17 @@ int encode_tmap_u8_sw128(CUtensorMap* out, const void* base, uint64_t inner_elem
 // General form: box = box_inner x box_rows elements, swizzle_bytes in {0, 32, 64, 128} (box_inner * 2 <= swizzle span).
 int encode_tmap_bf16(CUtensorMap* out, const void* base, uint64_t inner_elems, uint64_t rows, uint64_t row_stride_elems,
                      uint32_t box_inner, uint32_t box_rows, int swizzle_bytes);
+// Attention head tiles: a 3-D bf16 map {d, heads, rows} with byte strides {2d, 2 * row_stride_elems}, box {64, 1, box_rows},
+// 128-byte swizzle.  Box columns at or past d (a head narrower than its 64-column tile block) load as zeros and are never stored.
+int encode_tmap_heads(CUtensorMap* out, const void* base, int d, int heads, uint64_t rows, uint64_t row_stride_elems, uint32_t box_rows);
+
+// Head dims of the attention kernels and the block path: d % 8 == 0 (a TMA stride is a multiple of 16 bytes) and d <= 128 (the
+// d = 128 kernel already uses all 512 TMEM columns).  A head runs on the kernel of the next tile width, 64 or 128.
+__host__ __device__ inline bool head_dim_supported(int d) { return d >= 8 && d <= 128 && d % 8 == 0; }
+__host__ __device__ inline int head_tile(int d) { return d <= 64 ? 64 : 128; }
+// QKV GEMM epilogue: QK-norm + RoPE run inside it for these d only (its walk over a tile's heads needs whole heads per 64- or
+// d-column unit); at other head dims it copies q and k raw and launch_qk_norm_rope_fwd normalises them in place.
+__host__ __device__ inline bool qk_norm_fused(int d) { return d == 32 || d == 64 || d == 128; }
 
 // ---------------------------------------------------------------------------------------------
 // GEMM  out = epilogue(A[M,K] * B[N,K]^T), bf16 in, fp32 accumulate in TMEM (vtk_gemm.cu)

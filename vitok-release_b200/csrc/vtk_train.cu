@@ -92,6 +92,52 @@ __global__ void __launch_bounds__(256) qk_norm_rope_fwd_kernel(const bf16* __res
   }
 }
 
+// The same for any head dim d % 8 == 0, d <= 128 (pairs lane and lane + 32 of the head).  Also safe in place (zraw == qkv, ldz == ldq:
+// the inference path of the head dims whose QK-norm + RoPE the QKV GEMM epilogue does not fuse): a thread reads every element it writes
+// before writing it, and no other thread touches it.  nseg = 3 copies v as well, nseg = 2 (in place) leaves it.
+__global__ void __launch_bounds__(256) qk_norm_rope_fwd_any_kernel(const bf16* zraw, long long ldz, const bf16* __restrict__ wq,
+                                                                   const bf16* __restrict__ wk, const bf16* __restrict__ rope, bf16* qkv,
+                                                                   long long ldq, int M, int heads, int d, int nseg, float eps) {
+  const int lane = threadIdx.x & 31;
+  const int np = d >> 1;   // pairs per head
+  const long long slots = (long long)M * nseg * heads;
+  const int D = heads * d;
+  for (long long s = (long long)blockIdx.x * 8 + (threadIdx.x >> 5); s < slots; s += (long long)gridDim.x * 8) {
+    const int m = (int)(s / (nseg * heads));
+    const int hs = (int)(s - (long long)m * nseg * heads);
+    const int seg = hs / heads, head = hs - seg * heads;
+    const uint32_t* src = reinterpret_cast<const uint32_t*>(zraw + (long long)m * ldz + seg * D + head * d);
+    uint32_t* dst = reinterpret_cast<uint32_t*>(qkv + (long long)m * ldq + seg * D + head * d);
+    uint32_t t[2];
+#pragma unroll
+    for (int i = 0; i < 2; ++i) t[i] = lane + 32 * i < np ? src[lane + 32 * i] : 0u;
+    if (seg == 2) {
+#pragma unroll
+      for (int i = 0; i < 2; ++i)
+        if (lane + 32 * i < np) dst[lane + 32 * i] = t[i];
+      continue;
+    }
+    float ss = 0.f;
+#pragma unroll
+    for (int i = 0; i < 2; ++i) ss += bf16_lo(t[i]) * bf16_lo(t[i]) + bf16_hi(t[i]) * bf16_hi(t[i]);
+    ss = warp_sum(ss);
+    const float rstd = rsqrtf(ss / (float)d + eps);
+    const uint32_t* w = reinterpret_cast<const uint32_t*>(seg == 0 ? wq : wk);
+    const uint32_t* tw = reinterpret_cast<const uint32_t*>(rope) + ((long long)(m >> 5) * (d >> 2)) * 128 + (m & 31) * 4;
+#pragma unroll
+    for (int i = 0; i < 2; ++i) {
+      const int pr = lane + 32 * i;
+      if (pr >= np) break;
+      const uint32_t wv = w[pr];
+      const float y0 = bf16_lo(t[i]) * rstd * bf16_lo(wv), y1 = bf16_hi(t[i]) * rstd * bf16_hi(wv);
+      const uint32_t Y = bf2_cvt(y0, y1);
+      const uint32_t c2 = tw[(pr >> 2) * 128 + (pr & 3)];
+      const uint32_t s2 = tw[((np + pr) >> 2) * 128 + (pr & 3)];
+      dst[pr] = bf2_add(bf2_mul(Y, c2), bf2_mul(bf2_swap(Y), s2));
+    }
+  }
+}
+
 // zraw[:, qp:] -> act [M, Hf] = bf16(bf16(silu(g)) * v).  layout 0: 16-column groups (value16 | gate16) -- the packed
 // w_in of the inference path; layout 1: [value Hf | gate Hf], fc1's own row order (training: no weight repack).
 __device__ __forceinline__ void swiglu_cols(int o, int qp, int Hf, int layout, long long& voff, long long& goff) {
@@ -357,6 +403,85 @@ __global__ void __launch_bounds__(256) qk_norm_rope_bwd_kernel(bf16* __restrict_
 #pragma unroll
     for (int wp = 0; wp < 8; ++wp) s += red[wp][e / DH][e % DH];
     atomicAdd(&dw[e], s);
+  }
+}
+
+// The same for any head dim d % 8 == 0, d <= 128 (pairs lane and lane + 32 of the head).  dw = [2][d].
+__global__ void __launch_bounds__(256) qk_norm_rope_bwd_any_kernel(bf16* __restrict__ dz, long long lddz, const bf16* __restrict__ zraw,
+                                                                   long long ldz, const bf16* __restrict__ wq, const bf16* __restrict__ wk,
+                                                                   const bf16* __restrict__ rope, float* __restrict__ dw, int M, int heads,
+                                                                   int d, float eps) {
+  __shared__ float red[8][2][128];
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  const int np = d >> 1;
+  const int D = heads * d;
+  float acc[2][2][2];
+#pragma unroll
+  for (int a = 0; a < 2; ++a)
+#pragma unroll
+    for (int i = 0; i < 2; ++i) acc[a][i][0] = acc[a][i][1] = 0.f;
+  const long long slots = (long long)M * 2 * heads;
+  for (long long s = (long long)blockIdx.x * 8 + warp; s < slots; s += (long long)gridDim.x * 8) {
+    const int m = (int)(s / (2 * heads));
+    const int hs = (int)(s - (long long)m * 2 * heads);
+    const int seg = hs / heads, head = hs - seg * heads;
+    const uint32_t* xs = reinterpret_cast<const uint32_t*>(zraw + (long long)m * ldz + seg * D + head * d);
+    uint32_t* dp = reinterpret_cast<uint32_t*>(dz + (long long)m * lddz + seg * D + head * d);
+    const uint32_t* w = reinterpret_cast<const uint32_t*>(seg == 0 ? wq : wk);
+    const uint32_t* tw = reinterpret_cast<const uint32_t*>(rope) + ((long long)(m >> 5) * (d >> 2)) * 128 + (m & 31) * 4;
+    float x0[2], x1[2], g0[2], g1[2];
+    float ss = 0.f;
+#pragma unroll
+    for (int i = 0; i < 2; ++i) {
+      const int pr = lane + 32 * i;
+      x0[i] = x1[i] = g0[i] = g1[i] = 0.f;
+      if (pr < np) {
+        const uint32_t xv = xs[pr], dv = dp[pr];
+        x0[i] = bf16_lo(xv); x1[i] = bf16_hi(xv);
+        const uint32_t c2 = tw[(pr >> 2) * 128 + (pr & 3)];
+        const uint32_t s2 = tw[((np + pr) >> 2) * 128 + (pr & 3)];
+        const float c = bf16_lo(c2), sn = bf16_hi(s2);   // C2 = (c, c), S2 = (-s, +s)
+        const float d0 = bf16_lo(dv), d1 = bf16_hi(dv);
+        g0[i] = c * d0 + sn * d1;
+        g1[i] = -sn * d0 + c * d1;
+      }
+      ss += x0[i] * x0[i] + x1[i] * x1[i];
+    }
+    ss = warp_sum(ss);
+    const float rstd = rsqrtf(ss / (float)d + eps);
+    float dot = 0.f;
+    float gw0[2], gw1[2];
+#pragma unroll
+    for (int i = 0; i < 2; ++i) {
+      const int pr = lane + 32 * i;
+      const uint32_t wv = pr < np ? w[pr] : 0u;
+      x0[i] *= rstd; x1[i] *= rstd;                       // xh
+      const float isq = seg == 0 ? 1.f : 0.f;             // (no dynamic indexing of the register accumulators)
+      acc[0][i][0] += isq * g0[i] * x0[i];
+      acc[0][i][1] += isq * g1[i] * x1[i];
+      acc[1][i][0] += (1.f - isq) * g0[i] * x0[i];
+      acc[1][i][1] += (1.f - isq) * g1[i] * x1[i];
+      gw0[i] = g0[i] * bf16_lo(wv); gw1[i] = g1[i] * bf16_hi(wv);
+      dot += gw0[i] * x0[i] + gw1[i] * x1[i];
+    }
+    dot = warp_sum(dot) / (float)d;
+#pragma unroll
+    for (int i = 0; i < 2; ++i)
+      if (lane + 32 * i < np) dp[lane + 32 * i] = bf2_cvt(rstd * (gw0[i] - x0[i] * dot), rstd * (gw1[i] - x1[i] * dot));
+  }
+#pragma unroll
+  for (int a = 0; a < 2; ++a)
+#pragma unroll
+    for (int i = 0; i < 2; ++i) {
+      red[warp][a][2 * (lane + 32 * i)] = acc[a][i][0];
+      red[warp][a][2 * (lane + 32 * i) + 1] = acc[a][i][1];
+    }
+  __syncthreads();
+  for (int e = threadIdx.x; e < 2 * d; e += blockDim.x) {
+    float sum = 0.f;
+#pragma unroll
+    for (int wp = 0; wp < 8; ++wp) sum += red[wp][e / d][e % d];
+    atomicAdd(&dw[e], sum);
   }
 }
 
@@ -627,22 +752,19 @@ __global__ void __launch_bounds__(256) scale_by_dev_kernel(bf16* __restrict__ x,
   for (long long i = (nvec << 3) + tid; i < n; i += stride) x[i] = __float2bfloat16_rn(__bfloat162float(x[i]) * s);
 }
 
-// per attention row and head: delta = sum_d dO * O   (the softmax-backward row term), fp32 [M, heads]
-template <int DH>
+// per attention row and head: delta = sum_d dO * O   (the softmax-backward row term), fp32 [M, heads]; lane <-> pairs lane, lane + 32
 __global__ void __launch_bounds__(256) attn_delta_kernel(const bf16* __restrict__ o, long long ldo, const bf16* __restrict__ dob,
-                                                         long long lddo, float* __restrict__ delta, int M, int heads) {
-  constexpr int PPL = DH / 64;
+                                                         long long lddo, float* __restrict__ delta, int M, int heads, int d) {
   const int lane = threadIdx.x & 31;
   const long long slots = (long long)M * heads;
   for (long long s = (long long)blockIdx.x * 8 + (threadIdx.x >> 5); s < slots; s += (long long)gridDim.x * 8) {
     const long long m = s / heads;
     const int head = (int)(s - m * heads);
-    const uint32_t* a = reinterpret_cast<const uint32_t*>(o + m * ldo + head * DH);
-    const uint32_t* b = reinterpret_cast<const uint32_t*>(dob + m * lddo + head * DH);
+    const uint32_t* a = reinterpret_cast<const uint32_t*>(o + m * ldo + head * d);
+    const uint32_t* b = reinterpret_cast<const uint32_t*>(dob + m * lddo + head * d);
     float acc = 0.f;
-#pragma unroll
-    for (int i = 0; i < PPL; ++i) {
-      const uint32_t x = a[lane + 32 * i], y = b[lane + 32 * i];
+    for (int pr = lane; pr < (d >> 1); pr += 32) {
+      const uint32_t x = a[pr], y = b[pr];
       acc += bf16_lo(x) * bf16_lo(y) + bf16_hi(x) * bf16_hi(y);
     }
     acc = warp_sum(acc);
@@ -938,8 +1060,16 @@ __global__ void __launch_bounds__(MAXT, MINB) rmsnorm_bwd_cols_kernel(const bf16
 
 int launch_qk_norm_rope_fwd(const bf16* zraw, long long ldz, const bf16* wq, const bf16* wk, const bf16* rope, bf16* qkv,
                             long long ldq, int M, int heads, int d, float eps, cudaStream_t st) {
-  VTK_TRAIN_CHECK(d == 64 || d == 128, "qk_norm_rope: head_dim %d unsupported (64 or 128)", d);
+  VTK_TRAIN_CHECK(head_dim_supported(d), "qk_norm_rope: head_dim %d unsupported (supported: multiples of 8 from 8 to 128)", d);
   if (M <= 0) return 0;
+  const bool in_place = zraw == qkv;
+  VTK_TRAIN_CHECK(!in_place || ldz == ldq, "qk_norm_rope: in place needs ldz == ldq");
+  if (in_place || (d != 64 && d != 128)) {
+    const int nseg = in_place ? 2 : 3;
+    qk_norm_rope_fwd_any_kernel<<<grid_for((long long)M * nseg * heads, 8), 256, 0, st>>>(zraw, ldz, wq, wk, rope, qkv, ldq, M, heads, d,
+                                                                                           nseg, eps);
+    return check_cuda(cudaGetLastError(), "qk_norm_rope_fwd (any d) launch");
+  }
   const int hpw = 32 / (d / 8);
   if (heads % hpw == 0 && ldz % 8 == 0 && ldq % 8 == 0 && (long long)M * (3 * heads / hpw) < (1ll << 31) &&
       ((reinterpret_cast<uintptr_t>(zraw) | reinterpret_cast<uintptr_t>(qkv) | reinterpret_cast<uintptr_t>(wq) | reinterpret_cast<uintptr_t>(wk) |
@@ -1003,8 +1133,13 @@ int launch_swiglu_bwd(const bf16* dact, long long ldd, const bf16* zraw, long lo
 }
 int launch_qk_norm_rope_bwd(bf16* dz, long long lddz, const bf16* zraw, long long ldz, const bf16* wq, const bf16* wk,
                             const bf16* rope, float* dw, int M, int heads, int d, float eps, cudaStream_t st) {
-  VTK_TRAIN_CHECK(d == 64 || d == 128, "qk_norm_rope_bwd: head_dim %d unsupported (64 or 128)", d);
+  VTK_TRAIN_CHECK(head_dim_supported(d), "qk_norm_rope_bwd: head_dim %d unsupported (supported: multiples of 8 from 8 to 128)", d);
   if (M <= 0) return 0;
+  if (d != 64 && d != 128) {
+    qk_norm_rope_bwd_any_kernel<<<grid_for((long long)M * 2 * heads, 8, 8), 256, 0, st>>>(dz, lddz, zraw, ldz, wq, wk, rope, dw, M, heads,
+                                                                                            d, eps);
+    return check_cuda(cudaGetLastError(), "qk_norm_rope_bwd (any d) launch");
+  }
   const int hpw = 32 / (d / 8);
   if (heads % hpw == 0 && ldz % 8 == 0 && lddz % 8 == 0 && (long long)M * (2 * heads / hpw) < (1ll << 31) &&
       ((reinterpret_cast<uintptr_t>(zraw) | reinterpret_cast<uintptr_t>(dz) | reinterpret_cast<uintptr_t>(wq) | reinterpret_cast<uintptr_t>(wk) |
@@ -1094,11 +1229,9 @@ int launch_scale_by_dev(bf16* x, const float* scale, long long n, cudaStream_t s
 }
 int launch_attn_delta(const bf16* o, long long ldo, const bf16* dob, long long lddo, float* delta, int M, int heads, int d,
                       cudaStream_t st) {
-  VTK_TRAIN_CHECK(d == 64 || d == 128, "attn_delta: head_dim %d unsupported", d);
+  VTK_TRAIN_CHECK(head_dim_supported(d), "attn_delta: head_dim %d unsupported (supported: multiples of 8 from 8 to 128)", d);
   if (M <= 0) return 0;
-  const int grid = grid_for((long long)M * heads, 8);
-  if (d == 64) attn_delta_kernel<64><<<grid, 256, 0, st>>>(o, ldo, dob, lddo, delta, M, heads);
-  else attn_delta_kernel<128><<<grid, 256, 0, st>>>(o, ldo, dob, lddo, delta, M, heads);
+  attn_delta_kernel<<<grid_for((long long)M * heads, 8), 256, 0, st>>>(o, ldo, dob, lddo, delta, M, heads, d);
   return check_cuda(cudaGetLastError(), "attn_delta launch");
 }
 

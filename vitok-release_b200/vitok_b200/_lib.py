@@ -134,7 +134,7 @@ def load() -> ctypes.CDLL:
 
 def set_flag(name: str, value: int) -> None:
     """Process-wide kernel switch (include/vitok_b200.h: vtk_set_flag): "pdl", "gemm_splitk", "reserve_sms" (the persistent
-    kernels -- GEMMs and d = 64 attention -- size their grids for that many SMs fewer)."""
+    kernels -- GEMMs and attention at d <= 64 -- size their grids for that many SMs fewer)."""
     check(load().vtk_set_flag(name.encode(), int(value)))
 
 
@@ -376,6 +376,8 @@ def proj_residual_fp8(a8, a_scale, w8, w_scale: float, gamma, x):
 
 @_on_device
 def qkv_swiglu(h, w_packed, D, d, Hf, qp, norm_q, norm_k, table, eps=1e-6):
+    """QKV + fc1 GEMM with QK-norm, RoPE and SwiGLU (vtk_qkv_swiglu_bf16); d % 8 == 0, 8 <= d <= 128.  At d other than 32, 64 and
+    128 the QK-norm + RoPE run as a second kernel after the GEMM."""
     M = h.shape[0]
     qkv = torch.empty(M, 3 * D, dtype=torch.bfloat16, device=h.device)
     act = torch.empty(M, Hf, dtype=torch.bfloat16, device=h.device)
@@ -400,7 +402,8 @@ def attention(qkv: torch.Tensor, B: int, N: int, heads: int, d: int, mask: Optio
     """qkv [B*N, 3*heads*d] (q | k | v).  mask [B,N] bool -> sdpa semantics (masked query rows read 0); None -> flash semantics.
     The mask must be a prefix mask (every image's valid tokens first, what patchify emits): a mask with holes raises ValueError
     (a host check; masked batches with holes run on the packed layout, see ``attention_packed``).
-    window >= 0: sliding window |i - j| <= window (flash_attn window_size=(window, window))."""
+    window >= 0: sliding window |i - j| <= window (flash_attn window_size=(window, window)).
+    head_dim d: d % 8 == 0 and 8 <= d <= 128 (NotImplementedError otherwise)."""
     D = heads * d
     out = torch.empty(B * N, D, dtype=torch.bfloat16, device=qkv.device)
     kl = None
@@ -426,7 +429,7 @@ def umma_probe(a: torch.Tensor, b: torch.Tensor, n: int, k: int, b_mn_major: boo
 def attention_packed(qkv: torch.Tensor, plan: dict, B: int, N: int, heads: int, d: int, lse: Optional[torch.Tensor] = None,
                      out: Optional[torch.Tensor] = None) -> torch.Tensor:
     """Attention over the packed NaFlex layout of ``pack_plan`` (qkv [row capacity, 3*heads*d]; the plan's qrows must be 128 for
-    d = 64, 256 for d = 128).  Without ``lse`` the pad rows of ``out`` are never written; with ``lse`` ([rows, heads] fp32) they
+    d <= 64, 256 for 64 < d <= 128).  Without ``lse`` the pad rows of ``out`` are never written; with ``lse`` ([rows, heads] fp32) they
     are written as 0 and lse as +inf.  ``out`` (optional) = a preallocated [rows, heads*d]."""
     D = heads * d
     if out is None:

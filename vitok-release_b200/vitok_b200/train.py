@@ -283,7 +283,7 @@ def _block_forward(lib, blk, x: torch.Tensor, rope, kv, B: int, N: int, dims, wi
         _check(lib.vtk_attention_bf16(base, base + 2 * D, base + 4 * D, 3 * D, a2.data_ptr(), kp, _lib.ptr(kv), B, N, heads, d,
                                       1 if kv is not None else 0, window, lse.data_ptr(), st))
     else:
-        qrows = 128 if d == 64 else 256
+        qrows = 128 if d <= 64 else 256                  # d <= 64 runs on the 128-row kernel, 64 < d <= 128 on the 256-row one
         pl = pk.attn_plan(qrows)
         _check(lib.vtk_attention_packed_lse_bf16(base, base + 2 * D, base + 4 * D, 3 * D, a2.data_ptr(), kp, pl["n_valid"].data_ptr(),
                                                  pl["cu"].data_ptr(), pl["cuq"].data_ptr(), pl["grp_img"].data_ptr(),
