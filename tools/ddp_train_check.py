@@ -6,6 +6,8 @@ Every rank runs model(batch) -> Charbonnier -> backward on ITS OWN batch under D
   * after backward every rank holds the same gradients (bit-identical), and they equal the mean of the per-rank local
     gradients computed without DDP (all-reduce(mean) semantics);
   * after FusedAdamW steps the parameters stay identical across ranks and the loss goes down.
+With ``--frozen-encoder`` it checks instead the overlapped all-reduce (vb.enable_grad_sync) of a model whose encoder is frozen: every
+rank holds identical decoder gradients equal to the mean of the local ones, and the encoder has no gradient and stays identical.
 """
 import os
 import sys
@@ -20,12 +22,60 @@ from torch.nn.parallel import DistributedDataParallel as DDP  # noqa: E402
 import vitok_b200 as vb  # noqa: E402
 
 
+def _same_on_ranks(t, world):
+    chk = t.float().sum().double().reshape(1)
+    lst = [torch.zeros_like(chk) for _ in range(world)]
+    dist.all_gather(lst, chk)
+    return all(float(x) == float(lst[0]) for x in lst)
+
+
+def frozen_encoder(cfg, dev, rank, world):
+    enc = ("patch_embed.", "to_code.", "encoder_blocks.")
+
+    def make():
+        torch.manual_seed(0)
+        m = vb.AE(**cfg, attn_backend="flash").train().to(dev, torch.bfloat16)
+        for mod in (m.patch_embed, m.encoder_blocks, m.to_code):
+            mod.requires_grad_(False)
+        return m
+
+    g = torch.Generator().manual_seed(100 + rank)
+    imgs = torch.rand(4, 3, 256, 256, generator=g) * 2 - 1
+    pd = vb.patchify_batch(imgs.to(dev), 16, 256, out_dtype=torch.bfloat16, device=dev)
+    twin = make()
+    vb.charbonnier_loss(twin(pd)["patches"], pd["patches"], pd["patch_mask"]).backward()
+    local_g = {n: p.grad.float().clone() for n, p in twin.named_parameters() if p.grad is not None}
+    assert not any(n.startswith(enc) for n in local_g) and len(local_g) == sum(1 for n, _ in twin.named_parameters() if not n.startswith(enc))
+    for t in local_g.values():
+        dist.all_reduce(t, op=dist.ReduceOp.SUM)
+        t /= world
+    m = make()
+    vb.enable_grad_sync(m)
+    vb.charbonnier_loss(m(pd)["patches"], pd["patches"], pd["patch_mask"]).backward()
+    worst = 0.0
+    for n, p in m.named_parameters():
+        if n.startswith(enc):
+            assert p.grad is None, f"{n}: a frozen parameter got a gradient"
+            assert _same_on_ranks(p.detach(), world), f"{n}: frozen parameters differ across ranks"
+            continue
+        worst = max(worst, float((p.grad.float() - local_g[n]).norm() / local_g[n].norm().clamp_min(1e-30)))
+        assert _same_on_ranks(p.grad, world), f"{n}: overlapped-sync gradients differ across ranks"
+    assert worst < 2e-2, worst
+    if rank == 0:
+        print(f"grad_sync frozen encoder OK: world={world} worst decoder grad rel err vs hand-made mean {worst:.3e}")
+
+
 def main():
     rank, world, local = int(os.environ["RANK"]), int(os.environ["WORLD_SIZE"]), int(os.environ["LOCAL_RANK"])
     torch.cuda.set_device(local)
     dev = torch.device("cuda", local)
     dist.init_process_group("nccl", device_id=dev)
-    variant = sys.argv[1] if len(sys.argv) > 1 else "w256_d2_h4-w512_d3_h4/1x16x16"
+    args = [a for a in sys.argv[1:] if a != "--frozen-encoder"]
+    variant = args[0] if args else "w256_d2_h4-w512_d3_h4/1x16x16"
+    if "--frozen-encoder" in sys.argv[1:]:
+        frozen_encoder(vb.decode_variant(variant), dev, rank, world)
+        dist.destroy_process_group()
+        return
     cfg = vb.decode_variant(variant)
     torch.manual_seed(0)
     model = vb.AE(**cfg, attn_backend="flash").train().to(dev, torch.bfloat16)

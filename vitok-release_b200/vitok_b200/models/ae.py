@@ -16,8 +16,10 @@ Semantics kept from the reference (file:line in the reference tree):
   * unknown kwargs ignored (ae.py:92); ``sw <= 0`` -> None (ae.py:99).
 ``sw``: sliding-window attention |i-j| <= sw on the token index with the flash backend (attention.py:113-116);
     ignored by the sdpa backend, as in the reference.
-Training: ``model(batch)`` in train mode builds one autograd node (vitok_b200/train.py); encode/decode alone are
-    inference-only.  ``quantize()`` (FP8 block GEMMs) needs widths that are multiples of 256 and raises otherwise.
+Training: ``model(batch)`` in train mode builds one autograd node (vitok_b200/train.py) that computes only the gradients
+    autograd asks for: frozen parameters (``requires_grad=False``) cost no weight-gradient GEMM and get no ``.grad``, and the
+    backward pass stops below the lowest block that needs one.  ``AE(encoder=False)`` trains on ``batch["z"]``, ``AE(decoder=False)``
+    returns the encode dict with z carrying the graph.  encode/decode alone are inference-only.  ``quantize()`` (FP8 block GEMMs) needs widths that are multiples of 256 and raises otherwise.
 """
 from __future__ import annotations
 
@@ -483,8 +485,11 @@ class AE(nn.Module):
         return self.training and torch.is_grad_enabled() and any(p.requires_grad for p in self.parameters())
 
     def forward(self, x: Dict[str, torch.Tensor]) -> Dict[str, torch.Tensor]:
-        """encode then decode (ae.py:245-251).  In training mode with gradients enabled this is the training step's
-        forward: one autograd node whose backward runs the sm_100a backward kernels (vitok_b200/train.py)."""
+        """encode then decode (ae.py:245-251); a model with one half runs that half.  In training mode with gradients enabled
+        (some parameter requires grad) this is the training step's forward: one autograd node whose backward runs the sm_100a
+        backward kernels for exactly the gradients autograd asks for (vitok_b200/train.py).  ``AE(encoder=False)`` decodes
+        ``x["z"]`` (z gets a gradient when it requires grad); ``AE(decoder=False)`` returns the encode dict, whose ``z`` carries the
+        graph back to the encoder parameters (and to ``x["patches"]`` when they require grad)."""
         if self._wants_grad():
             from ..train import train_forward
             return train_forward(self, x)

@@ -25,11 +25,15 @@ mask the attention backward understands; the output is permuted back.
 include/vitok_b200.h: vtk_pack_plan) -- every image's valid tokens, in token order, padded to 16 rows, so every GEMM, elementwise
 kernel and saved activation covers the valid tokens only; attention forward / backward are the packed kernels
 (vtk_attention_packed_lse_bf16, vtk_attention_bwd_packed_bf16).  No permutation is needed for masks with holes.
+Only the gradients autograd asks for are computed (``_grad_plan``): a parameter with ``requires_grad=False`` gets no
+weight-gradient GEMM, no all-reduce and no ``.grad``, and the backward pass stops at the deepest block whose input gradient
+something below still needs -- blocks below it keep no activations.  ``AE(encoder=False)`` trains on ``batch["z"]``,
+``AE(decoder=False)`` returns z with its graph.
 """
 from __future__ import annotations
 
 import ctypes
-from typing import Dict, List, Optional
+from typing import Dict, NamedTuple, Optional, Tuple
 
 import torch
 
@@ -256,6 +260,74 @@ class _Packing:
         return keep[self._row_img].contiguous()
 
 
+# the four matrices of a block, in the order of its flat weight-gradient buffer
+_BLOCK_MATS = ("attn.qkv_proj.weight", "ffn.fc1.weight", "attn.out_proj.weight", "ffn.fc2.weight")
+_SIDE_NAMES = {0: ("patch_embed", "to_code", "encoder_blocks"), 1: ("decoder_embed", "to_pixels", "decoder_blocks")}
+
+
+class SidePlan(NamedTuple):
+    """What the backward pass of one side computes.
+
+    ``stages[i]`` -- how deep block i's backward goes: 0 nothing; 1 ``resid_bwd``; 2 also the dgrad to [attn | act], the SwiGLU and
+    attention backward and ``qk_norm_rope_bwd``; 3 also the dgrad to h and ``rmsnorm_bwd`` (the block's input gradient).
+    ``wgrads[i]`` -- which of block i's weight-gradient GEMMs run: (qkv_proj, fc1, out_proj, fc2).
+    ``save_from`` -- the first block that keeps its activations; blocks below it run their forward and keep nothing.
+    ``top`` -- the gradient w.r.t. the last block's output is needed (the dgrad through the side's output projection runs).
+    ``dinput`` -- the gradient w.r.t. the side's input (patches, or z) is needed (the dgrad through the input projection runs).
+    ``embed`` / ``head`` -- (weight, bias) gradients of the input projection (patch_embed / decoder_embed) and of the output
+    projection (to_code / to_pixels)."""
+    stages: Tuple[int, ...]
+    wgrads: Tuple[Tuple[bool, bool, bool, bool], ...]
+    save_from: int
+    top: bool
+    dinput: bool
+    embed: Tuple[bool, bool]
+    head: Tuple[bool, bool]
+
+
+def _grad_plan(needs: Dict[str, bool], depths: Dict[int, int], input_grad: bool) -> Dict[int, SidePlan]:
+    """The backward pass's work list from what autograd asks for: ``needs`` maps every parameter name to its requires_grad
+    (``ctx.needs_input_grad``), ``depths`` the present sides (0 encoder, 1 decoder) to their block counts, ``input_grad``
+    says whether the step's input (patches, or z for a decoder-only model) requires grad.
+
+    A block's input gradient is needed when anything below it needs a gradient: a trainable parameter of an earlier block or of the
+    input projection, or the side's input -- for the decoder that is z, needed when anything of the encoder is trainable (or the
+    patches require grad), for a decoder-only model when z requires grad.  A block then runs all three stages; otherwise it stops at
+    the deepest stage that produces a gradient of one of its own trainable parameters."""
+
+    def side(s: int, below: bool) -> SidePlan:
+        emb, head, blk = _SIDE_NAMES[s]
+        embed = (needs[emb + ".weight"], needs[emb + ".bias"])
+        need = below or any(embed)                     # the gradient w.r.t. the current block's input is consumed below it
+        trainable = {int(k.split(".")[1]) for k, v in needs.items() if v and k.startswith(blk + ".")}
+        stages, wgrads = [], []
+        for i in range(depths[s]):
+            p = f"{blk}.{i}."
+            w = tuple(needs[p + m] for m in _BLOCK_MATS)
+            if need or needs[p + "norm1.weight"]:
+                st = 3
+            elif w[0] or w[1] or needs[p + "attn.norm_q.weight"] or needs[p + "attn.norm_k.weight"]:
+                st = 2
+            elif w[2] or w[3] or needs.get(p + "layer_scale.gamma", False):
+                st = 1
+            else:
+                st = 0
+            stages.append(st)
+            wgrads.append(w)
+            need = need or i in trainable
+        save_from = next((i for i, st in enumerate(stages) if st), len(stages))
+        return SidePlan(tuple(stages), tuple(wgrads), save_from, need, below, embed, (needs[head + ".weight"], needs[head + ".bias"]))
+
+    plans = {}
+    z_grad = input_grad
+    if 0 in depths:
+        plans[0] = side(0, input_grad)
+        z_grad = plans[0].top or any(plans[0].head)    # the bottleneck backward (layernorm_bwd, to_code) runs
+    if 1 in depths:
+        plans[1] = side(1, z_grad)
+    return plans
+
+
 def _block_forward(lib, blk, x: torch.Tensor, rope, kv, B: int, N: int, dims, window: int, keep, keep_prob: float,
                    pk: Optional[_Packing] = None):
     """One transformer block (ae.py:55-65) with everything the backward needs: returns (x_new, (h, zraw, qkv, a2, lse, y)).
@@ -297,7 +369,8 @@ def _block_forward(lib, blk, x: torch.Tensor, rope, kv, B: int, N: int, dims, wi
 
 
 def _side_forward(lib, model, sw: _SideWeights, side: int, xin: torch.Tensor, row, col, kv, window: int, B: int, N: int, saved: Dict,
-                  pk: Optional[_Packing] = None):
+                  save_from: int, pk: Optional[_Packing] = None):
+    """Blocks ``save_from`` and up keep what their backward needs (``saved["layers"]``); the blocks below keep nothing."""
     width = model.encoder_width if side == 0 else model.decoder_width
     heads = model.encoder_heads if side == 0 else model.decoder_heads
     d = width // heads
@@ -330,23 +403,32 @@ def _side_forward(lib, model, sw: _SideWeights, side: int, xin: torch.Tensor, ro
             if pk is not None:
                 keep = pk.per_row(keep)
         x_new, inner = _block_forward(lib, blk, x, rope, kv, B, N, dims, window, keep, keep_prob, pk)
-        # activation checkpointing (ae.py:159-160): block i with i % checkpoint == 0 keeps its input only
-        layers.append((x, None if (ck > 0 and li % ck == 0) else inner, keep, keep_prob))
+        if li < save_from:             # no backward reaches this block
+            layers.append(None)
+        else:                          # activation checkpointing (ae.py:159-160): block i with i % checkpoint == 0 keeps its input only
+            layers.append((x, None if (ck > 0 and li % ck == 0) else inner, keep, keep_prob))
         x = x_new
-    saved.update(dict(layers=layers, x_final=x, rope=rope, kv=kv, window=window, xin=xin, dims=dims, pk=pk))
+    saved.update(dict(layers=layers, x_final=x, rope=rope if save_from < len(sw.blocks) else None, kv=kv, window=window, xin=xin,
+                      dims=dims, pk=pk))
     return x
 
 
-def _side_backward(lib, model, sw: _SideWeights, side: int, dx: torch.Tensor, saved: Dict, B: int, N: int, need_dxin: bool,
+def _side_backward(lib, model, sw: _SideWeights, side: int, dx: Optional[torch.Tensor], saved: Dict, B: int, N: int, plan: SidePlan,
                    sync: Optional[_GradSync] = None):
-    """dx = gradient w.r.t. the output of the last block.  Returns (block grads, dW_a, db_a, d_input)."""
+    """dx = gradient w.r.t. the output of the last block (None when ``plan.top`` is False).  Runs the stages and weight gradients of
+    ``plan``.  Returns ({block index: grads}, dW_a, db_a, d_input); the block grads include the vector gradients of every stage that
+    ran, trainable or not (the caller keeps the trainable ones), and entries not computed are None."""
     dims = saved["dims"]
     M, D, heads, d, Hf, qp, ZP, kp = dims
     st = _lib.stream_ptr()
-    dev = dx.device
     rope, kv, window, pk = saved["rope"], saved["kv"], saved["window"], saved["pk"]
-    grads: List[Dict[str, torch.Tensor]] = []
-    for li in range(len(sw.blocks) - 1, -1, -1):
+    grads: Dict[int, Dict[str, torch.Tensor]] = {}
+    if dx is None:
+        return grads, None, None, None
+    dev = dx.device
+    for li in range(len(sw.blocks) - 1, plan.save_from - 1, -1):
+        stage = plan.stages[li]
+        want = dict(zip(("qkv", "fc1", "out", "fc2"), plan.wgrads[li]))
         wqkv, w1, w_o, w_2, n1, nq, nk, gamma = sw.blocks[li]
         x, inner, keep, keep_prob = saved["layers"][li]
         if inner is None:      # checkpointed block: re-run its forward from x (same stochastic-depth draw)
@@ -357,110 +439,140 @@ def _side_backward(lib, model, sw: _SideWeights, side: int, dx: torch.Tensor, sa
         dgamma = torch.zeros(D, dtype=torch.float32, device=dev)
         _check(lib.vtk_resid_bwd_dp(dx.data_ptr(), y.data_ptr(), gamma.data_ptr(), dy.data_ptr(), dgamma.data_ptr(), M, D,
                                     _lib.ptr(keep), N if pk is None else 1, float(keep_prob), st))
-        # the four weight gradients of the block live in ONE flat buffer so that they leave as one all-reduce
-        n_qkv, n_fc1, n_o, n_f2 = 3 * D * D, 2 * Hf * D, D * D, D * Hf
-        flat = torch.empty(n_qkv + n_fc1 + n_o + n_f2, dtype=BF, device=dev)
-        dw_qkv = flat[:n_qkv].view(3 * D, D)
-        dw_fc1 = flat[n_qkv:n_qkv + n_fc1].view(2 * Hf, D)
-        dw_o = flat[n_qkv + n_fc1:n_qkv + n_fc1 + n_o].view(D, D)
-        dw_f2 = flat[n_qkv + n_fc1 + n_o:].view(D, Hf)
-        da2 = torch.empty(M, kp, dtype=BF, device=dev)                            # d[attn | act] = dy @ [out_proj | fc2]
-        _dgrad(dy, D, w_o, M, D, D, out=da2[:, :D])
-        _dgrad(dy, D, w_2, M, Hf, D, out=da2[:, D:D + Hf])
-        _wgrad(dy, D, D, a2, kp, D, M, out=dw_o)                                  # out_proj.weight grad [D, D] = dy^T attn
-        _wgrad(dy, D, D, a2[:, D:], kp, Hf, M, out=dw_f2)                         # fc2.weight grad [D, Hf] = dy^T act
-        dz = torch.empty(M, ZP, dtype=BF, device=dev)
-        if qp > 3 * D:
-            dz[:, 3 * D:qp].zero_()
-        _check(lib.vtk_swiglu_bwd(da2.data_ptr() + 2 * D, kp, zraw.data_ptr(), ZP, qp, dz.data_ptr(), ZP, M, Hf, 1, st))
-        delta = torch.empty(M, heads, dtype=torch.float32, device=dev)
-        _check(lib.vtk_attn_delta(a2.data_ptr(), kp, da2.data_ptr(), kp, delta.data_ptr(), M, heads, d, st))
-        qb, zb = qkv.data_ptr(), dz.data_ptr()
-        if pk is None:
-            _check(lib.vtk_attention_bwd_bf16(qb, qb + 2 * D, qb + 4 * D, 3 * D, da2.data_ptr(), kp, lse.data_ptr(), delta.data_ptr(),
-                                              zb, zb + 2 * D, zb + 4 * D, ZP, _lib.ptr(kv), B, N, heads, d,
-                                              1 if kv is not None else 0, window, st))
-        else:
-            pl = pk.plan
-            _check(lib.vtk_attention_bwd_packed_bf16(qb, qb + 2 * D, qb + 4 * D, 3 * D, da2.data_ptr(), kp, lse.data_ptr(),
-                                                     delta.data_ptr(), zb, zb + 2 * D, zb + 4 * D, ZP, pl["n_valid"].data_ptr(),
-                                                     pl["cu"].data_ptr(), pl["cuq"].data_ptr(), pl["grp_img"].data_ptr(),
-                                                     pl["grp_order"].data_ptr(), B, heads, d, M, pk.groups[128], st))
-        dwqk = torch.zeros(2, d, dtype=torch.float32, device=dev)
-        _check(lib.vtk_qk_norm_rope_bwd(dz.data_ptr(), ZP, zraw.data_ptr(), ZP, nq.data_ptr(), nk.data_ptr(), rope.data_ptr(),
-                                        dwqk.data_ptr(), M, heads, d, 1e-6, st))
-        dh = _dgrad(dz, ZP, wqkv, M, D, 3 * D)                                    # dz[:, :3D] @ Wqkv ...
-        _dgrad(dz[:, qp:], ZP, w1, M, D, 2 * Hf, out=dh, accumulate=True)         # ... + dz[:, qp:] @ W1, added in the GEMM epilogue
-        _wgrad(dz, ZP, 3 * D, h, D, D, M, out=dw_qkv)                             # qkv_proj.weight grad [3D, D]
-        _wgrad(dz[:, qp:], ZP, 2 * Hf, h, D, D, M, out=dw_fc1)                    # fc1.weight grad [2Hf, D], fc1's own row order
-        dx_in = torch.empty(M, D, dtype=BF, device=dev)
-        dw1 = torch.zeros(D, dtype=torch.float32, device=dev)
-        _check(lib.vtk_rmsnorm_bwd(x.data_ptr(), dh.data_ptr(), n1.data_ptr(), dx.data_ptr(), dx_in.data_ptr(), dw1.data_ptr(),
-                                   M, D, 1e-6, st))
-        bg = dict(
-            qkv=dw_qkv, fc1=dw_fc1, out=dw_o, fc2=dw_f2,
-            norm1=dw1, norm_q=dwqk[0], norm_k=dwqk[1], gamma=dgamma)
-        if sync is not None:          # this block's weight gradients leave for the all-reduce while the next block computes
+        bg = dict(gamma=dgamma)
+        # the trainable weight gradients of the block live in ONE flat buffer so that they leave as one all-reduce
+        sizes = dict(qkv=(3 * D, D), fc1=(2 * Hf, D), out=(D, D), fc2=(D, Hf))
+        flat = torch.empty(sum(r * c for k, (r, c) in sizes.items() if want[k]), dtype=BF, device=dev)
+        off = 0
+        for k, (r, c) in sizes.items():
+            if want[k]:
+                bg[k] = flat[off:off + r * c].view(r, c)
+                off += r * c
+        if stage >= 2:
+            da2 = torch.empty(M, kp, dtype=BF, device=dev)                        # d[attn | act] = dy @ [out_proj | fc2]
+            _dgrad(dy, D, w_o, M, D, D, out=da2[:, :D])
+            _dgrad(dy, D, w_2, M, Hf, D, out=da2[:, D:D + Hf])
+        if want["out"]:
+            _wgrad(dy, D, D, a2, kp, D, M, out=bg["out"])                         # out_proj.weight grad [D, D] = dy^T attn
+        if want["fc2"]:
+            _wgrad(dy, D, D, a2[:, D:], kp, Hf, M, out=bg["fc2"])                 # fc2.weight grad [D, Hf] = dy^T act
+        if stage >= 2:
+            dz = torch.empty(M, ZP, dtype=BF, device=dev)
+            if qp > 3 * D:
+                dz[:, 3 * D:qp].zero_()
+            _check(lib.vtk_swiglu_bwd(da2.data_ptr() + 2 * D, kp, zraw.data_ptr(), ZP, qp, dz.data_ptr(), ZP, M, Hf, 1, st))
+            delta = torch.empty(M, heads, dtype=torch.float32, device=dev)
+            _check(lib.vtk_attn_delta(a2.data_ptr(), kp, da2.data_ptr(), kp, delta.data_ptr(), M, heads, d, st))
+            qb, zb = qkv.data_ptr(), dz.data_ptr()
+            if pk is None:
+                _check(lib.vtk_attention_bwd_bf16(qb, qb + 2 * D, qb + 4 * D, 3 * D, da2.data_ptr(), kp, lse.data_ptr(),
+                                                  delta.data_ptr(), zb, zb + 2 * D, zb + 4 * D, ZP, _lib.ptr(kv), B, N, heads, d,
+                                                  1 if kv is not None else 0, window, st))
+            else:
+                pl = pk.plan
+                _check(lib.vtk_attention_bwd_packed_bf16(qb, qb + 2 * D, qb + 4 * D, 3 * D, da2.data_ptr(), kp, lse.data_ptr(),
+                                                         delta.data_ptr(), zb, zb + 2 * D, zb + 4 * D, ZP, pl["n_valid"].data_ptr(),
+                                                         pl["cu"].data_ptr(), pl["cuq"].data_ptr(), pl["grp_img"].data_ptr(),
+                                                         pl["grp_order"].data_ptr(), B, heads, d, M, pk.groups[128], st))
+            dwqk = torch.zeros(2, d, dtype=torch.float32, device=dev)
+            _check(lib.vtk_qk_norm_rope_bwd(dz.data_ptr(), ZP, zraw.data_ptr(), ZP, nq.data_ptr(), nk.data_ptr(), rope.data_ptr(),
+                                            dwqk.data_ptr(), M, heads, d, 1e-6, st))
+            bg["norm_q"], bg["norm_k"] = dwqk[0], dwqk[1]
+        if stage >= 3:
+            dh = _dgrad(dz, ZP, wqkv, M, D, 3 * D)                                # dz[:, :3D] @ Wqkv ...
+            _dgrad(dz[:, qp:], ZP, w1, M, D, 2 * Hf, out=dh, accumulate=True)     # ... + dz[:, qp:] @ W1, added in the GEMM epilogue
+        if want["qkv"]:
+            _wgrad(dz, ZP, 3 * D, h, D, D, M, out=bg["qkv"])                      # qkv_proj.weight grad [3D, D]
+        if want["fc1"]:
+            _wgrad(dz[:, qp:], ZP, 2 * Hf, h, D, D, M, out=bg["fc1"])             # fc1.weight grad [2Hf, D], fc1's own row order
+        dx_in = None
+        if stage >= 3:
+            dx_in = torch.empty(M, D, dtype=BF, device=dev)
+            dw1 = torch.zeros(D, dtype=torch.float32, device=dev)
+            _check(lib.vtk_rmsnorm_bwd(x.data_ptr(), dh.data_ptr(), n1.data_ptr(), dx.data_ptr(), dx_in.data_ptr(), dw1.data_ptr(),
+                                       M, D, 1e-6, st))
+            bg["norm1"] = dw1
+        if sync is not None and flat.numel():   # this block's weight gradients leave for the all-reduce while the next block computes
             sync.reduce(flat)
             for k in ("qkv", "fc1", "out", "fc2"):
-                bg[k]._vtk_reduced = True
-        grads.append(bg)
+                if want[k]:
+                    bg[k]._vtk_reduced = True
+        grads[li] = bg
         dx = dx_in
-    grads.reverse()
     xin = saved["xin"]
-    cin = xin.shape[-1]
-    dwa = _wgrad(dx, D, D, xin.reshape(M, cin), cin, cin, M)                     # [D, cin]
-    dba = _colsum(dx, D, M, D)
-    dxin = _dgrad(dx, D, sw.wa, M, cin, D) if need_dxin else None               # [M, cin]
+    cin = xin.shape[-1] if xin is not None else 0
+    dwa = _wgrad(dx, D, D, xin.reshape(M, cin), cin, cin, M) if plan.embed[0] else None       # [D, cin]
+    dba = _colsum(dx, D, M, D) if plan.embed[1] else None
+    dxin = _dgrad(dx, D, sw.wa, M, sw.wa.shape[1], D) if plan.dinput else None                 # [M, cin]
     return grads, dwa, dba, dxin
 
 
 class AETrainFunction(torch.autograd.Function):
-    """patches -> reconstructed patches with gradients for every AE parameter (reference AE.forward, ae.py:245-251)."""
+    """The training forward of the sides the model has (reference AE.forward, ae.py:245-251): patches -> reconstructed patches,
+    patches -> z (``AE(decoder=False)``) or z -> patches (``AE(encoder=False)``), with the gradients ``ctx.needs_input_grad`` asks
+    for -- of the parameters and of the input -- and no others (``_grad_plan``)."""
 
     @staticmethod
-    def forward(ctx, model, patches, row, col, mask, *params):
-        with _lib.device_of(patches, *params):
-            return AETrainFunction._forward(ctx, model, patches, row, col, mask, *params)
+    def forward(ctx, model, x, row, col, mask, *params):
+        with _lib.device_of(x, *params):
+            return AETrainFunction._forward(ctx, model, x, row, col, mask, *params)
 
     @staticmethod
-    def _forward(ctx, model, patches, row, col, mask, *params):
+    def _forward(ctx, model, x_in, row, col, mask, *params):
         lib = _lib.load()
-        B, N, P = patches.shape
-        dev = patches.device
+        B, N, cin = x_in.shape
+        want = model.pixels_per_token if model.is_encoder else model.channels_per_token
+        if cin != want:
+            raise RuntimeError(f"shape mismatch: last dim {cin} != {want}")
+        dev = x_in.device
+        names = [n for n, _ in model.named_parameters()]
+        needs = dict(zip(names, ctx.needs_input_grad[5:]))
+        sides = {s[0]: len(s[3]) for s in model._sides()}
+        plan = _grad_plan(needs, sides, bool(ctx.needs_input_grad[1]))
         pk = _Packing(mask.to(dev), B, N) if _packs(model, mask) else None    # (packed row counts are multiples of 16)
         if pk is None and (B * N) % 8:
             raise ValueError("vitok_b200 training: B * N must be a multiple of 8 (token count is the K dimension of the wgrad GEMMs)")
-        enc_w, dec_w = _SideWeights(model, 0), _SideWeights(model, 1)
+        sw_ = {side: _SideWeights(model, side) for side in sorted(sides)}
         row = row.to(device=dev, dtype=torch.int64).contiguous()
         col = col.to(device=dev, dtype=torch.int64).contiguous()
         # padded step: each image's key length (train_forward has made every mask a prefix mask); the packed step's attention
         # reads the lengths from its plan.  The sdpa backend (a mask given) ignores the sliding window.
         kv = _lib.kv_len(mask.to(dev).bool()) if mask is not None and pk is None else None
         window = int(model.sw) if (model.sw and mask is None) else -1
-        xin = (_lib.cast_to_bf16(patches) if patches.dtype == torch.float32 else patches).contiguous().view(B * N, P)
+        x = (_lib.cast_to_bf16(x_in) if x_in.dtype == torch.float32 else x_in).contiguous().view(B * N, cin)
         M, C = B * N, model.channels_per_token
         if pk is not None:
-            xin, row, col, M = pk.pack(xin), pk.pack_index(row), pk.pack_index(col), pk.M
-        s_enc, s_dec = {}, {}
-        x = _side_forward(lib, model, enc_w, 0, xin, row, col, kv, window, B, N, s_enc, pk)
-        zlin = _linear(x, x.shape[1], enc_w.wb, enc_w.bb, M, C, x.shape[1])
-        z = torch.empty(M, C, dtype=BF, device=dev)
-        _check(lib.vtk_layernorm_fwd(zlin.data_ptr(), z.data_ptr(), M, C, 1e-6, _lib.stream_ptr()))
-        xd = _side_forward(lib, model, dec_w, 1, z, row, col, kv, window, B, N, s_dec, pk)
-        out = _linear(xd, xd.shape[1], dec_w.wb, dec_w.bb, M, P, xd.shape[1])
+            x, row, col, M = pk.pack(x), pk.pack_index(row), pk.pack_index(col), pk.M
+        saved = {}
+        ctx.zlin = None
+        for side, w in sw_.items():
+            s = saved[side] = {}
+            sp = plan[side]
+            h = _side_forward(lib, model, w, side, x, row, col, kv, window, B, N, s, sp.save_from, pk)
+            if not sp.embed[0]:
+                s["xin"] = None
+            if not sp.head[0]:
+                s["x_final"] = None
+            if side == 0:          # latent bottleneck: to_code, then LayerNorm without affine
+                zlin = _linear(h, h.shape[1], w.wb, w.bb, M, C, h.shape[1])
+                x = torch.empty(M, C, dtype=BF, device=dev)
+                _check(lib.vtk_layernorm_fwd(zlin.data_ptr(), x.data_ptr(), M, C, 1e-6, _lib.stream_ptr()))
+                if sp.top or any(sp.head):
+                    ctx.zlin = zlin
+            else:
+                x = _linear(h, h.shape[1], w.wb, w.bb, M, model.pixels_per_token, h.shape[1])
         # activations live on ctx (not save_for_backward: they are workspace of the backward kernels, freed block by block while it
         # runs); a second backward through the same graph is therefore refused with a clear error in backward()
-        ctx.model, ctx.enc_w, ctx.dec_w, ctx.s_enc, ctx.s_dec = model, enc_w, dec_w, s_enc, s_dec
-        ctx.zlin, ctx.shape, ctx.names = zlin, (B, N, P, C), [n for n, _ in model.named_parameters()]
+        ctx.model, ctx.sw, ctx.saved, ctx.plan = model, sw_, saved, plan
+        ctx.shape, ctx.names, ctx.needs = (B, N, cin, C), names, needs
         ctx.param_dtypes = [p.dtype for p in params]
-        ctx.patches_dtype = patches.dtype
+        ctx.in_dtype = x_in.dtype
         ctx.pk = pk
-        return out.view(B, N, P) if pk is None else pk.unpack(out)
+        return x.view(B, N, x.shape[1]) if pk is None else pk.unpack(x)
 
     @staticmethod
     def backward(ctx, dout):
-        if ctx.s_dec is None:
+        if ctx.saved is None:
             raise RuntimeError("vitok_b200 training: backward was already run through this forward pass -- its activations are "
                                "released while the backward kernels consume them (retain_graph / double backward is not "
                                "supported; run model(batch) again)")
@@ -470,60 +582,68 @@ class AETrainFunction(torch.autograd.Function):
     @staticmethod
     def _backward(ctx, dout):
         lib = _lib.load()
-        model, enc_w, dec_w = ctx.model, ctx.enc_w, ctx.dec_w
-        B, N, P, C = ctx.shape
+        model, plan, sw_, saved = ctx.model, ctx.plan, ctx.sw, ctx.saved
+        B, N, cin, C = ctx.shape
         pk = ctx.pk
         M = B * N if pk is None else pk.M
-        dout = dout.to(BF).contiguous().view(B * N, P)
+        cout = dout.shape[-1]
+        dout = dout.to(BF).contiguous().view(B * N, cout)
         if pk is not None:
             dout = pk.pack(dout)           # pad rows 0: no gradient enters them, every weight gradient sums over valid tokens only
-        g: Dict[str, torch.Tensor] = {}
-        # decoder: to_pixels, blocks, decoder_embed
-        xd = ctx.s_dec["x_final"]
-        Dd = xd.shape[1]
-        g["to_pixels.weight"] = _wgrad(dout, P, P, xd, Dd, Dd, M)
-        g["to_pixels.bias"] = _colsum(dout, P, M, P)
-        dx = _dgrad(dout, P, dec_w.wb, M, Dd, P)
+        g: Dict[str, Optional[torch.Tensor]] = {}
         grp = getattr(model, "_grad_sync_group", None)
         sync = _GradSync(grp[0]) if grp is not None else None
-        blocks, dwa, dba, dz = _side_backward(lib, model, dec_w, 1, dx, ctx.s_dec, B, N, True, sync)
-        g["decoder_embed.weight"], g["decoder_embed.bias"] = dwa, dba
-        for i, bg in enumerate(blocks):
-            _name_block(g, f"decoder_blocks.{i}.", bg)
-        # latent bottleneck: LayerNorm (no affine) + to_code
-        dzlin = torch.empty(M, C, dtype=BF, device=dout.device)
-        _check(lib.vtk_layernorm_bwd(ctx.zlin.data_ptr(), dz.data_ptr(), dzlin.data_ptr(), M, C, 1e-6, _lib.stream_ptr()))
-        xe = ctx.s_enc["x_final"]
-        De = xe.shape[1]
-        g["to_code.weight"] = _wgrad(dzlin, C, C, xe, De, De, M)
-        g["to_code.bias"] = _colsum(dzlin, C, M, C)
-        dx = _dgrad(dzlin, C, enc_w.wb, M, De, C)
-        need_dpatches = bool(ctx.needs_input_grad[1])
-        blocks, dwa, dba, dpatches = _side_backward(lib, model, enc_w, 0, dx, ctx.s_enc, B, N, need_dpatches, sync)
-        g["patch_embed.weight"], g["patch_embed.bias"] = dwa, dba
-        for i, bg in enumerate(blocks):
-            _name_block(g, f"encoder_blocks.{i}.", bg)
+        dz = dout                          # gradient w.r.t. z (None: nothing below z needs one)
+        dinput = None
+        if 1 in plan:                      # decoder: to_pixels, blocks, decoder_embed
+            sp, w, s = plan[1], sw_[1], saved[1]
+            Dd = w.wb.shape[1]
+            if sp.head[0]:
+                g["to_pixels.weight"] = _wgrad(dout, cout, cout, s["x_final"], Dd, Dd, M)
+            if sp.head[1]:
+                g["to_pixels.bias"] = _colsum(dout, cout, M, cout)
+            dx = _dgrad(dout, cout, w.wb, M, Dd, cout) if sp.top else None
+            blocks, g["decoder_embed.weight"], g["decoder_embed.bias"], dz = _side_backward(lib, model, w, 1, dx, s, B, N, sp, sync)
+            for i in sorted(blocks):
+                _name_block(g, f"decoder_blocks.{i}.", blocks[i])
+            dinput = dz
+        if ctx.zlin is not None:           # latent bottleneck: LayerNorm (no affine) + to_code, then the encoder
+            sp, w, s = plan[0], sw_[0], saved[0]
+            dzlin = torch.empty(M, C, dtype=BF, device=dout.device)
+            _check(lib.vtk_layernorm_bwd(ctx.zlin.data_ptr(), dz.data_ptr(), dzlin.data_ptr(), M, C, 1e-6, _lib.stream_ptr()))
+            De = w.wb.shape[1]
+            if sp.head[0]:
+                g["to_code.weight"] = _wgrad(dzlin, C, C, s["x_final"], De, De, M)
+            if sp.head[1]:
+                g["to_code.bias"] = _colsum(dzlin, C, M, C)
+            dx = _dgrad(dzlin, C, w.wb, M, De, C) if sp.top else None
+            blocks, g["patch_embed.weight"], g["patch_embed.bias"], dinput = _side_backward(lib, model, w, 0, dx, s, B, N, sp, sync)
+            for i in sorted(blocks):
+                _name_block(g, f"encoder_blocks.{i}.", blocks[i])
+        # frozen parameters get no gradient: drop what fell out of a stage that ran for another reason
+        g = {n: t for n, t in g.items() if t is not None and ctx.needs.get(n, False)}
         if sync is not None:
             sync.finish(g)
         grads = []
         for name, dt in zip(ctx.names, ctx.param_dtypes):
             t = g.get(name)
             grads.append(None if t is None else t.to(dt).contiguous())
-        ctx.s_enc = ctx.s_dec = ctx.zlin = ctx.pk = None
-        if dpatches is not None:
-            dpatches = (dpatches.view(B, N, P) if pk is None else pk.unpack(dpatches)).to(ctx.patches_dtype)
-        return (None, dpatches, None, None, None, *grads)
+        ctx.saved = ctx.sw = ctx.zlin = ctx.pk = None
+        if dinput is not None and ctx.needs_input_grad[1]:
+            dinput = (dinput.view(B, N, cin) if pk is None else pk.unpack(dinput)).to(ctx.in_dtype)
+        else:
+            dinput = None
+        return (None, dinput, None, None, None, *grads)
+
+
+_BLOCK_GRAD_NAMES = dict(qkv="attn.qkv_proj.weight", out="attn.out_proj.weight", fc1="ffn.fc1.weight", fc2="ffn.fc2.weight",
+                         norm1="norm1.weight", norm_q="attn.norm_q.weight", norm_k="attn.norm_k.weight", gamma="layer_scale.gamma")
 
 
 def _name_block(g: Dict[str, torch.Tensor], prefix: str, bg: Dict[str, torch.Tensor]) -> None:
-    g[prefix + "attn.qkv_proj.weight"] = bg["qkv"]
-    g[prefix + "attn.out_proj.weight"] = bg["out"]
-    g[prefix + "ffn.fc1.weight"] = bg["fc1"]
-    g[prefix + "ffn.fc2.weight"] = bg["fc2"]
-    g[prefix + "norm1.weight"] = bg["norm1"]
-    g[prefix + "attn.norm_q.weight"] = bg["norm_q"]
-    g[prefix + "attn.norm_k.weight"] = bg["norm_k"]
-    g[prefix + "layer_scale.gamma"] = bg["gamma"]
+    for k, n in _BLOCK_GRAD_NAMES.items():
+        if k in bg:
+            g[prefix + n] = bg[k]
 
 
 def _packs(model, mask: Optional[torch.Tensor]) -> bool:
@@ -546,30 +666,34 @@ def _prefix_permutation(mask: torch.Tensor):
 
 
 def train_forward(model, patch_dict: Dict[str, torch.Tensor]) -> Dict[str, torch.Tensor]:
-    """AE.forward in training mode (ae.py:245-251): same dict contract as encode -> decode."""
-    if not (model.is_encoder and model.is_decoder):
-        raise NotImplementedError("vitok_b200: the training step needs both halves (encoder=True, decoder=True)")
-    patches = patch_dict["patches"]
-    if not patches.is_cuda:
+    """AE.forward in training mode (ae.py:245-251): same dict contract as encode -> decode.  ``AE(encoder=False)`` decodes
+    ``patch_dict["z"]``; ``AE(decoder=False)`` returns the encode dict, whose z carries the graph."""
+    x = patch_dict["patches" if model.is_encoder else "z"]
+    if not x.is_cuda:
         raise RuntimeError("vitok_b200.AE: inputs must be CUDA tensors (there is no CPU path)")
     mask = patch_dict.get("patch_mask") if model.attn_backend == "sdpa" else None
     params = [p for _, p in model.named_parameters()]
     row, col = patch_dict["row_idx"], patch_dict["col_idx"]
     # (the packed layout keeps every image's valid tokens in order for any mask: no permutation)
-    pp = _prefix_permutation(mask.to(patches.device)) if mask is not None and not _packs(model, mask) else None
+    pp = _prefix_permutation(mask.to(x.device)) if mask is not None and not _packs(model, mask) else None
     if pp is None:
-        out = AETrainFunction.apply(model, patches, row, col, mask, *params)
+        out = AETrainFunction.apply(model, x, row, col, mask, *params)
     else:
         # a mask with holes: move every image's valid tokens to the front (pure index plumbing; the model only sees positions
         # through row_idx / col_idx, which travel with the tokens), run the prefix-mask path, and move the outputs back
         perm, inv = pp
-        pe = perm[:, :, None].expand(-1, -1, patches.shape[-1])
-        out_p = AETrainFunction.apply(model, patches.gather(1, pe), row.to(perm.device).gather(1, perm), col.to(perm.device).gather(1, perm),
+        pe = perm[:, :, None].expand(-1, -1, x.shape[-1])
+        out_p = AETrainFunction.apply(model, x.gather(1, pe), row.to(perm.device).gather(1, perm), col.to(perm.device).gather(1, perm),
                                       mask.to(perm.device).gather(1, perm), *params)
         out = out_p.gather(1, inv[:, :, None].expand(-1, -1, out_p.shape[-1]))
     pdtype = params[0].dtype
     if pdtype == torch.float32 and not torch.is_autocast_enabled():
         out = out.float()
+    if not model.is_decoder:
+        return {
+            "patch_mask": patch_dict.get("patch_mask"), "row_idx": patch_dict["row_idx"], "col_idx": patch_dict["col_idx"],
+            "orig_height": patch_dict.get("orig_height"), "orig_width": patch_dict.get("orig_width"), "z": out,
+        }
     return {
         "patch_mask": patch_dict.get("patch_mask"), "row_idx": patch_dict.get("row_idx"), "col_idx": patch_dict.get("col_idx"),
         "orig_height": patch_dict.get("orig_height"), "orig_width": patch_dict.get("orig_width"), "patches": out,
