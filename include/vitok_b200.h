@@ -105,6 +105,31 @@ int vtk_unpatchify(const void* patches, int dtype, const uint8_t* patch_mask, co
                    const int64_t* col_idx, int B, int N, int patch, int gy, int gx, int* cell_map, void* out,
                    int out_format, int* status, void* stream);
 
+/* Per-tile SSIM of a NaFlex patch batch against its target, forward and backward: the SSIM tile loss of
+ * scripts/train_vae.py:328-368 (the reference unpatchifies with torch fold / scatter, crops tiles and runs torchmetrics'
+ * StructuralSimilarityIndexMeasure on them).  The canvas is read straight from the token layout, never written: pixel (y, x) of
+ * image b is unpatchify's (vtk_unpatchify's cell map on the grid gy x gx; masked tokens and empty cells read 0), mapped to
+ * [0, 1] by format 0 = minus_one_to_one ((v + 1) / 2) or 1 = zero_to_one (v), no clamping.  SSIM: 11 x 11 gaussian window,
+ * sigma 1.5, K1 = 0.01, K2 = 0.03, data_range 1, per channel, averaged over the 3 channels and every window position lying
+ * entirely inside the tile.
+ * pred / target: [B, N, 3 p^2], dtype 0 = float32, 1 = bfloat16 each; patch_mask [B, N] bool bytes; row / col [B, N] int64.
+ * tiles      : [T, 5] int32 (image, y0, x0, h, w) in canvas pixels; the caller keeps each inside its image (h, w >= 11).
+ *              max_tile_h / max_tile_w bound every tile's h / w (they size the forward grid and the workspace).
+ * out        : [T] fp32 tile values (vtk_ssim_fwd).  Per-tile sums run in a fixed order with no float atomics: bit-identical run to
+ *              run, and a tile's value does not depend on the other tiles of the call.
+ * gout, dpred: vtk_ssim_bwd writes dpred [B, N, 3 p^2] in pred's dtype = sum_t gout[t] d out[t] / d pred (recomputing the
+ *              moments, nothing is kept from the forward); 0 for masked tokens, tokens that own no canvas pixel and pixels outside
+ *              every tile.
+ * workspace  : vtk_ssim_workspace_bytes(B, gy, gx, T, max_tile_h, max_tile_w) bytes of device memory (cell map + block sums). */
+size_t vtk_ssim_workspace_bytes(int B, int gy, int gx, int T, int max_tile_h, int max_tile_w);
+int vtk_ssim_fwd(const void* pred, int pred_dtype, const void* target, int target_dtype, const uint8_t* patch_mask,
+                 const int64_t* row_idx, const int64_t* col_idx, int B, int N, int patch, int gy, int gx, const int* tiles, int T,
+                 int max_tile_h, int max_tile_w, int format, float* out, void* workspace, size_t workspace_bytes, void* stream);
+int vtk_ssim_bwd(const void* pred, int pred_dtype, const void* target, int target_dtype, const uint8_t* patch_mask,
+                 const int64_t* row_idx, const int64_t* col_idx, int B, int N, int patch, int gy, int gx, const int* tiles, int T,
+                 int max_tile_h, int max_tile_w, int format, const float* gout, void* dpred, void* workspace, size_t workspace_bytes,
+                 void* stream);
+
 /* ------------------------------------------------------------------------------------------------
  * Kernel-level entry points (used by the parity tests and by vtk_ae_* internally)
  * ---------------------------------------------------------------------------------------------- */

@@ -19,7 +19,7 @@ CSRC = os.path.join(HERE, "csrc")
 OUT_DIR = os.path.join(HERE, "vitok_b200")
 LIB = os.path.join(OUT_DIR, "libvitok_b200.so")
 OBJ_DIR = os.path.join(HERE, "build")
-SOURCES = ["vtk_api.cu", "vtk_gemm.cu", "vtk_attention.cu", "vtk_elementwise.cu", "vtk_pp.cu", "vtk_train.cu", "vtk_attention_bwd.cu"]
+SOURCES = ["vtk_api.cu", "vtk_gemm.cu", "vtk_attention.cu", "vtk_elementwise.cu", "vtk_pp.cu", "vtk_train.cu", "vtk_attention_bwd.cu", "vtk_ssim.cu"]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-std=c++17", "-lineinfo",
     "-Xcompiler", "-fPIC,-fvisibility=hidden", "--expt-relaxed-constexpr",

@@ -347,6 +347,43 @@ int vtk_unpatchify(const void* patches, int dtype, const uint8_t* patch_mask, co
   return launch_unpatchify(a, (cudaStream_t)stream);
 }
 
+static int ssim_call(const void* pred, int pred_dtype, const void* target, int target_dtype, const uint8_t* patch_mask,
+                     const int64_t* row_idx, const int64_t* col_idx, int B, int N, int patch, int gy, int gx, const int* tiles, int T,
+                     int max_tile_h, int max_tile_w, int format, float* out, const float* gout, void* dpred, void* workspace,
+                     size_t workspace_bytes, void* stream) {
+  VTK_REQUIRE(pred && target && patch_mask && row_idx && col_idx && tiles && workspace, "vtk_ssim: null pointer");
+  VTK_REQUIRE((pred_dtype == 0 || pred_dtype == 1) && (target_dtype == 0 || target_dtype == 1),
+              "vtk_ssim: dtypes must be 0 (f32) or 1 (bf16)");
+  VTK_REQUIRE(format == 0 || format == 1, "vtk_ssim: format must be 0 (minus_one_to_one) or 1 (zero_to_one)");
+  SsimArgs a;
+  a.pred = pred; a.pred_dtype = pred_dtype; a.target = target; a.target_dtype = target_dtype;
+  a.patch_mask = patch_mask; a.row_idx = row_idx; a.col_idx = col_idx;
+  a.B = B; a.N = N; a.patch = patch; a.gy = gy; a.gx = gx; a.tiles = tiles; a.T = T; a.max_tile_h = max_tile_h;
+  a.max_tile_w = max_tile_w; a.format = format; a.out = out; a.gout = gout; a.dpred = dpred;
+  return launch_ssim(a, out == nullptr, workspace, workspace_bytes, (cudaStream_t)stream);
+}
+
+size_t vtk_ssim_workspace_bytes(int B, int gy, int gx, int T, int max_tile_h, int max_tile_w) {
+  return ssim_workspace_bytes(B, gy, gx, T, max_tile_h, max_tile_w);
+}
+
+int vtk_ssim_fwd(const void* pred, int pred_dtype, const void* target, int target_dtype, const uint8_t* patch_mask,
+                 const int64_t* row_idx, const int64_t* col_idx, int B, int N, int patch, int gy, int gx, const int* tiles, int T,
+                 int max_tile_h, int max_tile_w, int format, float* out, void* workspace, size_t workspace_bytes, void* stream) {
+  VTK_REQUIRE(out, "vtk_ssim_fwd: null pointer");
+  return ssim_call(pred, pred_dtype, target, target_dtype, patch_mask, row_idx, col_idx, B, N, patch, gy, gx, tiles, T, max_tile_h,
+                   max_tile_w, format, out, nullptr, nullptr, workspace, workspace_bytes, stream);
+}
+
+int vtk_ssim_bwd(const void* pred, int pred_dtype, const void* target, int target_dtype, const uint8_t* patch_mask,
+                 const int64_t* row_idx, const int64_t* col_idx, int B, int N, int patch, int gy, int gx, const int* tiles, int T,
+                 int max_tile_h, int max_tile_w, int format, const float* gout, void* dpred, void* workspace, size_t workspace_bytes,
+                 void* stream) {
+  VTK_REQUIRE(gout && dpred, "vtk_ssim_bwd: null pointer");
+  return ssim_call(pred, pred_dtype, target, target_dtype, patch_mask, row_idx, col_idx, B, N, patch, gy, gx, tiles, T, max_tile_h,
+                   max_tile_w, format, nullptr, gout, dpred, workspace, workspace_bytes, stream);
+}
+
 int vtk_rmsnorm_bf16(const void* x, int64_t ldx, const void* w, void* y, int64_t ldy, int M, int D, float eps,
                      void* stream) {
   VTK_REQUIRE(x && w && y, "vtk_rmsnorm_bf16: null pointer");

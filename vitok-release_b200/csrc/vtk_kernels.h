@@ -263,6 +263,9 @@ struct UnpatchifyArgs {
   int* status;                 // set to 1 when a valid token falls outside the canvas
 };
 int launch_unpatchify(const UnpatchifyArgs& a, cudaStream_t stream);
+// unpatchify's cell -> token map alone (memset to -1, then the scatter of the valid tokens); uses patch_mask, row_idx, col_idx,
+// B, N, gy, gx, cell_map and status of `a`
+int launch_cellmap(const UnpatchifyArgs& a, cudaStream_t stream);
 int launch_grid_extent(const uint8_t* mask, const int64_t* row, const int64_t* col, int B, int N, int* out2,
                        cudaStream_t stream);
 
@@ -287,6 +290,21 @@ int launch_rmsnorm_bwd(const bf16* x, const bf16* dh, const bf16* w, const bf16*
 int launch_ln_bwd(const bf16* zlin, const bf16* dz, bf16* dx, int M, int C, float eps, cudaStream_t st);
 int launch_charbonnier(const bf16* pred, const bf16* target, const uint8_t* mask, const int* n_valid, float* loss_sum, bf16* dpred,
                        int B, int N, int P, float eps, cudaStream_t st);
+// per-tile SSIM on the token layout (vtk_ssim.cu; include/vitok_b200.h: vtk_ssim_fwd / vtk_ssim_bwd)
+struct SsimArgs {
+  const void* pred; int pred_dtype;       // [B, N, 3 p^2], 0 = fp32, 1 = bf16
+  const void* target; int target_dtype;
+  const uint8_t* patch_mask; const int64_t* row_idx; const int64_t* col_idx;   // [B, N]
+  int B, N, patch, gy, gx;                // canvas grid (unpatchify's)
+  const int* tiles; int T;                // [T, 5] int32 (image, y0, x0, h, w)
+  int max_tile_h, max_tile_w;             // bounds of the tiles' h / w (size the forward grid and workspace)
+  int format;                             // 0 = minus_one_to_one, 1 = zero_to_one
+  float* out;                             // forward: [T] fp32
+  const float* gout; void* dpred;         // backward: [T] fp32, [B, N, 3 p^2] in pred's dtype
+  int* cell_map = nullptr; float* partial = nullptr;   // carved from the workspace by launch_ssim
+};
+size_t ssim_workspace_bytes(int B, int gy, int gx, int T, int max_tile_h, int max_tile_w);
+int launch_ssim(const SsimArgs& a, bool backward, void* workspace, size_t workspace_bytes, cudaStream_t st);
 int launch_attn_delta(const bf16* o, long long ldo, const bf16* dob, long long lddo, float* delta, int M, int heads, int d,
                       cudaStream_t st);
 // one tensor of a multi-tensor AdamW step (mirrors vtk_adamw_tensor of include/vitok_b200.h)

@@ -921,18 +921,22 @@ static void unpatchify_dispatch(const UnpatchifyArgs& a, int blocks, cudaStream_
   else (void)launch_k(unpatchify_kernel<T>, dim3(blocks), dim3(256), 0, stream, a);
 }
 
+int launch_cellmap(const UnpatchifyArgs& a, cudaStream_t stream) {
+  const long long cells = (long long)a.B * a.gy * a.gx;
+  if (check_cuda(cudaMemsetAsync(a.cell_map, 0xFF, cells * sizeof(int), stream), "cell_map memset")) return -1;
+  const long long cap = (long long)num_sms() * 16;
+  long long blocks = ((long long)a.B * a.N + 255) / 256;
+  if (blocks > cap) blocks = cap;
+  (void)launch_k(cellmap_kernel, dim3((int)blocks), dim3(256), 0, stream, a);
+  return 0;
+}
+
 int launch_unpatchify(const UnpatchifyArgs& a, cudaStream_t stream) {
   if (a.patch % 4 || a.patch <= 0) { set_error("unpatchify: patch size must be a positive multiple of 4 (got %d)", a.patch); return -2; }
   if (a.gy <= 0 || a.gx <= 0) { set_error("unpatchify: empty canvas %dx%d", a.gy, a.gx); return -2; }
   if (a.B <= 0) return 0;
+  if (int rc = launch_cellmap(a, stream)) return rc;
   const long long cells = (long long)a.B * a.gy * a.gx;
-  if (check_cuda(cudaMemsetAsync(a.cell_map, 0xFF, cells * sizeof(int), stream), "cell_map memset")) return -1;
-  const long long cap = (long long)num_sms() * 16;
-  {
-    long long blocks = ((long long)a.B * a.N + 255) / 256;
-    if (blocks > cap) blocks = cap;
-    (void)launch_k(cellmap_kernel, dim3((int)blocks), dim3(256), 0, stream, a);
-  }
   if (cells >= (1ll << 31)) { set_error("unpatchify: canvas too large"); return -2; }
   long long blocks = (cells + 7) / 8;                    // one warp per cell, 8 warps per CTA
   const long long cap2 = (long long)num_sms() * 8 * 16;

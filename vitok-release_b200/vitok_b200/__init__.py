@@ -12,9 +12,9 @@ from .data import patch_collate_fn
 from .graphs import GraphedAE, GraphedCodec
 from .parallel import shard_by_tokens, shard_range
 from .pretrained import list_pretrained, load_pretrained, save_pretrained
-from .train import FusedAdamW, charbonnier_loss, enable_grad_sync
+from .train import FusedAdamW, charbonnier_loss, enable_grad_sync, ssim
 
 __version__ = "0.1.0"
 __all__ = ["AE", "Model", "decode_variant", "build_transform", "parse_op", "OPS", "patch_collate_fn", "preprocess",
-           "postprocess", "unpatchify", "unpack", "patchify_batch", "pack_images", "patchify_packed", "charbonnier_loss", "FusedAdamW", "enable_grad_sync", "load_pretrained", "list_pretrained",
+           "postprocess", "unpatchify", "unpack", "patchify_batch", "pack_images", "patchify_packed", "charbonnier_loss", "ssim", "FusedAdamW", "enable_grad_sync", "load_pretrained", "list_pretrained",
            "save_pretrained", "shard_range", "shard_by_tokens", "GraphedAE", "GraphedCodec"]

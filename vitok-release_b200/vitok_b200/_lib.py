@@ -56,6 +56,11 @@ SIGNATURES = {
     "vtk_patchify_selftest": (c_int, [c_vp, c_vp]),
     "vtk_grid_extent": (c_int, [c_vp, c_vp, c_vp, c_int, c_int, c_vp, c_vp]),
     "vtk_unpatchify": (c_int, [c_vp, c_int, c_vp, c_vp, c_vp, c_int, c_int, c_int, c_int, c_int, c_vp, c_vp, c_int, c_vp, c_vp]),
+    "vtk_ssim_workspace_bytes": (c_sz, [c_int, c_int, c_int, c_int, c_int, c_int]),
+    "vtk_ssim_fwd": (c_int, [c_vp, c_int, c_vp, c_int, c_vp, c_vp, c_vp, c_int, c_int, c_int, c_int, c_int, c_vp, c_int, c_int, c_int,
+                             c_int, c_vp, c_vp, c_sz, c_vp]),
+    "vtk_ssim_bwd": (c_int, [c_vp, c_int, c_vp, c_int, c_vp, c_vp, c_vp, c_int, c_int, c_int, c_int, c_int, c_vp, c_int, c_int, c_int,
+                             c_int, c_vp, c_vp, c_vp, c_sz, c_vp]),
     "vtk_rmsnorm_bf16": (c_int, [c_vp, c_i64, c_vp, c_vp, c_i64, c_int, c_int, c_f32, c_vp]),
     "vtk_rope_table": (c_int, [c_vp, c_vp, c_vp, c_vp, c_int, c_int, c_vp]),
     "vtk_cast_f32_to_bf16": (c_int, [c_vp, c_vp, c_i64, c_vp]),

@@ -7,7 +7,7 @@ GEMM (data gradients against the weights as stored, weight gradients on transpos
 streams, the autograd graph edge, the random draw of stochastic depth and -- under DDP (train_vae.py:172) -- the NCCL
 gradient all-reduce.
 
-Also here: ``charbonnier_loss`` (train_vae.py:314-320) and ``FusedAdamW`` (train_vae.py:200-208: AdamW with fp32 master
+Also here: ``charbonnier_loss`` (train_vae.py:314-320), ``ssim`` (the SSIM tile loss term, train_vae.py:328-368; csrc/vtk_ssim.cu) and ``FusedAdamW`` (train_vae.py:200-208: AdamW with fp32 master
 weights and fp32 moments, multi-tensor).
 
 Saved per block (bf16 unless noted): x (block input), h = RMSNorm(x), zraw = [h Wqkv^T | pad | h W1^T], qkv (normed + roped),
@@ -738,6 +738,159 @@ def charbonnier_loss(pred: torch.Tensor, target: torch.Tensor, patch_mask: Optio
     """sqrt(diff^2 + eps^2) averaged over pixels, then over each image's valid tokens, then over the batch
     (scripts/train_vae.py:314-320), forward and gradient in one kernel."""
     return _Charbonnier.apply(pred, target, patch_mask, eps)
+
+
+_SSIM_FORMATS = {"minus_one_to_one": (0, 0.5), "zero_to_one": (1, 1.0)}
+_SSIM_WIN = 11
+
+
+def _ssim_format(current_format: str) -> int:
+    """Format code of the SSIM kernels: values are mapped to [0, 1] before SSIM, (v + 1) / 2 for "minus_one_to_one" and v for
+    "zero_to_one"; anything else is a ValueError (SSIM's luminance term is not shift-invariant, so the mapping is part of the
+    definition)."""
+    if current_format not in _SSIM_FORMATS:
+        raise ValueError(f"vitok_b200.ssim: current_format must be one of {sorted(_SSIM_FORMATS)}, got {current_format!r}")
+    return _SSIM_FORMATS[current_format][0]
+
+
+def _ssim_default_tiles(orig_height: torch.Tensor, orig_width: torch.Tensor) -> torch.Tensor:
+    """One tile per image, (b, 0, 0, orig_height[b], orig_width[b]): the region ``unpack`` returns.  [B, 5] int32 on the device of
+    the sizes."""
+    oh = torch.as_tensor(orig_height).reshape(-1)
+    ow = torch.as_tensor(orig_width).reshape(-1).to(oh.device)
+    if oh.numel() != ow.numel():
+        raise ValueError("vitok_b200.ssim: orig_height and orig_width differ in length")
+    b = torch.arange(oh.numel(), device=oh.device)
+    z = torch.zeros_like(b)
+    return torch.stack([b, z, z, oh.to(b.dtype), ow.to(b.dtype)], dim=1).to(torch.int32)
+
+
+def _ssim_check_tiles(tiles: torch.Tensor, orig_height, orig_width) -> None:
+    """Host-side validation of a [T, 5] tile table (image, y0, x0, h, w) against the images' orig_height x orig_width: every tile
+    lies inside its image and is at least 11 x 11 (one whole window).  Raises ValueError."""
+    if tiles.ndim != 2 or tiles.shape[1] != 5:
+        raise ValueError(f"vitok_b200.ssim: tiles must be [T, 5] (image, y0, x0, h, w), got {tuple(tiles.shape)}")
+    if tiles.dtype.is_floating_point or tiles.dtype == torch.bool:
+        raise ValueError(f"vitok_b200.ssim: tiles must be an integer tensor, got {tiles.dtype}")
+    if tiles.shape[0] == 0:
+        raise ValueError("vitok_b200.ssim: no tiles")
+    if tiles.shape[0] > 65535:
+        raise ValueError(f"vitok_b200.ssim: at most 65535 tiles per call, got {tiles.shape[0]}")
+    t = tiles.to(torch.int64)
+    oh = torch.as_tensor(orig_height).reshape(-1).to(torch.int64)
+    ow = torch.as_tensor(orig_width).reshape(-1).to(torch.int64)
+    b, y0, x0, h, w = t.unbind(1)
+    bad_b = (b < 0) | (b >= oh.numel())
+    if bool(bad_b.any()):
+        i = int(bad_b.nonzero()[0])
+        raise ValueError(f"vitok_b200.ssim: tile {i} names image {int(b[i])} of a batch of {oh.numel()}")
+    small = (h < _SSIM_WIN) | (w < _SSIM_WIN)
+    if bool(small.any()):
+        i = int(small.nonzero()[0])
+        raise ValueError(f"vitok_b200.ssim: tile {i} is {int(h[i])} x {int(w[i])}; tiles must be at least {_SSIM_WIN} x {_SSIM_WIN}")
+    outside = (y0 < 0) | (x0 < 0) | (y0 + h > oh[b]) | (x0 + w > ow[b])
+    if bool(outside.any()):
+        i = int(outside.nonzero()[0])
+        raise ValueError(f"vitok_b200.ssim: tile {i} = {t[i].tolist()} does not lie inside its image's "
+                         f"{int(oh[b[i]])} x {int(ow[b[i]])} pixels")
+
+
+class _SSIM(torch.autograd.Function):
+    @staticmethod
+    def forward(ctx, pred, target, m8, row, col, tiles, geo, fmt):
+        B, N, patch, gy, gx, max_h, max_w = geo
+        dev = pred.device
+        T = tiles.shape[0]
+        lib = _lib.load()
+        out = torch.empty(T, dtype=torch.float32, device=dev)
+        with _lib.device_of(pred, target, tiles):
+            ws_bytes = lib.vtk_ssim_workspace_bytes(B, gy, gx, T, max_h, max_w)
+            ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
+            _check(lib.vtk_ssim_fwd(pred.data_ptr(), 0 if pred.dtype == torch.float32 else 1, target.data_ptr(),
+                                    0 if target.dtype == torch.float32 else 1, m8.data_ptr(), row.data_ptr(), col.data_ptr(), B, N, patch,
+                                    gy, gx, tiles.data_ptr(), T, max_h, max_w, fmt, out.data_ptr(), ws.data_ptr(), ws_bytes,
+                                    _lib.stream_ptr()))
+        ctx.save_for_backward(pred, target, m8, row, col, tiles)
+        ctx.geo, ctx.fmt = geo, fmt
+        return out
+
+    @staticmethod
+    def backward(ctx, gout):
+        pred, target, m8, row, col, tiles = ctx.saved_tensors
+        B, N, patch, gy, gx, max_h, max_w = ctx.geo
+        T = tiles.shape[0]
+        lib = _lib.load()
+        with _lib.device_of(pred):
+            g = gout.detach().to(device=pred.device, dtype=torch.float32).contiguous()
+            dpred = torch.empty_like(pred)
+            ws_bytes = lib.vtk_ssim_workspace_bytes(B, gy, gx, T, max_h, max_w)
+            ws = torch.empty(ws_bytes, dtype=torch.uint8, device=pred.device)
+            _check(lib.vtk_ssim_bwd(pred.data_ptr(), 0 if pred.dtype == torch.float32 else 1, target.data_ptr(),
+                                    0 if target.dtype == torch.float32 else 1, m8.data_ptr(), row.data_ptr(), col.data_ptr(), B, N, patch,
+                                    gy, gx, tiles.data_ptr(), T, max_h, max_w, ctx.fmt, g.data_ptr(), dpred.data_ptr(), ws.data_ptr(),
+                                    ws_bytes, _lib.stream_ptr()))
+        return dpred, None, None, None, None, None, None, None
+
+
+def ssim(pred: torch.Tensor, batch: dict, patch: int = 16, tiles: Optional[torch.Tensor] = None,
+         current_format: str = "minus_one_to_one") -> torch.Tensor:
+    """Per-tile SSIM of ``pred`` against ``batch["patches"]`` on the images' canvases: the SSIM tile loss term of the reference's
+    training loop (scripts/train_vae.py:328-368), ``loss = charbonnier + w * (1 - ssim(out["patches"], batch)).mean()``.
+
+    pred   : [B, N, 3 p^2] bf16 / fp32 (e.g. ``model(batch)["patches"]``); the gradient flows to it, in its dtype and token layout.
+    batch  : the NaFlex dict; "patches" (the target, must not require grad), "patch_mask", "row_idx", "col_idx", "orig_height",
+             "orig_width" are used.
+    tiles  : int [T, 5] of (image, y0, x0, h, w) in canvas pixels, each inside its image's orig_height x orig_width and at least
+             11 x 11; None = one tile per image covering (0, 0, orig_height, orig_width), the region ``unpack`` returns.
+    Returns fp32 [T].
+
+    The canvas is the one ``unpatchify(batch, patch)`` builds (masked tokens read 0; where two valid tokens share a cell the
+    later one wins), its values mapped to [0, 1] ((v + 1) / 2 for "minus_one_to_one", v for "zero_to_one", no clamping).  SSIM is
+    torchmetrics' default (11 x 11 gaussian window, sigma 1.5, K1 = 0.01, K2 = 0.03, data_range 1) per channel, averaged over the 3
+    channels and the window positions lying entirely inside the tile.  The kernels read pixels from the token layout and never
+    write a canvas; forward and backward are deterministic (fixed reduction order, no float atomics), and a tile's value does not
+    depend on the other images of the batch.  One device-to-host copy per call (the tile table, the image sizes and the canvas
+    grid, for validation)."""
+    fmt = _ssim_format(current_format)
+    target = batch["patches"]
+    if target.requires_grad:
+        raise ValueError("vitok_b200.ssim: batch['patches'] requires grad; the SSIM gradient goes to pred only")
+    if not isinstance(patch, int) or patch <= 0:
+        raise ValueError(f"vitok_b200.ssim: patch must be a positive int, got {patch!r}")
+    if pred.ndim != 3 or pred.shape[-1] != 3 * patch * patch:
+        raise ValueError(f"vitok_b200.ssim: pred must be [B, N, 3 * patch^2] = [B, N, {3 * patch * patch}] for patch {patch}, "
+                         f"got {tuple(pred.shape)}")
+    if tuple(target.shape) != tuple(pred.shape):
+        raise ValueError(f"vitok_b200.ssim: pred {tuple(pred.shape)} and batch['patches'] {tuple(target.shape)} differ in shape")
+    for name, t in (("pred", pred), ("batch['patches']", target)):
+        if t.dtype not in (torch.float32, BF):
+            raise ValueError(f"vitok_b200.ssim: {name} must be float32 or bfloat16, got {t.dtype}")
+    if not pred.is_cuda or not target.is_cuda:
+        raise RuntimeError("vitok_b200.ssim: pred and batch['patches'] must be CUDA tensors (there is no CPU path)")
+    dev = pred.device
+    B, N, _ = pred.shape
+    m8 = batch["patch_mask"].to(dev).bool().contiguous().view(torch.uint8)
+    row = batch["row_idx"].to(device=dev, dtype=torch.int64).contiguous()
+    col = batch["col_idx"].to(device=dev, dtype=torch.int64).contiguous()
+    oh = torch.as_tensor(batch["orig_height"]).reshape(-1).to(device=dev, dtype=torch.int64)
+    ow = torch.as_tensor(batch["orig_width"]).reshape(-1).to(device=dev, dtype=torch.int64)
+    if oh.numel() != B or ow.numel() != B:
+        raise ValueError(f"vitok_b200.ssim: orig_height / orig_width must hold one size per image ({B})")
+    tl = _ssim_default_tiles(oh, ow) if tiles is None else torch.as_tensor(tiles)
+    if tl.ndim != 2 or tl.shape[1] != 5 or tl.dtype.is_floating_point or tl.dtype == torch.bool:
+        _ssim_check_tiles(tl, [1], [1])      # raises the shape / dtype error
+    tl = tl.to(device=dev, dtype=torch.int32).contiguous()
+    with _lib.device_of(pred, target, m8, row, col):
+        ext = torch.empty(2, dtype=torch.int32, device=dev)
+        _check(_lib.load().vtk_grid_extent(m8.data_ptr(), row.data_ptr(), col.data_ptr(), B, N, ext.data_ptr(), _lib.stream_ptr()))
+        host = torch.cat([ext.long(), oh, ow, tl.reshape(-1).long()]).cpu()     # the one sync of the call
+    gy, gx = int(host[0]), int(host[1])
+    oh_h, ow_h, tl_h = host[2:2 + B], host[2 + B:2 + 2 * B], host[2 + 2 * B:].reshape(-1, 5)
+    _ssim_check_tiles(tl_h, oh_h, ow_h)
+    if gy == 0 or gx == 0:
+        raise ValueError("vitok_b200.ssim: the batch has no valid token")
+    geo = (B, N, patch, gy, gx, int(tl_h[:, 3].max()), int(tl_h[:, 4].max()))
+    return _SSIM.apply(pred.contiguous(), target.contiguous(), m8, row, col, tl, geo, fmt)
 
 
 class FusedAdamW(torch.optim.Optimizer):
