@@ -296,6 +296,25 @@ typedef struct {
 } vtk_adamw_tensor;
 int vtk_adamw_multi(const vtk_adamw_tensor* tensors, int n_tensors, float lr, float beta1, float beta2, float eps, int step,
                     float grad_scale, void* stream);
+/* vtk_adamw_multi with gradient clipping and an EMA of the master weights in the same pass (vtk_adamw_multi = this with NULL, NULL).
+ *   coef (optional): fp32 device scalar, e.g. norm_coef + 1 of vtk_grad_norm_finish; every gradient is multiplied by it after
+ *     grad_scale (coef == 1 gives the unclipped step bit for bit).
+ *   ema (optional): one fp32 device pointer of n elements per table entry (host array); after the update
+ *     ema = lerp(ema, master, w) with w = (float)(1 - ema_decay), 0 <= ema_decay < 1, in torch.lerp's fp32 arithmetic -- the
+ *     weight is formed in double, as torch._foreach_lerp_(ema, master, 1 - ema_decay) forms it from a Python float.
+ * HBM traffic per bf16 parameter: 28 bytes; with ema 36. */
+int vtk_adamw_multi_ex(const vtk_adamw_tensor* tensors, float* const* ema, int n_tensors, float lr, float beta1, float beta2, float eps,
+                       int step, float grad_scale, const float* coef, double ema_decay, void* stream);
+/* Global L2 norm of the gradients of a vtk_adamw_tensor table (only g, n and g_is_f32 are read), deterministic and without a host
+ * sync.  vtk_grad_sumsq_multi writes partials[slot0 + j] = fp32 sum of g^2 over the j-th 8192-element chunk of the table
+ * (chunks numbered tensor by tensor; vtk_grad_norm_slots(table) of them), so several calls can fill one workspace;
+ * vtk_grad_norm_finish then sums partials[0, n_slots) in a fixed order in double and writes norm_coef[0] = the norm (fp32) and
+ * norm_coef[1] = clamp(max_norm / (norm + 1e-6), max = 1), the clip coefficient of torch.nn.utils.clip_grad_norm_ (NaN for a NaN
+ * norm, 0 for an inf norm; max_norm = inf never clips a finite norm).  HBM traffic: one read of the gradients, 2 bytes per bf16
+ * value and 4 per fp32 value. */
+int64_t vtk_grad_norm_slots(const vtk_adamw_tensor* tensors, int n_tensors);
+int vtk_grad_sumsq_multi(const vtk_adamw_tensor* tensors, int n_tensors, float* partials, int64_t slot0, void* stream);
+int vtk_grad_norm_finish(const float* partials, int64_t n_slots, float max_norm, float* norm_coef, void* stream);
 /* x [n] bf16 *= *scale (fp32 scalar in device memory): the loss gradient arriving at vtk_charbonnier's dpred */
 int vtk_scale_by_dev(void* x, const float* scale, int64_t n, void* stream);
 /* delta [M, heads] fp32 = rowsum over d of dO * O; d % 8 == 0, 8 <= d <= 128 */

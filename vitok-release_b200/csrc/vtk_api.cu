@@ -640,12 +640,31 @@ int vtk_charbonnier(const void* pred, const void* target, const uint8_t* patch_m
   return launch_charbonnier((const bf16*)pred, (const bf16*)target, patch_mask, n_valid, loss_sum, (bf16*)dpred, B, N, P, eps,
                             (cudaStream_t)stream);
 }
-int vtk_adamw_multi(const vtk_adamw_tensor* tensors, int n_tensors, float lr, float beta1, float beta2, float eps, int step,
-                    float grad_scale, void* stream) {
+int vtk_adamw_multi_ex(const vtk_adamw_tensor* tensors, float* const* ema, int n_tensors, float lr, float beta1, float beta2, float eps,
+                       int step, float grad_scale, const float* coef, double ema_decay, void* stream) {
   VTK_REQUIRE(tensors || n_tensors == 0, "vtk_adamw_multi: null tensor table");
   static_assert(sizeof(vtk_adamw_tensor) == sizeof(AdamwTensor), "vtk_adamw_tensor layout");
-  return launch_adamw_multi(reinterpret_cast<const AdamwTensor*>(tensors), n_tensors, lr, beta1, beta2, eps, step, grad_scale,
-                            (cudaStream_t)stream);
+  return launch_adamw_multi(reinterpret_cast<const AdamwTensor*>(tensors), ema, n_tensors, lr, beta1, beta2, eps, step, grad_scale, coef,
+                            ema_decay, (cudaStream_t)stream);
+}
+int vtk_adamw_multi(const vtk_adamw_tensor* tensors, int n_tensors, float lr, float beta1, float beta2, float eps, int step,
+                    float grad_scale, void* stream) {
+  return vtk_adamw_multi_ex(tensors, nullptr, n_tensors, lr, beta1, beta2, eps, step, grad_scale, nullptr, 0.0, stream);
+}
+int64_t vtk_grad_norm_slots(const vtk_adamw_tensor* tensors, int n_tensors) {
+  if (!tensors || n_tensors <= 0) return 0;
+  return grad_norm_slots(reinterpret_cast<const AdamwTensor*>(tensors), n_tensors);
+}
+int vtk_grad_sumsq_multi(const vtk_adamw_tensor* tensors, int n_tensors, float* partials, int64_t slot0, void* stream) {
+  VTK_REQUIRE(tensors || n_tensors == 0, "vtk_grad_sumsq_multi: null tensor table");
+  VTK_REQUIRE(partials || n_tensors == 0, "vtk_grad_sumsq_multi: null partials");
+  VTK_REQUIRE(slot0 >= 0, "vtk_grad_sumsq_multi: slot0 must be >= 0");
+  return launch_grad_sumsq(reinterpret_cast<const AdamwTensor*>(tensors), n_tensors, partials + slot0, (cudaStream_t)stream);
+}
+int vtk_grad_norm_finish(const float* partials, int64_t n_slots, float max_norm, float* norm_coef, void* stream) {
+  VTK_REQUIRE(norm_coef && (partials || n_slots == 0), "vtk_grad_norm_finish: null pointer");
+  VTK_REQUIRE(n_slots >= 0, "vtk_grad_norm_finish: n_slots must be >= 0");
+  return launch_grad_norm_finish(partials, n_slots, max_norm, norm_coef, (cudaStream_t)stream);
 }
 int vtk_scale_by_dev(void* x, const float* scale, int64_t n, void* stream) {
   VTK_REQUIRE(x && scale, "vtk_scale_by_dev: null pointer");

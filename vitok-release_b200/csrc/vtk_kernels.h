@@ -311,8 +311,12 @@ int launch_attn_delta(const bf16* o, long long ldo, const bf16* dob, long long l
 struct AdamwTensor {
   float* master; void* p16; const void* g; float* m; float* v; long long n; float weight_decay; int g_is_f32;
 };
-int launch_adamw_multi(const AdamwTensor* tensors, int n_tensors, float lr, float b1, float b2, float eps, int step, float grad_scale,
-                       cudaStream_t st);
+// ema (optional, one fp32 pointer per tensor) follows the new master with decay ema_decay; coef (optional, device) scales every gradient
+int launch_adamw_multi(const AdamwTensor* tensors, float* const* ema, int n_tensors, float lr, float b1, float b2, float eps, int step,
+                       float grad_scale, const float* coef, double ema_decay, cudaStream_t st);
+long long grad_norm_slots(const AdamwTensor* tensors, int n_tensors);
+int launch_grad_sumsq(const AdamwTensor* tensors, int n_tensors, float* partials, cudaStream_t st);
+int launch_grad_norm_finish(const float* partials, long long n_slots, float max_norm, float* norm_coef, cudaStream_t st);
 int launch_scale_by_dev(bf16* x, const float* scale, long long n, cudaStream_t st);
 
 }  // namespace vtk

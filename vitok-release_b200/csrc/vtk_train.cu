@@ -15,6 +15,7 @@
 #include <stdlib.h>
 
 #include <algorithm>
+#include <type_traits>
 
 #include "vtk_common.cuh"
 #include "vtk_kernels.h"
@@ -653,6 +654,12 @@ __device__ __forceinline__ void adamw_one(float& pf, float gf, float& mf, float&
   pf -= (lr / bc1) * (mf / denom);
 }
 
+// ema + w (master - ema) with torch.lerp's formula (ATen/native/Lerp.h), the fp32 arithmetic torch._foreach_lerp_(ema, master, w)
+// runs: the two branches keep the result exact at w = 0 and w = 1
+__device__ __forceinline__ float ema_lerp(float e, float m, float w) {
+  return fabsf(w) < 0.5f ? e + w * (m - e) : m - (m - e) * (1.f - w);
+}
+
 // ------------------------------------------------------------------------------------------------
 // Multi-tensor AdamW with the reference's optimizer precision (scripts/train_vae.py:200-208 keeps fp32 parameters and fp32
 // Adam moments under autocast): per tensor an fp32 MASTER copy of the parameter and fp32 exp_avg / exp_avg_sq are updated
@@ -660,7 +667,11 @@ __device__ __forceinline__ void adamw_one(float& pf, float gf, float& mf, float&
 // ulp of the weight is therefore not lost (it accumulates in the master).  fp32 model parameters are their own master
 // (p16 == nullptr).  Up to ADAMW_MAX_T tensors per launch travel in the kernel parameters; work is cut into chunks of
 // ADAMW_CHUNK elements and dealt to the blocks round-robin, so one launch covers tensors of any size mix.
-// HBM traffic per parameter: 4 + 4 + 4 (master, m, v) + 2 (bf16 grad) read, 4 + 4 + 4 + 2 written = 28 bytes.
+//   kClip: every gradient is multiplied by *coef (device memory: the clip coefficient of grad_norm_finish_kernel) after
+//          grad_scale; coef == 1 leaves the step bit-identical to the unclipped one.
+//   kEma:  the fp32 EMA of the master follows the new master value in the same pass, ema = lerp(ema, master, ema_w).
+// HBM traffic per parameter: 4 + 4 + 4 (master, m, v) + 2 (bf16 grad) read, 4 + 4 + 4 + 2 written = 28 bytes; kEma adds the
+// EMA's 4 read + 4 written = 36 bytes; kClip adds nothing here (one coefficient per launch).
 // ------------------------------------------------------------------------------------------------
 static constexpr int ADAMW_MAX_T = 64;
 static constexpr int ADAMW_CHUNK = 8192;   // elements per (block, iteration): 256 threads x 4 vectors of 8
@@ -676,20 +687,39 @@ struct AdamwBatch {
   unsigned char g_f32[ADAMW_MAX_T];
   int nt;
 };
+struct AdamwEmaBatch : AdamwBatch {
+  float* ema[ADAMW_MAX_T];
+};
+template <bool kEma>
+using AdamwBatchT = typename std::conditional<kEma, AdamwEmaBatch, AdamwBatch>::type;
 
-__global__ void __launch_bounds__(256) adamw_multi_kernel(const __grid_constant__ AdamwBatch b, float lr, float b1, float b2, float eps,
-                                                          float bc1, float bc2_sqrt, float grad_scale) {
+// tensor of global chunk ch: binary search in chunk0 (nt <= 64)
+__device__ __forceinline__ int chunk_tensor(const AdamwBatch& b, int ch) {
+  int lo = 0, hi = b.nt;
+  while (hi - lo > 1) {
+    const int mid = (lo + hi) >> 1;
+    if (b.chunk0[mid] <= ch) lo = mid; else hi = mid;
+  }
+  return lo;
+}
+
+// gradient as the update sees it: times the host scale, then (clipping) times the device coefficient
+template <bool kClip>
+__device__ __forceinline__ float scaled(float grad_scale, float coef, float g) {
+  float x = g * grad_scale;
+  if constexpr (kClip) x *= coef;
+  return x;
+}
+
+template <bool kClip, bool kEma>
+__global__ void __launch_bounds__(256) adamw_multi_kernel(const __grid_constant__ AdamwBatchT<kEma> b, float lr, float b1, float b2,
+                                                          float eps, float bc1, float bc2_sqrt, float grad_scale,
+                                                          const float* __restrict__ coef, float ema_w) {
   const int total = b.chunk0[b.nt];
+  float cf = 1.f;
+  if constexpr (kClip) cf = __ldg(coef);
   for (int ch = blockIdx.x; ch < total; ch += gridDim.x) {
-    int t = 0;   // tensor of this chunk: binary search in chunk0 (nt <= 64)
-    {
-      int lo = 0, hi = b.nt;
-      while (hi - lo > 1) {
-        const int mid = (lo + hi) >> 1;
-        if (b.chunk0[mid] <= ch) lo = mid; else hi = mid;
-      }
-      t = lo;
-    }
+    const int t = chunk_tensor(b, ch);
     const long long e0 = (long long)(ch - b.chunk0[t]) * ADAMW_CHUNK;
     const long long n = b.n[t];
     const long long e1 = e0 + ADAMW_CHUNK < n ? e0 + ADAMW_CHUNK : n;
@@ -697,10 +727,13 @@ __global__ void __launch_bounds__(256) adamw_multi_kernel(const __grid_constant_
     bf16* __restrict__ pp = b.p16[t];
     float* __restrict__ mm = b.m[t];
     float* __restrict__ vv = b.v[t];
+    float* __restrict__ ee = nullptr;
+    if constexpr (kEma) ee = b.ema[t];
     const float wd = b.wd[t];
     const bool gf32 = b.g_f32[t] != 0;
     const bool vec = ((reinterpret_cast<uintptr_t>(mp) | reinterpret_cast<uintptr_t>(mm) | reinterpret_cast<uintptr_t>(vv) |
-                       reinterpret_cast<uintptr_t>(b.g[t])) & 15) == 0 && (pp == nullptr || (reinterpret_cast<uintptr_t>(pp) & 7) == 0);
+                       reinterpret_cast<uintptr_t>(b.g[t]) | reinterpret_cast<uintptr_t>(ee)) & 15) == 0 &&
+                     (pp == nullptr || (reinterpret_cast<uintptr_t>(pp) & 7) == 0);
     long long i = e0 + 4 * (long long)threadIdx.x;
     if (vec) {
       for (; i + 3 < e1; i += 4 * 256) {   // 4 elements per thread and iteration: 16-byte fp32 vectors, 8-byte bf16 vectors
@@ -713,14 +746,20 @@ __global__ void __launch_bounds__(256) adamw_multi_kernel(const __grid_constant_
           const uint2 q = __ldg(reinterpret_cast<const uint2*>(static_cast<const bf16*>(b.g[t]) + i));
           g4[0] = bf16_lo(q.x); g4[1] = bf16_hi(q.x); g4[2] = bf16_lo(q.y); g4[3] = bf16_hi(q.y);
         }
-        adamw_one(pf.x, g4[0] * grad_scale, mf.x, vf.x, lr, b1, b2, eps, wd, bc1, bc2_sqrt);
-        adamw_one(pf.y, g4[1] * grad_scale, mf.y, vf.y, lr, b1, b2, eps, wd, bc1, bc2_sqrt);
-        adamw_one(pf.z, g4[2] * grad_scale, mf.z, vf.z, lr, b1, b2, eps, wd, bc1, bc2_sqrt);
-        adamw_one(pf.w, g4[3] * grad_scale, mf.w, vf.w, lr, b1, b2, eps, wd, bc1, bc2_sqrt);
+        adamw_one(pf.x, scaled<kClip>(grad_scale, cf, g4[0]), mf.x, vf.x, lr, b1, b2, eps, wd, bc1, bc2_sqrt);
+        adamw_one(pf.y, scaled<kClip>(grad_scale, cf, g4[1]), mf.y, vf.y, lr, b1, b2, eps, wd, bc1, bc2_sqrt);
+        adamw_one(pf.z, scaled<kClip>(grad_scale, cf, g4[2]), mf.z, vf.z, lr, b1, b2, eps, wd, bc1, bc2_sqrt);
+        adamw_one(pf.w, scaled<kClip>(grad_scale, cf, g4[3]), mf.w, vf.w, lr, b1, b2, eps, wd, bc1, bc2_sqrt);
         *reinterpret_cast<float4*>(mp + i) = pf;
         *reinterpret_cast<float4*>(mm + i) = mf;
         *reinterpret_cast<float4*>(vv + i) = vf;
         if (pp) *reinterpret_cast<uint2*>(pp + i) = make_uint2(bf2_cvt(pf.x, pf.y), bf2_cvt(pf.z, pf.w));
+        if constexpr (kEma) {
+          float4 ef = *reinterpret_cast<const float4*>(ee + i);
+          ef.x = ema_lerp(ef.x, pf.x, ema_w); ef.y = ema_lerp(ef.y, pf.y, ema_w);
+          ef.z = ema_lerp(ef.z, pf.z, ema_w); ef.w = ema_lerp(ef.w, pf.w, ema_w);
+          *reinterpret_cast<float4*>(ee + i) = ef;
+        }
       }
       // tail of the chunk (n % 4 elements of the last chunk)
       i = e0 + ((e1 - e0) & ~3LL) + threadIdx.x;
@@ -729,11 +768,87 @@ __global__ void __launch_bounds__(256) adamw_multi_kernel(const __grid_constant_
     }
     for (; i < e1; i += vec ? 256 * 1024 : 256) {
       float pf = mp[i], mf = mm[i], vf = vv[i];
-      const float gf = (gf32 ? static_cast<const float*>(b.g[t])[i] : __bfloat162float(static_cast<const bf16*>(b.g[t])[i])) * grad_scale;
+      const float gf = scaled<kClip>(grad_scale, cf, gf32 ? static_cast<const float*>(b.g[t])[i] : __bfloat162float(static_cast<const bf16*>(b.g[t])[i]));
       adamw_one(pf, gf, mf, vf, lr, b1, b2, eps, wd, bc1, bc2_sqrt);
       mp[i] = pf; mm[i] = mf; vv[i] = vf;
       if (pp) pp[i] = __float2bfloat16_rn(pf);
+      if constexpr (kEma) ee[i] = ema_lerp(ee[i], pf, ema_w);
     }
+  }
+}
+
+// ------------------------------------------------------------------------------------------------
+// Global L2 gradient norm for clipping (torch.nn.utils.clip_grad_norm_), deterministic: grad_sumsq_kernel writes one fp32 sum of
+// squares per ADAMW_CHUNK chunk to its own slot (thread-sequential, then a fixed shuffle tree: no atomics), and the one-CTA
+// grad_norm_finish_kernel adds the slots in a fixed order in fp64.  A chunk's partial depends only on that chunk's gradient values,
+// and its slot only on its position in the tensor table, so the norm does not depend on how the table is cut into launches.
+// HBM traffic per parameter: the gradient read once, 2 bytes (bf16) or 4 (fp32).
+// ------------------------------------------------------------------------------------------------
+__global__ void __launch_bounds__(256) grad_sumsq_kernel(const __grid_constant__ AdamwBatch b, float* __restrict__ partials) {
+  __shared__ float red[8];
+  const int total = b.chunk0[b.nt];
+  for (int ch = blockIdx.x; ch < total; ch += gridDim.x) {
+    const int t = chunk_tensor(b, ch);
+    const long long e0 = (long long)(ch - b.chunk0[t]) * ADAMW_CHUNK;
+    const long long n = b.n[t];
+    const long long e1 = e0 + ADAMW_CHUNK < n ? e0 + ADAMW_CHUNK : n;
+    const bool gf32 = b.g_f32[t] != 0;
+    const char* gp = static_cast<const char*>(b.g[t]);
+    const int esz = gf32 ? 4 : 2;
+    float s = 0.f;
+    long long i = e0 + threadIdx.x;
+    if ((reinterpret_cast<uintptr_t>(gp) & 15) == 0) {   // 16-byte loads: 8 bf16 or 4 fp32 values; 32 values per thread and chunk
+      const int per = 16 / esz;
+      const long long nvec = (e1 - e0) / per;
+      for (long long v = threadIdx.x; v < nvec; v += 256) {
+        const uint4 q = ld_global_nc_v4(gp + (e0 + v * per) * esz);
+        if (gf32) {
+          const float f0 = __uint_as_float(q.x), f1 = __uint_as_float(q.y), f2 = __uint_as_float(q.z), f3 = __uint_as_float(q.w);
+          s = fmaf(f0, f0, s); s = fmaf(f1, f1, s); s = fmaf(f2, f2, s); s = fmaf(f3, f3, s);
+        } else {
+          float f[8];
+          unpack8(q, f);
+#pragma unroll
+          for (int k = 0; k < 8; ++k) s = fmaf(f[k], f[k], s);
+        }
+      }
+      i = e0 + nvec * per + threadIdx.x;                 // the last chunk's n % per values
+    }
+    for (; i < e1; i += 256) {
+      const float x = gf32 ? reinterpret_cast<const float*>(gp)[i] : __bfloat162float(reinterpret_cast<const bf16*>(gp)[i]);
+      s = fmaf(x, x, s);
+    }
+    s = warp_sum(s);
+    if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = s;
+    __syncthreads();
+    if (threadIdx.x < 32) {
+      float r = threadIdx.x < 8 ? red[threadIdx.x] : 0.f;
+      r = warp_sum(r);
+      if (threadIdx.x == 0) partials[ch] = r;
+    }
+    __syncthreads();
+  }
+}
+
+// norm_coef[0] = sqrt(sum of the partials), norm_coef[1] = clamp(max_norm / (norm + 1e-6), max = 1) -- evaluated as torch evaluates
+// it for an fp32 norm (Tensor.__rtruediv__: reciprocal, then times max_norm; clamp keeps NaN), so inf and NaN norms give torch's
+// coefficient (an inf norm: 0; a NaN norm: NaN).
+__global__ void __launch_bounds__(256) grad_norm_finish_kernel(const float* __restrict__ partials, long long n_slots, float max_norm,
+                                                               float* __restrict__ norm_coef) {
+  __shared__ double red[256];
+  double s = 0.0;
+  for (long long i = threadIdx.x; i < n_slots; i += 256) s += (double)partials[i];
+  red[threadIdx.x] = s;
+  __syncthreads();
+  for (int w = 128; w > 0; w >>= 1) {
+    if (threadIdx.x < w) red[threadIdx.x] += red[threadIdx.x + w];
+    __syncthreads();
+  }
+  if (threadIdx.x == 0) {
+    const float norm = (float)sqrt(red[0]);
+    const float c = (1.f / (norm + 1e-6f)) * max_norm;
+    norm_coef[0] = norm;
+    norm_coef[1] = c > 1.f ? 1.f : c;
   }
 }
 
@@ -1193,34 +1308,92 @@ int launch_charbonnier(const bf16* pred, const bf16* target, const uint8_t* mask
   charbonnier_kernel<<<grid_for((long long)B * N, 8), 256, 0, st>>>(pred, target, mask, n_valid, loss_sum, dpred, B, N, P, eps);
   return check_cuda(cudaGetLastError(), "charbonnier launch");
 }
-int launch_adamw_multi(const AdamwTensor* tensors, int n_tensors, float lr, float b1, float b2, float eps, int step, float grad_scale,
-                       cudaStream_t st) {
-  VTK_TRAIN_CHECK(step >= 1, "adamw: step must be >= 1");
-  const float bc1 = 1.f - powf(b1, (float)step), bc2s = sqrtf(1.f - powf(b2, (float)step));
+// The next launch's share of the tensor table from tensors[i] on: at most ADAMW_MAX_T non-empty tensors and fewer than 2^30
+// chunks.  Fills g / n / g_f32 / chunk0 of `bt` (all the norm pass reads) and src[k] = the table index of slot k; returns the
+// batch's chunk count.
+static long long next_adamw_batch(const AdamwTensor* tensors, int n_tensors, int& i, AdamwBatch& bt, int (&src)[ADAMW_MAX_T]) {
+  bt.nt = 0;
+  long long chunks = 0;
+  for (; i < n_tensors && bt.nt < ADAMW_MAX_T; ++i) {
+    const AdamwTensor& t = tensors[i];
+    if (t.n <= 0) continue;
+    const long long c = (t.n + ADAMW_CHUNK - 1) / ADAMW_CHUNK;
+    if (chunks + c >= (1ll << 30)) break;
+    const int k = bt.nt++;
+    src[k] = i;
+    bt.g[k] = t.g; bt.n[k] = t.n; bt.g_f32[k] = t.g_is_f32 ? 1 : 0;
+    bt.chunk0[k] = (int)chunks;
+    chunks += c;
+  }
+  bt.chunk0[bt.nt] = (int)chunks;
+  return chunks;
+}
+
+template <bool kClip, bool kEma>
+static int launch_adamw_t(const AdamwTensor* tensors, float* const* ema, int n_tensors, float lr, float b1, float b2, float eps,
+                          float bc1, float bc2s, float grad_scale, const float* coef, float ema_w, cudaStream_t st) {
   int i = 0;
   while (i < n_tensors) {
-    AdamwBatch bt;
-    bt.nt = 0;
-    long long chunks = 0;
-    for (; i < n_tensors && bt.nt < ADAMW_MAX_T; ++i) {
-      const AdamwTensor& t = tensors[i];
-      if (t.n <= 0) continue;
-      VTK_TRAIN_CHECK(t.master && t.g && t.m && t.v, "adamw: null pointer in tensor %d", i);
-      const long long c = (t.n + ADAMW_CHUNK - 1) / ADAMW_CHUNK;
-      if (chunks + c >= (1ll << 30)) break;
-      const int k = bt.nt++;
-      bt.master[k] = t.master; bt.p16[k] = (bf16*)t.p16; bt.g[k] = t.g; bt.m[k] = t.m; bt.v[k] = t.v; bt.n[k] = t.n;
-      bt.wd[k] = t.weight_decay; bt.g_f32[k] = t.g_is_f32 ? 1 : 0;
-      bt.chunk0[k] = (int)chunks;
-      chunks += c;
-    }
+    AdamwBatchT<kEma> bt;
+    int src[ADAMW_MAX_T];
+    const long long chunks = next_adamw_batch(tensors, n_tensors, i, bt, src);
     if (bt.nt == 0) continue;
-    bt.chunk0[bt.nt] = (int)chunks;
+    for (int k = 0; k < bt.nt; ++k) {
+      const AdamwTensor& t = tensors[src[k]];
+      VTK_TRAIN_CHECK(t.master && t.g && t.m && t.v, "adamw: null pointer in tensor %d", src[k]);
+      bt.master[k] = t.master; bt.p16[k] = (bf16*)t.p16; bt.m[k] = t.m; bt.v[k] = t.v; bt.wd[k] = t.weight_decay;
+      if constexpr (kEma) {
+        VTK_TRAIN_CHECK(ema[src[k]], "adamw: null ema pointer for tensor %d", src[k]);
+        bt.ema[k] = ema[src[k]];
+      }
+    }
     const int grid = (int)std::min<long long>(chunks, (long long)num_sms() * 8);
-    adamw_multi_kernel<<<grid, 256, 0, st>>>(bt, lr, b1, b2, eps, bc1, bc2s, grad_scale);
+    adamw_multi_kernel<kClip, kEma><<<grid, 256, 0, st>>>(bt, lr, b1, b2, eps, bc1, bc2s, grad_scale, coef, ema_w);
     if (check_cuda(cudaGetLastError(), "adamw_multi launch")) return -1;
   }
   return 0;
+}
+
+int launch_adamw_multi(const AdamwTensor* tensors, float* const* ema, int n_tensors, float lr, float b1, float b2, float eps, int step,
+                       float grad_scale, const float* coef, double ema_decay, cudaStream_t st) {
+  VTK_TRAIN_CHECK(step >= 1, "adamw: step must be >= 1");
+  VTK_TRAIN_CHECK(!ema || (ema_decay >= 0.0 && ema_decay < 1.0), "adamw: ema_decay must lie in [0, 1) (got %g)", ema_decay);
+  const float bc1 = 1.f - powf(b1, (float)step), bc2s = sqrtf(1.f - powf(b2, (float)step));
+  const float ema_w = (float)(1.0 - ema_decay);   // the weight torch._foreach_lerp_(ema, master, 1 - decay) rounds to fp32
+  if (coef) {
+    return ema ? launch_adamw_t<true, true>(tensors, ema, n_tensors, lr, b1, b2, eps, bc1, bc2s, grad_scale, coef, ema_w, st)
+               : launch_adamw_t<true, false>(tensors, ema, n_tensors, lr, b1, b2, eps, bc1, bc2s, grad_scale, coef, ema_w, st);
+  }
+  return ema ? launch_adamw_t<false, true>(tensors, ema, n_tensors, lr, b1, b2, eps, bc1, bc2s, grad_scale, coef, ema_w, st)
+             : launch_adamw_t<false, false>(tensors, ema, n_tensors, lr, b1, b2, eps, bc1, bc2s, grad_scale, coef, ema_w, st);
+}
+
+long long grad_norm_slots(const AdamwTensor* tensors, int n_tensors) {
+  long long s = 0;
+  for (int i = 0; i < n_tensors; ++i)
+    if (tensors[i].n > 0) s += (tensors[i].n + ADAMW_CHUNK - 1) / ADAMW_CHUNK;
+  return s;
+}
+
+int launch_grad_sumsq(const AdamwTensor* tensors, int n_tensors, float* partials, cudaStream_t st) {
+  int i = 0;
+  while (i < n_tensors) {
+    AdamwBatch bt;
+    int src[ADAMW_MAX_T];
+    const long long chunks = next_adamw_batch(tensors, n_tensors, i, bt, src);
+    if (bt.nt == 0) continue;
+    for (int k = 0; k < bt.nt; ++k) VTK_TRAIN_CHECK(bt.g[k], "grad_norm: null gradient pointer in tensor %d", src[k]);
+    const int grid = (int)std::min<long long>(chunks, (long long)num_sms() * 8);
+    grad_sumsq_kernel<<<grid, 256, 0, st>>>(bt, partials);
+    if (check_cuda(cudaGetLastError(), "grad_sumsq launch")) return -1;
+    partials += chunks;
+  }
+  return 0;
+}
+
+int launch_grad_norm_finish(const float* partials, long long n_slots, float max_norm, float* norm_coef, cudaStream_t st) {
+  grad_norm_finish_kernel<<<1, 256, 0, st>>>(partials, n_slots, max_norm, norm_coef);
+  return check_cuda(cudaGetLastError(), "grad_norm_finish launch");
 }
 int launch_scale_by_dev(bf16* x, const float* scale, long long n, cudaStream_t st) {
   if (n <= 0) return 0;

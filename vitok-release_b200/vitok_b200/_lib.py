@@ -78,6 +78,11 @@ SIGNATURES = {
     "vtk_resid_fwd_dp": (c_int, [c_vp, c_vp, c_vp, c_vp, c_int, c_int, c_vp, c_int, c_f32, c_vp]),
     "vtk_resid_bwd_dp": (c_int, [c_vp, c_vp, c_vp, c_vp, c_vp, c_int, c_int, c_vp, c_int, c_f32, c_vp]),
     "vtk_adamw_multi": (c_int, [ctypes.POINTER(AdamwTensor), c_int, c_f32, c_f32, c_f32, c_f32, c_int, c_f32, c_vp]),
+    "vtk_adamw_multi_ex": (c_int, [ctypes.POINTER(AdamwTensor), ctypes.POINTER(c_vp), c_int, c_f32, c_f32, c_f32, c_f32, c_int, c_f32,
+                                   c_vp, ctypes.c_double, c_vp]),
+    "vtk_grad_norm_slots": (c_i64, [ctypes.POINTER(AdamwTensor), c_int]),
+    "vtk_grad_sumsq_multi": (c_int, [ctypes.POINTER(AdamwTensor), c_int, c_vp, c_i64, c_vp]),
+    "vtk_grad_norm_finish": (c_int, [c_vp, c_i64, c_f32, c_vp, c_vp]),
     "vtk_scale_by_dev": (c_int, [c_vp, c_vp, c_i64, c_vp]),
     "vtk_linear_ln_bf16": (c_int, [c_vp, c_i64, c_vp, c_i64, c_vp, c_vp, c_i64, c_int, c_int, c_int, c_f32, c_vp]),
     "vtk_qkv_swiglu_bf16": (c_int, [c_vp, c_i64, c_vp, c_i64, c_i64, c_int, c_int, c_int, c_int, c_int, c_vp, c_vp, c_vp,

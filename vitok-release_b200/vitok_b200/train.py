@@ -32,6 +32,7 @@ something below still needs -- blocks below it keep no activations.  ``AE(encode
 """
 from __future__ import annotations
 
+import contextlib
 import ctypes
 from typing import Dict, NamedTuple, Optional, Tuple
 
@@ -900,10 +901,75 @@ class FusedAdamW(torch.optim.Optimizer):
     bf16 ulp of the weight is not lost (at lr 1e-4 that is every weight above ~0.05 and all norm weights).  fp32 model
     parameters are their own master.  torch.optim.AdamW semantics (decoupled weight decay, bias correction); one kernel launch
     per 64 tensors of a param group; 28 bytes of HBM traffic per bf16 parameter.  ``state_dict()`` holds step, master (bf16
-    parameters only), exp_avg, exp_avg_sq per parameter."""
+    parameters only), exp_avg, exp_avg_sq (and ema) per parameter; ``load_state_dict`` keeps them fp32.
 
-    def __init__(self, params, lr=1e-3, betas=(0.9, 0.999), eps=1e-8, weight_decay=1e-2):
+    ``max_grad_norm``: clip by the global L2 norm of every gradient of the step (all groups), as
+    ``torch.nn.utils.clip_grad_norm_(params, max_grad_norm)`` before the step would -- coefficient
+    ``min(max_grad_norm / (norm + 1e-6), 1)`` in fp32 -- but the gradients are scaled inside the AdamW pass, so ``.grad`` is NOT
+    rewritten.  The norm comes from a deterministic pass over the gradients (fp32 sums per 8192-value chunk, added in fp64;
+    bit-identical from run to run, however the tensors are grouped) and stays on the device with the coefficient: no host sync.
+    ``grad_norm`` is the pre-clip norm of the last step as a 0-dim fp32 CUDA tensor (reading it syncs).  ``float("inf")`` computes
+    the norm and never clips.  The parameters must all live on one device.
+
+    ``ema_decay`` (0 <= decay < 1): ``state[p]["ema"]``, an fp32 exponential moving average of the fp32 master weights (not of the
+    bf16-rounded parameters, which stand still at small lr while the master moves), updated in the same pass after every step in
+    which p has a gradient: ``ema = lerp(ema, master, 1 - decay)`` with torch.lerp's fp32 arithmetic.  It starts at the parameter's
+    value when the parameter first gets optimizer state.  ``ema_state_dict(model)`` exports it, ``swap_ema(model)`` evaluates with it.
+    HBM traffic: +8 bytes per parameter for the EMA, +2 (bf16 gradients) or +4 (fp32) for the norm pass."""
+
+    def __init__(self, params, lr=1e-3, betas=(0.9, 0.999), eps=1e-8, weight_decay=1e-2, max_grad_norm=None, ema_decay=None):
+        if max_grad_norm is not None:
+            max_grad_norm = _real_arg("max_grad_norm", max_grad_norm)
+            if not max_grad_norm > 0.0:
+                raise ValueError(f"FusedAdamW: max_grad_norm must be > 0 (float('inf') computes the norm and never clips), got {max_grad_norm}")
+        if ema_decay is not None:
+            ema_decay = _real_arg("ema_decay", ema_decay)
+            if not 0.0 <= ema_decay < 1.0:
+                raise ValueError(f"FusedAdamW: ema_decay must satisfy 0 <= ema_decay < 1, got {ema_decay}")
+        self.max_grad_norm, self.ema_decay = max_grad_norm, ema_decay
+        self.grad_norm: Optional[torch.Tensor] = None
+        self._norm_ws: Optional[torch.Tensor] = None
         super().__init__(params, dict(lr=lr, betas=betas, eps=eps, weight_decay=weight_decay))
+
+    def add_param_group(self, param_group):
+        super().add_param_group(param_group)
+        if self.max_grad_norm is not None:
+            devs = {p.device for g in self.param_groups for p in g["params"]}
+            if len(devs) > 1:
+                raise ValueError(f"FusedAdamW: max_grad_norm needs every parameter on one device (the global norm is not reduced across "
+                                 f"devices); got {sorted(str(d) for d in devs)}")
+
+    @staticmethod
+    def _table(items) -> ctypes.Array:
+        table = (_lib.AdamwTensor * len(items))()
+        for e, (group, p, gr, stt) in zip(table, items):
+            master = stt.get("master")
+            e.master = (master if master is not None else p).data_ptr()
+            e.p16 = p.data_ptr() if master is not None else None
+            e.g = gr.data_ptr()
+            e.m, e.v = stt["exp_avg"].data_ptr(), stt["exp_avg_sq"].data_ptr()
+            e.n = p.numel()
+            e.weight_decay = float(group["weight_decay"])
+            e.g_is_f32 = 1 if gr.dtype == torch.float32 else 0
+        return table
+
+    def _clip_coef(self, lib, items) -> torch.Tensor:
+        """Queue the norm pass over every gradient of ``items``; returns the device coefficient [1] and sets ``grad_norm``."""
+        devs = {it[1].device for it in items}
+        if len(devs) > 1:
+            raise ValueError(f"FusedAdamW: max_grad_norm needs every parameter on one device; got {sorted(str(d) for d in devs)}")
+        dev = devs.pop()
+        table = self._table(items)
+        slots = int(lib.vtk_grad_norm_slots(table, len(items)))
+        if self._norm_ws is None or self._norm_ws.numel() != max(slots, 1) or self._norm_ws.device != dev:
+            self._norm_ws = torch.empty(max(slots, 1), dtype=torch.float32, device=dev)
+        norm_coef = torch.empty(2, dtype=torch.float32, device=dev)     # fresh per step: a grad_norm the caller holds stays valid
+        with torch.cuda.device(dev):
+            st = _lib.stream_ptr()
+            _check(lib.vtk_grad_sumsq_multi(table, len(items), self._norm_ws.data_ptr(), 0, st))
+            _check(lib.vtk_grad_norm_finish(self._norm_ws.data_ptr(), slots, float(self.max_grad_norm), norm_coef.data_ptr(), st))
+        self.grad_norm = norm_coef[0]
+        return norm_coef[1:]
 
     @torch.no_grad()
     def step(self, closure=None):
@@ -912,9 +978,9 @@ class FusedAdamW(torch.optim.Optimizer):
             with torch.enable_grad():
                 loss = closure()
         lib = _lib.load()
+        per_group = []            # (group, p, grad, state) of every parameter with a gradient, group by group
         for group in self.param_groups:
-            b1, b2 = group["betas"]
-            by_dev: Dict[torch.device, list] = {}
+            items = []
             for p in group["params"]:
                 if p.grad is None:
                     continue
@@ -929,30 +995,104 @@ class FusedAdamW(torch.optim.Optimizer):
                         stt["master"] = p.detach().float()
                     stt["exp_avg"] = torch.zeros(p.shape, dtype=torch.float32, device=p.device)
                     stt["exp_avg_sq"] = torch.zeros(p.shape, dtype=torch.float32, device=p.device)
+                if self.ema_decay is not None and "ema" not in stt:
+                    stt["ema"] = p.detach().to(torch.float32, copy=True)
                 stt["step"] += 1
                 gr = p.grad
                 if gr.dtype not in (BF, torch.float32):
                     gr = gr.float()
                 gr = gr.contiguous()
-                by_dev.setdefault(p.device, []).append((p, gr, stt))
-            for dev, items in by_dev.items():
+                items.append((group, p, gr, stt))
+            per_group.append(items)
+        coef = None
+        if self.max_grad_norm is not None and any(per_group):
+            coef = self._clip_coef(lib, [it for items in per_group for it in items])
+        for group, items in zip(self.param_groups, per_group):
+            b1, b2 = group["betas"]
+            by_dev: Dict[torch.device, list] = {}
+            for it in items:
+                by_dev.setdefault(it[1].device, []).append(it)
+            for dev, dev_items in by_dev.items():
                 # parameters of a group share lr / betas / eps / weight decay; their step counts agree unless a parameter
                 # got its first gradient later -- launch per distinct step
-                for step in sorted({it[2]["step"] for it in items}):
-                    sel = [it for it in items if it[2]["step"] == step]
-                    table = (_lib.AdamwTensor * len(sel))()
-                    for e, (p, gr, stt) in zip(table, sel):
-                        master = stt.get("master")
-                        e.master = (master if master is not None else p).data_ptr()
-                        e.p16 = p.data_ptr() if master is not None else None
-                        e.g = gr.data_ptr()
-                        e.m, e.v = stt["exp_avg"].data_ptr(), stt["exp_avg_sq"].data_ptr()
-                        e.n = p.numel()
-                        e.weight_decay = float(group["weight_decay"])
-                        e.g_is_f32 = 1 if gr.dtype == torch.float32 else 0
+                for step in sorted({it[3]["step"] for it in dev_items}):
+                    sel = [it for it in dev_items if it[3]["step"] == step]
+                    table = self._table(sel)
+                    ema = None
+                    if self.ema_decay is not None:
+                        ema = (ctypes.c_void_p * len(sel))(*[it[3]["ema"].data_ptr() for it in sel])
                     with torch.cuda.device(dev):
-                        _check(lib.vtk_adamw_multi(table, len(sel), float(group["lr"]), float(b1), float(b2), float(group["eps"]),
-                                                   int(step), 1.0, _lib.stream_ptr()))
-                    for p, _, _ in sel:
+                        _check(lib.vtk_adamw_multi_ex(table, ema, len(sel), float(group["lr"]), float(b1), float(b2), float(group["eps"]),
+                                                      int(step), 1.0, _lib.ptr(coef), float(self.ema_decay or 0.0), _lib.stream_ptr()))
+                    for _, p, _, _ in sel:
                         torch.autograd.graph.increment_version(p)   # the kernel wrote p in place: invalidate packed copies
         return loss
+
+    def load_state_dict(self, state_dict):
+        """torch.optim.Optimizer.load_state_dict, except that the fp32 state (master, exp_avg, exp_avg_sq, ema) stays fp32: the base
+        class casts floating-point state to each parameter's dtype, which would round it to bf16 for bf16 parameters."""
+        super().load_state_dict(state_dict)
+        saved_ids = [i for g in state_dict["param_groups"] for i in g["params"]]
+        params = [p for g in self.param_groups for p in g["params"]]
+        for i, p in zip(saved_ids, params):
+            saved = state_dict["state"].get(i)
+            if not saved:
+                continue
+            for k in _FP32_STATE:
+                if k in saved:
+                    self.state[p][k] = saved[k].to(device=p.device, dtype=torch.float32, copy=True)
+
+    def _ema_params(self, model, remove_duplicate: bool = True):
+        if self.ema_decay is None:
+            raise ValueError("FusedAdamW: this optimizer keeps no EMA (construct it with ema_decay)")
+        return [(n, p, self.state[p]) for n, p in model.named_parameters(remove_duplicate=remove_duplicate)
+                if p in self.state and "ema" in self.state[p]]
+
+    @torch.no_grad()
+    def ema_state_dict(self, model) -> Dict[str, torch.Tensor]:
+        """``model.state_dict()`` with every parameter that has an EMA replaced by the EMA cast to the parameter's dtype (the release
+        weights of the run); parameters without optimizer state (frozen, or never given a gradient) and buffers keep their current
+        values.  The EMA tensors are copied, never aliased."""
+        sd = model.state_dict()
+        for n, p, stt in self._ema_params(model, remove_duplicate=False):
+            sd[n] = stt["ema"].to(dtype=p.dtype, copy=True)
+        return sd
+
+    @contextlib.contextmanager
+    def swap_ema(self, model):
+        """Evaluate ``model`` with its EMA weights, in place and without extra memory::
+
+            with opt.swap_ema(model):
+                model.eval(); ...
+
+        On entry a bf16 parameter with an EMA is overwritten by bf16(ema) and an fp32 one swaps storage with its EMA; on exit a bf16
+        parameter is re-emitted from its fp32 master and an fp32 one swaps back.  The bf16 exit is exact because after every step a
+        bf16 parameter equals bf16(master) -- the invariant this relies on: do not write a bf16 parameter other than through this
+        optimizer while it has state (a change made inside the block is lost on exit).  Version counters are bumped both ways, so
+        AE's packed inference weights rebuild.  Parameters without an EMA are left alone."""
+        swapped = []
+        try:
+            for _, p, stt in self._ema_params(model):
+                if p.dtype == BF:
+                    p.data.copy_(stt["ema"])
+                else:
+                    p.data, stt["ema"] = stt["ema"], p.data
+                torch.autograd.graph.increment_version(p)
+                swapped.append((p, stt))
+            yield model
+        finally:
+            for p, stt in swapped:
+                if p.dtype == BF:
+                    p.data.copy_(stt["master"])
+                else:
+                    p.data, stt["ema"] = stt["ema"], p.data
+                torch.autograd.graph.increment_version(p)
+
+
+_FP32_STATE = ("master", "exp_avg", "exp_avg_sq", "ema")
+
+
+def _real_arg(name: str, value) -> float:
+    if isinstance(value, bool) or not isinstance(value, (int, float)):
+        raise ValueError(f"FusedAdamW: {name} must be a real number or None, got {value!r}")
+    return float(value)
